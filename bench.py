@@ -7,8 +7,8 @@ batches of 4096.  One STEP = one pass of the fused eval kernel chain over one ba
 
   value   graphs/s, whole job, batches already resident in HBM (reference tensor layout:
           fp32 x, int64 edge_index), evaluated by LightpathGNN.forward_stream (one launch of the
-          persistent kernel per run of batches), replayed from CUDA graphs, timed with CUDA events
-          over a region of >= 100 ms whatever --steps is (`repeats`)
+          persistent kernel per run of batches), --steps steps replayed from one CUDA graph, timed
+          with CUDA events
   e2e     graphs/s through the public host-facing API (LightpathInferencePipeline): pinned HOST
           batches (compact wire format) -> H2D -> kernels -> D2H of (out, lut_batch) every step
   secondary  time-boxed cfg 3 (DDP training step) and cfg 5 (stress graph) blocks
@@ -18,6 +18,8 @@ batches of 4096.  One STEP = one pass of the fused eval kernel chain over one ba
 `--impl reference` times that CPU oracle alone, all host threads, same config and metric.
 N>1 (torchrun): every rank owns a disjoint shard of graphs (weak scaling, no collective on the
 data path); time = max over ranks.
+`--dump-outputs DIR` writes what the last timed step returned (rank 0) as DIR/out.npy (float32) and
+DIR/lut_batch.npy (float64); the inputs are seeded, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -57,13 +59,16 @@ def parse_args():
     ap.add_argument("--workload", default="lightpath_infer", choices=["lightpath_infer", "topo_train", "topo_stress", "lightpath_train"],
                     help="lightpath_infer = BASELINE configs[1] (the headline line); topo_train = configs[2] "
                          "(TopologicalGNN DDP training, batch 1024/GPU); topo_stress = configs[4] (10k nodes, hidden 256)")
-    ap.add_argument("--min-timed-ms", type=float, default=100.0,
-                    help="the K-step unit is repeated until the timed region is at least this long")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (lightpath_infer only)")
     ap.add_argument("--secondary-box-s", type=float, default=150.0,
                     help="wall-clock box of the secondary blocks; past it the headline line is printed without them")
     ap.add_argument("--no-secondary", action="store_true",
                     help="skip the time-boxed cfg 3 (DDP training) and cfg 5 (stress graph) blocks of the default line")
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.dump_outputs and args.workload != "lightpath_infer":
+        ap.error("--dump-outputs is implemented for --workload lightpath_infer only")
+    return args
 
 
 def workload_config(args, world: int) -> dict:
@@ -72,8 +77,8 @@ def workload_config(args, world: int) -> dict:
     return {"workload": "BASELINE cfg2: LightpathGNN eval (GAT->BN->ReLU->LUT->MLP), "
                         f"{args.graphs} synthetic lightpath graphs per GPU, n~U{{8..56}}, batch {args.batch}",
             "batch": args.batch, "graphs_per_gpu": args.graphs, "weights": "lightpath_training/models/model_1.pth",
-            "l2": f"no flush: every repeat of the K-step unit starts at a different batch of the shard's {nb} "
-                  "distinct batches (~1.7 KB/graph; the bytes actually cycled are reported as l2_cycled_bytes)",
+            "l2": f"evicted before the timed region; the timed steps walk the shard's {nb} distinct batches in order "
+                  "(~1.7 KB/graph; the bytes actually cycled are reported as l2_cycled_bytes)",
             "parallelism": f"graph-sharded x{world}, no collective"}
 
 
@@ -142,6 +147,23 @@ def algorithmic_bytes(batch) -> int:
     return 20 * N + 8 * E + 24 * (B + 1) + 24 * L + 4
 
 
+def dump_outputs(out_dir: str, arrays: dict, cap: int = 60 << 20) -> None:
+    """Writes tensors that share their first dimension as out_dir/<name>.npy: float32 and float64 as they are,
+    anything else as float64.  Past `cap` bytes in all, the same seeded sample of rows is taken from every
+    tensor and the sampled row indices are written as rows.npy."""
+    import numpy as np
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    total = sum(v.nbytes for v in arrays.values())
+    if total > cap:
+        rows = np.sort(np.random.default_rng(0).choice(n, int(n * cap / (total + 8 * n)), replace=False))
+        arrays = {**{k: v[rows] for k, v in arrays.items()}, "rows": rows.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def peaks():
     p = ROOT / "MEASURED_PEAKS.json"
     if p.exists():
@@ -194,9 +216,11 @@ def run_reference(args):
         t0 = time.perf_counter()
         g = 0
         for i in range(steps):
-            m(hbs[i % n_b])
+            out, lut_batch = m(hbs[i % n_b])
             g += hbs[i % n_b].num_graphs
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"out": out, "lut_batch": lut_batch})
     v = g / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus,
@@ -212,26 +236,19 @@ def run_reference(args):
 
 # --------------------------------------------------------------------------- B200 arm
 class ResidentRunner:
-    """The K timed steps as CUDA graphs over batches resident in HBM.
+    """The K timed steps as one CUDA graph over batches resident in HBM.
 
     A step = one 4096-graph batch through the persistent eval kernel (LightpathGNN.forward_stream: ONE launch
-    of lp_stream_kernel covers a whole run of consecutive batches).  A *unit* is a captured graph of
-    `unit_steps` consecutive steps (a multiple of K, at least `min_unit` steps so that a replay is long
-    against the CPU's graph-launch cost).  Successive units start at successive batches of the shard
-    (wrapping), so consecutive replays read different bytes.  Every distinct unit graph is replayed once
-    before the timed region: no cold replay is ever timed."""
+    of lp_stream_kernel covers a whole run of consecutive batches).  Step s evaluates batch s modulo the shard:
+    the W warm-up steps run eagerly, the K timed steps that follow them are captured as one graph, and that
+    graph is replayed once before the timed region, so no cold replay is ever timed."""
 
-    def __init__(self, model, plan, K: int, min_unit: int = 256, max_variants: int = 16):
+    def __init__(self, model, plan, K: int, W: int):
         self.model, self.plan = model, plan
-        self.nb, self.K = len(plan), K
+        self.nb, self.K, self.W = len(plan), K, W
         self.side = torch.cuda.Stream()
-        if K >= self.nb:                                          # a unit = one pass over the shard
-            self.unit_steps, self.n_var = self.nb, 1
-        else:
-            self.unit_steps = K * max(1, -(-min_unit // K))       # a multiple of K, >= min_unit steps
-            self.n_var = 1 if self.unit_steps >= self.nb else min(-(-self.nb // self.unit_steps), max_variants)
-        self.graphs = []
-        self.launches_per_unit = []
+        self.graph = None
+        self.launches = 0
 
     def run_steps(self, first: int, count: int) -> int:
         """Enqueues steps [first, first + count) (batch index modulo the shard); returns the launches made."""
@@ -243,42 +260,28 @@ class ResidentRunner:
             first, count, n = first + c, count - c, n + 1
         return n
 
-    def capture(self, warmup_steps: int):
+    def capture(self):
         with torch.cuda.stream(self.side):
-            self.run_steps(0, max(warmup_steps, 3))                # eager warm-up on the stream captured below
+            self.run_steps(0, self.W)                              # eager warm-up on the stream captured below
             torch.cuda.synchronize()
-            for v in range(self.n_var):
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g, stream=self.side):
-                    self.launches_per_unit.append(self.run_steps(v * self.unit_steps, self.unit_steps))
-                self.graphs.append(g)
-            for g in self.graphs:                                  # upload + first replay outside the timed region
-                g.replay()
+            self.graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(self.graph, stream=self.side):
+                self.launches = self.run_steps(self.W, self.K)
+            self.graph.replay()                                    # upload + first replay outside the timed region
             torch.cuda.synchronize()
 
-    def timed(self, n_units: int, ev0, ev1):
+    def timed(self, ev0, ev1, l2_flush):
         with torch.cuda.stream(self.side):
+            # reading a buffer larger than L2 evicts the batches the untimed replay left there, and keeps the GPU
+            # busy while the host enqueues the replay: the region starts with the first kernel, not a launch gap
+            l2_flush.sum()
             ev0.record(self.side)
-            for r in range(n_units):
-                self.graphs[r % self.n_var].replay()
+            self.graph.replay()
             ev1.record(self.side)
 
-    def launches_in(self, n_units: int) -> int:
-        return sum(self.launches_per_unit[r % self.n_var] for r in range(n_units))
-
-    def graphs_in(self, n_units: int) -> int:
-        tot = 0
-        for r in range(n_units):
-            f = (r % self.n_var) * self.unit_steps
-            tot += sum(self.plan.batches[s % self.nb].num_graphs for s in range(f, f + self.unit_steps))
-        return tot
-
-    def distinct_batches(self, n_units: int):
-        seen = set()
-        for r in range(min(n_units, self.n_var)):
-            f = r * self.unit_steps
-            seen.update(s % self.nb for s in range(f, f + self.unit_steps))
-        return sorted(seen)
+    def batches(self) -> list:
+        """Batch index of every timed step, in order."""
+        return [s % self.nb for s in range(self.W, self.W + self.K)]
 
 
 def run_b200(args):
@@ -337,37 +340,34 @@ def run_b200(args):
 
     K, W = max(1, args.steps), max(args.warmup, 3)
     mark("shard resident; capturing")
-    runner = ResidentRunner(model, plan, K)
-    runner.capture(W)
-    mark("calibrating")
-    # ---- calibrate: how many unit replays make the timed region >= --min-timed-ms (same count on every rank)
+    runner = ResidentRunner(model, plan, K, W)
+    runner.capture()
+    steps = runner.batches()
+    graphs_done = sum(plan.batches[i].num_graphs for i in steps)
+    l2_flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)      # > 126 MB L2
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    barrier()
-    n_cal = max(runner.n_var, 2)
-    runner.timed(n_cal, ev0, ev1)
-    torch.cuda.synchronize()
-    unit_ms = max(all_ranks(ev0.elapsed_time(ev1) / n_cal))
-    n_units = max(1, int(-(-args.min_timed_ms // max(unit_ms, 1e-6))), -(-K // runner.unit_steps))
-    n_units = min(n_units, 1_000_000)
-    timed_steps = n_units * runner.unit_steps
-    graphs_done = runner.graphs_in(n_units)
     barrier()
     prof = bool(os.environ.get("QOT_PROFILE_TIMED_REGION"))      # `ncu --profile-from-start off`: only the timed launches
     if prof:
         torch.cuda.profiler.start()
     with ClockSampler(local) as clk:
-        runner.timed(n_units, ev0, ev1)
+        runner.timed(ev0, ev1, l2_flush)
         torch.cuda.synchronize()
     if prof:
         torch.cuda.profiler.stop()
     barrier()
     mark("timed region done")
+    if args.dump_outputs and rank == 0:
+        last = plan.result(steps[-1])
+        n = int(last.n_lut.item())
+        dump_outputs(args.dump_outputs, {"out": last.out[:n], "lut_batch": last.lut_batch[:n]})
+    del l2_flush
     ms = ev0.elapsed_time(ev1)
     per_rank_ms = all_ranks(ms)
     ms_max = max(per_rank_ms)
     graphs_all = sum(all_ranks(float(graphs_done)))
     value = graphs_all / (ms_max * 1e-3)
-    cycled = runner.distinct_batches(n_units)
+    cycled = sorted(set(steps))
     l2_cycled_bytes = sum(batches[i].nbytes(("x", "ptr", "edge_ptr", "lut_ptr")) + batches[i].num_edges * 8 for i in cycled)
 
     # ---- the replays against an eager run through the oracle-checked module path (one launch per batch): same rows
@@ -385,11 +385,11 @@ def run_b200(args):
     # ---- roofline of the dominant kernel: its average duration over the timed region, measured live
     # (CUDA events on the launching stream; the region is nothing but launches of that kernel)
     alg = sum(algorithmic_bytes(batches[i]) for i in cycled) / len(cycled)
-    step_s = ms * 1e-3 / timed_steps
+    step_s = ms * 1e-3 / K
     peak, peak_kind = peaks()
     achieved = alg / step_s / 1e9
-    n_launch = runner.launches_in(n_units)
-    per_launch = timed_steps / n_launch                          # batches one launch of the persistent kernel covers
+    n_launch = runner.launches
+    per_launch = K / n_launch                                    # batches one launch of the persistent kernel covers
     traffic = None
     tp = ROOT / "profiles" / "lp_infer_traffic.json"             # dram__bytes_{read,write}.sum of one ncu --set full capture
     if tp.exists() and Bsz == 4096:
@@ -458,9 +458,9 @@ def run_b200(args):
     if rank == 0:
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
-            "ms_per_step": ms_max / timed_steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+            "ms_per_step": ms_max / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": workload_config(args, world),
-            "repeats": timed_steps / K, "timed_steps": timed_steps, "timed_region_ms": ms_max,
+            "timed_steps": K, "timed_region_ms": ms_max,
             "per_rank_ms": per_rank_ms, "l2_cycled_bytes": l2_cycled_bytes, "host": numa,
             "roofline": roofline, "cpu_baseline": cpu_base, "e2e": e2e,
             "gpu_launches": n_launch, "clocks": clk.summary(), "secondary": None,
