@@ -122,6 +122,8 @@ SIGNATURES = {
     "qot_ddp_sgd_step": (C.c_int, [P, P, i32, i32, i64, P, i32, P, P, P, P, vp]),
     "qot_lightpath_stream_tiles": (i64, [i64]),
     "qot_lightpath_infer_stream": (C.c_int, [P, i32, i64, i64, i64, P, i32, i32, vp]),
+    "qot_lightpath_every_node_tiles": (i64, [i64]),
+    "qot_lightpath_infer_every_node": (C.c_int, [P, i32, i64, i64, P, i32, i32, vp]),
     "qot_lightpath_wire_bytes": (sz, [i64, i64, i64, i64]),
     "qot_lightpath_wire_result_bytes": (sz, [i64]),
     "qot_lightpath_infer_wire_host": (C.c_int, [P, i64, i64, i64, i64, P, i32, C.POINTER(QotLpWireSlot), P,

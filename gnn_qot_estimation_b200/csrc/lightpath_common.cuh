@@ -1,7 +1,7 @@
 // Device helpers shared by the LightpathGNN eval sources (lightpath_infer.cu: parameter folding and lut_ptr;
-// lightpath_stream.cu: the persistent kernel):
+// lightpath_stream.cu: the persistent kernel; lightpath_every_node.cu: every node as the LUT):
 // layout of the prepared parameter block, TF32 split helpers, the warp-per-row attention used by
-// the generic path, the FP32 readout head of one row.
+// the generic path, the FP32 readout head of one row, the mma.sync readout head of 16 rows.
 #pragma once
 #include "common.cuh"
 
@@ -104,11 +104,12 @@ __device__ __forceinline__ void attn_consume(AttnState& st, const int* msg, int 
     st.m = mn;
   }
 }
-// z[h][f] = acc / (sum + 1e-16) into slot h*8+f of s_z (lane (m,h) stores feature m)
+// z[h][f] = acc / (sum + 1e-16) into slot h*kPitch+f of s_z (lane (m,h) stores feature m)
+template <int kPitch = 8>
 __device__ __forceinline__ void attn_finish(const AttnState& st, float* s_z, int lane) {
   const int slot = lane >> 2, h = lane & 3;
   const float den = st.ssum + 1e-16f;
-  if (slot < kF) s_z[h * 8 + slot] = pick5(st.acc, slot) / den;
+  if (slot < kF) s_z[h * kPitch + slot] = pick5(st.acc, slot) / den;
 }
 
 // z (slot h*8+f of s_z) -> folded projection + BatchNorm + ReLU -> MLP head; lanes 0..2 return out[k].
@@ -171,10 +172,26 @@ __device__ __forceinline__ float lut_row_head(const float* __restrict__ w, const
   return (lane == 0 ? o3[0] : lane == 1 ? o3[1] : o3[2]) + b2;
 }
 
+// x accessors of the generic row: XRaw reads x as stored; XAsLut reads it with the LUT flag column overridden --
+// 1.0 for node `lut` and 0.0 for every other node (every-node mode: row `lut` evaluated as the LUT)
+struct XRaw {
+  const float* __restrict__ x;
+  __device__ __forceinline__ float operator()(int64_t j, int k) const { return x[j * kF + k]; }
+};
+struct XAsLut {
+  const float* __restrict__ x;
+  int64_t lut;
+  int col;
+  __device__ __forceinline__ float operator()(int64_t j, int k) const {
+    return k == col ? (j == lut ? 1.0f : 0.0f) : x[j * kF + k];
+  }
+};
+
 // Generic row evaluation straight from global memory: graphs beyond the fast-path caps, further
 // LUT rows of a graph, rows with more than kMsgCap-1 in-edges or a source outside their slab.
-template <bool kHead = true>
-__device__ __noinline__ float lut_row_global(const float* __restrict__ x, const int64_t* __restrict__ esrc,
+// kHead = false: z only, into slot h*8+f of s_z.
+template <bool kHead = true, typename XF = XRaw>
+__device__ __noinline__ float lut_row_global(XF xg, const int64_t* __restrict__ esrc,
                                              const int64_t* __restrict__ edst, int64_t e0, int64_t e1,
                                              int64_t N, int64_t i, const float* __restrict__ prep,
                                              const float* __restrict__ w, int* s_msg, float* s_z,
@@ -184,9 +201,9 @@ __device__ __noinline__ float lut_row_global(const float* __restrict__ x, const 
 #pragma unroll
   for (int k = 0; k < kF; ++k) {
     As[k] = __ldg(prep + kOffAsrc + k * kHeads + h);
-    d_i = fmaf(x[i * kF + k], __ldg(prep + kOffAdst + k * kHeads + h), d_i);
+    d_i = fmaf(xg(i, k), __ldg(prep + kOffAdst + k * kHeads + h), d_i);
   }
-  auto xf = [&](int j, int k) { return x[static_cast<int64_t>(j) * kF + k]; };
+  auto xf = [&](int j, int k) { return xg(static_cast<int64_t>(j), k); };
   AttnState st;
   int cnt = 0;
   for (int64_t eb = e0; eb < e1; eb += 32) {
@@ -215,6 +232,116 @@ __device__ __noinline__ float lut_row_global(const float* __restrict__ x, const 
   const float ov = lut_row_head(w, s_z, s_y, lane);
   __syncwarp();
   return ov;
+}
+
+// ------------------------------------------------------------------------------------------------
+// readout head of 16 z rows on the tensor cores (mma.sync m16n8k8 TF32, split-fp32 operands: hi*lo + lo*hi
+// + hi*hi), one warp: folded projection + BN + ReLU -> mlp.0 -> LeakyReLU -> mlp.3.  Row g8 = lane >> 2 of the
+// tile is `za` (20 floats, [h][f]), row g8 + 8 is `zb`; `va` / `vb`: the row exists (else zeros go in).  `f1` /
+// `f2`: the B1f / B2f fragment tables of `prepared` (kStHeadFrag4 float4, shared memory in the kernels).
+// Lanes t4 = lane & 3 < 3 return output t4 of both rows in oa / ob.
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ void st_mma_tf32(float (&c)[4], const unsigned (&a)[4], float b0, float b1) {
+  asm volatile(
+      "mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
+      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(__float_as_uint(b0)), "r"(__float_as_uint(b1)));
+}
+constexpr int kStHeadFrag4 = (kOffAsP - kOffB1f) / 4;   // float4 entries of B1f | B2f (contiguous in `prepared`)
+
+__device__ __forceinline__ void head_rows16_tf32x3(const float4* __restrict__ f1, const float4* __restrict__ f2,
+                                                   const float* za, const float* zb, bool va, bool vb,
+                                                   const float* __restrict__ prep, int lane, float& oa_out,
+                                                   float& ob_out) {
+  const int t4 = lane & 3;
+  float H[4][4], Hc[4][4];                             // fp32 sums of the hi x hi tiles; compensation chains
+#pragma unroll
+  for (int q = 0; q < 4; ++q)
+#pragma unroll
+    for (int i = 0; i < 4; ++i) H[q][i] = Hc[q][i] = 0.f;
+#pragma unroll 1
+  for (int h = 0; h < kHeads; ++h) {
+    unsigned ahi[4], alo[4];
+    {
+      float a[4];
+      a[0] = va ? za[h * kF + t4] : 0.f;
+      a[1] = vb ? zb[h * kF + t4] : 0.f;
+      a[2] = t4 == 0 ? (va ? za[h * kF + 4] : 0.f) : (t4 == 1 ? 1.0f : 0.f);
+      a[3] = t4 == 0 ? (vb ? zb[h * kF + 4] : 0.f) : (t4 == 1 ? 1.0f : 0.f);
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        ahi[i] = tf32_rna(a[i]);
+        alo[i] = tf32_rna(a[i] - __uint_as_float(ahi[i]));
+      }
+    }
+#pragma unroll
+    for (int jj = 0; jj < 4; ++jj) {
+      const int j = 4 * h + jj;
+      const float4 b = f1[j * 32 + lane];
+      float c[4] = {0.f, 0.f, 0.f, 0.f};
+      st_mma_tf32(c, alo, b.x, b.y);
+      st_mma_tf32(c, ahi, b.z, b.w);
+      st_mma_tf32(c, ahi, b.x, b.y);
+      const float y[4] = {fmaxf(c[0], 0.f), fmaxf(c[2], 0.f), fmaxf(c[1], 0.f), fmaxf(c[3], 0.f)};
+      unsigned yhi[4], ylo[4];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        yhi[i] = tf32_rna_finite(y[i]);
+        ylo[i] = tf32_rna_finite(y[i] - __uint_as_float(yhi[i]));
+      }
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const float4 b2 = f2[(j * 4 + q) * 32 + lane];
+        st_mma_tf32(Hc[q], ylo, b2.x, b2.y);
+        st_mma_tf32(Hc[q], yhi, b2.z, b2.w);
+        float t[4] = {0.f, 0.f, 0.f, 0.f};
+        st_mma_tf32(t, yhi, b2.x, b2.y);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) H[q][i] += t[i];
+      }
+    }
+  }
+  float oa[QOT_OUT] = {0.f, 0.f, 0.f}, ob[QOT_OUT] = {0.f, 0.f, 0.f};
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    const int o = 8 * q + 2 * t4;
+    const float2 b1 = __ldg(reinterpret_cast<const float2*>(prep + kOffB1 + o));
+    float hv[4] = {H[q][0] + Hc[q][0] + b1.x, H[q][1] + Hc[q][1] + b1.y, H[q][2] + Hc[q][2] + b1.x,
+                   H[q][3] + Hc[q][3] + b1.y};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) hv[i] = hv[i] > 0.f ? hv[i] : 0.01f * hv[i];
+#pragma unroll
+    for (int k = 0; k < QOT_OUT; ++k) {
+      const float2 w2 = __ldg(reinterpret_cast<const float2*>(prep + kOffW2 + k * kHid + o));
+      oa[k] = fmaf(hv[0], w2.x, oa[k]);
+      oa[k] = fmaf(hv[1], w2.y, oa[k]);
+      ob[k] = fmaf(hv[2], w2.x, ob[k]);
+      ob[k] = fmaf(hv[3], w2.y, ob[k]);
+    }
+  }
+#pragma unroll
+  for (int s = 1; s <= 2; s <<= 1) {
+#pragma unroll
+    for (int k = 0; k < QOT_OUT; ++k) {
+      oa[k] += __shfl_xor_sync(kFull, oa[k], s);
+      ob[k] += __shfl_xor_sync(kFull, ob[k], s);
+    }
+  }
+  const float b2 = t4 < QOT_OUT ? __ldg(prep + kOffB2 + t4) : 0.f;
+  oa_out = (t4 == 0 ? oa[0] : t4 == 1 ? oa[1] : oa[2]) + b2;
+  ob_out = (t4 == 0 ? ob[0] : t4 == 1 ? ob[1] : ob[2]) + b2;
+}
+
+// descriptor of the batch tile T of the launch belongs to (uniform tile count per batch, or prefix search)
+// T is absolute (tile0 units); the launch covers tiles [base, base + total)
+__device__ __forceinline__ int st_batch_of(const qot_lp_batch_t* __restrict__ bt, int nb, int64_t tpb, int64_t base, int64_t T) {
+  if (tpb > 0) return static_cast<int>(min((T - base) / tpb, static_cast<int64_t>(nb - 1)));
+  int lo = 0, hi = nb - 1;                 // last b with tile0[b] <= T
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (bt[mid].tile0 <= T) lo = mid; else hi = mid - 1;
+  }
+  return lo;
 }
 
 constexpr int kSubMsg = 16;               // fast path: sources of the LUT row + its self loop

@@ -225,18 +225,6 @@ __device__ __forceinline__ void st_mbar_init(unsigned long long* bar, int count)
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(st_smem_u32(bar)), "r"(count) : "memory");
 }
 
-// descriptor of the batch tile T of the launch belongs to (uniform tile count per batch, or prefix search)
-// T is absolute (tile0 units); the launch covers tiles [base, base + total)
-__device__ __forceinline__ int st_batch_of(const qot_lp_batch_t* __restrict__ bt, int nb, int64_t tpb, int64_t base, int64_t T) {
-  if (tpb > 0) return static_cast<int>(min((T - base) / tpb, static_cast<int64_t>(nb - 1)));
-  int lo = 0, hi = nb - 1;                 // last b with tile0[b] <= T
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (bt[mid].tile0 <= T) lo = mid; else hi = mid - 1;
-  }
-  return lo;
-}
-
 // ------------------------------------------------------------------------------------------------
 // producer: one warp
 // ------------------------------------------------------------------------------------------------
@@ -384,10 +372,10 @@ __device__ __noinline__ void st_generic(int cw, unsigned todo, const float* __re
           if (orow < gl1) {                                      // never write past this graph's rows
             const int64_t i = nbq + bit;
             if constexpr (kHead) {
-              const float ov = lut_row_global<true>(gx, ga.esrc, ga.edst, ge0, ge1, N, i, prep, prep + kOffWf, s_m, s_z, s_y, lane);
+              const float ov = lut_row_global<true>(XRaw{gx}, ga.esrc, ga.edst, ge0, ge1, N, i, prep, prep + kOffWf, s_m, s_z, s_y, lane);
               if (lane < QOT_OUT) ga.out[orow * QOT_OUT + lane] = ov;
             } else {
-              lut_row_global<false>(gx, ga.esrc, ga.edst, ge0, ge1, N, i, prep, nullptr, s_m, s_z, nullptr, lane);
+              lut_row_global<false>(XRaw{gx}, ga.esrc, ga.edst, ge0, ge1, N, i, prep, nullptr, s_m, s_z, nullptr, lane);
               if (lane < kHeads * kF) ga.z[orow * (kHeads * kF) + lane] = s_z[(lane / kF) * 8 + lane % kF];
             }
             if (lane == 0) {
@@ -1065,14 +1053,6 @@ lp_stream_kernel(const qot_lp_batch_t* __restrict__ batches, int n_batches, int6
 // readout head over the z rows of every batch of the launch (grid.y = batch): folded projection + BN + ReLU
 // -> mlp.0 -> LeakyReLU -> mlp.3 on the tensor cores (mma.sync TF32 x3), 64 rows per block
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void st_mma_tf32(float (&c)[4], const unsigned (&a)[4], float b0, float b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(__float_as_uint(b0)), "r"(__float_as_uint(b1)));
-}
-constexpr int kStHeadFrag4 = (kOffAsP - kOffB1f) / 4;   // float4 entries of B1f | B2f (contiguous in `prepared`)
-
 __global__ void __launch_bounds__(128)
 lp_stream_head_kernel(const qot_lp_batch_t* __restrict__ batches, const float* __restrict__ prep) {
   __shared__ float4 frag[kStHeadFrag4];
@@ -1090,85 +1070,11 @@ lp_stream_head_kernel(const qot_lp_batch_t* __restrict__ batches, const float* _
        tile += static_cast<int64_t>(gridDim.x) * 4) {
     const int64_t ra = tile * 16 + g8, rb = ra + 8;
     const bool va = ra < L, vb = rb < L;
-    const float* za = zbuf + ra * (kHeads * kF);
-    const float* zb = zbuf + rb * (kHeads * kF);
-    float H[4][4], Hc[4][4];                           // fp32 sums of the hi x hi tiles; compensation chains
-#pragma unroll
-    for (int q = 0; q < 4; ++q)
-#pragma unroll
-      for (int i = 0; i < 4; ++i) H[q][i] = Hc[q][i] = 0.f;
-#pragma unroll 1
-    for (int h = 0; h < kHeads; ++h) {
-      unsigned ahi[4], alo[4];
-      {
-        float a[4];
-        a[0] = va ? za[h * kF + t4] : 0.f;
-        a[1] = vb ? zb[h * kF + t4] : 0.f;
-        a[2] = t4 == 0 ? (va ? za[h * kF + 4] : 0.f) : (t4 == 1 ? 1.0f : 0.f);
-        a[3] = t4 == 0 ? (vb ? zb[h * kF + 4] : 0.f) : (t4 == 1 ? 1.0f : 0.f);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          ahi[i] = tf32_rna(a[i]);
-          alo[i] = tf32_rna(a[i] - __uint_as_float(ahi[i]));
-        }
-      }
-#pragma unroll
-      for (int jj = 0; jj < 4; ++jj) {
-        const int j = 4 * h + jj;
-        const float4 b = f1[j * 32 + lane];
-        float c[4] = {0.f, 0.f, 0.f, 0.f};
-        st_mma_tf32(c, alo, b.x, b.y);
-        st_mma_tf32(c, ahi, b.z, b.w);
-        st_mma_tf32(c, ahi, b.x, b.y);
-        const float y[4] = {fmaxf(c[0], 0.f), fmaxf(c[2], 0.f), fmaxf(c[1], 0.f), fmaxf(c[3], 0.f)};
-        unsigned yhi[4], ylo[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          yhi[i] = tf32_rna_finite(y[i]);
-          ylo[i] = tf32_rna_finite(y[i] - __uint_as_float(yhi[i]));
-        }
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          const float4 b2 = f2[(j * 4 + q) * 32 + lane];
-          st_mma_tf32(Hc[q], ylo, b2.x, b2.y);
-          st_mma_tf32(Hc[q], yhi, b2.z, b2.w);
-          float t[4] = {0.f, 0.f, 0.f, 0.f};
-          st_mma_tf32(t, yhi, b2.x, b2.y);
-#pragma unroll
-          for (int i = 0; i < 4; ++i) H[q][i] += t[i];
-        }
-      }
-    }
-    float oa[QOT_OUT] = {0.f, 0.f, 0.f}, ob[QOT_OUT] = {0.f, 0.f, 0.f};
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      const int o = 8 * q + 2 * t4;
-      const float2 b1 = __ldg(reinterpret_cast<const float2*>(prep + kOffB1 + o));
-      float hv[4] = {H[q][0] + Hc[q][0] + b1.x, H[q][1] + Hc[q][1] + b1.y, H[q][2] + Hc[q][2] + b1.x,
-                     H[q][3] + Hc[q][3] + b1.y};
-#pragma unroll
-      for (int i = 0; i < 4; ++i) hv[i] = hv[i] > 0.f ? hv[i] : 0.01f * hv[i];
-#pragma unroll
-      for (int k = 0; k < QOT_OUT; ++k) {
-        const float2 w2 = __ldg(reinterpret_cast<const float2*>(prep + kOffW2 + k * kHid + o));
-        oa[k] = fmaf(hv[0], w2.x, oa[k]);
-        oa[k] = fmaf(hv[1], w2.y, oa[k]);
-        ob[k] = fmaf(hv[2], w2.x, ob[k]);
-        ob[k] = fmaf(hv[3], w2.y, ob[k]);
-      }
-    }
-#pragma unroll
-    for (int s = 1; s <= 2; s <<= 1) {
-#pragma unroll
-      for (int k = 0; k < QOT_OUT; ++k) {
-        oa[k] += __shfl_xor_sync(kFull, oa[k], s);
-        ob[k] += __shfl_xor_sync(kFull, ob[k], s);
-      }
-    }
+    float oa, ob;
+    head_rows16_tf32x3(f1, f2, zbuf + ra * (kHeads * kF), zbuf + rb * (kHeads * kF), va, vb, prep, lane, oa, ob);
     if (t4 < QOT_OUT) {
-      const float b2 = __ldg(prep + kOffB2 + t4);
-      if (va) out[ra * QOT_OUT + t4] = (t4 == 0 ? oa[0] : t4 == 1 ? oa[1] : oa[2]) + b2;
-      if (vb) out[rb * QOT_OUT + t4] = (t4 == 0 ? ob[0] : t4 == 1 ? ob[1] : ob[2]) + b2;
+      if (va) out[ra * QOT_OUT + t4] = oa;
+      if (vb) out[rb * QOT_OUT + t4] = ob;
     }
   }
 }

@@ -7,7 +7,8 @@ the shipped checkpoints (``conv1.lin.weight``, ``conv1.att_src``, ``conv1.att_ds
 ``lightpath_training/test.py:63`` loads ``models/model_N.pth`` with strict=True.
 
 eval(): one launch of the persistent kernel (csrc/lightpath_stream.cu) per batch -- or per MANY
-batches through ``stream_plan`` / ``forward_stream``.
+batches through ``stream_plan`` / ``forward_stream``.  ``forward_every_node`` / ``stream_plan(..., every_node=True)``:
+every node of a graph evaluated as the LUT in one pass (csrc/lightpath_every_node.cu).
 train(): GAT forward -> batch statistics -> LUT head, with the matching backward
 kernels (csrc/lightpath_train.cu) through ``torch.autograd.Function``.
 """
@@ -85,11 +86,59 @@ class LightpathGNN(torch.nn.Module):
         plan.launch(self.prepared())
         return plan.result(0)
 
-    def stream_plan(self, batches, split_head: bool = False) -> "ops.LightpathStreamPlan":
+    def stream_plan(self, batches, split_head: bool = False, every_node: bool = False) -> "ops.LightpathStreamPlan":
         """Plan for evaluating many resident batches with one launch of the persistent kernel each time
-        ``forward_stream`` is called (the streaming form of lightpath_training/test.py:77-94)."""
+        ``forward_stream`` is called (the streaming form of lightpath_training/test.py:77-94).
+        ``every_node``: every node of every graph as the LUT (see ``forward_every_node``)."""
         self._check_supported()
-        return ops.LightpathStreamPlan(batches, self.is_lut_index, split_head)
+        return ops.LightpathStreamPlan(batches, self.is_lut_index, split_head, every_node)
+
+    @_lib.on_tensor_device
+    def forward_every_node(self, data) -> torch.Tensor:
+        """QoT of every lightpath of every graph of ONE batch, one pass over each graph (eval mode only).
+
+        Returns ``out [N, 3]``: row i is what ``forward`` under ``eval()`` returns for node i's graph, given a copy of
+        that graph in which node i's flag column ``x[:, is_lut_index]`` is 1.0 and every other node's flag column is
+        0.0.  Whatever the stored flag column holds (0, 1, several ones, any value) has no effect.  Rows are in node
+        order; the graph of row i is ``data.batch[i]``.  From raw samples: ``to_graph.create_lightpath_graphs(...,
+        return_conn_ids=True)``, then ``collate``, then this call -- row i is lightpath ``conn_ids[i]`` of sample
+        ``batch[i]``.  Foreign batches (PyG / pyg_compat) get ``ptr`` / ``edge_ptr`` derived; their edges must be
+        grouped by graph.  The plan (output buffer + device descriptor) is cached on the batch object; the call reads
+        one status word back (a synchronisation) and raises on malformed input."""
+        if self.training:
+            raise RuntimeError("LightpathGNN.forward_every_node is eval-only (in training mode BatchNorm couples the "
+                               "nodes): call model.eval()")
+        if not data.x.is_cuda or not data.edge_index.is_cuda:
+            raise RuntimeError("LightpathGNN (B200) needs the batch on a CUDA device; there is no CPU path")
+        self._check_supported()
+        from ..batch import Batch
+        cache = ops.batch_cache(data)
+        key = ("every_node_plan", self.is_lut_index, data.x.data_ptr(), data.edge_index.data_ptr(),
+               tuple(data.x.shape), tuple(data.edge_index.shape))
+        plan = cache.get(key)
+        if plan is None:
+            gptr = ops.batch_graph_ptr(data)
+            eptr = getattr(data, "edge_ptr", None)
+            if eptr is None:
+                if "eptr" not in cache:
+                    cache["eptr"] = ops.edge_ptr(data.edge_index, data.batch, gptr.numel() - 1)
+                eptr = cache["eptr"][0]
+            view = Batch(x=data.x, edge_index=data.edge_index, batch=getattr(data, "batch", None), ptr=gptr,
+                         edge_ptr=eptr, num_graphs=int(gptr.numel() - 1),
+                         sym_by_src=bool(getattr(data, "sym_by_src", False)))
+            plan = cache[key] = ops.LightpathStreamPlan([view], self.is_lut_index, every_node=True)
+        plan.launch(self.prepared())
+        flags = [plan.status[:1]]
+        if getattr(data, "edge_ptr", None) is None:
+            flags.append(cache["eptr"][1])                         # "edges grouped by graph" check
+        vals = torch.cat(flags).tolist()                          # the one D2H of this call
+        if len(vals) > 1 and vals[1]:
+            raise RuntimeError("LightpathGNN.forward_every_node: the batch's edges are not grouped by graph "
+                               "(every-node mode reads each graph's edges as one contiguous range)")
+        if vals[0]:
+            raise RuntimeError("LightpathGNN.forward_every_node: malformed graph offsets (ptr / edge_ptr outside "
+                               "the batch)")
+        return plan.result(0).out.clone()                         # the plan's buffer is reused by the next call
 
     @_lib.on_tensor_device
     def forward_stream(self, plan, first: int = 0, count=None) -> None:

@@ -216,15 +216,28 @@ class LightpathStreamPlan:
     the batches' readout-row counts (one device->host read of the nb counts here, none afterwards), one
     status word and one row count per batch, and the DEVICE array of batch descriptors the kernel walks.
     ``launch(prepared, first, count)`` enqueues batches [first, first+count) on the current stream: no
-    synchronisation, CUDA-graph capturable.  ``result(i)`` gives views of batch i's outputs."""
+    synchronisation, CUDA-graph capturable.  ``result(i)`` gives views of batch i's outputs.
 
-    def __init__(self, batches, is_lut_index: int, split_head: bool = False):
+    ``every_node=True`` (qot_lightpath_infer_every_node): every node of every graph is evaluated as the LUT.  Row i of
+    batch b's output [N_b, 3] is what the reference forward under eval() returns for node i's graph with node i's flag
+    column set to 1.0 and every other node's to 0.0; the stored flag column has no effect.  Rows are in node order, the
+    graph of row i is ``batch[i]``.  Buffers are sized by N: no lut_ptr is needed and nothing is read from the device."""
+
+    def __init__(self, batches, is_lut_index: int, split_head: bool = False, every_node: bool = False):
         """``split_head``: QOT_LP_SPLIT_HEAD -- the readout head as a second launch instead of inside the kernel."""
         L = _lib.lib()
         if not batches:
             raise ValueError("LightpathStreamPlan: no batches")
+        if every_node and split_head:
+            raise ValueError("LightpathStreamPlan: split_head does not apply to every_node mode")
         dev = batches[0].x.device
         for b in batches:
+            if every_node:
+                if b.ptr is None or b.edge_ptr is None:
+                    raise RuntimeError("LightpathStreamPlan(every_node=True) needs batches carrying ptr and edge_ptr "
+                                       "(PackedGraphStore.collate provides them)")
+                _require_cuda(b.x, b.edge_index, b.ptr, b.edge_ptr)
+                continue
             if b.ptr is None or b.edge_ptr is None or b.lut_ptr is None or getattr(b, "lut_col", None) != is_lut_index:
                 raise RuntimeError("LightpathStreamPlan needs batches carrying ptr, edge_ptr and lut_ptr for "
                                    "is_lut_index (PackedGraphStore.collate provides them)")
@@ -232,20 +245,27 @@ class LightpathStreamPlan:
         self.batches = list(batches)                 # keeps the input tensors alive
         self.device = dev                            # (_lib.on_tensor_device makes it current around forward_stream)
         self.is_lut_index = int(is_lut_index)
+        self.every_node = bool(every_node)
         # QOT_LP_SYMMETRIC_BY_SOURCE only when EVERY batch carries the verified-layout mark
         self.flags = (1 if all(getattr(b, "sym_by_src", False) for b in batches) else 0) | (2 if split_head else 0)
         nb = len(batches)
-        rows = torch.stack([b.lut_ptr[-1] for b in batches]).tolist()          # the one sync
-        self.rows = [int(r) for r in rows]
+        if every_node:
+            self.rows = [int(b.x.shape[0]) for b in batches]
+        else:
+            rows = torch.stack([b.lut_ptr[-1] for b in batches]).tolist()      # the one sync
+            self.rows = [int(r) for r in rows]
         cap = [max(r, 1) for r in self.rows]
         off = [0]
         for c in cap:
             off.append(off[-1] + c)
         tot = off[-1]
         self.out = torch.empty(tot, 3, dtype=torch.float32, device=dev)
-        self.lut_batch = torch.empty(tot, dtype=torch.int64, device=dev)
-        self.lut_node = torch.empty(tot, dtype=torch.int32, device=dev)
-        self.z = torch.empty(tot, 20, dtype=torch.float32, device=dev)
+        if every_node:                               # the kernel writes `out` only
+            self.lut_batch = self.lut_node = self.z = None
+        else:
+            self.lut_batch = torch.empty(tot, dtype=torch.int64, device=dev)
+            self.lut_node = torch.empty(tot, dtype=torch.int32, device=dev)
+            self.z = torch.empty(tot, 20, dtype=torch.float32, device=dev)
         self.n_lut = torch.zeros(nb, dtype=torch.int32, device=dev)
         self.status = torch.zeros(nb, dtype=torch.int32, device=dev)
         self.off = off
@@ -254,25 +274,32 @@ class LightpathStreamPlan:
         tile0 = [0]
         for i, b in enumerate(batches):
             x, ei = _f32(b.x), _i64(b.edge_index)
-            gp, ep, lp = _i64(b.ptr), _i64(b.edge_ptr), _i64(b.lut_ptr)
-            self.keep += [x, ei, gp, ep, lp]
+            gp, ep = _i64(b.ptr), _i64(b.edge_ptr)
+            self.keep += [x, ei, gp, ep]
             d = descs[i]
-            d.x, d.edge_index, d.ptr, d.edge_ptr, d.lut_ptr = ptr(x), ptr(ei), ptr(gp), ptr(ep), ptr(lp)
+            d.x, d.edge_index, d.ptr, d.edge_ptr = ptr(x), ptr(ei), ptr(gp), ptr(ep)
             d.N, d.E, d.B = int(x.shape[0]), int(ei.shape[1]), int(gp.numel() - 1)
             o = off[i]
             d.out = self.out.data_ptr() + o * 12
-            d.lut_batch = self.lut_batch.data_ptr() + o * 8
-            d.lut_node = self.lut_node.data_ptr() + o * 4
             d.n_lut = self.n_lut.data_ptr() + i * 4
             d.status = self.status.data_ptr() + i * 4
-            d.z = self.z.data_ptr() + o * 80
             d.tile0 = tile0[-1]
+            if every_node:
+                tile0.append(tile0[-1] + int(L.qot_lightpath_every_node_tiles(d.B)))
+                continue
+            lp = _i64(b.lut_ptr)
+            self.keep.append(lp)
+            d.lut_ptr = ptr(lp)
+            d.lut_batch = self.lut_batch.data_ptr() + o * 8
+            d.lut_node = self.lut_node.data_ptr() + o * 4
+            d.z = self.z.data_ptr() + o * 80
             tile0.append(tile0[-1] + int(L.qot_lightpath_stream_tiles(d.B)))
         self.tile0 = tile0
         self.desc_size = C.sizeof(_lib.QotLpBatch)
         raw = torch.frombuffer(bytearray(bytes(descs)), dtype=torch.uint8)
         self.descs = raw.to(dev)
-        _track_status("qot_lightpath_infer_stream (lut_ptr does not describe x, or a pipeline barrier timed out)",
+        _track_status("qot_lightpath_infer_every_node (malformed graph offsets)" if every_node else
+                      "qot_lightpath_infer_stream (lut_ptr does not describe x, or a pipeline barrier timed out)",
                       self.status)
 
     def __len__(self):
@@ -286,13 +313,23 @@ class LightpathStreamPlan:
         tiles = [self.tile0[i + 1] - self.tile0[i] for i in range(first, first + count)]
         uniform = tiles[0] if all(t == tiles[0] for t in tiles[:-1]) and tiles[-1] <= tiles[0] else 0
         self.status[first:first + count].zero_()
+        if self.every_node:
+            check(_lib.lib().qot_lightpath_infer_every_node(
+                self.descs.data_ptr() + first * self.desc_size, count, self.tile0[first + count] - self.tile0[first],
+                uniform, ptr(prepared), self.is_lut_index, self.flags, stream()), "qot_lightpath_infer_every_node")
+            return
         check(_lib.lib().qot_lightpath_infer_stream(
             self.descs.data_ptr() + first * self.desc_size, count, self.tile0[first + count] - self.tile0[first],
             uniform, max(self.rows[first:first + count]), ptr(prepared), self.is_lut_index, self.flags, stream()),
             "qot_lightpath_infer_stream")
 
     def result(self, i: int) -> LightpathInferOut:
+        """every_node: ``out`` holds batch i's N rows, ``lut_batch`` is the batch's ``batch`` vector (or None),
+        ``lut_node`` / ``n_lut`` are None."""
         a, b = self.off[i], self.off[i + 1]
+        if self.every_node:
+            return LightpathInferOut(self.out[a:a + self.rows[i]], getattr(self.batches[i], "batch", None), None, None,
+                                     self.status[i:i + 1])
         return LightpathInferOut(self.out[a:b], self.lut_batch[a:b], self.lut_node[a:b], self.n_lut[i:i + 1],
                                  self.status[i:i + 1])
 

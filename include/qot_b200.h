@@ -348,6 +348,21 @@ int qot_lightpath_infer_stream(const qot_lp_batch_t* batches, int32_t n_batches,
                                int64_t uniform_tiles, int64_t max_rows, const float* prepared,
                                int32_t is_lut_index, int32_t flags, void* stream);
 
+/* Every-node mode (csrc/lightpath_every_node.cu, lp_every_node_kernel): every node of every graph evaluated as the
+ * LUT, one pass over each graph.  For a batch with N nodes, row i of out [N,3] is what the reference
+ * LightpathGNN.forward under eval() returns for node i's graph, given a copy of that graph in which node i's flag
+ * column x[:, is_lut_index] is 1.0 and every other node's flag column is 0.0.  Whatever the stored flag column holds
+ * has no effect.  Rows are in node order; the graph of row i is batch[i].
+ * Same descriptor array as qot_lightpath_infer_stream, with tile0 counted in qot_lightpath_every_node_tiles(B) units.
+ * Reads x, edge_index, ptr, edge_ptr, N, E, B, out (>= N rows), status (ZERO on entry; bit 0: malformed graph
+ * offsets, the graph's rows are not written) and tile0; ignores lut_ptr / lut_batch / lut_node / n_lut / z, which
+ * may be NULL.  `prepared` as for qot_lightpath_infer_stream (qot_lightpath_prepare); flags: 0 or
+ * QOT_LP_SYMMETRIC_BY_SOURCE (same bits either way on a verified layout).  No host synchronisation: capturable. */
+int64_t qot_lightpath_every_node_tiles(int64_t B);
+int qot_lightpath_infer_every_node(const qot_lp_batch_t* batches, int32_t n_batches, int64_t total_tiles,
+                                   int64_t uniform_tiles, const float* prepared, int32_t is_lut_index,
+                                   int32_t flags, void* stream);
+
 /* The evaluation loop of lightpath_training/test.py:77-94 for batches arriving from the HOST: one call per batch
  * replaces `data.to(device)` -> `model(data)` -> `.cpu()`.  The batch travels in the COMPACT WIRE FORMAT of a
  * verified-layout batch (see QOT_LP_SYMMETRIC_BY_SOURCE; PackedGraphStore.host_wire_batch packs it), one contiguous
