@@ -141,6 +141,30 @@ class LightpathGNN(torch.nn.Module):
         return plan.result(0).out.clone()                         # the plan's buffer is reused by the next call
 
     @_lib.on_tensor_device
+    def forward_candidates(self, state, cands, max_impact: int = 64) -> "ops.CandidateQoT":
+        """QoT of candidate lightpaths against a network state, and what each candidate does to the lightpaths
+        already set up (eval mode only; csrc/lightpath_candidates.cu).
+
+        ``state``: ``to_graph.lightpath_network_state(data, freqs, lp_feat)``; ``cands``: ``to_graph.LightpathCandidates``
+        on the state's device.  For candidate k, let sample' be sample ``cands.sample[k]`` with the candidate written
+        into every channel of its path and slot range (a new conn_id, features ``cands.feat[k]``, unknown metrics).  In
+        sample''s lightpath graph with the flag column ``x[:, is_lut_index]`` one-hot:
+        ``out[k]`` is ``forward`` under ``eval()`` with the flag at the candidate; ``impact_out[k, i]`` is the same with
+        the flag at the i-th lightpath the candidate interferes with (``impact_node[k, i]``, a node of ``state.batch``,
+        ascending) -- compare it with ``forward_every_node(state.batch)`` for the "before" value.  Candidates are
+        evaluated independently, each against the state alone.  ``status`` holds ``ops.CAND_*`` bits: a bad sample,
+        a bad path or slot range, or an occupied channel gives a NaN row and no impact rows; more than ``max_impact``
+        neighbours keeps the first ``max_impact`` rows and reports the true count in ``n_impact``.
+        One launch, nothing read back: capturable in a CUDA graph.  Malformed arguments raise on the host."""
+        if self.training:
+            raise RuntimeError("LightpathGNN.forward_candidates is eval-only (in training mode BatchNorm couples the "
+                               "nodes): call model.eval()")
+        if not state.batch.x.is_cuda:
+            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
+        self._check_supported()
+        return ops.lightpath_candidates(state, cands, self.prepared(), self.is_lut_index, max_impact)
+
+    @_lib.on_tensor_device
     def forward_stream(self, plan, first: int = 0, count=None) -> None:
         """Enqueues batches [first, first+count) of ``plan`` (eval mode; no host synchronisation)."""
         if self.training:

@@ -185,3 +185,44 @@ def network_status_samples(num_samples: int, num_links: int = 40, num_freqs: int
                 data[s, fi["osnr"], l, q] = data[s, fi["snr"], l, q] = data[s, fi["ber"], l, q] = -1.0
         target[s] = [rng.uniform(12.47, 33.49), rng.uniform(8.96, 29.98), rng.uniform(1.7e-12, 1.98e-2), rng.integers(0, 3)]
     return {"data": data, "target": target, "freqs": freqs, "lp_feat": list(LP_FEAT), "metric": list(METRICS)}
+
+
+def lightpath_candidates(samples, per_sample: int, seed: int = 0):
+    """Seeded candidate lightpaths for the network-status ``samples`` (the dict ``network_status_samples`` returns):
+    ``per_sample`` candidates per sample, each on 1..6 distinct random links with one slot (or two adjacent slots,
+    probability 0.1) that is free on every link of its path; ``feat = (float32(freqs[q0]), mod_order, num_spans,
+    path_len)`` as ``network_status_samples`` writes a lightpath's first channel.  A sample too full to place a
+    candidate after 64 draws gets fewer.  Returns ``to_graph.LightpathCandidates`` of CPU tensors (``.to(device)``)."""
+    import numpy as np
+    from .to_graph import LightpathCandidates
+    rng = np.random.default_rng(seed)
+    data, freqs = samples["data"], samples["freqs"]
+    S, _, L, Q = data.shape
+    occupied = np.any(data != 0, axis=1)                       # [S, L, Q]
+    smp, lptr, links, q0s, widths, feats = [], [0], [], [], [], []
+    for s in range(S):
+        for _ in range(per_sample):
+            for _try in range(64):
+                width = 2 if rng.random() < 0.1 else 1
+                path = rng.choice(L, size=min(int(rng.integers(1, 7)), L), replace=False)
+                free = ~occupied[s, path].any(axis=0)          # [Q]
+                ok = free[:Q - width + 1].copy()
+                for u in range(1, width):
+                    ok &= free[u:Q - width + 1 + u]
+                cand = np.flatnonzero(ok)
+                if cand.size:
+                    break
+            else:
+                continue
+            q0 = int(rng.choice(cand))
+            smp.append(s)
+            links.extend(int(l) for l in path)
+            lptr.append(len(links))
+            q0s.append(q0)
+            widths.append(width)
+            feats.append([np.float32(freqs[q0]), rng.choice([4, 8, 16, 32, 64]), int(rng.integers(1, 107)),
+                          int(rng.integers(24214, 7834746))])
+    return LightpathCandidates(torch.tensor(smp, dtype=torch.int64), torch.tensor(lptr, dtype=torch.int64),
+                               torch.tensor(links, dtype=torch.int32), torch.tensor(q0s, dtype=torch.int32),
+                               torch.tensor(widths, dtype=torch.int32),
+                               torch.tensor(np.array(feats, dtype=np.float32).reshape(-1, 4)))

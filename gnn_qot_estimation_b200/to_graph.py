@@ -14,13 +14,13 @@ against golden vectors made by the reference's own code); edges are emitted sort
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional, Sequence
+from typing import NamedTuple, Optional, Sequence
 
 import torch
 
 from . import _lib
 from .batch import PackedGraphStore
-from .ops import check, ptr, stream
+from .ops import _track_status, check, ptr, stream
 
 # constants.py:1-12 of the reference
 FEATURE_RANGES = {"mod_order": (0.0, 64.0), "path_len": (24214.0, 7834746.0), "num_spans": (1.0, 106.0),
@@ -133,3 +133,65 @@ def create_topological_graphs(data: torch.Tensor, target: torch.Tensor, lp_feat:
                                          ptr(status), stream()), "qot_topological_graph_fill")
     node_ptr = torch.arange(S + 1, dtype=torch.int64, device=dev) * int(num_nodes)
     return PackedGraphStore(node_ptr, edge_ptr, edge_src, edge_dst, None, edge_feat, y)
+
+
+class LightpathNetworkState(NamedTuple):
+    """A resident network state: raw samples turned into graphs once, plus the index structures candidate QoT needs
+    (``lightpath_network_state``; ``LightpathGNN.forward_candidates``)."""
+    batch: "object"               # Batch of all S graphs in sample order (works with forward_every_node)
+    conn_ids: torch.Tensor        # [N] int64: lightpath of each node of ``batch``
+    chan_node: torch.Tensor       # [S, L, Q] int32: node of ``batch`` on each channel, -1 = free
+    rowptr: torch.Tensor          # [N+1] int64: node v's out-edges are [rowptr[v], rowptr[v+1]) of batch.edge_index
+    freqs: torch.Tensor           # [Q] float64
+    cfg: "object"                 # the QotLpGraphCfg the graphs were built with (scaling ranges, threshold)
+    S: int
+    L: int
+    Q: int
+
+
+class LightpathCandidates(NamedTuple):
+    """Candidate lightpaths (device tensors).  Candidate k: sample ``sample[k]`` of the state, the path
+    ``links[link_ptr[k]:link_ptr[k+1]]``, slots ``[q0[k], q0[k] + width[k])`` on every link of the path, raw channel
+    vector ``feat[k] = (freq, mod_order, num_spans, path_len)``."""
+    sample: torch.Tensor          # [K] int64
+    link_ptr: torch.Tensor        # [K+1] int64
+    links: torch.Tensor           # [sum of path lengths] int32
+    q0: torch.Tensor              # [K] int32
+    width: torch.Tensor           # [K] int32
+    feat: torch.Tensor            # [K, 4] float32
+
+    def to(self, device) -> "LightpathCandidates":
+        return LightpathCandidates(*(t.to(device) for t in self))
+
+
+@_lib.on_tensor_device
+def lightpath_network_state(data: torch.Tensor, freqs: torch.Tensor, lp_feat: Sequence[str],
+                            freq_threshold: float = 0.05) -> LightpathNetworkState:
+    """data [S, F, L, Q] float32 (CUDA, 0 = free channel), freqs [Q] float64 -> the network state candidate lightpaths
+    are evaluated against.  Builds the S graphs with ``create_lightpath_graphs`` (its one host synchronisation; no
+    targets needed), collates them in sample order, and maps every channel to its node (qot_lightpath_channel_map).
+    ``state.batch`` goes straight into ``LightpathGNN.forward_every_node`` (the QoT of the lightpaths already set up)."""
+    if not data.is_cuda:
+        raise RuntimeError("lightpath_network_state needs CUDA tensors (gnn_qot_estimation_b200 has no CPU path)")
+    dev = data.device
+    data = data.to(torch.float32).contiguous()
+    freqs = freqs.to(dev, torch.float64).contiguous()
+    S, F, L, Q = (int(v) for v in data.shape)
+    metric = ["osnr", "snr", "ber"]
+    store, conn_ids = create_lightpath_graphs(data, torch.zeros(S, 3, dtype=torch.float64, device=dev), freqs, lp_feat,
+                                              metric, freq_threshold, return_conn_ids=True)
+    # edges come out sorted by (source, target), both directions of every interaction, no repeated pair: the layout
+    # verify_layout() checks, by construction
+    store.sym_by_src = True
+    batch = store.collate(range(S))
+    N = int(batch.x.shape[0])
+    rowptr = torch.zeros(N + 1, dtype=torch.int64, device=dev)
+    rowptr[1:] = torch.cumsum(torch.bincount(batch.edge_index[0], minlength=N), 0)
+    cfg = _cfg(lp_feat, metric, F, L, Q, 3, freq_threshold)
+    chan_node = torch.empty(S, L, Q, dtype=torch.int32, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    check(_lib.lib().qot_lightpath_channel_map(ptr(data), S, C.byref(cfg), ptr(batch.ptr), ptr(conn_ids), N,
+                                               ptr(chan_node), ptr(status), stream()), "qot_lightpath_channel_map")
+    _track_status("qot_lightpath_channel_map (an occupied channel's conn_id is not among its sample's lightpaths)",
+                  status)
+    return LightpathNetworkState(batch, conn_ids, chan_node, rowptr, freqs, cfg, S, L, Q)

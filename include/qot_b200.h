@@ -511,6 +511,56 @@ int qot_lightpath_graph_fill(const void* scratch, int64_t S, const int64_t* node
                              const int64_t* edge_ptr, float* node_feat, int64_t* conn_ids,
                              int32_t* edge_src, int32_t* edge_dst, int32_t* status, void* stream);
 
+/* Candidate QoT (csrc/lightpath_candidates.cu): candidate lightpaths evaluated against a resident NETWORK STATE -- raw
+ * samples data [S, F, L, Q] float32 (0 = free channel), the grid freqs [Q] float64 and the qot_lp_graph_cfg_t they
+ * were turned into graphs with (qot_lightpath_graph_count / _fill, then qot_collate of all S samples in order) --
+ * without rebuilding the state's graphs.
+ *
+ * qot_lightpath_channel_map (lp_channel_map_kernel, once per state): chan_node [S, L, Q] int32 = the state-batch node
+ * index of the lightpath on each channel, -1 on a free channel.  A channel is occupied when any of its F features is
+ * non-zero; its lightpath is the conn_id row truncated toward zero (both as qot_lightpath_graph_count reads them),
+ * looked up in conn_ids [N] int64 over the sample's nodes [node_ptr[s], node_ptr[s+1]) (node_ptr [S+1] int64).
+ * status (optional, int32[1], zeroed by the caller): bit 0 = an occupied channel whose conn_id the sample's node list
+ * lacks, or malformed node offsets; such a channel holds INT_MIN (occupied, no neighbour). */
+int qot_lightpath_channel_map(const float* data, int64_t S, const qot_lp_graph_cfg_t* cfg, const int64_t* node_ptr,
+                              const int64_t* conn_ids, int64_t N, int32_t* chan_node, int32_t* status, void* stream);
+
+/* qot_lightpath_candidates (lp_candidate_kernel): K candidates, one warp each, one launch.  Candidate k names sample
+ * sample[k], a path links[link_ptr[k] .. link_ptr[k+1]) (int32 link indices; duplicates change nothing), the slot
+ * range [q0[k], q0[k] + width[k]) used on every link of the path and its raw channel vector feat [K,4] = (freq,
+ * mod_order, num_spans, path_len), the values to_graph would read from its channels.  sample' = data[sample[k]] with
+ * the candidate written into every channel of its path and slot range (new conn_id, features feat[k], osnr = snr =
+ * ber = -1).  In sample''s lightpath graph, with the flag column x[:, is_lut_index] one-hot:
+ *   out [K,3]          row k: the reference LightpathGNN.forward under eval() with the flag at the candidate's node;
+ *   impact rows        one per existing lightpath j adjacent to the candidate (sharing a link at 0 < |freqs[qc] -
+ *                      freqs[qj]| < cfg->freq_threshold in fp64): the same forward with the flag at j, in ascending
+ *                      order of j's state-batch node index.  impact_node [K,max_impact] int64 = j, impact_out
+ *                      [K,max_impact,3]; slots past the rows written hold -1 / NaN.  n_impact [K] int32 = the number
+ *                      of neighbours (may exceed max_impact).
+ * Candidates are independent of each other.  The candidate's x row is feat scaled as qot_lightpath_graph_count scales
+ * node features (min-max in fp64 of the float32 value with cfg->feat_lo / feat_hi, then fp32).
+ * State: freqs [Q] float64, x [N,5], node_ptr [S+1], rowptr [N+1] int64 (node v's out-edges are
+ * [rowptr[v], rowptr[v+1]) of edge_index [2,E] int64, which must be the layout qot_lightpath_graph_fill produces:
+ * sorted by source, every edge in both directions, so a node's in-neighbours are the destinations of its out-run),
+ * chan_node from qot_lightpath_channel_map.  n_links: entries of `links`.  `prepared` as for
+ * qot_lightpath_infer_stream.  status [K] int32 (written for every candidate), bits QOT_CAND_*: with BAD_SAMPLE,
+ * BAD_PATH, OCCUPIED or BAD_STATE before the scan ends the out row is NaN and n_impact is 0; with IMPACT_OVERFLOW the
+ * out row and the first max_impact impact rows are written.  No host synchronisation: capturable; a malformed
+ * candidate never faults and never stops the launch. */
+#define QOT_CAND_BAD_SAMPLE 1        /* sample[k] outside [0, S)                                                  */
+#define QOT_CAND_BAD_PATH 2          /* empty path, a link outside [0, L), width < 1 or slot range outside [0, Q) */
+#define QOT_CAND_OCCUPIED 4          /* a channel of the candidate is occupied on some link of its path           */
+#define QOT_CAND_IMPACT_OVERFLOW 8   /* more neighbours than max_impact                                           */
+#define QOT_CAND_BAD_STATE 16        /* the state arrays are inconsistent (offsets, chan_node, rowptr); the
+                                        affected rows are NaN                                                     */
+int qot_lightpath_candidates(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
+                             const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N,
+                             int64_t E, const int32_t* chan_node, int64_t K, const int64_t* sample,
+                             const int64_t* link_ptr, const int32_t* links, int64_t n_links, const int32_t* q0,
+                             const int32_t* width, const float* feat, const float* prepared, int32_t is_lut_index,
+                             int32_t max_impact, float* out, int32_t* status, int32_t* n_impact,
+                             int64_t* impact_node, float* impact_out, void* stream);
+
 /* The topological representation: to_graph.py::create_topological_graph (:62-184: one edge per
  * lightpath between its source and destination network node, lightpaths added in ascending conn_id,
  * nx.Graph keeps one edge per node pair -- position from the first, attributes from the last) fused
