@@ -22,6 +22,15 @@
 //                      source-sorted edge list (self loop dropped, flag 0), the candidate (flag 0), j's self loop.
 //     Every z row goes through the warp's 16-row buffer and head_rows16_tf32x3 (the mma.sync head of every-node mode).
 //
+// Reconfiguration (qot_lightpath_reconfigure, the kMove instantiation): a change is a candidate that also names the
+// lightpath j it moves (-1: a plain insertion, bit-identical to the candidate path).  j's old channels count as free,
+// its old neighbours (the destinations of its out-run, self loop dropped) go into a second 256-bit mask, and the impact
+// rows are the union of both masks, ranked ascending, with kind bits old | new << 1:
+//       j's row:         query flag 1, j's new neighbours (flag 0), the appended self loop (none for a teardown);
+//       impact row i:    query flag 1, i's state in-row without j (flag 0), j with its new x if i is a new
+//                        neighbour (flag 0), i's self loop.
+// Every other row of the sample is unchanged, for the same locality reason as a candidate's.
+//
 // Deterministic: integer mask bits only, fixed message order, no float atomics.  A malformed candidate gets status
 // bits and a NaN row; it never faults and never stops the launch.
 #include <algorithm>
@@ -79,9 +88,10 @@ static_assert(kCdMaskWords <= 32, "one mask word per lane");
 struct CdWarpSmem {
   float z[16 * kCdZPitch];                 // staged z rows of the head
   long long orow[16];                      // where each staged row's 3 outputs go
-  int nbr[kCdMaxN + 1];                    // neighbours (sample-local, ascending), then the candidate's self loop
-  int msg[kCdMsgCap];                      // message list of one impact row
-  unsigned mask[kCdMaskWords];             // neighbour bits
+  int nbr[kCdMaxN + 1];                    // impact rows (sample-local, ascending), then the candidate's self loop
+  int msg[kCdMsgCap];                      // message list of one row
+  unsigned mask[kCdMaskWords];             // neighbour bits of the new placement
+  unsigned omask[kCdMaskWords];            // old neighbour bits of the moved lightpath (reconfiguration only)
   float cx[8];                             // the candidate's scaled x row
 };
 struct CdSmem {
@@ -139,6 +149,20 @@ __device__ __forceinline__ int cd_row(CdWarpSmem& ws, int w, int zc, const int* 
   return zc;
 }
 
+// ranks the set bits of a 256-bit mask (lane t < 8 holds word t) ascending into dst[0, count); returns the count
+__device__ __forceinline__ int cd_rank(unsigned mw, int* dst, int lane) {
+  int pos = __popc(mw);
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int up = __shfl_up_sync(kFull, pos, o);
+    if (lane >= o) pos += up;
+  }
+  const int cnt = __shfl_sync(kFull, pos, 31);
+  pos -= __popc(mw);
+  for (unsigned m = mw; m; m &= m - 1) dst[pos++] = 32 * lane + __ffs(m) - 1;
+  return cnt;
+}
+
 struct CdArgs {
   qot_lp_graph_cfg_t cfg;
   int64_t S, N, E, K, n_links;
@@ -148,6 +172,7 @@ struct CdArgs {
   const int64_t* rowptr;
   const int64_t* edst;                     // destination row of the state's source-sorted edge_index
   const int32_t* chan_node;
+  const int64_t* node;                     // moved lightpath of each change (kMove only)
   const int64_t* sample;
   const int64_t* link_ptr;
   const int32_t* links;
@@ -160,9 +185,12 @@ struct CdArgs {
   int32_t* status;
   int32_t* n_impact;
   int64_t* impact_node;
+  int8_t* impact_kind;                     // optional (kMove only)
   float* impact_out;
 };
 
+// kMove = false: qot_lightpath_candidates; true: qot_lightpath_reconfigure (a.node, a.impact_kind)
+template <bool kMove>
 __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __grid_constant__ CdArgs a) {
   CdSmem& sm = cd_smem();
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
@@ -188,15 +216,20 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
     int st = 0;
     const int64_t s = a.sample[k];
     if (s < 0 || s >= a.S) st |= QOT_CAND_BAD_SAMPLE;
+    const int64_t jg = kMove ? a.node[k] : -1;            // moved lightpath (state-batch node), -1 = an insertion
     const int64_t p0 = a.link_ptr[k], p1 = a.link_ptr[k + 1];
+    const bool tear = kMove && jg >= 0 && p1 == p0;       // a teardown: no new placement, q0 / width / feat unused
     const int c0 = a.q0[k], cw = a.width[k];
     bool badp = !(p0 >= 0 && p1 > p0 && p1 <= a.n_links) || cw < 1 || c0 < 0 || static_cast<int64_t>(c0) + cw > Q;
+    if (kMove && tear) badp = !(p0 >= 0 && p0 <= a.n_links);
     if (!badp)
       for (int64_t e = p0 + lane; e < p1; e += 32) {
         const int l = a.links[e];
         badp |= l < 0 || l >= L;
       }
     if (__any_sync(kFull, badp)) st |= QOT_CAND_BAD_PATH;
+    if (kMove && jg != -1 && !(st & QOT_CAND_BAD_SAMPLE) && (jg < a.node_ptr[s] || jg >= a.node_ptr[s + 1]))
+      st |= QOT_CAND_BAD_NODE;
     int64_t n0 = 0;
     int n = 0;
     if (st == 0) {
@@ -205,8 +238,12 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
       if (n0 >= 0 && n1 >= n0 && n1 <= a.N && n1 - n0 <= kCdMaxN) n = static_cast<int>(n1 - n0);
       else st |= QOT_CAND_BAD_STATE;
     }
+    const int jm = kMove && st == 0 && jg >= 0 ? static_cast<int>(jg - n0) : -1;   // sample-local; -1 matches no node
     // ---- neighbours: chan_node rows of the path's links, the fp64 df test of to_graph.cu
-    if (lane < kCdMaskWords) ws.mask[lane] = 0u;
+    if (lane < kCdMaskWords) {
+      ws.mask[lane] = 0u;
+      if (kMove) ws.omask[lane] = 0u;
+    }
     __syncwarp();
     if (st == 0) {
       bool occ = false, bad = false;
@@ -214,7 +251,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
         const int32_t* __restrict__ row = a.chan_node + (s * L + a.links[e]) * Q;
         for (int q = lane; q < Q; q += 32) {
           const int32_t v = row[q];
-          if (v == -1) continue;
+          if (v == -1 || (kMove && v == jg)) continue;            // free, or the moved lightpath's own channel
           if (q >= c0 && q < c0 + cw) { occ = true; continue; }
           if (v < -1) continue;                                   // occupied by an unknown lightpath: no edge
           const int64_t j = v - n0;
@@ -228,33 +265,38 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
           if (hit) atomicOr(&ws.mask[j >> 5], 1u << (j & 31));
         }
       }
+      if (kMove && jm >= 0) {                 // old neighbours: destinations of j's out-run, self loop dropped
+        const int64_t r0 = a.rowptr[n0 + jm], r1 = a.rowptr[n0 + jm + 1];
+        if (!(r0 >= 0 && r1 >= r0 && r1 <= a.E)) bad = true;
+        else
+          for (int64_t e = r0 + lane; e < r1; e += 32) {
+            const int64_t dg = a.edst[e] - n0;
+            if (dg < 0 || dg >= n) bad = true;
+            else if (dg != jm) atomicOr(&ws.omask[dg >> 5], 1u << (dg & 31));
+          }
+      }
       if (__any_sync(kFull, occ)) st |= QOT_CAND_OCCUPIED;
       if (__any_sync(kFull, bad)) st |= QOT_CAND_BAD_STATE;
     }
     __syncwarp();
-    if (st & (QOT_CAND_BAD_SAMPLE | QOT_CAND_BAD_PATH | QOT_CAND_OCCUPIED | QOT_CAND_BAD_STATE)) {
+    if (st & (QOT_CAND_BAD_SAMPLE | QOT_CAND_BAD_PATH | QOT_CAND_OCCUPIED | QOT_CAND_BAD_STATE | QOT_CAND_BAD_NODE)) {
       if (lane < QOT_OUT) a.out[k * QOT_OUT + lane] = nan;
       if (lane == 0) {
         a.status[k] = st;
         a.n_impact[k] = 0;
       }
       for (int i = lane; i < MI; i += 32) a.impact_node[k * MI + i] = -1;
+      if (kMove && a.impact_kind)
+        for (int i = lane; i < MI; i += 32) a.impact_kind[k * MI + i] = 0;
       for (int i = lane; i < MI * QOT_OUT; i += 32) a.impact_out[k * MI * QOT_OUT + i] = nan;
       continue;
     }
-    // ---- neighbours ranked ascending: lane t < 8 owns mask word t
+    // ---- neighbours of the new placement ranked ascending: lane t < 8 owns mask word t.  A candidate's impact rows
+    // are exactly these; a change's own row takes them from msg and its impact rows are ranked below.
     const unsigned mw = lane < kCdMaskWords ? ws.mask[lane] : 0u;
-    int pos = __popc(mw);
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int up = __shfl_up_sync(kFull, pos, o);
-      if (lane >= o) pos += up;
-    }
-    const int cnt = __shfl_sync(kFull, pos, 31);
-    pos -= __popc(mw);
-    for (unsigned m = mw; m; m &= m - 1) ws.nbr[pos++] = 32 * lane + __ffs(m) - 1;
-    if (lane == 0) ws.nbr[cnt] = kCand;                           // the candidate's appended self loop
-    if (cnt > MI) st |= QOT_CAND_IMPACT_OVERFLOW;
+    int* own = kMove ? ws.msg : ws.nbr;
+    const int nn = cd_rank(mw, own, lane);
+    if (lane == 0) own[nn] = kCand;                               // the candidate's appended self loop
     // ---- the candidate's x row [freq, is_lut, mod_order, num_spans, path_len]: min-max in fp64 of the float32
     // value, then fp32 (dataset.py's scaling; feat_lo / feat_hi in feat's order)
     if (lane < 4) {
@@ -266,15 +308,31 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
     __syncwarp();
     const float* xs = a.x + n0 * kF;
     // ---- candidate row: neighbours (flag 0), then its self loop (flag 1)
-    zc = cd_row(ws, w, zc, ws.nbr, cnt + 1, kCand, CdX{xs, ws.cx, kCand, a.lut_col}, As, Ad, a.out + k * QOT_OUT,
-                prep, lane);
+    if (kMove && tear) {
+      if (lane < QOT_OUT) a.out[k * QOT_OUT + lane] = nan;
+    } else {
+      zc = cd_row(ws, w, zc, own, nn + 1, kCand, CdX{xs, ws.cx, kCand, a.lut_col}, As, Ad, a.out + k * QOT_OUT,
+                  prep, lane);
+    }
+    int cnt = nn;
+    if (kMove) {                             // impact rows of a change: old and new neighbours
+      cnt = cd_rank(mw | (lane < kCdMaskWords ? ws.omask[lane] : 0u), ws.nbr, lane);
+      __syncwarp();
+    }
+    if (cnt > MI) st |= QOT_CAND_IMPACT_OVERFLOW;
     // ---- impact rows: neighbour j's in-row (flag 0), the candidate (flag 0), j's self loop (flag 1)
     const int rows = min(cnt, MI);
     for (int i = 0; i < rows; ++i) {
       const int j = ws.nbr[i];
+      const int kind = kMove ? static_cast<int>((ws.omask[j >> 5] >> (j & 31) & 1u) |
+                                                (ws.mask[j >> 5] >> (j & 31) & 1u) << 1)
+                             : 2;            // bit 0: was a neighbour of the moved lightpath, bit 1: is one now
       const int64_t r0 = a.rowptr[n0 + j], r1 = a.rowptr[n0 + j + 1];
       float* dst = a.impact_out + (k * MI + i) * QOT_OUT;
-      if (lane == 0) a.impact_node[k * MI + i] = n0 + j;
+      if (lane == 0) {
+        a.impact_node[k * MI + i] = n0 + j;
+        if (kMove && a.impact_kind) a.impact_kind[k * MI + i] = static_cast<int8_t>(kind);
+      }
       bool bad = !(r0 >= 0 && r1 >= r0 && r1 <= a.E && r1 - r0 <= kCdMaxN);
       int m = 0;
       if (!bad) {
@@ -283,7 +341,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
           const int64_t dg = e < r1 ? a.edst[e] - n0 : -1;
           const bool inside = dg >= 0 && dg < n;
           bad |= e < r1 && !inside;
-          const bool keep = inside && dg != j;
+          const bool keep = inside && dg != j && (!kMove || dg != jm);
           const unsigned ball = __ballot_sync(kFull, keep);
           if (keep) ws.msg[m + __popc(ball & ((1u << lane) - 1u))] = static_cast<int>(dg);
           m += __popc(ball);
@@ -295,14 +353,18 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
         __syncwarp();
         continue;
       }
+      const int mc = kind >> 1;               // the candidate / moved lightpath is a message of new neighbours only
       if (lane == 0) {
-        ws.msg[m] = kCand;
-        ws.msg[m + 1] = j;
+        if (mc) ws.msg[m] = kCand;
+        ws.msg[m + mc] = j;
       }
       __syncwarp();
-      zc = cd_row(ws, w, zc, ws.msg, m + 2, j, CdX{xs, ws.cx, j, a.lut_col}, As, Ad, dst, prep, lane);
+      zc = cd_row(ws, w, zc, ws.msg, m + mc + 1, j, CdX{xs, ws.cx, j, a.lut_col}, As, Ad, dst, prep, lane);
     }
-    for (int i = rows + lane; i < MI; i += 32) a.impact_node[k * MI + i] = -1;
+    for (int i = rows + lane; i < MI; i += 32) {
+      a.impact_node[k * MI + i] = -1;
+      if (kMove && a.impact_kind) a.impact_kind[k * MI + i] = 0;
+    }
     for (int i = rows * QOT_OUT + lane; i < MI * QOT_OUT; i += 32) a.impact_out[k * MI * QOT_OUT + i] = nan;
     if (lane == 0) {
       a.status[k] = st;
@@ -317,6 +379,51 @@ static int cfg_check(const qot_lp_graph_cfg_t* cfg, const char* who) {
   QOT_REQUIRE(cfg->F > 0 && cfg->L > 0 && cfg->Q > 0 && cfg->L <= 65535 && cfg->Q <= 65535 &&
                   static_cast<int64_t>(cfg->L) * cfg->Q < (1ll << 30), "%s: bad tensor extents", who);
   QOT_REQUIRE(cfg->i_conn >= 0 && cfg->i_conn < cfg->F, "%s: conn_id row out of range", who);
+  return QOT_OK;
+}
+
+// shared by both entry points: argument checks, the once-per-device shared-memory opt-in, the launch
+template <bool kMove>
+static int cd_launch(const char* who, const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
+                     const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N, int64_t E,
+                     const int32_t* chan_node, int64_t K, const int64_t* node, const int64_t* sample,
+                     const int64_t* link_ptr, const int32_t* links, int64_t n_links, const int32_t* q0,
+                     const int32_t* width, const float* feat, const float* prepared, int32_t is_lut_index,
+                     int32_t max_impact, float* out, int32_t* status, int32_t* n_impact, int64_t* impact_node,
+                     int8_t* impact_kind, float* impact_out, cudaStream_t stream) {
+  if (int rc = cfg_check(cfg, who)) return rc;
+  QOT_REQUIRE(S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && K >= 0 && n_links >= 0 && max_impact >= 0,
+              "%s: bad size", who);
+  QOT_REQUIRE(prepared && (reinterpret_cast<uintptr_t>(prepared) & 15) == 0, "%s: prepared must be 16-byte aligned",
+              who);
+  QOT_REQUIRE(is_lut_index >= 0 && is_lut_index < kF, "%s: is_lut_index out of range", who);
+  if (K == 0) return QOT_OK;
+  QOT_REQUIRE(sample && link_ptr && q0 && width && feat && out && status && n_impact && (n_links == 0 || links) &&
+                  (max_impact == 0 || (impact_node && impact_out)) && (!kMove || node),
+              "%s: null candidate or output array", who);
+  QOT_REQUIRE(S == 0 || (freqs && x && node_ptr && rowptr && chan_node && (E == 0 || edge_index)),
+              "%s: null state array", who);
+  static std::atomic<unsigned long long> done{0};
+  constexpr int smem = static_cast<int>(sizeof(CdSmem));
+  if (int rc = once_per_device(done, [] {
+        QOT_CUDA(cudaFuncSetAttribute(lp_candidate_kernel<kMove>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        return static_cast<int>(QOT_OK);
+      }))
+    return rc;
+  CdArgs a;
+  a.cfg = *cfg;
+  a.S = S; a.N = N; a.E = E; a.K = K; a.n_links = n_links;
+  a.freqs = freqs; a.x = x; a.node_ptr = node_ptr; a.rowptr = rowptr;
+  a.edst = edge_index ? edge_index + E : nullptr;
+  a.chan_node = chan_node;
+  a.node = node;
+  a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = q0; a.width = width; a.feat = feat;
+  a.prep = prepared; a.lut_col = is_lut_index; a.max_impact = max_impact;
+  a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_node;
+  a.impact_kind = max_impact ? impact_kind : nullptr; a.impact_out = impact_out;
+  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, cdiv(K, kCdWarps)));
+  lp_candidate_kernel<kMove><<<grid, kCdThreads, smem, stream>>>(a);
+  QOT_LAUNCH_CHECK();
   return QOT_OK;
 }
 
@@ -348,37 +455,23 @@ extern "C" int qot_lightpath_candidates(const qot_lp_graph_cfg_t* cfg, int64_t S
                                         int32_t is_lut_index, int32_t max_impact, float* out, int32_t* status,
                                         int32_t* n_impact, int64_t* impact_node, float* impact_out,
                                         void* stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (int rc = cfg_check(cfg, "qot_lightpath_candidates")) return rc;
-  QOT_REQUIRE(S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && K >= 0 && n_links >= 0 && max_impact >= 0,
-              "qot_lightpath_candidates: bad size");
-  QOT_REQUIRE(prepared && (reinterpret_cast<uintptr_t>(prepared) & 15) == 0,
-              "qot_lightpath_candidates: prepared must be 16-byte aligned");
-  QOT_REQUIRE(is_lut_index >= 0 && is_lut_index < kF, "qot_lightpath_candidates: is_lut_index out of range");
-  if (K == 0) return QOT_OK;
-  QOT_REQUIRE(sample && link_ptr && q0 && width && feat && out && status && n_impact && (n_links == 0 || links) &&
-                  (max_impact == 0 || (impact_node && impact_out)),
-              "qot_lightpath_candidates: null candidate or output array");
-  QOT_REQUIRE(S == 0 || (freqs && x && node_ptr && rowptr && chan_node && (E == 0 || edge_index)),
-              "qot_lightpath_candidates: null state array");
-  static std::atomic<unsigned long long> done{0};
-  constexpr int smem = static_cast<int>(sizeof(CdSmem));
-  if (int rc = once_per_device(done, [] {
-        QOT_CUDA(cudaFuncSetAttribute(lp_candidate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        return static_cast<int>(QOT_OK);
-      }))
-    return rc;
-  CdArgs a;
-  a.cfg = *cfg;
-  a.S = S; a.N = N; a.E = E; a.K = K; a.n_links = n_links;
-  a.freqs = freqs; a.x = x; a.node_ptr = node_ptr; a.rowptr = rowptr;
-  a.edst = edge_index ? edge_index + E : nullptr;
-  a.chan_node = chan_node;
-  a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = q0; a.width = width; a.feat = feat;
-  a.prep = prepared; a.lut_col = is_lut_index; a.max_impact = max_impact;
-  a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_node; a.impact_out = impact_out;
-  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, cdiv(K, kCdWarps)));
-  lp_candidate_kernel<<<grid, kCdThreads, smem, stream>>>(a);
-  QOT_LAUNCH_CHECK();
-  return QOT_OK;
+  return cd_launch<false>("qot_lightpath_candidates", cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node,
+                          K, nullptr, sample, link_ptr, links, n_links, q0, width, feat, prepared, is_lut_index,
+                          max_impact, out, status, n_impact, impact_node, nullptr, impact_out,
+                          static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int qot_lightpath_reconfigure(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs,
+                                         const float* x, const int64_t* node_ptr, const int64_t* rowptr,
+                                         const int64_t* edge_index, int64_t N, int64_t E, const int32_t* chan_node,
+                                         int64_t K, const int64_t* node, const int64_t* sample,
+                                         const int64_t* link_ptr, const int32_t* links, int64_t n_links,
+                                         const int32_t* q0, const int32_t* width, const float* feat,
+                                         const float* prepared, int32_t is_lut_index, int32_t max_impact, float* out,
+                                         int32_t* status, int32_t* n_impact, int64_t* impact_node,
+                                         int8_t* impact_kind, float* impact_out, void* stream_) {
+  return cd_launch<true>("qot_lightpath_reconfigure", cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E,
+                         chan_node, K, node, sample, link_ptr, links, n_links, q0, width, feat, prepared,
+                         is_lut_index, max_impact, out, status, n_impact, impact_node, impact_kind, impact_out,
+                         static_cast<cudaStream_t>(stream_));
 }

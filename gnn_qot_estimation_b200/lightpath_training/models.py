@@ -165,6 +165,31 @@ class LightpathGNN(torch.nn.Module):
         return ops.lightpath_candidates(state, cands, self.prepared(), self.is_lut_index, max_impact)
 
     @_lib.on_tensor_device
+    def forward_reconfigurations(self, state, changes, max_impact: int = 64) -> "ops.ReconfigQoT":
+        """QoT after moving, retuning, rerouting or tearing down a lightpath of a network state, and what each change
+        does to the other lightpaths (eval mode only; csrc/lightpath_candidates.cu, qot_lightpath_reconfigure).
+
+        ``changes``: ``to_graph.LightpathChanges`` on the state's device (``to_graph.lightpath_nodes`` turns conn_ids
+        into its ``node`` entries).  For change k with moved lightpath j (conn_id c), let sample' be sample
+        ``changes.sample[k]`` with every channel of c cleared and, unless the path is empty (a teardown), j written on
+        every channel of the new path and slot range with features ``changes.feat[k]`` (its other rows as on its first
+        channel).  In sample''s lightpath graph with the flag column one-hot: ``out[k]`` is ``forward`` under ``eval()``
+        with the flag at j (NaN for a teardown); ``impact_out[k, r]`` is the same with the flag at ``impact_node[k, r]``,
+        each lightpath that was or is adjacent to j, ascending, and ``impact_kind[k, r]`` says which (``ops.KIND_LOST``
+        1, ``KIND_GAINED`` 2, ``KIND_KEPT`` 3).  Every other lightpath's QoT is unchanged:
+        ``forward_every_node(state.batch)`` gives it.  ``node[k] = -1`` is an insertion, bit-identical to
+        ``forward_candidates``.  Changes are evaluated independently, each against the state alone.  ``status`` holds
+        ``ops.CAND_*`` bits (``CAND_BAD_NODE``: the node is not in the sample; j's own channels are not OCCUPIED).
+        One launch, nothing read back: capturable in a CUDA graph.  Malformed arguments raise on the host."""
+        if self.training:
+            raise RuntimeError("LightpathGNN.forward_reconfigurations is eval-only (in training mode BatchNorm couples "
+                               "the nodes): call model.eval()")
+        if not state.batch.x.is_cuda:
+            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
+        self._check_supported()
+        return ops.lightpath_reconfigure(state, changes, self.prepared(), self.is_lut_index, max_impact)
+
+    @_lib.on_tensor_device
     def forward_stream(self, plan, first: int = 0, count=None) -> None:
         """Enqueues batches [first, first+count) of ``plan`` (eval mode; no host synchronisation)."""
         if self.training:

@@ -334,8 +334,11 @@ class LightpathStreamPlan:
                                  self.status[i:i + 1])
 
 
-# status bits of qot_lightpath_candidates (include/qot_b200.h)
+# status bits of qot_lightpath_candidates / qot_lightpath_reconfigure (include/qot_b200.h)
 CAND_BAD_SAMPLE, CAND_BAD_PATH, CAND_OCCUPIED, CAND_IMPACT_OVERFLOW, CAND_BAD_STATE = 1, 2, 4, 8, 16
+CAND_BAD_NODE = 32
+# impact_kind bits of qot_lightpath_reconfigure
+KIND_LOST, KIND_GAINED, KIND_KEPT = 1, 2, 3
 
 
 class CandidateQoT(NamedTuple):
@@ -346,32 +349,59 @@ class CandidateQoT(NamedTuple):
     impact_out: torch.Tensor     # [K, max_impact, 3]: their QoT with the candidate set up; NaN past the rows
 
 
+class ReconfigQoT(NamedTuple):
+    out: torch.Tensor            # [K,3]: the moved lightpath's QoT at its new placement (NaN for a teardown)
+    status: torch.Tensor         # [K] int32, CAND_* bits
+    n_impact: torch.Tensor       # [K] int32: lightpaths that lose, gain or keep the moved one (may exceed max_impact)
+    impact_node: torch.Tensor    # [K, max_impact] int64: their nodes in the state batch, ascending; -1 past the rows
+    impact_kind: torch.Tensor    # [K, max_impact] int8: KIND_LOST / KIND_GAINED / KIND_KEPT; 0 past the rows
+    impact_out: torch.Tensor     # [K, max_impact, 3]: their QoT after the change; NaN past the rows
+
+
+_CAND_DTYPES = {"sample": torch.int64, "link_ptr": torch.int64, "links": torch.int32, "q0": torch.int32,
+                "width": torch.int32, "feat": torch.float32}
+
+
+def _check_candidate_args(state, c, prepared, max_impact, who: str, arg: str, want: dict) -> int:
+    """Host-side checks shared by forward_candidates and forward_reconfigurations; returns K."""
+    if int(max_impact) != max_impact or max_impact < 0:
+        raise ValueError(f"{who}: max_impact must be a non-negative integer")
+    dev = state.batch.x.device
+    for name, dt in want.items():
+        t = getattr(c, name)
+        if not torch.is_tensor(t) or not t.is_cuda:
+            raise RuntimeError(f"{who}: {arg}.{name} must be a CUDA tensor (no CPU path)")
+        if t.device != dev:
+            raise ValueError(f"{who}: {arg}.{name} is on {t.device}, the state on {dev}")
+        if t.dtype != dt:
+            raise TypeError(f"{who}: {arg}.{name} must be {dt}, got {t.dtype}")
+    if prepared.device != dev:
+        raise ValueError(f"{who}: the model is on {prepared.device}, the state on {dev}")
+    K = int(c.sample.shape[0]) if c.sample.dim() == 1 else -1
+    shapes_ok = (K >= 0 and c.link_ptr.shape == (K + 1,) and c.links.dim() == 1 and
+                 c.q0.shape == (K,) and c.width.shape == (K,) and c.feat.shape == (K, 4))
+    if not shapes_ok:
+        raise ValueError(f"{who}: need sample [K], link_ptr [K+1], links [n], q0 [K], width [K], feat [K,4]")
+    if "node" in want and c.node.shape != (K,):
+        raise ValueError(f"{who}: need node [K] with K = sample.shape[0]")
+    return K
+
+
+def _state_args(state, keep: list):
+    """The state's leading arguments of qot_lightpath_candidates / _reconfigure; converted tensors go into `keep`."""
+    b = state.batch
+    x, ei = _f32(b.x), _i64(b.edge_index)
+    keep += [x, ei]
+    return (C.byref(state.cfg), state.S, ptr(state.freqs), ptr(x), ptr(b.ptr), ptr(state.rowptr),
+            ptr(ei) if ei.numel() else None, int(x.shape[0]), int(ei.shape[1]), ptr(state.chan_node))
+
+
 def lightpath_candidates(state, cands, prepared: torch.Tensor, is_lut_index: int, max_impact: int) -> CandidateQoT:
     """One launch of qot_lightpath_candidates; nothing is read back (CUDA-graph capturable).  Refuses CPU tensors and
     mismatched devices, dtypes or shapes; what can only be judged on the device comes back as status bits."""
-    if int(max_impact) != max_impact or max_impact < 0:
-        raise ValueError("forward_candidates: max_impact must be a non-negative integer")
+    K = _check_candidate_args(state, cands, prepared, max_impact, "forward_candidates", "cands", _CAND_DTYPES)
     max_impact = int(max_impact)
-    b = state.batch
-    dev = b.x.device
-    want = {"sample": torch.int64, "link_ptr": torch.int64, "links": torch.int32, "q0": torch.int32,
-            "width": torch.int32, "feat": torch.float32}
-    for name, dt in want.items():
-        t = getattr(cands, name)
-        if not torch.is_tensor(t) or not t.is_cuda:
-            raise RuntimeError(f"forward_candidates: cands.{name} must be a CUDA tensor (no CPU path)")
-        if t.device != dev:
-            raise ValueError(f"forward_candidates: cands.{name} is on {t.device}, the state on {dev}")
-        if t.dtype != dt:
-            raise TypeError(f"forward_candidates: cands.{name} must be {dt}, got {t.dtype}")
-    if prepared.device != dev:
-        raise ValueError(f"forward_candidates: the model is on {prepared.device}, the state on {dev}")
-    K = int(cands.sample.shape[0]) if cands.sample.dim() == 1 else -1
-    shapes_ok = (K >= 0 and cands.link_ptr.shape == (K + 1,) and cands.links.dim() == 1 and
-                 cands.q0.shape == (K,) and cands.width.shape == (K,) and cands.feat.shape == (K, 4))
-    if not shapes_ok:
-        raise ValueError("forward_candidates: need sample [K], link_ptr [K+1], links [n], q0 [K], width [K], "
-                         "feat [K,4]")
+    dev = state.batch.x.device
     out = torch.empty(K, 3, dtype=torch.float32, device=dev)
     status = torch.empty(K, dtype=torch.int32, device=dev)
     n_impact = torch.empty(K, dtype=torch.int32, device=dev)
@@ -380,16 +410,41 @@ def lightpath_candidates(state, cands, prepared: torch.Tensor, is_lut_index: int
     if K == 0:
         return CandidateQoT(out, status, n_impact, impact_node, impact_out)
     c = lambda t: ptr(t.contiguous()) if t.numel() else None
-    ei = b.edge_index
     keep = [t.contiguous() for t in cands]           # alive until the launch is enqueued
     with torch.cuda.device(dev):                     # stream() of the state's device
         check(_lib.lib().qot_lightpath_candidates(
-            C.byref(state.cfg), state.S, ptr(state.freqs), ptr(_f32(b.x)), ptr(b.ptr), ptr(state.rowptr),
-            ptr(_i64(ei)) if ei.numel() else None, int(b.x.shape[0]), int(ei.shape[1]), ptr(state.chan_node), K,
+            *_state_args(state, keep), K,
             ptr(keep[0]), ptr(keep[1]), c(keep[2]), int(keep[2].numel()), ptr(keep[3]), ptr(keep[4]), ptr(keep[5]),
             ptr(prepared), int(is_lut_index), max_impact, ptr(out), ptr(status), ptr(n_impact),
             c(impact_node), c(impact_out), stream()), "qot_lightpath_candidates")
     return CandidateQoT(out, status, n_impact, impact_node, impact_out)
+
+
+def lightpath_reconfigure(state, changes, prepared: torch.Tensor, is_lut_index: int, max_impact: int) -> ReconfigQoT:
+    """One launch of qot_lightpath_reconfigure (moves, teardowns and insertions of lightpaths, each against the state
+    alone); nothing is read back (CUDA-graph capturable).  Same host-side checks as ``lightpath_candidates``."""
+    want = dict(_CAND_DTYPES, node=torch.int64)
+    K = _check_candidate_args(state, changes, prepared, max_impact, "forward_reconfigurations", "changes", want)
+    max_impact = int(max_impact)
+    dev = state.batch.x.device
+    out = torch.empty(K, 3, dtype=torch.float32, device=dev)
+    status = torch.empty(K, dtype=torch.int32, device=dev)
+    n_impact = torch.empty(K, dtype=torch.int32, device=dev)
+    impact_node = torch.empty(K, max_impact, dtype=torch.int64, device=dev)
+    impact_kind = torch.empty(K, max_impact, dtype=torch.int8, device=dev)
+    impact_out = torch.empty(K, max_impact, 3, dtype=torch.float32, device=dev)
+    if K == 0:
+        return ReconfigQoT(out, status, n_impact, impact_node, impact_kind, impact_out)
+    c = lambda t: ptr(t.contiguous()) if t.numel() else None
+    ch = changes
+    keep = [t.contiguous() for t in (ch.node, ch.sample, ch.link_ptr, ch.links, ch.q0, ch.width, ch.feat)]
+    with torch.cuda.device(dev):
+        check(_lib.lib().qot_lightpath_reconfigure(
+            *_state_args(state, keep), K, ptr(keep[0]),
+            ptr(keep[1]), ptr(keep[2]), c(keep[3]), int(keep[3].numel()), ptr(keep[4]), ptr(keep[5]), ptr(keep[6]),
+            ptr(prepared), int(is_lut_index), max_impact, ptr(out), ptr(status), ptr(n_impact),
+            c(impact_node), c(impact_kind), c(impact_out), stream()), "qot_lightpath_reconfigure")
+    return ReconfigQoT(out, status, n_impact, impact_node, impact_kind, impact_out)
 
 
 class GraphIndex:

@@ -226,3 +226,94 @@ def lightpath_candidates(samples, per_sample: int, seed: int = 0):
                                torch.tensor(links, dtype=torch.int32), torch.tensor(q0s, dtype=torch.int32),
                                torch.tensor(widths, dtype=torch.int32),
                                torch.tensor(np.array(feats, dtype=np.float32).reshape(-1, 4)))
+
+
+def lightpath_changes(samples, state, per_sample: int, seed: int = 0):
+    """Seeded changes to the lightpaths of ``samples`` (the dict ``network_status_samples`` returns), whose network
+    state ``state`` is (``to_graph.lightpath_network_state``; its node numbering gives ``node``).  ``per_sample``
+    changes per sample, a mix of
+      - retunes (0.35): the lightpath on its own links at another slot of its own width; half of them take the nearest
+        slot, which overlaps its own slots for a super-channel;
+      - reroutes (0.30): onto 1..6 distinct random links, its own width, new num_spans and path_len;
+      - teardowns (0.20): an empty path (q0, width and feat are the lightpath's own, and unused);
+      - insertions (0.15): node -1, as ``lightpath_candidates`` draws them.
+    A move keeps the lightpath's mod_order and sets ``freq = float32(freqs[q0])``; its channels are free or its own on
+    every link of its path.  A sample without lightpaths gets insertions only; a draw that finds no room after 64 tries
+    is dropped.  Returns ``to_graph.LightpathChanges`` of CPU tensors (``.to(device)``)."""
+    import numpy as np
+    from .to_graph import LightpathChanges
+    rng = np.random.default_rng(seed)
+    data, freqs = samples["data"], samples["freqs"]
+    fi = {k: i for i, k in enumerate(samples["lp_feat"])}
+    S, _, L, Q = data.shape
+    occupied = np.any(data != 0, axis=1)                       # [S, L, Q]
+    conn_ids = state.conn_ids.cpu().numpy()
+    ptr = state.batch.ptr.cpu().numpy()
+    nodes, smp, lptr, links, q0s, widths, feats = [], [], [0], [], [], [], []
+
+    def slots_ok(free, path, width):
+        """[Q - width + 1] bool: start slots whose width slots are free on every link of path."""
+        f = free[path].all(axis=0)
+        ok = f[:Q - width + 1].copy()
+        for u in range(1, width):
+            ok &= f[u:Q - width + 1 + u]
+        return np.flatnonzero(ok)
+
+    def emit(node, s, path, q0, width, feat):
+        nodes.append(node)
+        smp.append(s)
+        links.extend(int(l) for l in path)
+        lptr.append(len(links))
+        q0s.append(int(q0))
+        widths.append(int(width))
+        feats.append(feat)
+
+    for s in range(S):
+        conn = np.trunc(data[s, fi["conn_id"]])
+        n0, n1 = int(ptr[s]), int(ptr[s + 1])
+        for _ in range(per_sample):
+            r = rng.random() if n1 > n0 else 1.0
+            if r >= 0.85:                                          # insertion
+                for _try in range(64):
+                    width = 2 if rng.random() < 0.1 else 1
+                    path = rng.choice(L, size=min(int(rng.integers(1, 7)), L), replace=False)
+                    cand = slots_ok(~occupied[s], path, width)
+                    if cand.size:
+                        q0 = int(rng.choice(cand))
+                        emit(-1, s, path, q0, width, [np.float32(freqs[q0]), rng.choice([4, 8, 16, 32, 64]),
+                                                      int(rng.integers(1, 107)), int(rng.integers(24214, 7834746))])
+                        break
+                continue
+            j = int(rng.integers(n0, n1))
+            mine = occupied[s] & (conn == conn_ids[j])
+            ls, qs = np.nonzero(mine)                              # row-major: (ls[0], qs[0]) is the first channel
+            own_links = np.unique(ls)
+            q_own, w = int(qs.min()), int(qs.max() - qs.min() + 1)
+            mod, spans, plen = (data[s, fi[k], ls[0], qs[0]] for k in ("mod_order", "num_spans", "path_len"))
+            free = ~occupied[s] | mine
+            if r < 0.35:                                           # retune on its own links
+                cand = slots_ok(free, own_links, w)
+                other = cand[cand != q_own]
+                if other.size == 0:
+                    q0 = q_own
+                elif rng.random() < 0.5:
+                    d = np.abs(other - q_own)
+                    q0 = int(rng.choice(other[d == d.min()]))
+                else:
+                    q0 = int(rng.choice(other))
+                emit(j, s, own_links, q0, w, [np.float32(freqs[q0]), mod, spans, plen])
+            elif r < 0.65:                                         # reroute
+                for _try in range(64):
+                    path = rng.choice(L, size=min(int(rng.integers(1, 7)), L), replace=False)
+                    cand = slots_ok(free, path, w)
+                    if cand.size:
+                        q0 = int(rng.choice(cand))
+                        emit(j, s, path, q0, w, [np.float32(freqs[q0]), mod, int(rng.integers(1, 107)),
+                                                 int(rng.integers(24214, 7834746))])
+                        break
+            else:                                                  # teardown
+                emit(j, s, [], q_own, w, [np.float32(freqs[q_own]), mod, spans, plen])
+    return LightpathChanges(torch.tensor(nodes, dtype=torch.int64), torch.tensor(smp, dtype=torch.int64),
+                            torch.tensor(lptr, dtype=torch.int64), torch.tensor(links, dtype=torch.int32),
+                            torch.tensor(q0s, dtype=torch.int32), torch.tensor(widths, dtype=torch.int32),
+                            torch.tensor(np.array(feats, dtype=np.float32).reshape(-1, 4)))

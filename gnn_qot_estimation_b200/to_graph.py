@@ -164,6 +164,42 @@ class LightpathCandidates(NamedTuple):
         return LightpathCandidates(*(t.to(device) for t in self))
 
 
+class LightpathChanges(NamedTuple):
+    """Changes to a network state (device tensors): change k moves lightpath ``node[k]`` (a node of ``state.batch`` in
+    sample ``sample[k]``, see ``lightpath_nodes``; -1 = a new lightpath, as a candidate) onto the path
+    ``links[link_ptr[k]:link_ptr[k+1]]`` and slots ``[q0[k], q0[k] + width[k])`` with raw channel vector ``feat[k] =
+    (freq, mod_order, num_spans, path_len)``.  An empty path with ``node[k] >= 0`` tears the lightpath down."""
+    node: torch.Tensor            # [K] int64
+    sample: torch.Tensor          # [K] int64
+    link_ptr: torch.Tensor        # [K+1] int64
+    links: torch.Tensor           # [sum of path lengths] int32
+    q0: torch.Tensor              # [K] int32
+    width: torch.Tensor           # [K] int32
+    feat: torch.Tensor            # [K, 4] float32
+
+    def to(self, device) -> "LightpathChanges":
+        return LightpathChanges(*(t.to(device) for t in self))
+
+
+def lightpath_nodes(state: LightpathNetworkState, sample: torch.Tensor, conn_id: torch.Tensor) -> torch.Tensor:
+    """[K] int64: the node of ``state.batch`` that holds lightpath ``conn_id[k]`` in sample ``sample[k]``, -1 where the
+    sample has no such lightpath (or ``sample[k]`` is outside the state).  Device tensor ops, no host synchronisation:
+    one sort of the state's (sample, conn_id) keys and a binary search per query."""
+    b = state.batch
+    dev = b.x.device
+    sample = sample.to(dev, torch.int64)
+    conn_id = conn_id.to(dev, torch.int64)
+    lo, span = -(1 << 31), 1 << 32                           # conn_ids are int32 values (a float32 row truncated)
+    key = b.batch.to(torch.int64) * span + (state.conn_ids - lo)
+    skey, order = torch.sort(key)
+    ok = (sample >= 0) & (sample < state.S) & (conn_id >= lo) & (conn_id < lo + span)
+    q = torch.where(ok, sample * span + (conn_id - lo), torch.full_like(sample, -1))
+    if skey.numel() == 0:
+        return torch.full_like(sample, -1)
+    i = torch.searchsorted(skey, q).clamp(max=skey.numel() - 1)
+    return torch.where(ok & (skey[i] == q), order[i], torch.full_like(sample, -1))
+
+
 @_lib.on_tensor_device
 def lightpath_network_state(data: torch.Tensor, freqs: torch.Tensor, lp_feat: Sequence[str],
                             freq_threshold: float = 0.05) -> LightpathNetworkState:

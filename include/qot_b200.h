@@ -561,6 +561,34 @@ int qot_lightpath_candidates(const qot_lp_graph_cfg_t* cfg, int64_t S, const dou
                              int32_t max_impact, float* out, int32_t* status, int32_t* n_impact,
                              int64_t* impact_node, float* impact_out, void* stream);
 
+/* qot_lightpath_reconfigure (lp_candidate_kernel, the same launch shape): K changes to the state, evaluated
+ * independently, each against the state alone.  Change k takes the candidate arguments above plus node [K] int64:
+ * the lightpath it moves, a node of the state batch in [node_ptr[s], node_ptr[s+1]) for s = sample[k], or -1 for a
+ * plain insertion (then every output is bit-identical to qot_lightpath_candidates and every impact_kind is 2).  Let c
+ * be the moved lightpath j's conn_id.  sample' = data[s] with every channel of conn_id c zeroed and then, unless the
+ * change is a teardown, one vector written on every channel of the path and slot range: conn_id c, the feat[k] values,
+ * and j's other rows (src/dst, metrics) from j's first channel.  AN EMPTY PATH WITH node[k] >= 0 IS A TEARDOWN, not
+ * BAD_PATH: q0, width and feat are not read, the out row is NaN.  A channel of the new placement is occupied when its
+ * chan_node is neither -1 nor j (j's own channels are free; INT_MIN is occupied).  In sample''s graph:
+ *   out [K,3]          the forward with the flag at j's new node (NaN for a teardown);
+ *   impact rows        every lightpath i != j that was adjacent to j in the state graph or is adjacent to j in
+ *                      sample''s graph, ascending in node order of the state batch: impact_node = i, impact_out = the
+ *                      forward with the flag at i, impact_kind [K,max_impact] int8 (optional, may be NULL) = bit 0: i
+ *                      was j's neighbour, bit 1: i is j's neighbour after the change (1 lost j, 2 gained j, 3 kept j
+ *                      with its new features); slots past the rows written hold -1 / 0 / NaN.  n_impact [K] = the
+ *                      number of such rows (may exceed max_impact).
+ * Every other row of sample' equals its row in the state.  Message order: j's row = its new neighbours ascending, then
+ * its self loop; row i = i's state in-row ascending without j and without i's self loop, then j if bit 1 is set, then
+ * i's self loop.  Status bits QOT_CAND_*, plus BAD_NODE; with BAD_NODE the out row is NaN and n_impact is 0. */
+#define QOT_CAND_BAD_NODE 32         /* node[k] is neither -1 nor a node of sample[k]                             */
+int qot_lightpath_reconfigure(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
+                              const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N,
+                              int64_t E, const int32_t* chan_node, int64_t K, const int64_t* node,
+                              const int64_t* sample, const int64_t* link_ptr, const int32_t* links, int64_t n_links,
+                              const int32_t* q0, const int32_t* width, const float* feat, const float* prepared,
+                              int32_t is_lut_index, int32_t max_impact, float* out, int32_t* status, int32_t* n_impact,
+                              int64_t* impact_node, int8_t* impact_kind, float* impact_out, void* stream);
+
 /* The topological representation: to_graph.py::create_topological_graph (:62-184: one edge per
  * lightpath between its source and destination network node, lightpaths added in ascending conn_id,
  * nx.Graph keeps one edge per node pair -- position from the first, attributes from the last) fused
