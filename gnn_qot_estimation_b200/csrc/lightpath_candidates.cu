@@ -131,7 +131,8 @@ __device__ __noinline__ void cd_flush(int w, int cnt, const float* __restrict__ 
 }
 
 // attention of query node q over msg[0, M) into the next staged z row; the row's outputs go to `dst`
-__device__ __forceinline__ int cd_row(CdWarpSmem& ws, int w, int zc, const int* msg, int M, int q, const CdX& xf,
+template <typename XF>
+__device__ __forceinline__ int cd_row(CdWarpSmem& ws, int w, int zc, const int* msg, int M, int q, const XF& xf,
                                       const float (&As)[kF], const float (&Ad)[kF], float* dst,
                                       const float* __restrict__ prep, int lane) {
   float d_q = 0.f;
@@ -374,6 +375,380 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
   if (zc) cd_flush(w, zc, prep, lane);
 }
 
+// ------------------------------------------------------------------------------------------------ change sets
+// lp_change_set_kernel: persistent, one warp per set of changes to one sample (qot_lightpath_change_sets).  The set's
+// removed lightpaths R (the nodes its changes move or tear down) go into a 256-bit mask; each placed change scans its
+// path's chan_node rows with R counted as free, its new neighbours into its own 256-bit mask; the placed changes are
+// tested pairwise (a shared link and 0 < |df| < threshold: adjacent; a shared channel: a conflict); R's out-runs give
+// the old neighbours.  The impact rows are the union of all masks without R, ranked ascending.  Changed lightpath c is
+// message source -1 - c (its scaled x row in the warp's table), so a set of one change runs the reconfiguration rows
+// with the same message order and values: bit-identical to lp_candidate_kernel<true>.
+constexpr int kCsMaxChanges = QOT_SET_MAX_CHANGES;
+constexpr int kCsMsgCap = kCdMaxN + kCsMaxChanges + 8;  // in-row (<= kCdMaxN) + changed lightpaths + self loop
+constexpr int kCsFatal = QOT_CAND_BAD_SAMPLE | QOT_CAND_BAD_PATH | QOT_CAND_OCCUPIED | QOT_CAND_BAD_STATE |
+                         QOT_CAND_BAD_NODE | QOT_SET_BAD_SET | QOT_SET_DUPLICATE | QOT_SET_CONFLICT;
+static_assert(kCsMaxChanges == 64, "the pairwise matrix and the per-set bit words hold 64 changes");
+
+struct CsWarpSmem {
+  unsigned nmask[kCsMaxChanges][kCdMaskWords];  // new-neighbour bits of each change
+  float cx[kCsMaxChanges][8];                   // scaled x row of each change
+  unsigned long long adj[kCsMaxChanges];        // bit d of row c: changes c and d are adjacent
+  int msg[kCsMsgCap];                           // message list of one row
+  int st[kCsMaxChanges];                        // status bits of each change
+  int jm[kCsMaxChanges];                        // sample-local node each change moves or tears down, -1: none
+  unsigned rmask[kCdMaskWords];                 // R: the lightpaths the set moves or tears down
+  unsigned char tear[kCsMaxChanges];            // the change is a teardown
+  long long k0, n0;                             // the set's first change and its sample's first node
+  int nc, cnt, any;                             // changes, impact rows, OR of the status words
+};
+struct CsSmem {
+  CdSmem cd;                                    // head fragments and the candidate kernel's per-warp state
+  CsWarpSmem w[kCdWarps];
+};
+static_assert(sizeof(CsSmem) + 16 <= 227 * 1024, "lp_change_set_kernel: shared memory over the 227 KB block limit");
+
+// x of a message source: sample-local node j >= 0 of the state, or changed lightpath -1 - j of the set
+struct CsX {
+  const float* __restrict__ xs;
+  const float (*cx)[8];
+  int lut, col;
+  __device__ __forceinline__ float operator()(int j, int k) const {
+    if (k == col) return j == lut ? 1.0f : 0.0f;
+    return j < 0 ? cx[-1 - j][k] : __ldg(xs + static_cast<int64_t>(j) * kF + k);
+  }
+};
+
+struct CsArgs {
+  CdArgs c;                                // the reconfiguration arguments; status, n_impact and impact_* are per set
+  int64_t G;
+  const int64_t* set_ptr;
+  float* chg_out;                          // [K,3]
+  int32_t* chg_status;                     // [K]
+};
+
+__device__ __forceinline__ bool cs_bit(const unsigned* m, int j) { return m[j >> 5] >> (j & 31) & 1u; }
+
+__global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __grid_constant__ CsArgs ca) {
+  const CdArgs& a = ca.c;
+  CsSmem& sm = *reinterpret_cast<CsSmem*>(cd_smem_raw);
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  CdWarpSmem& ws = sm.cd.w[w];
+  CsWarpSmem& xw = sm.w[w];
+  for (int i = tid; i < kStHeadFrag4; i += kCdThreads)
+    sm.cd.frag[i] = __ldg(reinterpret_cast<const float4*>(a.prep + kOffB1f) + i);
+  // set_ptr must partition [0, K): non-decreasing from 0 to K.  Otherwise sets could overlap, so none is evaluated:
+  // every change and every set gets BAD_SET, each output written by exactly one thread of the grid.
+  bool bad_ptr = false;
+  for (int64_t g = tid; g <= ca.G; g += kCdThreads) {
+    const int64_t v = ca.set_ptr[g];
+    bad_ptr |= (g == 0 && v != 0) || (g == ca.G && v != a.K) || (g < ca.G && ca.set_ptr[g + 1] < v);
+  }
+  bad_ptr = __syncthreads_or(bad_ptr);
+  const float* __restrict__ prep = a.prep;
+  const float nan = __int_as_float(0x7fc00000);
+  if (bad_ptr) {
+    const int64_t gt = static_cast<int64_t>(blockIdx.x) * kCdThreads + tid;
+    const int64_t gs = static_cast<int64_t>(gridDim.x) * kCdThreads;
+    for (int64_t k = gt; k < a.K; k += gs) {
+      ca.chg_status[k] = QOT_SET_BAD_SET;
+      for (int o = 0; o < QOT_OUT; ++o) ca.chg_out[k * QOT_OUT + o] = nan;
+    }
+    for (int64_t g = gt; g < ca.G; g += gs) {
+      a.status[g] = QOT_SET_BAD_SET;
+      a.n_impact[g] = 0;
+      for (int i = 0; i < a.max_impact; ++i) {
+        a.impact_node[g * a.max_impact + i] = -1;
+        if (a.impact_kind) a.impact_kind[g * a.max_impact + i] = 0;
+        for (int o = 0; o < QOT_OUT; ++o) a.impact_out[(g * a.max_impact + i) * QOT_OUT + o] = nan;
+      }
+    }
+    return;
+  }
+  const int h = lane & 3;
+  float As[kF], Ad[kF];
+#pragma unroll
+  for (int k = 0; k < kF; ++k) {
+    As[k] = __ldg(prep + kOffAsrc + k * kHeads + h);
+    Ad[k] = __ldg(prep + kOffAdst + k * kHeads + h);
+  }
+  // L, Q, the threshold and max_impact are read from the kernel parameters where used: hoisted, they spill
+  int zc = 0;                                       // rows staged in this warp's head buffer
+  for (int64_t g = static_cast<int64_t>(blockIdx.x) * kCdWarps + w; g < ca.G;
+       g += static_cast<int64_t>(gridDim.x) * kCdWarps) {
+    const int64_t k0 = ca.set_ptr[g], nk = ca.set_ptr[g + 1] - k0;
+    const int nc = nk > kCsMaxChanges ? 0 : static_cast<int>(nk);   // a set over the limit is not examined
+    const int64_t s = nc ? a.sample[k0] : -1;
+    int64_t n0 = 0;
+    int n = 0;
+    bool state_ok = s >= 0 && s < a.S;
+    if (state_ok) {
+      n0 = a.node_ptr[s];
+      const int64_t n1 = a.node_ptr[s + 1];
+      if (n0 >= 0 && n1 >= n0 && n1 <= a.N && n1 - n0 <= kCdMaxN) n = static_cast<int>(n1 - n0);
+      else state_ok = false;
+    }
+    if (lane < kCdMaskWords) {
+      xw.rmask[lane] = 0u;
+      ws.mask[lane] = 0u;
+      ws.omask[lane] = 0u;
+    }
+    __syncwarp();
+    // ---- each change: the reconfiguration checks, the set's sample, R, the scaled x row
+    for (int c = 0; c < nc; ++c) {
+      const int64_t k = k0 + c;
+      int st = 0;
+      const int64_t sk = a.sample[k];
+      if (sk < 0 || sk >= a.S) st |= QOT_CAND_BAD_SAMPLE;
+      if (sk != s) st |= QOT_SET_BAD_SET;
+      const int64_t jg = a.node[k];
+      const int64_t p0 = a.link_ptr[k], p1 = a.link_ptr[k + 1];
+      const bool tear = jg >= 0 && p1 == p0;        // a teardown: no new placement, q0 / width / feat unused
+      const int c0 = a.q0[k], cw = a.width[k];
+      bool badp = tear ? !(p0 >= 0 && p0 <= a.n_links)
+                       : !(p0 >= 0 && p1 > p0 && p1 <= a.n_links) || cw < 1 || c0 < 0 ||
+                             static_cast<int64_t>(c0) + cw > a.cfg.Q;
+      if (!badp)
+        for (int64_t e = p0 + lane; e < p1; e += 32) {
+          const int l = a.links[e];
+          badp |= l < 0 || l >= a.cfg.L;
+        }
+      if (__any_sync(kFull, badp)) st |= QOT_CAND_BAD_PATH;
+      if (jg != -1 && !(st & QOT_CAND_BAD_SAMPLE) && (jg < a.node_ptr[sk] || jg >= a.node_ptr[sk + 1]))
+        st |= QOT_CAND_BAD_NODE;
+      if (st == 0 && !state_ok) st |= QOT_CAND_BAD_STATE;
+      const int jm = st == 0 && jg >= 0 ? static_cast<int>(jg - n0) : -1;
+      if (lane == 0) {
+        if (jm >= 0) {
+          if (cs_bit(xw.rmask, jm)) st |= QOT_SET_DUPLICATE;
+          xw.rmask[jm >> 5] |= 1u << (jm & 31);
+        }
+        xw.st[c] = st;
+        xw.jm[c] = jm;
+        xw.tear[c] = tear;
+      }
+      if (lane < kCdMaskWords) xw.nmask[c][lane] = 0u;
+      // x row [freq, is_lut, mod_order, num_spans, path_len]: dataset.py's scaling, as the candidate kernel
+      if (lane < 4) {
+        const double v = static_cast<double>(a.feat[k * 4 + lane]);
+        xw.cx[c][lane == 0 ? 0 : lane + 1] =
+            static_cast<float>((v - a.cfg.feat_lo[lane]) / (a.cfg.feat_hi[lane] - a.cfg.feat_lo[lane]));
+      }
+      if (lane == 4) xw.cx[c][1] = 1.0f;
+      __syncwarp();
+    }
+    if (lane == 0)                                  // every change removing a lightpath removed twice
+      for (int c = 1; c < nc; ++c)
+        if (xw.st[c] & QOT_SET_DUPLICATE)
+          for (int d = 0; d < c; ++d)
+            if (xw.jm[d] == xw.jm[c]) xw.st[d] |= QOT_SET_DUPLICATE;
+    __syncwarp();
+    int any = nk > kCsMaxChanges ? QOT_SET_BAD_SET : 0;
+    for (int c = 0; c < nc; ++c) any |= xw.st[c];
+    if (!(any & kCsFatal)) {
+      // ---- new neighbours of each placed change; R's channels are free and R is no neighbour
+      for (int c = 0; c < nc; ++c) {
+        if (xw.tear[c]) continue;
+        const int64_t k = k0 + c;
+        const int64_t p0 = a.link_ptr[k], p1 = a.link_ptr[k + 1];
+        const int c0 = a.q0[k], cw = a.width[k];
+        bool occ = false, bad = false;
+        for (int64_t e = p0; e < p1; ++e) {
+          const int32_t* __restrict__ row = a.chan_node + (s * a.cfg.L + a.links[e]) * a.cfg.Q;
+          for (int q = lane; q < a.cfg.Q; q += 32) {
+            const int32_t v = row[q];
+            if (v == -1) continue;
+            const int64_t j = v - n0;
+            const bool inside = v >= 0 && j >= 0 && j < n;
+            if (inside && cs_bit(xw.rmask, static_cast<int>(j))) continue;
+            if (q >= c0 && q < c0 + cw) { occ = true; continue; }
+            if (v < -1) continue;                   // occupied by an unknown lightpath: no edge
+            if (!inside) { bad = true; continue; }
+            const double fq = a.freqs[q];
+            bool hit = false;
+            for (int cc = c0; cc < c0 + cw && !hit; ++cc) {
+              const double df = fabs(a.freqs[cc] - fq);
+              hit = df < a.cfg.freq_threshold && df > 0.0;
+            }
+            if (hit) atomicOr(&xw.nmask[c][j >> 5], 1u << (j & 31));
+          }
+        }
+        const bool o = __any_sync(kFull, occ), b = __any_sync(kFull, bad);
+        if (lane == 0) xw.st[c] |= (o ? QOT_CAND_OCCUPIED : 0) | (b ? QOT_CAND_BAD_STATE : 0);
+      }
+      // ---- old neighbours: the destinations of R's out-runs, self loops dropped
+      for (int c = 0; c < nc; ++c) {
+        const int jm = xw.jm[c];
+        if (jm < 0) continue;
+        const int64_t r0 = a.rowptr[n0 + jm], r1 = a.rowptr[n0 + jm + 1];
+        bool bad = !(r0 >= 0 && r1 >= r0 && r1 <= a.E);
+        if (!bad)
+          for (int64_t e = r0 + lane; e < r1; e += 32) {
+            const int64_t dg = a.edst[e] - n0;
+            if (dg < 0 || dg >= n) bad = true;
+            else if (dg != jm) atomicOr(&ws.omask[dg >> 5], 1u << (dg & 31));
+          }
+        if (__any_sync(kFull, bad) && lane == 0) xw.st[c] |= QOT_CAND_BAD_STATE;
+      }
+      // ---- pairs of placed changes, one lane per pair: a shared link and a shared slot is a conflict, a shared link
+      // and 0 < |df| < threshold (to_graph's test on the grid) an edge
+      for (int c = lane; c < nc; c += 32) xw.adj[c] = 0ull;
+      __syncwarp();
+      for (int pr = lane; pr < nc * nc; pr += 32) {
+        const int c = pr / nc, d = pr - c * nc;
+        if (d <= c || xw.tear[c] || xw.tear[d]) continue;
+        const int64_t kc = k0 + c, kd = k0 + d;
+        bool share = false;
+        for (int64_t e = a.link_ptr[kc]; e < a.link_ptr[kc + 1] && !share; ++e)
+          for (int64_t f = a.link_ptr[kd]; f < a.link_ptr[kd + 1] && !share; ++f) share = a.links[e] == a.links[f];
+        if (!share) continue;
+        const int c0 = a.q0[kc], cw = a.width[kc], d0 = a.q0[kd], dw = a.width[kd];
+        if (c0 < d0 + dw && d0 < c0 + cw) {
+          atomicOr(&xw.st[c], QOT_SET_CONFLICT);
+          atomicOr(&xw.st[d], QOT_SET_CONFLICT);
+          continue;
+        }
+        bool hit = false;
+        for (int qc = c0; qc < c0 + cw && !hit; ++qc)
+          for (int qd = d0; qd < d0 + dw && !hit; ++qd) {
+            const double df = fabs(a.freqs[qc] - a.freqs[qd]);
+            hit = df < a.cfg.freq_threshold && df > 0.0;
+          }
+        if (hit) {
+          atomicOr(&xw.adj[c], 1ull << d);
+          atomicOr(&xw.adj[d], 1ull << c);
+        }
+      }
+      __syncwarp();
+      any = 0;
+      for (int c = 0; c < nc; ++c) any |= xw.st[c];
+    }
+    // ---- impact rows: every lightpath outside R adjacent to a changed one before or after, ascending; their in-rows
+    // are checked before any row is emitted, so that a bad state leaves the whole set NaN
+    int cnt = 0;
+    if (!(any & kCsFatal)) {
+      if (lane < kCdMaskWords) {
+        unsigned nw = 0u;
+        for (int c = 0; c < nc; ++c) nw |= xw.nmask[c][lane];
+        ws.mask[lane] = nw;
+        ws.omask[lane] &= ~xw.rmask[lane];
+      }
+      __syncwarp();
+      const unsigned uw = lane < kCdMaskWords ? ws.mask[lane] | ws.omask[lane] : 0u;
+      cnt = cd_rank(uw, ws.nbr, lane);
+      __syncwarp();
+      bool bad = false;
+      for (int i = 0; i < min(cnt, a.max_impact); ++i) {
+        const int64_t r0 = a.rowptr[n0 + ws.nbr[i]], r1 = a.rowptr[n0 + ws.nbr[i] + 1];
+        if (!(r0 >= 0 && r1 >= r0 && r1 <= a.E && r1 - r0 <= kCdMaxN)) { bad = true; break; }
+        for (int64_t e = r0 + lane; e < r1; e += 32) {
+          const int64_t dg = a.edst[e] - n0;
+          bad |= dg < 0 || dg >= n;
+        }
+      }
+      if (__any_sync(kFull, bad)) {
+        if (lane == 0) xw.st[0] |= QOT_CAND_BAD_STATE;
+        any |= QOT_CAND_BAD_STATE;
+      }
+      if (cnt > a.max_impact && lane == 0)
+        for (int c = 0; c < nc; ++c) xw.st[c] |= QOT_CAND_IMPACT_OVERFLOW;
+      if (cnt > a.max_impact) any |= QOT_CAND_IMPACT_OVERFLOW;
+      __syncwarp();
+    }
+    if (any & kCsFatal) {                           // a partial joint answer is meaningless: the whole set is NaN
+      for (int64_t k = k0 + lane; k < k0 + nk; k += 32) {
+        ca.chg_status[k] = nc ? xw.st[k - k0] : QOT_SET_BAD_SET;
+        for (int o = 0; o < QOT_OUT; ++o) ca.chg_out[k * QOT_OUT + o] = nan;
+      }
+      if (lane == 0) {
+        a.status[g] = any;
+        a.n_impact[g] = 0;
+      }
+      for (int i = lane; i < a.max_impact; i += 32) {
+        a.impact_node[g * a.max_impact + i] = -1;
+        if (a.impact_kind) a.impact_kind[g * a.max_impact + i] = 0;
+      }
+      for (int i = lane; i < a.max_impact * QOT_OUT; i += 32) a.impact_out[g * a.max_impact * QOT_OUT + i] = nan;
+      __syncwarp();
+      continue;
+    }
+    // ---- the rows, one attention call site: the changes in set order (new neighbours ascending, the adjacent
+    // changes in set order, the self loop), then the impact rows (the state in-row without R and the self loop, the
+    // adjacent changes in set order, the self loop).  The set's scalars live in shared memory across the rows.
+    if (lane == 0) {
+      xw.k0 = k0;
+      xw.n0 = n0;
+      xw.nc = nc;
+      xw.cnt = cnt;
+      xw.any = any;
+    }
+    __syncwarp();
+    for (int r = 0; r < nc + min(cnt, a.max_impact); ++r) {
+      const int64_t n0r = xw.n0;
+      const int ncr = xw.nc;
+      int m = 0, q;
+      float* dst;
+      if (r < ncr) {                                // the row of change c = r
+        dst = ca.chg_out + (xw.k0 + r) * QOT_OUT;
+        if (xw.tear[r]) {
+          if (lane < QOT_OUT) dst[lane] = nan;
+          continue;
+        }
+        m = cd_rank(lane < kCdMaskWords ? xw.nmask[r][lane] : 0u, xw.msg, lane);
+        if (lane == 0) {
+          for (unsigned long long b = xw.adj[r]; b; b &= b - 1) xw.msg[m++] = -(__ffsll(static_cast<long long>(b)));
+          xw.msg[m++] = -1 - r;
+        }
+        m = __shfl_sync(kFull, m, 0);
+        q = -1 - r;
+      } else {                                      // impact row i = r - nc
+        const int i = r - ncr, j = ws.nbr[i];
+        const int kind = static_cast<int>(cs_bit(ws.omask, j)) | static_cast<int>(cs_bit(ws.mask, j)) << 1;
+        const int64_t r0 = a.rowptr[n0r + j], r1 = a.rowptr[n0r + j + 1];
+        if (lane == 0) {
+          a.impact_node[g * a.max_impact + i] = n0r + j;
+          if (a.impact_kind) a.impact_kind[g * a.max_impact + i] = static_cast<int8_t>(kind);
+        }
+        for (int64_t eb = r0; eb < r1; eb += 32) {
+          const int64_t e = eb + lane;
+          const int dg = e < r1 ? static_cast<int>(a.edst[e] - n0r) : -1;
+          const bool keep = dg >= 0 && dg != j && !cs_bit(xw.rmask, dg);
+          const unsigned ball = __ballot_sync(kFull, keep);
+          if (keep) xw.msg[m + __popc(ball & ((1u << lane) - 1u))] = dg;
+          m += __popc(ball);
+        }
+        if (kind >> 1)
+          for (int cb = 0; cb < ncr; cb += 32) {
+            const int c = cb + lane;
+            const bool hit = c < ncr && !xw.tear[c] && cs_bit(xw.nmask[c], j);
+            const unsigned ball = __ballot_sync(kFull, hit);
+            if (hit) xw.msg[m + __popc(ball & ((1u << lane) - 1u))] = -1 - c;
+            m += __popc(ball);
+          }
+        if (lane == 0) xw.msg[m] = j;
+        ++m;
+        q = j;
+        dst = a.impact_out + (g * a.max_impact + i) * QOT_OUT;
+      }
+      __syncwarp();
+      zc = cd_row(ws, w, zc, xw.msg, m, q, CsX{a.x + n0r * kF, xw.cx, q, a.lut_col}, As, Ad, dst, prep, lane);
+    }
+    const int rows = min(xw.cnt, a.max_impact);
+    for (int i = rows + lane; i < a.max_impact; i += 32) {
+      a.impact_node[g * a.max_impact + i] = -1;
+      if (a.impact_kind) a.impact_kind[g * a.max_impact + i] = 0;
+    }
+    for (int i = rows * QOT_OUT + lane; i < a.max_impact * QOT_OUT; i += 32)
+      a.impact_out[g * a.max_impact * QOT_OUT + i] = nan;
+    for (int c = lane; c < xw.nc; c += 32) ca.chg_status[xw.k0 + c] = xw.st[c];
+    if (lane == 0) {
+      a.status[g] = xw.any;
+      a.n_impact[g] = xw.cnt;
+    }
+    __syncwarp();
+  }
+  if (zc) cd_flush(w, zc, prep, lane);
+}
+
 static int cfg_check(const qot_lp_graph_cfg_t* cfg, const char* who) {
   QOT_REQUIRE(cfg, "%s: null cfg", who);
   QOT_REQUIRE(cfg->F > 0 && cfg->L > 0 && cfg->Q > 0 && cfg->L <= 65535 && cfg->Q <= 65535 &&
@@ -427,6 +802,54 @@ static int cd_launch(const char* who, const qot_lp_graph_cfg_t* cfg, int64_t S, 
   return QOT_OK;
 }
 
+static int cs_launch(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
+                     const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N, int64_t E,
+                     const int32_t* chan_node, int64_t K, const int64_t* node, const int64_t* sample,
+                     const int64_t* link_ptr, const int32_t* links, int64_t n_links, const int32_t* q0,
+                     const int32_t* width, const float* feat, int64_t G, const int64_t* set_ptr, const float* prepared,
+                     int32_t is_lut_index, int32_t max_impact, float* out, int32_t* status, int32_t* set_status,
+                     int32_t* n_impact, int64_t* impact_node, int8_t* impact_kind, float* impact_out,
+                     cudaStream_t stream) {
+  const char* who = "qot_lightpath_change_sets";
+  if (int rc = cfg_check(cfg, who)) return rc;
+  QOT_REQUIRE(S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && K >= 0 && G >= 0 && n_links >= 0 && max_impact >= 0,
+              "%s: bad size", who);
+  QOT_REQUIRE(prepared && (reinterpret_cast<uintptr_t>(prepared) & 15) == 0, "%s: prepared must be 16-byte aligned",
+              who);
+  QOT_REQUIRE(is_lut_index >= 0 && is_lut_index < kF, "%s: is_lut_index out of range", who);
+  if (G == 0 && K == 0) return QOT_OK;
+  QOT_REQUIRE(set_ptr && (G == 0 || (set_status && n_impact && (max_impact == 0 || (impact_node && impact_out)))),
+              "%s: null set or set output array", who);
+  QOT_REQUIRE(K == 0 || (node && sample && link_ptr && q0 && width && feat && out && status && (n_links == 0 || links)),
+              "%s: null change or change output array", who);
+  QOT_REQUIRE(S == 0 || (freqs && x && node_ptr && rowptr && chan_node && (E == 0 || edge_index)),
+              "%s: null state array", who);
+  static std::atomic<unsigned long long> done{0};
+  constexpr int smem = static_cast<int>(sizeof(CsSmem));
+  if (int rc = once_per_device(done, [] {
+        QOT_CUDA(cudaFuncSetAttribute(lp_change_set_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        return static_cast<int>(QOT_OK);
+      }))
+    return rc;
+  CsArgs ca;
+  CdArgs& a = ca.c;
+  a.cfg = *cfg;
+  a.S = S; a.N = N; a.E = E; a.K = K; a.n_links = n_links;
+  a.freqs = freqs; a.x = x; a.node_ptr = node_ptr; a.rowptr = rowptr;
+  a.edst = edge_index ? edge_index + E : nullptr;
+  a.chan_node = chan_node;
+  a.node = node;
+  a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = q0; a.width = width; a.feat = feat;
+  a.prep = prepared; a.lut_col = is_lut_index; a.max_impact = max_impact;
+  a.out = nullptr; a.status = set_status; a.n_impact = n_impact; a.impact_node = impact_node;
+  a.impact_kind = max_impact ? impact_kind : nullptr; a.impact_out = impact_out;
+  ca.G = G; ca.set_ptr = set_ptr; ca.chg_out = out; ca.chg_status = status;
+  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, std::max<int64_t>(1, cdiv(G, kCdWarps))));
+  lp_change_set_kernel<<<grid, kCdThreads, smem, stream>>>(ca);
+  QOT_LAUNCH_CHECK();
+  return QOT_OK;
+}
+
 }  // namespace qot
 
 using namespace qot;
@@ -474,4 +897,19 @@ extern "C" int qot_lightpath_reconfigure(const qot_lp_graph_cfg_t* cfg, int64_t 
                          chan_node, K, node, sample, link_ptr, links, n_links, q0, width, feat, prepared,
                          is_lut_index, max_impact, out, status, n_impact, impact_node, impact_kind, impact_out,
                          static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int qot_lightpath_change_sets(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs,
+                                         const float* x, const int64_t* node_ptr, const int64_t* rowptr,
+                                         const int64_t* edge_index, int64_t N, int64_t E, const int32_t* chan_node,
+                                         int64_t K, const int64_t* node, const int64_t* sample,
+                                         const int64_t* link_ptr, const int32_t* links, int64_t n_links,
+                                         const int32_t* q0, const int32_t* width, const float* feat, int64_t G,
+                                         const int64_t* set_ptr, const float* prepared, int32_t is_lut_index,
+                                         int32_t max_impact, float* out, int32_t* status, int32_t* set_status,
+                                         int32_t* n_impact, int64_t* impact_node, int8_t* impact_kind,
+                                         float* impact_out, void* stream_) {
+  return cs_launch(cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, K, node, sample, link_ptr, links,
+                   n_links, q0, width, feat, G, set_ptr, prepared, is_lut_index, max_impact, out, status, set_status,
+                   n_impact, impact_node, impact_kind, impact_out, static_cast<cudaStream_t>(stream_));
 }

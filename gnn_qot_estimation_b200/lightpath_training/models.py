@@ -190,6 +190,34 @@ class LightpathGNN(torch.nn.Module):
         return ops.lightpath_reconfigure(state, changes, self.prepared(), self.is_lut_index, max_impact)
 
     @_lib.on_tensor_device
+    def forward_change_sets(self, state, changes, set_ptr, max_impact: int = 64) -> "ops.ChangeSetQoT":
+        """QoT after several changes to one sample applied together -- batch provisioning, defragmentation with swaps,
+        failure restoration -- and what each set does to the other lightpaths (eval mode only;
+        csrc/lightpath_candidates.cu, qot_lightpath_change_sets).
+
+        ``changes``: ``to_graph.LightpathChanges`` as for ``forward_reconfigurations``; ``set_ptr`` [G+1] int64 on the
+        state's device: set g is changes ``[set_ptr[g], set_ptr[g+1])``, all naming one sample, at most
+        ``ops.SET_MAX_CHANGES``.  sample' = the sample with every lightpath the set moves or tears down cleared, then
+        every non-teardown change written on its path and slots (a move keeps its conn_id and other rows; an insertion
+        gets a new conn_id, one above the sample's largest, +1 per insertion in set order).  In sample''s lightpath graph
+        with the flag column one-hot: ``out[k]`` is the changed lightpath's row (NaN for a teardown);
+        ``impact_out[g, r]`` is the row of ``impact_node[g, r]``, each lightpath the set does not move that is adjacent
+        to a changed lightpath before or after it, ascending, with ``impact_kind[g, r]`` bit 0 (it loses a neighbour)
+        | bit 1 (a changed lightpath is its neighbour now).  Every other lightpath's QoT is unchanged:
+        ``forward_every_node(state.batch)`` gives it.  A channel is occupied only by a lightpath the set does not move,
+        so swaps are legal.  ``status`` holds ``ops.CAND_*`` and ``ops.SET_*`` bits per change, ``set_status`` their
+        OR; any bit but ``CAND_IMPACT_OVERFLOW`` makes the whole set NaN with ``n_impact`` 0.  A set of one change is
+        bit-identical to ``forward_reconfigurations``.  One launch, nothing read back: capturable in a CUDA graph.
+        Malformed arguments raise on the host."""
+        if self.training:
+            raise RuntimeError("LightpathGNN.forward_change_sets is eval-only (in training mode BatchNorm couples the "
+                               "nodes): call model.eval()")
+        if not state.batch.x.is_cuda:
+            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
+        self._check_supported()
+        return ops.lightpath_change_sets(state, changes, set_ptr, self.prepared(), self.is_lut_index, max_impact)
+
+    @_lib.on_tensor_device
     def forward_stream(self, plan, first: int = 0, count=None) -> None:
         """Enqueues batches [first, first+count) of ``plan`` (eval mode; no host synchronisation)."""
         if self.training:

@@ -339,6 +339,9 @@ CAND_BAD_SAMPLE, CAND_BAD_PATH, CAND_OCCUPIED, CAND_IMPACT_OVERFLOW, CAND_BAD_ST
 CAND_BAD_NODE = 32
 # impact_kind bits of qot_lightpath_reconfigure
 KIND_LOST, KIND_GAINED, KIND_KEPT = 1, 2, 3
+# status bits of qot_lightpath_change_sets, on top of the CAND_* bits; a set holds at most SET_MAX_CHANGES changes
+SET_BAD_SET, SET_DUPLICATE, SET_CONFLICT = 64, 128, 256
+SET_MAX_CHANGES = 64
 
 
 class CandidateQoT(NamedTuple):
@@ -356,6 +359,16 @@ class ReconfigQoT(NamedTuple):
     impact_node: torch.Tensor    # [K, max_impact] int64: their nodes in the state batch, ascending; -1 past the rows
     impact_kind: torch.Tensor    # [K, max_impact] int8: KIND_LOST / KIND_GAINED / KIND_KEPT; 0 past the rows
     impact_out: torch.Tensor     # [K, max_impact, 3]: their QoT after the change; NaN past the rows
+
+
+class ChangeSetQoT(NamedTuple):
+    out: torch.Tensor            # [K,3]: each changed lightpath's QoT at its new placement (NaN: teardown, fatal set)
+    status: torch.Tensor         # [K] int32, CAND_* | SET_* bits of each change
+    set_status: torch.Tensor     # [G] int32, the OR over the set's changes
+    n_impact: torch.Tensor       # [G] int32: lightpaths the set disturbs (may exceed max_impact)
+    impact_node: torch.Tensor    # [G, max_impact] int64: their nodes in the state batch, ascending; -1 past the rows
+    impact_kind: torch.Tensor    # [G, max_impact] int8: KIND_LOST / KIND_GAINED / KIND_KEPT; 0 past the rows
+    impact_out: torch.Tensor     # [G, max_impact, 3]: their QoT after the set; NaN past the rows
 
 
 _CAND_DTYPES = {"sample": torch.int64, "link_ptr": torch.int64, "links": torch.int32, "q0": torch.int32,
@@ -445,6 +458,47 @@ def lightpath_reconfigure(state, changes, prepared: torch.Tensor, is_lut_index: 
             ptr(prepared), int(is_lut_index), max_impact, ptr(out), ptr(status), ptr(n_impact),
             c(impact_node), c(impact_kind), c(impact_out), stream()), "qot_lightpath_reconfigure")
     return ReconfigQoT(out, status, n_impact, impact_node, impact_kind, impact_out)
+
+
+def lightpath_change_sets(state, changes, set_ptr: torch.Tensor, prepared: torch.Tensor, is_lut_index: int,
+                          max_impact: int) -> "ChangeSetQoT":
+    """One launch of qot_lightpath_change_sets (sets of changes to one sample each, evaluated jointly); nothing is read
+    back (CUDA-graph capturable).  The host checks of ``lightpath_reconfigure`` plus set_ptr's device, dtype and shape;
+    set_ptr's values are judged on the device (``SET_BAD_SET``)."""
+    who = "forward_change_sets"
+    want = dict(_CAND_DTYPES, node=torch.int64)
+    K = _check_candidate_args(state, changes, prepared, max_impact, who, "changes", want)
+    max_impact = int(max_impact)
+    dev = state.batch.x.device
+    if not torch.is_tensor(set_ptr) or not set_ptr.is_cuda:
+        raise RuntimeError(f"{who}: set_ptr must be a CUDA tensor (no CPU path)")
+    if set_ptr.device != dev:
+        raise ValueError(f"{who}: set_ptr is on {set_ptr.device}, the state on {dev}")
+    if set_ptr.dtype != torch.int64:
+        raise TypeError(f"{who}: set_ptr must be torch.int64, got {set_ptr.dtype}")
+    if set_ptr.dim() != 1 or set_ptr.shape[0] < 1:
+        raise ValueError(f"{who}: need set_ptr [G+1] with G >= 0")
+    G = int(set_ptr.shape[0]) - 1
+    out = torch.empty(K, 3, dtype=torch.float32, device=dev)
+    status = torch.empty(K, dtype=torch.int32, device=dev)
+    set_status = torch.empty(G, dtype=torch.int32, device=dev)
+    n_impact = torch.empty(G, dtype=torch.int32, device=dev)
+    impact_node = torch.empty(G, max_impact, dtype=torch.int64, device=dev)
+    impact_kind = torch.empty(G, max_impact, dtype=torch.int8, device=dev)
+    impact_out = torch.empty(G, max_impact, 3, dtype=torch.float32, device=dev)
+    res = ChangeSetQoT(out, status, set_status, n_impact, impact_node, impact_kind, impact_out)
+    if K == 0 and G == 0:
+        return res
+    c = lambda t: ptr(t.contiguous()) if t.numel() else None
+    ch = changes
+    keep = [t.contiguous() for t in (ch.node, ch.sample, ch.link_ptr, ch.links, ch.q0, ch.width, ch.feat, set_ptr)]
+    with torch.cuda.device(dev):
+        check(_lib.lib().qot_lightpath_change_sets(
+            *_state_args(state, keep), K, c(keep[0]),
+            c(keep[1]), ptr(keep[2]), c(keep[3]), int(keep[3].numel()), c(keep[4]), c(keep[5]), c(keep[6]), G,
+            ptr(keep[7]), ptr(prepared), int(is_lut_index), max_impact, c(out), c(status), c(set_status),
+            c(n_impact), c(impact_node), c(impact_kind), c(impact_out), stream()), "qot_lightpath_change_sets")
+    return res
 
 
 class GraphIndex:

@@ -317,3 +317,182 @@ def lightpath_changes(samples, state, per_sample: int, seed: int = 0):
                             torch.tensor(lptr, dtype=torch.int64), torch.tensor(links, dtype=torch.int32),
                             torch.tensor(q0s, dtype=torch.int32), torch.tensor(widths, dtype=torch.int32),
                             torch.tensor(np.array(feats, dtype=np.float32).reshape(-1, 4)))
+
+
+def lightpath_change_sets(samples, state, per_sample: int, seed: int = 0):
+    """Seeded sets of simultaneous changes to the lightpaths of ``samples`` (as ``lightpath_changes``), for
+    ``LightpathGNN.forward_change_sets``.  ``per_sample`` sets per sample, a mix of
+      - restoration (0.25): a random link that carries lightpaths fails; each lightpath crossing it (at most
+        ``ops.SET_MAX_CHANGES``) is rerouted onto 1..6 links that avoid it, its own width, at slots free once all of
+        them are cleared and not taken by an earlier reroute of the set, or torn down when there is no room;
+      - batch insertion (0.25): 2..8 new lightpaths; after the first, half of them share a link with an earlier one of
+        the set at the slot right next to it, so that the two interfere;
+      - defragmentation (0.25): 2..8 retunes of distinct lightpaths on their own links, starting with a slot swap of two
+        lightpaths of equal width whenever the sample has a pair that can swap;
+      - single changes (0.25): one change drawn as ``lightpath_changes`` draws it.
+    Every placement is free once the set's moved and torn-down lightpaths are cleared, and the placements of a set are
+    disjoint.  A sample without lightpaths gets batch insertions; a draw that finds no room is dropped, so a set may
+    come out smaller (never empty).  Returns ``(to_graph.LightpathChanges, set_ptr [G+1] int64)`` of CPU tensors."""
+    import numpy as np
+    from .to_graph import LightpathChanges
+    rng = np.random.default_rng(seed)
+    data, freqs = samples["data"], samples["freqs"]
+    fi = {k: i for i, k in enumerate(samples["lp_feat"])}
+    S, _, L, Q = data.shape
+    occupied = np.any(data != 0, axis=1)
+    conn_ids = state.conn_ids.cpu().numpy()
+    ptr = state.batch.ptr.cpu().numpy()
+    rows, set_ptr = [], [0]
+
+    def starts(free, path, width):
+        f = free[np.asarray(path)].all(axis=0)
+        ok = f[:Q - width + 1].copy()
+        for u in range(1, width):
+            ok &= f[u:Q - width + 1 + u]
+        return np.flatnonzero(ok)
+
+    def own(s, j):
+        """(channels [L, Q] bool, own links, q0, width, (mod, spans, plen)) of node j of sample s."""
+        mine = occupied[s] & (np.trunc(data[s, fi["conn_id"]]) == conn_ids[j])
+        ls, qs = np.nonzero(mine)
+        rest = tuple(data[s, fi[k], ls[0], qs[0]] for k in ("mod_order", "num_spans", "path_len"))
+        return mine, np.unique(ls), int(qs.min()), int(qs.max() - qs.min() + 1), rest
+
+    def take(free, path, q0, width):
+        free[np.ix_(np.asarray(path), range(q0, q0 + width))] = False
+
+    def rand_path():
+        return rng.choice(L, size=min(int(rng.integers(1, 7)), L), replace=False)
+
+    def new_feat(q0):
+        return [np.float32(freqs[q0]), rng.choice([4, 8, 16, 32, 64]), int(rng.integers(1, 107)),
+                int(rng.integers(24214, 7834746))]
+
+    def restoration(s, n0, n1):
+        carried = np.flatnonzero(occupied[s].any(axis=1))
+        l_fail = int(rng.choice(carried))
+        hit = [j for j in range(n0, n1) if own(s, j)[0][l_fail].any()][:64]
+        info = {j: own(s, j) for j in hit}
+        free = ~occupied[s]
+        for j in hit:
+            free |= info[j][0]
+        out = []
+        for j in hit:
+            _, _, _, w, (mod, _, _) = info[j]
+            for _try in range(16):
+                path = rand_path()
+                if l_fail in path:
+                    continue
+                cand = starts(free, path, w)
+                if cand.size:
+                    q0 = int(rng.choice(cand))
+                    take(free, path, q0, w)
+                    out.append((j, s, path, q0, w, [np.float32(freqs[q0]), mod, int(rng.integers(1, 107)),
+                                                     int(rng.integers(24214, 7834746))]))
+                    break
+            else:
+                out.append((j, s, [], info[j][2], w, [np.float32(freqs[info[j][2]]), mod, 0, 0]))
+        return out
+
+    def batch_insertion(s):
+        free = ~occupied[s]
+        out = []
+        for i in range(int(rng.integers(2, 9))):
+            w = 2 if rng.random() < 0.1 else 1
+            placed = False
+            if out and rng.random() < 0.5:                 # next to an earlier one of the set, on one of its links
+                _, _, p, q, pw, _ = out[int(rng.integers(len(out)))]
+                l = int(rng.choice(p))
+                for q0 in (q + pw, q - w):
+                    if 0 <= q0 and q0 + w <= Q and free[l, q0:q0 + w].all():
+                        path = np.array([l] + [x for x in rand_path() if x != l][:2])
+                        if free[np.ix_(path, range(q0, q0 + w))].all():
+                            take(free, path, q0, w)
+                            out.append((-1, s, path, q0, w, new_feat(q0)))
+                            placed = True
+                            break
+            for _try in range(0 if placed else 16):
+                path = rand_path()
+                cand = starts(free, path, w)
+                if cand.size:
+                    q0 = int(rng.choice(cand))
+                    take(free, path, q0, w)
+                    out.append((-1, s, path, q0, w, new_feat(q0)))
+                    break
+        return out
+
+    def defragmentation(s, n0, n1):
+        info = {j: own(s, j) for j in range(n0, n1)}
+        order = [int(j) for j in rng.permutation(np.arange(n0, n1))]
+        want = int(rng.integers(2, 9))
+        out, moved = [], []
+        free = ~occupied[s]
+        for a in order:                                    # a swap: a onto b's slots on a's links, b onto a's
+            ma, la, qa, wa, ra = info[a]
+            for b in order:
+                mb, lb, qb, wb, rb = info[b]
+                if b == a or wb != wa or qb == qa:
+                    continue
+                others = occupied[s] & ~ma & ~mb
+                if others[np.ix_(la, range(qb, qb + wa))].any() or others[np.ix_(lb, range(qa, qa + wa))].any():
+                    continue
+                if set(la.tolist()) & set(lb.tolist()) and abs(qb - qa) < wa:
+                    continue                               # the two new placements would share a channel
+                free |= ma | mb
+                take(free, la, qb, wa)
+                take(free, lb, qa, wb)
+                out += [(a, s, la, qb, wa, [np.float32(freqs[qb]), *ra]),
+                        (b, s, lb, qa, wb, [np.float32(freqs[qa]), *rb])]
+                moved += [a, b]
+                break
+            if moved:
+                break
+        for j in order:
+            if len(out) >= want:
+                break
+            if j in moved:
+                continue
+            m, ls, q_own, w, r = info[j]
+            f = free | m
+            cand = starts(f, ls, w)
+            cand = cand[cand != q_own]
+            if cand.size:
+                q0 = int(rng.choice(cand))
+                free |= m
+                take(free, ls, q0, w)
+                out.append((j, s, ls, q0, w, [np.float32(freqs[q0]), *r]))
+                moved.append(j)
+        return out
+
+    single = lightpath_changes(samples, state, per_sample, seed=int(rng.integers(1 << 31)))
+    by_sample = {}
+    for k in range(single.sample.shape[0]):
+        a, b = int(single.link_ptr[k]), int(single.link_ptr[k + 1])
+        by_sample.setdefault(int(single.sample[k]), []).append(
+            (int(single.node[k]), int(single.sample[k]), single.links[a:b].tolist(), int(single.q0[k]),
+             int(single.width[k]), single.feat[k].tolist()))
+    for s in range(S):
+        n0, n1 = int(ptr[s]), int(ptr[s + 1])
+        singles = by_sample.get(s, [])
+        for _ in range(per_sample):
+            r = rng.random() if n1 > n0 else 0.3
+            if r < 0.25:
+                got = restoration(s, n0, n1)
+            elif r < 0.5:
+                got = batch_insertion(s)
+            elif r < 0.75:
+                got = defragmentation(s, n0, n1)
+            else:
+                got = [singles.pop(0)] if singles else []
+            if got:
+                rows.extend(got)
+                set_ptr.append(len(rows))
+    lptr = np.cumsum([0] + [len(r[2]) for r in rows])
+    return (LightpathChanges(torch.tensor([r[0] for r in rows], dtype=torch.int64),
+                             torch.tensor([r[1] for r in rows], dtype=torch.int64),
+                             torch.tensor(lptr, dtype=torch.int64),
+                             torch.tensor([int(l) for r in rows for l in r[2]], dtype=torch.int32),
+                             torch.tensor([r[3] for r in rows], dtype=torch.int32),
+                             torch.tensor([r[4] for r in rows], dtype=torch.int32),
+                             torch.tensor(np.array([r[5] for r in rows], dtype=np.float32).reshape(-1, 4))),
+            torch.tensor(set_ptr, dtype=torch.int64))

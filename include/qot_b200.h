@@ -589,6 +589,43 @@ int qot_lightpath_reconfigure(const qot_lp_graph_cfg_t* cfg, int64_t S, const do
                               int32_t is_lut_index, int32_t max_impact, float* out, int32_t* status, int32_t* n_impact,
                               int64_t* impact_node, int8_t* impact_kind, float* impact_out, void* stream);
 
+/* qot_lightpath_change_sets (lp_change_set_kernel, the same launch shape, one warp per set): G sets of changes, each
+ * evaluated jointly against the state.  The changes take the qot_lightpath_reconfigure arguments; set g is changes
+ * [set_ptr[g], set_ptr[g+1]) (set_ptr [G+1] int64), all naming one sample s, at most QOT_SET_MAX_CHANGES of them.
+ * sample' = data[s] with (1) every channel of every lightpath the set moves or tears down (node >= 0) zeroed, then
+ * (2) each non-teardown change written on its path x slot range: a move as qot_lightpath_reconfigure writes it (j's
+ * conn_id, feat, j's other rows from its first channel), an insertion with a new conn_id (one above the sample's
+ * largest, +1 per insertion in set order; metrics -1).  The placements of a set must be disjoint.  A channel is occupied
+ * only when its chan_node is a lightpath the set does not move (so swaps are legal; INT_MIN is occupied).  In sample''s
+ * graph, flag one-hot:
+ *   out [K,3]            the changed lightpath's row at its new placement; NaN for a teardown;
+ *   impact rows          per set, every lightpath i of the state that the set does not move and that is adjacent to a
+ *                        changed lightpath before or after the set, ascending in node order of the state batch:
+ *                        impact_node [G,M], impact_out [G,M,3], impact_kind [G,M] int8 (may be NULL) = bit 0: an
+ *                        in-neighbour of i is moved or torn down, bit 1: a changed lightpath is i's neighbour after the
+ *                        set; past the rows -1 / 0 / NaN.  n_impact [G] = the number of such rows (may exceed M).
+ * Every other row of sample' equals its row in the state.  Message order: the row of change c = its new neighbours in
+ * the state ascending, then the other changes adjacent to it in set order, then its self loop; impact row i = i's state
+ * in-row ascending without the removed lightpaths and without i's self loop, then the changes adjacent to i in set
+ * order, then i's self loop.  A set of one change is bit-identical to qot_lightpath_reconfigure.
+ * status [K] = the QOT_CAND_* bits of each change plus the QOT_SET_* bits below (IMPACT_OVERFLOW on every change of an
+ * overflowing set, BAD_STATE found in an impact row on the set's first change); set_status [G] = the OR over the set.
+ * Every bit but IMPACT_OVERFLOW is fatal for the whole set: all its out rows are NaN and n_impact is 0.  If set_ptr is
+ * not non-decreasing from 0 to K, no set is evaluated: every status and set_status is BAD_SET. */
+#define QOT_SET_MAX_CHANGES 64
+#define QOT_SET_BAD_SET 64           /* the set's changes name different samples (on the changes that differ from the
+                                        first), the set has more than 64 changes, or set_ptr is malformed            */
+#define QOT_SET_DUPLICATE 128        /* a lightpath is moved or torn down by two changes of the set (on both)       */
+#define QOT_SET_CONFLICT 256         /* this change's placement shares a channel with another change's placement    */
+int qot_lightpath_change_sets(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
+                              const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N,
+                              int64_t E, const int32_t* chan_node, int64_t K, const int64_t* node,
+                              const int64_t* sample, const int64_t* link_ptr, const int32_t* links, int64_t n_links,
+                              const int32_t* q0, const int32_t* width, const float* feat, int64_t G,
+                              const int64_t* set_ptr, const float* prepared, int32_t is_lut_index, int32_t max_impact,
+                              float* out, int32_t* status, int32_t* set_status, int32_t* n_impact,
+                              int64_t* impact_node, int8_t* impact_kind, float* impact_out, void* stream);
+
 /* The topological representation: to_graph.py::create_topological_graph (:62-184: one edge per
  * lightpath between its source and destination network node, lightpaths added in ascending conn_id,
  * nx.Graph keeps one edge per node pair -- position from the first, attributes from the last) fused
