@@ -1,10 +1,7 @@
 """Reference for LightpathGNN's candidate QoT (TEST INFRASTRUCTURE, like every_node_ref.py): a candidate lightpath
 written literally into a numpy copy of its sample, the graph rebuilt with the numpy restatement of to_graph
 (oracle.lightpath_data_ref), one one-hot copy of that graph per evaluated node, all run through the oracle model."""
-from types import SimpleNamespace
-
 import numpy as np
-import torch
 
 from oracle.to_graph_oracle import lightpath_data_ref
 
@@ -28,25 +25,15 @@ def insert_candidate(sample, lp_feat, links, q0, width, feat):
     return out, conn
 
 
-def candidates_ref(model, sample, freqs, lp_feat, links, q0, width, feat, freq_threshold=0.05):
+def candidates_ref(model, sample, freqs, lp_feat, links, q0, width, feat, freq_threshold=0.05, chunk=None, device=None):
     """Candidate QoT of one candidate, defined literally.  Returns ``(row [3], {conn_id: row [3]})``: the candidate's
     row (flag one-hot at its node) and, for every existing lightpath adjacent to it in the rebuilt graph, that
-    lightpath's row (flag one-hot there).  Runs on ``model``'s dtype, on the CPU."""
+    lightpath's row (flag one-hot there).  Runs on ``model``'s dtype, on ``device`` (default: the CPU), ``chunk`` copies
+    per oracle call (see ``reconfig_ref._rows``); rows come back on the CPU."""
+    from reconfig_ref import _rows
     s2, conn = insert_candidate(sample, lp_feat, links, q0, width, feat)
     conns, x, _, ei = lightpath_data_ref(s2, np.zeros(3), freqs, lp_feat, METRIC, freq_threshold)
     c = int(np.flatnonzero(conns == conn)[0])
     nbr = sorted({int(d) for s, d in ei.T if s == c and d != c})
-    rows = [c] + nbr
-    dt = next(model.parameters()).dtype
-    n, R = x.shape[0], len(rows)
-    xc = torch.from_numpy(np.tile(x, (R, 1))).to(dt)
-    flag = torch.zeros(R * n, dtype=dt)
-    flag[torch.arange(R) * n + torch.tensor(rows)] = 1.0
-    xc[:, model.is_lut_index] = flag
-    e = torch.from_numpy(ei)
-    eic = torch.cat([e + r * n for r in range(R)], 1)
-    bt = torch.repeat_interleave(torch.arange(R), n)
-    with torch.no_grad():
-        out, lut_batch = model(SimpleNamespace(x=xc, edge_index=eic, batch=bt, num_graphs=R))
-    assert torch.equal(lut_batch, torch.arange(R)), "every copy has exactly one readout row"
+    out = _rows(model, x, ei, [c] + nbr, chunk, device)
     return out[0], {int(conns[j]): out[i + 1] for i, j in enumerate(nbr)}

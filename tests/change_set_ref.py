@@ -41,13 +41,13 @@ def apply_set(sample, lp_feat, changes):
     return out, conns
 
 
-def change_set_ref(model, sample, freqs, lp_feat, changes, freq_threshold=0.05):
+def change_set_ref(model, sample, freqs, lp_feat, changes, freq_threshold=0.05, chunk=None, device=None):
     """Change-set QoT of one set, defined literally.  ``changes``: [(conn_id or None, links, q0, width, feat)], a move
     (conn_id and a path), a teardown (conn_id and an empty path) or an insertion (None).  Returns ``(rows, {conn_id:
     (kind, row [3])})``: per change its row at its new placement (flag one-hot there; None for a teardown) and, for
     every lightpath of the sample the set does not name that was adjacent to a removed one in the original graph (kind
     bit 0) or is adjacent to a changed one in the rebuilt graph (kind bit 1), its row.  Runs on ``model``'s dtype, on
-    the CPU."""
+    ``device`` (default: the CPU), ``chunk`` copies per oracle call (see ``reconfig_ref._rows``); rows come back on the CPU."""
     s2, conns = apply_set(sample, lp_feat, changes)
     removed = {int(c) for c, *_ in changes if c is not None}
     changed = {c for c, ch in zip(conns, changes) if c is not None and len(ch[1])}
@@ -58,7 +58,7 @@ def change_set_ref(model, sample, freqs, lp_feat, changes, freq_threshold=0.05):
     node_of = {int(v): i for i, v in enumerate(conns1)}
     others = sorted(old | new)
     own = [node_of[c] for c, ch in zip(conns, changes) if len(ch[1])]
-    out = _rows(model, x, ei, own + [node_of[o] for o in others])
+    out = _rows(model, x, ei, own + [node_of[o] for o in others], chunk, device)
     rows, r = [], 0
     for ch in changes:
         rows.append(out[r] if len(ch[1]) else None)

@@ -29,23 +29,32 @@ def rewrite_lightpath(sample, lp_feat, conn_id, links, q0, width, feat):
     return out
 
 
-def _rows(model, x, ei, rows):
-    """Eval forward of one one-hot copy of the graph per entry of ``rows`` -> [len(rows), 3]."""
+def _rows(model, x, ei, rows, chunk=None, device=None):
+    """Eval forward of one one-hot copy of the graph per entry of ``rows`` -> [len(rows), 3] on the CPU.  ``chunk``:
+    copies per oracle call (None: all at once; a dense graph's copies can outgrow memory), results concatenated.
+    ``device``: where the copies are evaluated (``model`` must be there; None: the CPU)."""
     dt = next(model.parameters()).dtype
     n, R = x.shape[0], len(rows)
     if R == 0:
         return torch.zeros(0, 3, dtype=dt)
-    xc = torch.from_numpy(np.tile(x, (R, 1))).to(dt)
-    flag = torch.zeros(R * n, dtype=dt)
-    flag[torch.arange(R) * n + torch.tensor(rows)] = 1.0
-    xc[:, model.is_lut_index] = flag
-    e = torch.from_numpy(ei)
-    eic = torch.cat([e + r * n for r in range(R)], 1)
-    bt = torch.repeat_interleave(torch.arange(R), n)
-    with torch.no_grad():
-        out, lut_batch = model(SimpleNamespace(x=xc, edge_index=eic, batch=bt, num_graphs=R))
-    assert torch.equal(lut_batch, torch.arange(R)), "every copy has exactly one readout row"
-    return out
+    step = R if chunk is None else int(chunk)
+    assert step > 0
+    outs = []
+    for c0 in range(0, R, step):
+        part = rows[c0:c0 + step]
+        P = len(part)
+        xc = torch.from_numpy(np.tile(x, (P, 1))).to(device=device, dtype=dt)
+        flag = torch.zeros(P * n, dtype=dt, device=device)
+        flag[torch.arange(P, device=device) * n + torch.tensor(part, device=device)] = 1.0
+        xc[:, model.is_lut_index] = flag
+        e = torch.from_numpy(ei).to(device)
+        eic = torch.cat([e + r * n for r in range(P)], 1)
+        bt = torch.repeat_interleave(torch.arange(P, device=device), n)
+        with torch.no_grad():
+            out, lut_batch = model(SimpleNamespace(x=xc, edge_index=eic, batch=bt, num_graphs=P))
+        assert torch.equal(lut_batch.cpu(), torch.arange(P)), "every copy has exactly one readout row"
+        outs.append(out.cpu())
+    return torch.cat(outs)
 
 
 def _neighbours(conns, ei, c):
@@ -57,13 +66,14 @@ def _neighbours(conns, ei, c):
     return {int(conns[d]) for s, d in ei.T if s == v and d != v}
 
 
-def reconfig_ref(model, sample, freqs, lp_feat, conn_id, links, q0, width, feat, freq_threshold=0.05):
+def reconfig_ref(model, sample, freqs, lp_feat, conn_id, links, q0, width, feat, freq_threshold=0.05, chunk=None,
+                 device=None):
     """Reconfiguration QoT of one change, defined literally.  ``conn_id`` is the moved lightpath (None: an insertion,
     written as candidates_ref.insert_candidate writes it); an empty ``links`` is a teardown.  Returns ``(row [3] or
     None, {conn_id: (kind, row [3])})``: the moved lightpath's row at its new placement (flag one-hot there; None for a
     teardown) and, for every other lightpath that was adjacent to it in the original graph (kind bit 0) or is adjacent
     to it in the rebuilt graph (kind bit 1), that lightpath's row (flag one-hot there).  Runs on ``model``'s dtype, on
-    the CPU."""
+    ``device`` (default: the CPU), ``chunk`` copies per oracle call (see ``_rows``); rows come back on the CPU."""
     if conn_id is None:
         s2, c = insert_candidate(sample, lp_feat, links, q0, width, feat)
         old = set()
@@ -77,7 +87,7 @@ def reconfig_ref(model, sample, freqs, lp_feat, conn_id, links, q0, width, feat,
     node_of = {int(v): i for i, v in enumerate(conns)}
     others = sorted(old | new)
     own = [node_of[c]] if len(links) else []
-    out = _rows(model, x, ei, own + [node_of[o] for o in others])
+    out = _rows(model, x, ei, own + [node_of[o] for o in others], chunk, device)
     row = out[0] if own else None
     rest = out[len(own):]
     return row, {o: (int(o in old) | int(o in new) << 1, rest[i]) for i, o in enumerate(others)}
