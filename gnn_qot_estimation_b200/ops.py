@@ -588,13 +588,31 @@ class _GatConvFn(torch.autograd.Function):
 
 
 def gat_conv(x, graph: GraphIndex, lin_w, att_src, att_dst, bias) -> torch.Tensor:
+    """GATConv with gradients for its parameters only: x is data (the lightpath features of
+    lightpath_training/models.py:30), so an x that requires grad raises instead of getting a silent zero."""
     _require_cuda(x, lin_w)
+    if torch.is_grad_enabled() and x.requires_grad:
+        raise NotImplementedError("libqot_b200 GATConv: no gradient with respect to x (the input features are data); "
+                                  "pass x.detach()")
     return _GatConvFn.apply(x, lin_w, att_src, att_dst, bias, graph)
 
 
 # --------------------------------------------------------------------------- #
 # BatchNorm statistics, LUT readout + MLP head
 # --------------------------------------------------------------------------- #
+def _bn_train_stats(h, bn: torch.nn.BatchNorm1d):
+    """Batch statistics of ``bn`` in train(), with torch's running-stat update: ``num_batches_tracked`` counts the
+    batch first, and ``momentum=None`` takes the cumulative average ``1 / num_batches_tracked`` -- a read of the
+    counter, like torch's own BatchNorm, so only a fixed momentum is capturable in a CUDA graph.  One row raises
+    torch's ValueError (its variance is 0); N is on the host, so that check costs nothing."""
+    if h.shape[0] == 1:
+        raise ValueError(f"Expected more than 1 value per channel when training, got input size {h.shape}")
+    with torch.no_grad():
+        bn.num_batches_tracked += 1
+    momentum = bn.momentum if bn.momentum is not None else 1.0 / float(bn.num_batches_tracked)
+    return bn_batch_stats(h.detach(), bn.running_mean, bn.running_var, momentum)
+
+
 def bn_batch_stats(h, running_mean=None, running_var=None, momentum: float = 0.1):
     L = _lib.lib()
     h = _f32(h)
@@ -672,16 +690,14 @@ def lut_bn_head(h, x_feat, batch, is_lut_index, bn: torch.nn.BatchNorm1d, W1, b1
     """norm1 -> relu -> LUT readout -> mlp of lightpath_training/models.py:31-43.
     Raises ``ValueError("No LUT node found in the batch.")`` like the reference."""
     _require_cuda(h, x_feat, batch)
+    # norm1 before the readout, as in the reference: a 1-node batch raises BatchNorm's error, not the LUT one
+    if training:
+        mean, var = _bn_train_stats(h, bn)
+    else:
+        mean, var = bn.running_mean, bn.running_var
     lut_node, lut_batch, n = lut_select(x_feat, batch, is_lut_index, n_known)
     if n == 0:
         raise ValueError("No LUT node found in the batch.")
-    if training:
-        mean, var = bn_batch_stats(h.detach(), bn.running_mean, bn.running_var,
-                                   bn.momentum if bn.momentum is not None else 0.1)
-        with torch.no_grad():
-            bn.num_batches_tracked += 1
-    else:
-        mean, var = bn.running_mean, bn.running_var
     hmask = None
     if training and dropout_p > 0.0:
         keep = 1.0 - dropout_p
@@ -727,10 +743,7 @@ def batch_norm(x, bn: torch.nn.BatchNorm1d, training: bool):
     if x.shape[0] == 0:
         return x
     if training:
-        mean, var = bn_batch_stats(x.detach(), bn.running_mean, bn.running_var,
-                                   bn.momentum if bn.momentum is not None else 0.1)
-        with torch.no_grad():
-            bn.num_batches_tracked += 1
+        mean, var = _bn_train_stats(x, bn)
     else:
         mean, var = bn.running_mean, bn.running_var
     return _BatchNormFn.apply(x, mean, var, bn.eps, bn.weight, bn.bias, training)
