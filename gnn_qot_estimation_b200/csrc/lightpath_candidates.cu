@@ -749,6 +749,458 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
   if (zc) cd_flush(w, zc, prep, lane);
 }
 
+// ------------------------------------------------------------------------------------------------ placements
+// lp_placement_kernel: persistent, one warp per demand (qot_lightpath_placements).  A demand offers up to 32 options
+// (a route, a width, the channel features); a placement is an option with a start slot q0 whose channels are free on
+// every link of the route, and its rows are by definition the candidate kernel's rows for that candidate (freq =
+// float32(freqs[q0])).  Per option the warp reads each chan_node row of the route once, coalesced: the ballots give the
+// occupied bitmap (lane t owns slots [32t, 32t + 32), Q <= 1024) and the occupied channels of known lightpaths are
+// collected as (slot, node) entries.  The free starts for the option's width come from log2(width) AND-shift steps
+// of the free bitmap, words carried across lanes by shuffles.  Each free start's neighbour mask is the candidate
+// kernel's fp64 0 < |df| < threshold test over the collected entries (over the chan_node rows again when the route
+// holds more than kPlEntCap of them), ranked as the candidate kernel ranks it.  Own rows (and, with a bound, every
+// impact row) go 16 at a time through the head; the staged outputs fold into the placement's margin (an ordered
+// integer key, so min and max are exact and order-free) and, once its last row is out, into the demand's running best
+// (policy key << 32 | ~(option << 10 | q0): the lower index wins a tie).  The winner is evaluated again at the end of
+// the demand for its first max_impact impact rows.
+constexpr int kPlMaxOptions = QOT_PLACE_MAX_OPTIONS;
+constexpr int kPlMaxQ = QOT_PLACE_MAX_SLOTS;
+constexpr int kPlEntCap = 768;                     // (slot, node) entries of one route; more: scan chan_node again
+constexpr int kPlRing = 32;                        // placements with rows in the head buffer: at most 17
+constexpr int kPlFatal = QOT_CAND_BAD_SAMPLE | QOT_CAND_BAD_PATH | QOT_CAND_BAD_STATE;
+static_assert(kPlMaxQ == 32 * 32, "one 32-bit free word per lane");
+static_assert(kPlMaxOptions <= 32 && kPlMaxQ <= 1024, "option << 10 | q0 fits the low key word");
+
+struct PlPending {                           // a placement whose rows are in flight
+  float own[3];
+  unsigned mkey;                             // min of the row margins' ordered keys (0: a NaN margin)
+  int left, p, q0;                           // rows not yet folded, option (global), start slot
+};
+struct PlWarpSmem {
+  int ent[kPlEntCap];                        // the route's occupied channels of known lightpaths: slot << 8 | node
+  PlPending ring[kPlRing];
+  float rout[16][4];                         // outputs of the staged rows of the search
+  long long rnode[16];                       // bound index of a staged impact row, -1: an own row
+  int rtag[16];                              // ring slot of a staged row, -1: a winner's row (written out directly)
+  unsigned long long key;                    // the demand's running best (0: none feasible yet)
+  float best[4];                             // its own row and margin
+  int n_free, n_feas;
+};
+struct PlSmem {
+  CdSmem cd;                                 // head fragments and the candidate kernel's per-warp state
+  PlWarpSmem w[kCdWarps];
+};
+static_assert(sizeof(PlSmem) + 16 <= 227 * 1024, "lp_placement_kernel: shared memory over the 227 KB block limit");
+
+struct PlArgs {
+  CdArgs c;                                // state, links, width, prep, max_impact, status / n_impact / impact_*
+  int64_t P;                               // options
+  const int64_t* opt_ptr;                  // [D+1]
+  const float* own_bound;                  // [P]
+  const float* bound;                      // [N] or null
+  int metric, maximize, policy;
+  int32_t* option;                         // [D]
+  int32_t* q0;                             // [D]
+  float* margin;                           // [D]
+  int32_t* n_free;
+  int32_t* n_feasible;
+  float* all_out;                          // [P,Q,3] or null
+  float* all_margin;                       // [P,Q] or null
+};
+
+// float -> unsigned, monotone (-0 counts as +0); NaN -> 0, below every number
+__device__ __forceinline__ unsigned pl_okey(float f) {
+  if (f != f) return 0u;
+  const unsigned u = __float_as_uint(__fadd_rn(f, 0.0f));
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float pl_unkey(unsigned k) {
+  if (k == 0u) return __int_as_float(0x7fc00000);
+  return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
+// bit i of lane t's word of the result = slot 32t + i + k of x (slots past the last word read as 0, occupied)
+__device__ __forceinline__ unsigned pl_shr(unsigned x, int k, int lane) {
+  const int d = k >> 5, b = k & 31;
+  unsigned lo = __shfl_down_sync(kFull, x, d), hi = __shfl_down_sync(kFull, x, d + 1);
+  if (lane + d > 31) lo = 0u;
+  if (lane + d + 1 > 31) hi = 0u;
+  return b ? (lo >> b) | (hi << (32 - b)) : lo;
+}
+
+// the staged rows' outputs, in staging order, into their placements' margins; a placement whose last row is out goes
+// into the demand's count and running best, and into all_out / all_margin.  Lane 0.
+__device__ __noinline__ void pl_fold(const PlArgs& a, PlWarpSmem& pw, int cnt, int64_t o0) {
+  const int Q = a.c.cfg.Q;
+  for (int r = 0; r < cnt; ++r) {
+    const int t = pw.rtag[r];
+    if (t < 0) continue;
+    PlPending& pp = pw.ring[t];
+    const float v = pw.rout[r][a.metric];
+    const long long nd = pw.rnode[r];
+    const float b = nd < 0 ? a.own_bound[pp.p] : a.bound[nd];
+    const unsigned k = pl_okey(a.maximize ? __fsub_rn(v, b) : __fsub_rn(b, v));
+    pp.mkey = min(pp.mkey, k);
+    if (nd < 0)
+      for (int o = 0; o < QOT_OUT; ++o) pp.own[o] = pw.rout[r][o];
+    if (--pp.left) continue;
+    const float mg = pl_unkey(pp.mkey);
+    const int64_t at = static_cast<int64_t>(pp.p) * Q + pp.q0;
+    if (a.all_out) {
+      for (int o = 0; o < QOT_OUT; ++o) a.all_out[at * QOT_OUT + o] = pp.own[o];
+      a.all_margin[at] = mg;
+    }
+    if (pp.mkey < 0x80000000u) continue;               // margin < 0 or NaN: not feasible
+    ++pw.n_feas;
+    const float ov = pp.own[a.metric];
+    const unsigned hi = a.policy == QOT_PLACE_FIRST_FIT ? 0u
+                        : a.policy == QOT_PLACE_BEST_QOT ? pl_okey(a.maximize ? ov : -ov)
+                                                         : pp.mkey;
+    const unsigned idx = static_cast<unsigned>(pp.p - o0) << 10 | static_cast<unsigned>(pp.q0);
+    const unsigned long long key = static_cast<unsigned long long>(hi) << 32 | (0xffffffffu - idx);
+    if (key > pw.key) {
+      pw.key = key;
+      for (int o = 0; o < QOT_OUT; ++o) pw.best[o] = pp.own[o];
+      pw.best[3] = mg;
+    }
+  }
+}
+
+__device__ __noinline__ void pl_flush(const PlArgs& a, PlWarpSmem& pw, int w, int cnt, int64_t o0, int lane) {
+  cd_flush(w, cnt, a.c.prep, lane);
+  if (lane == 0) pl_fold(a, pw, cnt, o0);
+  __syncwarp();
+}
+
+// cd_row with the row's destination, ring slot and bound index recorded for pl_fold
+template <typename XF>
+__device__ __forceinline__ int pl_row(const PlArgs& a, CdWarpSmem& ws, PlWarpSmem& pw, int w, int zc, const int* msg,
+                                      int M, int q, const XF& xf, const float (&As)[kF], const float (&Ad)[kF],
+                                      float* dst, int tag, long long node, int64_t o0, int lane) {
+  float d_q = 0.f;
+#pragma unroll
+  for (int k = 0; k < kF; ++k) d_q = fmaf(xf(q, k), Ad[k], d_q);
+  AttnState st;
+  attn_consume(st, msg, M, xf, As, d_q, lane);
+  attn_finish<kF>(st, ws.z + zc * kCdZPitch, lane);
+  if (lane == 0) {
+    ws.orow[zc] = reinterpret_cast<long long>(dst ? dst : pw.rout[zc]);
+    pw.rtag[zc] = tag;
+    pw.rnode[zc] = node;
+  }
+  __syncwarp();
+  if (++zc == 16) {
+    pl_flush(a, pw, w, 16, o0, lane);
+    zc = 0;
+  }
+  return zc;
+}
+
+// neighbours of placement [q0, q0 + cw) on a route, from the route's chan_node rows (the candidate kernel's scan; the
+// placement's own channels are free) into ws.mask
+__device__ __forceinline__ void pl_scan_mask(const CdArgs& a, CdWarpSmem& ws, int64_t s, int64_t n0, int64_t p0,
+                                             int64_t p1, int q0, int cw, int lane) {
+  const int Q = a.cfg.Q;
+  for (int64_t e = p0; e < p1; ++e) {
+    const int32_t* __restrict__ row = a.chan_node + (s * a.cfg.L + a.links[e]) * Q;
+    for (int q = lane; q < Q; q += 32) {
+      const int32_t v = row[q];
+      if (v < 0) continue;                                  // free, or occupied by an unknown lightpath
+      const int j = static_cast<int>(v - n0);               // inside the sample: checked when the route was read
+      const double fq = a.freqs[q];
+      bool hit = false;
+      for (int c = q0; c < q0 + cw && !hit; ++c) {
+        const double df = fabs(a.freqs[c] - fq);
+        hit = df < a.cfg.freq_threshold && df > 0.0;
+      }
+      if (hit) atomicOr(&ws.mask[j >> 5], 1u << (j & 31));
+    }
+  }
+}
+
+__global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __grid_constant__ PlArgs pa) {
+  const CdArgs& a = pa.c;
+  PlSmem& sm = *reinterpret_cast<PlSmem*>(cd_smem_raw);
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  CdWarpSmem& ws = sm.cd.w[w];
+  PlWarpSmem& pw = sm.w[w];
+  for (int i = tid; i < kStHeadFrag4; i += kCdThreads)
+    sm.cd.frag[i] = __ldg(reinterpret_cast<const float4*>(a.prep + kOffB1f) + i);
+  __syncthreads();
+  const float* __restrict__ prep = a.prep;
+  const int h = lane & 3;
+  float As[kF], Ad[kF];
+#pragma unroll
+  for (int k = 0; k < kF; ++k) {
+    As[k] = __ldg(prep + kOffAsrc + k * kHeads + h);
+    Ad[k] = __ldg(prep + kOffAdst + k * kHeads + h);
+  }
+  const float nan = __int_as_float(0x7fc00000);
+  int zc = 0;                                             // rows staged in this warp's head buffer
+  for (int64_t d = static_cast<int64_t>(blockIdx.x) * kCdWarps + w; d < a.K;
+       d += static_cast<int64_t>(gridDim.x) * kCdWarps) {
+    const int L = a.cfg.L, Q = a.cfg.Q;
+    // ---- validation: the sample, the option range, every option's route and width, the state offsets
+    int st = 0;
+    const int64_t s = a.sample[d];
+    if (s < 0 || s >= a.S) st |= QOT_CAND_BAD_SAMPLE;
+    const int64_t o0 = pa.opt_ptr[d], o1 = pa.opt_ptr[d + 1];
+    const bool opts_ok = o0 >= 0 && o1 > o0 && o1 <= pa.P && o1 - o0 <= kPlMaxOptions;
+    bool badp = !opts_ok;
+    if (opts_ok)
+      for (int64_t po = o0; po < o1 && !badp; ++po) {
+        const int64_t p0 = a.link_ptr[po], p1 = a.link_ptr[po + 1];
+        const int cw = a.width[po];
+        bool b = !(p0 >= 0 && p1 > p0 && p1 <= a.n_links) || cw < 1 || cw > Q;
+        if (!b)
+          for (int64_t e = p0 + lane; e < p1; e += 32) {
+            const int l = a.links[e];
+            b |= l < 0 || l >= L;
+          }
+        badp = __any_sync(kFull, b);
+      }
+    if (badp) st |= QOT_CAND_BAD_PATH;
+    int64_t n0 = 0;
+    int n = 0;
+    if (st == 0) {
+      n0 = a.node_ptr[s];
+      const int64_t n1 = a.node_ptr[s + 1];
+      if (n0 >= 0 && n1 >= n0 && n1 <= a.N && n1 - n0 <= kCdMaxN) n = static_cast<int>(n1 - n0);
+      else st |= QOT_CAND_BAD_STATE;
+    }
+    if (lane == 0) {
+      pw.key = 0ull;
+      pw.n_free = pw.n_feas = 0;
+    }
+    __syncwarp();
+    const float* xs = a.x + n0 * kF;
+    int seq = 0;                                          // placements of this demand, for the ring slots
+    for (int64_t po = o0; st == 0 && po < o1; ++po) {
+      const int64_t p0 = a.link_ptr[po], p1 = a.link_ptr[po + 1];
+      const int cw = a.width[po];
+      // ---- the route's occupied bitmap (lane t: word t) and its channels of known lightpaths, one read per row
+      unsigned occ = 0u;
+      int ne = 0;
+      bool bad = false;
+      for (int64_t e = p0; e < p1; ++e) {
+        const int32_t* __restrict__ row = a.chan_node + (s * L + a.links[e]) * Q;
+        for (int qb = 0; qb < Q; qb += 32) {
+          const int q = qb + lane;
+          const int32_t v = q < Q ? row[q] : -1;
+          const unsigned ob = __ballot_sync(kFull, v != -1);
+          if (lane == qb >> 5) occ |= ob;
+          const int64_t j = static_cast<int64_t>(v) - n0;
+          const bool known = v >= 0 && j >= 0 && j < n;
+          bad |= v >= 0 && !known;
+          const bool keep = known;                        // every link's channels of known lightpaths
+          const unsigned kb = __ballot_sync(kFull, keep);
+          const int at = ne + __popc(kb & ((1u << lane) - 1u));
+          if (keep && at < kPlEntCap) pw.ent[at] = q << 8 | static_cast<int>(j);
+          ne += __popc(kb);
+        }
+      }
+      if (__any_sync(kFull, bad)) {
+        st |= QOT_CAND_BAD_STATE;
+        break;
+      }
+      __syncwarp();
+      // ---- free starts for width cw: AND of the free bits over [q0, q0 + cw), in log2(cw) shift steps
+      const int tail = Q - 32 * lane;
+      const unsigned valid = tail >= 32 ? 0xffffffffu : tail > 0 ? (1u << tail) - 1u : 0u;
+      unsigned run = ~occ & valid;
+      for (int have = 1; have < cw;) {
+        const int step = min(have, cw - have);
+        run &= pl_shr(run, step, lane);
+        have += step;
+      }
+      if (pa.all_out)                                     // NaN at every start that is not free
+        for (int wd = 0; wd < 32 && 32 * wd < Q; ++wd) {
+          const unsigned bits = __shfl_sync(kFull, run, wd);
+          const int q = 32 * wd + lane;
+          if (q >= Q || (bits >> lane & 1u)) continue;
+          const int64_t at = po * Q + q;
+          pa.all_margin[at] = nan;
+          for (int o = 0; o < QOT_OUT; ++o) pa.all_out[at * QOT_OUT + o] = nan;
+        }
+      // ---- every free start in ascending order
+      for (int wd = 0; wd < 32 && 32 * wd < Q; ++wd) {
+        for (unsigned bits = __shfl_sync(kFull, run, wd); bits; bits &= bits - 1u) {
+          const int q0 = 32 * wd + __ffs(bits) - 1;
+          if (lane < kCdMaskWords) ws.mask[lane] = 0u;
+          __syncwarp();
+          if (ne <= kPlEntCap) {
+            for (int i = lane; i < ne; i += 32) {
+              const int en = pw.ent[i], q = en >> 8, j = en & 255;
+              const double fq = a.freqs[q];
+              bool hit = false;
+              for (int c = q0; c < q0 + cw && !hit; ++c) {
+                const double df = fabs(a.freqs[c] - fq);
+                hit = df < a.cfg.freq_threshold && df > 0.0;
+              }
+              if (hit) atomicOr(&ws.mask[j >> 5], 1u << (j & 31));
+            }
+          } else {
+            pl_scan_mask(a, ws, s, n0, p0, p1, q0, cw, lane);
+          }
+          __syncwarp();
+          const int nn = cd_rank(lane < kCdMaskWords ? ws.mask[lane] : 0u, ws.nbr, lane);
+          // x row of the placement: (float32(freqs[q0]), the option's features), scaled as the candidate kernel does
+          if (lane < 4) {
+            const double v = lane == 0 ? static_cast<double>(static_cast<float>(a.freqs[q0]))
+                                       : static_cast<double>(a.feat[po * 3 + lane - 1]);
+            ws.cx[lane == 0 ? 0 : lane + 1] =
+                static_cast<float>((v - a.cfg.feat_lo[lane]) / (a.cfg.feat_hi[lane] - a.cfg.feat_lo[lane]));
+          }
+          if (lane == 4) ws.cx[1] = 1.0f;
+          const int slot = seq++ & (kPlRing - 1);
+          const int nimp = pa.bound ? nn : 0;             // impact rows count against a bound, all of them
+          if (lane == 0) {
+            ws.nbr[nn] = kCand;
+            PlPending& pp = pw.ring[slot];
+            pp.mkey = 0xffffffffu;
+            pp.left = 1 + nimp;
+            pp.p = static_cast<int>(po);
+            pp.q0 = q0;
+            ++pw.n_free;
+          }
+          __syncwarp();
+          zc = pl_row(pa, ws, pw, w, zc, ws.nbr, nn + 1, kCand, CdX{xs, ws.cx, kCand, a.lut_col}, As, Ad, nullptr,
+                      slot, -1, o0, lane);
+          for (int i = 0; i < nimp; ++i) {                // whatever max_impact is
+            const int j = ws.nbr[i];
+            const int64_t r0 = a.rowptr[n0 + j], r1 = a.rowptr[n0 + j + 1];
+            bool rb = !(r0 >= 0 && r1 >= r0 && r1 <= a.E && r1 - r0 <= kCdMaxN);
+            int m = 0;
+            if (!rb)
+              for (int64_t eb = r0; eb < r1; eb += 32) {
+                const int64_t e = eb + lane;
+                const int64_t dg = e < r1 ? a.edst[e] - n0 : -1;
+                const bool inside = dg >= 0 && dg < n;
+                rb |= e < r1 && !inside;
+                const bool keep = inside && dg != j;
+                const unsigned ball = __ballot_sync(kFull, keep);
+                if (keep) ws.msg[m + __popc(ball & ((1u << lane) - 1u))] = static_cast<int>(dg);
+                m += __popc(ball);
+              }
+            if (__any_sync(kFull, rb)) {
+              st |= QOT_CAND_BAD_STATE;
+              break;
+            }
+            if (lane == 0) {
+              ws.msg[m] = kCand;
+              ws.msg[m + 1] = j;
+            }
+            __syncwarp();
+            zc = pl_row(pa, ws, pw, w, zc, ws.msg, m + 2, j, CdX{xs, ws.cx, j, a.lut_col}, As, Ad, nullptr, slot,
+                        n0 + j, o0, lane);
+          }
+          if (st) break;
+        }
+        if (st) break;
+      }
+    }
+    // ---- every placement of the demand folded: the winner
+    if (zc) {
+      pl_flush(pa, pw, w, zc, o0, lane);
+      zc = 0;
+    }
+    const int MI = a.max_impact;
+    const unsigned long long key = pw.key;
+    int cnt = 0, rows = 0, bp = -1, bq = -1;
+    int64_t wp0 = 0, wp1 = 0;
+    if (st == 0 && key) {
+      const unsigned idx = 0xffffffffu - static_cast<unsigned>(key);
+      bp = static_cast<int>(idx >> 10);
+      bq = static_cast<int>(idx & 1023u);
+      const int64_t po = o0 + bp;
+      wp0 = a.link_ptr[po];
+      wp1 = a.link_ptr[po + 1];
+      const int cw = a.width[po];
+      if (lane < kCdMaskWords) ws.mask[lane] = 0u;
+      __syncwarp();
+      pl_scan_mask(a, ws, s, n0, wp0, wp1, bq, cw, lane);
+      __syncwarp();
+      cnt = cd_rank(lane < kCdMaskWords ? ws.mask[lane] : 0u, ws.nbr, lane);
+      __syncwarp();
+      rows = min(cnt, MI);
+      bool bad = false;                                   // in-rows checked before any row is written
+      for (int i = 0; i < rows && !bad; ++i) {
+        const int64_t r0 = a.rowptr[n0 + ws.nbr[i]], r1 = a.rowptr[n0 + ws.nbr[i] + 1];
+        if (!(r0 >= 0 && r1 >= r0 && r1 <= a.E && r1 - r0 <= kCdMaxN)) { bad = true; break; }
+        for (int64_t e = r0 + lane; e < r1; e += 32) {
+          const int64_t dg = a.edst[e] - n0;
+          bad |= dg < 0 || dg >= n;
+        }
+        bad = __any_sync(kFull, bad);
+      }
+      if (__any_sync(kFull, bad)) st |= QOT_CAND_BAD_STATE;
+      if (lane < 4) {
+        const double v = lane == 0 ? static_cast<double>(static_cast<float>(a.freqs[bq]))
+                                   : static_cast<double>(a.feat[po * 3 + lane - 1]);
+        ws.cx[lane == 0 ? 0 : lane + 1] =
+            static_cast<float>((v - a.cfg.feat_lo[lane]) / (a.cfg.feat_hi[lane] - a.cfg.feat_lo[lane]));
+      }
+      if (lane == 4) ws.cx[1] = 1.0f;
+      __syncwarp();
+    }
+    if (st & kPlFatal) {
+      if (lane < QOT_OUT) a.out[d * QOT_OUT + lane] = nan;
+      if (lane == 0) {
+        a.status[d] = st;
+        a.n_impact[d] = 0;
+        pa.option[d] = pa.q0[d] = -1;
+        pa.margin[d] = nan;
+        pa.n_free[d] = pa.n_feasible[d] = 0;
+      }
+      for (int i = lane; i < MI; i += 32) a.impact_node[d * MI + i] = -1;
+      for (int i = lane; i < MI * QOT_OUT; i += 32) a.impact_out[d * MI * QOT_OUT + i] = nan;
+      if (pa.all_out && opts_ok)
+        for (int64_t i = o0 * Q + lane; i < o1 * Q; i += 32) {
+          pa.all_margin[i] = nan;
+          for (int o = 0; o < QOT_OUT; ++o) pa.all_out[i * QOT_OUT + o] = nan;
+        }
+      __syncwarp();
+      continue;
+    }
+    // ---- the winner's impact rows: its neighbour j's in-row (flag 0), the placement (flag 0), j's self loop (flag 1)
+    for (int i = 0; i < rows; ++i) {
+      const int j = ws.nbr[i];
+      const int64_t r0 = a.rowptr[n0 + j], r1 = a.rowptr[n0 + j + 1];
+      if (lane == 0) a.impact_node[d * MI + i] = n0 + j;
+      int m = 0;
+      for (int64_t eb = r0; eb < r1; eb += 32) {
+        const int64_t e = eb + lane;
+        const int64_t dg = e < r1 ? a.edst[e] - n0 : -1;
+        const bool keep = dg >= 0 && dg != j;
+        const unsigned ball = __ballot_sync(kFull, keep);
+        if (keep) ws.msg[m + __popc(ball & ((1u << lane) - 1u))] = static_cast<int>(dg);
+        m += __popc(ball);
+      }
+      if (lane == 0) {
+        ws.msg[m] = kCand;
+        ws.msg[m + 1] = j;
+      }
+      __syncwarp();
+      zc = pl_row(pa, ws, pw, w, zc, ws.msg, m + 2, j, CdX{xs, ws.cx, j, a.lut_col}, As, Ad,
+                  a.impact_out + (d * MI + i) * QOT_OUT, -1, -1, o0, lane);
+    }
+    for (int i = rows + lane; i < MI; i += 32) a.impact_node[d * MI + i] = -1;
+    for (int i = rows * QOT_OUT + lane; i < MI * QOT_OUT; i += 32) a.impact_out[d * MI * QOT_OUT + i] = nan;
+    if (lane < QOT_OUT) a.out[d * QOT_OUT + lane] = key ? pw.best[lane] : nan;
+    if (lane == 0) {
+      a.status[d] = st | (cnt > MI ? QOT_CAND_IMPACT_OVERFLOW : 0);
+      a.n_impact[d] = cnt;
+      pa.option[d] = bp;
+      pa.q0[d] = bq;
+      pa.margin[d] = key ? pw.best[3] : nan;
+      pa.n_free[d] = pw.n_free;
+      pa.n_feasible[d] = pw.n_feas;
+    }
+    __syncwarp();
+  }
+  if (zc) pl_flush(pa, pw, w, zc, 0, lane);
+}
+
 static int cfg_check(const qot_lp_graph_cfg_t* cfg, const char* who) {
   QOT_REQUIRE(cfg, "%s: null cfg", who);
   QOT_REQUIRE(cfg->F > 0 && cfg->L > 0 && cfg->Q > 0 && cfg->L <= 65535 && cfg->Q <= 65535 &&
@@ -850,6 +1302,63 @@ static int cs_launch(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* fre
   return QOT_OK;
 }
 
+static int pl_launch(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
+                     const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N, int64_t E,
+                     const int32_t* chan_node, int64_t D, const int64_t* sample, const int64_t* opt_ptr, int64_t P,
+                     const int64_t* link_ptr, const int32_t* links, int64_t n_links, const int32_t* width,
+                     const float* feat, const float* own_bound, const float* bound, int32_t metric, int32_t maximize,
+                     int32_t policy, const float* prepared, int32_t is_lut_index, int32_t max_impact, int32_t* option,
+                     int32_t* q0, float* out, float* margin, int32_t* n_free, int32_t* n_feasible, int32_t* status,
+                     int32_t* n_impact, int64_t* impact_node, float* impact_out, float* all_out, float* all_margin,
+                     cudaStream_t stream) {
+  const char* who = "qot_lightpath_placements";
+  if (int rc = cfg_check(cfg, who)) return rc;
+  QOT_REQUIRE(cfg->Q <= QOT_PLACE_MAX_SLOTS, "%s: Q = %d over QOT_PLACE_MAX_SLOTS", who, cfg->Q);
+  QOT_REQUIRE(S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && D >= 0 && P >= 0 && n_links >= 0 && max_impact >= 0,
+              "%s: bad size", who);
+  QOT_REQUIRE(metric >= 0 && metric < QOT_OUT, "%s: metric must be an output column 0..2", who);
+  QOT_REQUIRE(policy == QOT_PLACE_FIRST_FIT || policy == QOT_PLACE_BEST_QOT || policy == QOT_PLACE_MAX_MARGIN,
+              "%s: unknown policy %d", who, policy);
+  QOT_REQUIRE(prepared && (reinterpret_cast<uintptr_t>(prepared) & 15) == 0, "%s: prepared must be 16-byte aligned",
+              who);
+  QOT_REQUIRE(is_lut_index >= 0 && is_lut_index < kF, "%s: is_lut_index out of range", who);
+  if (D == 0) return QOT_OK;
+  QOT_REQUIRE(sample && opt_ptr && link_ptr && (P == 0 || (width && feat && own_bound)) && (n_links == 0 || links),
+              "%s: null demand array", who);
+  QOT_REQUIRE(option && q0 && out && margin && n_free && n_feasible && status && n_impact &&
+                  (max_impact == 0 || (impact_node && impact_out)) && (!all_out == !all_margin),
+              "%s: null output array", who);
+  QOT_REQUIRE(S == 0 || (freqs && x && node_ptr && rowptr && chan_node && (E == 0 || edge_index)),
+              "%s: null state array", who);
+  static std::atomic<unsigned long long> done{0};
+  constexpr int smem = static_cast<int>(sizeof(PlSmem));
+  if (int rc = once_per_device(done, [] {
+        QOT_CUDA(cudaFuncSetAttribute(lp_placement_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        return static_cast<int>(QOT_OK);
+      }))
+    return rc;
+  PlArgs pa;
+  CdArgs& a = pa.c;
+  a.cfg = *cfg;
+  a.S = S; a.N = N; a.E = E; a.K = D; a.n_links = n_links;
+  a.freqs = freqs; a.x = x; a.node_ptr = node_ptr; a.rowptr = rowptr;
+  a.edst = edge_index ? edge_index + E : nullptr;
+  a.chan_node = chan_node;
+  a.node = nullptr;
+  a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = nullptr; a.width = width; a.feat = feat;
+  a.prep = prepared; a.lut_col = is_lut_index; a.max_impact = max_impact;
+  a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_node;
+  a.impact_kind = nullptr; a.impact_out = impact_out;
+  pa.P = P; pa.opt_ptr = opt_ptr; pa.own_bound = own_bound; pa.bound = bound;
+  pa.metric = metric; pa.maximize = maximize != 0; pa.policy = policy;
+  pa.option = option; pa.q0 = q0; pa.margin = margin; pa.n_free = n_free; pa.n_feasible = n_feasible;
+  pa.all_out = all_out; pa.all_margin = all_margin;
+  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, cdiv(D, kCdWarps)));
+  lp_placement_kernel<<<grid, kCdThreads, smem, stream>>>(pa);
+  QOT_LAUNCH_CHECK();
+  return QOT_OK;
+}
+
 }  // namespace qot
 
 using namespace qot;
@@ -912,4 +1421,22 @@ extern "C" int qot_lightpath_change_sets(const qot_lp_graph_cfg_t* cfg, int64_t 
   return cs_launch(cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, K, node, sample, link_ptr, links,
                    n_links, q0, width, feat, G, set_ptr, prepared, is_lut_index, max_impact, out, status, set_status,
                    n_impact, impact_node, impact_kind, impact_out, static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int qot_lightpath_placements(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs,
+                                        const float* x, const int64_t* node_ptr, const int64_t* rowptr,
+                                        const int64_t* edge_index, int64_t N, int64_t E, const int32_t* chan_node,
+                                        int64_t D, const int64_t* sample, const int64_t* opt_ptr, int64_t P,
+                                        const int64_t* link_ptr, const int32_t* links, int64_t n_links,
+                                        const int32_t* width, const float* feat, const float* own_bound,
+                                        const float* bound, int32_t metric, int32_t maximize, int32_t policy,
+                                        const float* prepared, int32_t is_lut_index, int32_t max_impact,
+                                        int32_t* option, int32_t* q0, float* out, float* margin, int32_t* n_free,
+                                        int32_t* n_feasible, int32_t* status, int32_t* n_impact,
+                                        int64_t* impact_node, float* impact_out, float* all_out, float* all_margin,
+                                        void* stream_) {
+  return pl_launch(cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, D, sample, opt_ptr, P, link_ptr,
+                   links, n_links, width, feat, own_bound, bound, metric, maximize, policy, prepared, is_lut_index,
+                   max_impact, option, q0, out, margin, n_free, n_feasible, status, n_impact, impact_node, impact_out,
+                   all_out, all_margin, static_cast<cudaStream_t>(stream_));
 }

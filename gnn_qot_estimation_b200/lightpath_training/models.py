@@ -218,6 +218,40 @@ class LightpathGNN(torch.nn.Module):
         return ops.lightpath_change_sets(state, changes, set_ptr, self.prepared(), self.is_lut_index, max_impact)
 
     @_lib.on_tensor_device
+    def forward_placements(self, state, demands, policy: int, metric: int = 0, maximize: bool = True, bound=None,
+                           max_impact: int = 64, return_all: bool = False) -> "ops.PlacementQoT":
+        """QoT-aware placement of lightpath demands: for each demand, the free slot range on one of its routes that a
+        policy picks among those whose predicted QoT meets its bounds (eval mode only; csrc/lightpath_candidates.cu,
+        qot_lightpath_placements).
+
+        ``demands``: ``to_graph.LightpathDemands`` on the state's device.  A placement of demand d is an option p
+        (route, width, features) with a start slot q0 such that ``[q0, q0 + width)`` is free on every link of the
+        route; its rows are, by definition, what ``forward_candidates`` returns for the candidate (sample, route, q0,
+        width, feat = (float32(state.freqs[q0]), mod_order, num_spans, path_len)).  A row's margin on output column
+        ``metric`` is ``v - b`` if ``maximize`` (OSNR, SNR) and ``b - v`` otherwise (BER), in fp32, with b the
+        option's ``own_bound`` for the own row and ``bound[node]`` (``bound`` [N] float32 over ``state.batch``'s
+        nodes, or None: impact rows unconstrained) for every impact row, whatever ``max_impact`` is.  The placement's
+        margin is the minimum over its rows, and it is feasible iff that is >= 0 (never when NaN).  ``policy``:
+        ``ops.PLACE_FIRST_FIT`` (the first feasible placement in (option, q0) order), ``ops.PLACE_BEST_QOT`` (the best
+        own value) or ``ops.PLACE_MAX_MARGIN`` (the largest margin); ties go to the lower option, then the lower q0.
+        Returns ``ops.PlacementQoT``: ``option`` (relative to the demand's first option) and ``q0`` (-1 if none is
+        feasible), the chosen own row ``out`` and ``margin`` (NaN if none), ``n_free`` / ``n_feasible`` over every
+        placement of the demand, ``status`` (``ops.CAND_*``: a bad sample, a bad route, width or option range, or a
+        bad state give -1 / NaN and zero counts; ``CAND_IMPACT_OVERFLOW`` applies to the chosen placement) and the
+        chosen placement's impact rows laid out as in ``forward_candidates``.  ``return_all``: also ``all_out`` [P, Q,
+        3] and ``all_margin`` [P, Q], every free placement's own row and margin, NaN at the other slots of the demands'
+        options.  Q is at most ``ops.PLACE_MAX_SLOTS``.  One launch, nothing read back: capturable in a CUDA graph.
+        Malformed arguments raise on the host."""
+        if self.training:
+            raise RuntimeError("LightpathGNN.forward_placements is eval-only (in training mode BatchNorm couples the "
+                               "nodes): call model.eval()")
+        if not state.batch.x.is_cuda:
+            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
+        self._check_supported()
+        return ops.lightpath_placements(state, demands, policy, metric, maximize, bound, self.prepared(),
+                                        self.is_lut_index, max_impact, return_all)
+
+    @_lib.on_tensor_device
     def forward_stream(self, plan, first: int = 0, count=None) -> None:
         """Enqueues batches [first, first+count) of ``plan`` (eval mode; no host synchronisation)."""
         if self.training:

@@ -501,6 +501,96 @@ def lightpath_change_sets(state, changes, set_ptr: torch.Tensor, prepared: torch
     return res
 
 
+# placement policies of qot_lightpath_placements; a demand offers at most PLACE_MAX_OPTIONS options, Q is at most
+# PLACE_MAX_SLOTS
+PLACE_FIRST_FIT, PLACE_BEST_QOT, PLACE_MAX_MARGIN = 0, 1, 2
+PLACE_MAX_OPTIONS = 32
+PLACE_MAX_SLOTS = 1024
+
+
+class PlacementQoT(NamedTuple):
+    option: torch.Tensor         # [D] int32: the chosen option, relative to opt_ptr[d] (-1: no feasible placement)
+    q0: torch.Tensor             # [D] int32: its start slot (-1: none)
+    out: torch.Tensor            # [D,3]: the chosen placement's own QoT (NaN: none)
+    margin: torch.Tensor         # [D]: its margin (NaN: none)
+    n_free: torch.Tensor         # [D] int32: free placements over the demand's options
+    n_feasible: torch.Tensor     # [D] int32: feasible placements among them
+    status: torch.Tensor         # [D] int32, CAND_* bits
+    n_impact: torch.Tensor       # [D] int32: lightpaths the chosen placement interferes with (may exceed max_impact)
+    impact_node: torch.Tensor    # [D, max_impact] int64: their nodes in the state batch, ascending; -1 past the rows
+    impact_out: torch.Tensor     # [D, max_impact, 3]: their QoT with the placement set up; NaN past the rows
+    all_out: Optional[torch.Tensor] = None     # [P, Q, 3] (return_all): every free placement's own QoT, NaN elsewhere
+    all_margin: Optional[torch.Tensor] = None  # [P, Q] (return_all): every free placement's margin, NaN elsewhere
+
+
+_DEMAND_DTYPES = {"sample": torch.int64, "opt_ptr": torch.int64, "link_ptr": torch.int64, "links": torch.int32,
+                  "width": torch.int32, "feat": torch.float32, "own_bound": torch.float32}
+
+
+def lightpath_placements(state, demands, policy: int, metric: int, maximize: bool, bound, prepared: torch.Tensor,
+                         is_lut_index: int, max_impact: int, return_all: bool = False) -> PlacementQoT:
+    """One launch of qot_lightpath_placements (the placement of each demand chosen over every free slot of its
+    options); nothing is read back (CUDA-graph capturable).  Refuses CPU tensors and mismatched devices, dtypes or
+    shapes, an unknown policy or metric and Q over PLACE_MAX_SLOTS; what can only be judged on the device comes back
+    as status bits."""
+    who = "forward_placements"
+    if int(max_impact) != max_impact or max_impact < 0:
+        raise ValueError(f"{who}: max_impact must be a non-negative integer")
+    if policy not in (PLACE_FIRST_FIT, PLACE_BEST_QOT, PLACE_MAX_MARGIN):
+        raise ValueError(f"{who}: policy must be PLACE_FIRST_FIT, PLACE_BEST_QOT or PLACE_MAX_MARGIN")
+    if metric not in (0, 1, 2):
+        raise ValueError(f"{who}: metric must be an output column 0, 1 or 2")
+    if state.Q > PLACE_MAX_SLOTS:
+        raise ValueError(f"{who}: Q = {state.Q} slots, at most {PLACE_MAX_SLOTS} (one 32-bit free word per lane)")
+    dev = state.batch.x.device
+    want = dict(_DEMAND_DTYPES)
+    named = [(n, getattr(demands, n), dt) for n, dt in want.items()]
+    if bound is not None:
+        named.append(("bound", bound, torch.float32))
+    for name, t, dt in named:
+        arg = "" if name == "bound" else "demands."
+        if not torch.is_tensor(t) or not t.is_cuda:
+            raise RuntimeError(f"{who}: {arg}{name} must be a CUDA tensor (no CPU path)")
+        if t.device != dev:
+            raise ValueError(f"{who}: {arg}{name} is on {t.device}, the state on {dev}")
+        if t.dtype != dt:
+            raise TypeError(f"{who}: {arg}{name} must be {dt}, got {t.dtype}")
+    if prepared.device != dev:
+        raise ValueError(f"{who}: the model is on {prepared.device}, the state on {dev}")
+    d = demands
+    D = int(d.sample.shape[0]) if d.sample.dim() == 1 else -1
+    P = int(d.width.shape[0]) if d.width.dim() == 1 else -1
+    if not (D >= 0 and P >= 0 and d.opt_ptr.shape == (D + 1,) and d.link_ptr.shape == (P + 1,) and
+            d.links.dim() == 1 and d.feat.shape == (P, 3) and d.own_bound.shape == (P,)):
+        raise ValueError(f"{who}: need sample [D], opt_ptr [D+1], link_ptr [P+1], links [n], width [P], feat [P,3], "
+                         "own_bound [P]")
+    N = int(state.batch.x.shape[0])
+    if bound is not None and bound.shape != (N,):
+        raise ValueError(f"{who}: need bound [N] with N = {N} nodes of the state batch")
+    max_impact = int(max_impact)
+    Q = state.Q
+    i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=dev)
+    f32 = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)
+    res = PlacementQoT(i32(D), i32(D), f32(D, 3), f32(D), i32(D), i32(D), i32(D), i32(D),
+                       torch.empty(D, max_impact, dtype=torch.int64, device=dev), f32(D, max_impact, 3),
+                       f32(P, Q, 3) if return_all else None, f32(P, Q) if return_all else None)
+    if D == 0:
+        return res
+    c = lambda t: ptr(t.contiguous()) if t is not None and t.numel() else None
+    keep = [t.contiguous() for t in (d.sample, d.opt_ptr, d.link_ptr, d.links, d.width, d.feat, d.own_bound)]
+    if bound is not None:
+        keep.append(bound.contiguous())
+    with torch.cuda.device(dev):
+        check(_lib.lib().qot_lightpath_placements(
+            *_state_args(state, keep), D, ptr(keep[0]), ptr(keep[1]), P, ptr(keep[2]), c(keep[3]),
+            int(keep[3].numel()), c(keep[4]), c(keep[5]), c(keep[6]), c(bound), int(metric), int(bool(maximize)),
+            int(policy), ptr(prepared), int(is_lut_index), max_impact, ptr(res.option), ptr(res.q0), ptr(res.out),
+            ptr(res.margin), ptr(res.n_free), ptr(res.n_feasible), ptr(res.status), ptr(res.n_impact),
+            c(res.impact_node), c(res.impact_out), c(res.all_out), c(res.all_margin), stream()),
+            "qot_lightpath_placements")
+    return res
+
+
 class GraphIndex:
     """Lazily built, cached index structures of one batch: the destination-sorted CSR
     (forward), its GAT variant (self loops replaced) and the source-sorted transposed

@@ -496,3 +496,44 @@ def lightpath_change_sets(samples, state, per_sample: int, seed: int = 0):
                              torch.tensor([r[4] for r in rows], dtype=torch.int32),
                              torch.tensor(np.array([r[5] for r in rows], dtype=np.float32).reshape(-1, 4))),
             torch.tensor(set_ptr, dtype=torch.int64))
+
+
+def lightpath_demands(samples, per_sample: int, options=(1, 4), seed: int = 0, bound_range=(0.1, 0.6)):
+    """Seeded lightpath demands for the network-status ``samples`` (the dict ``network_status_samples`` returns), for
+    ``LightpathGNN.forward_placements``.  ``per_sample`` demands per sample, each in a random sample with
+    ``options[0]..options[1]`` options.  An option is a route of 1..6 distinct random links (free slots or not), a
+    width of 1..3 slots, ``feat = (mod_order, num_spans, path_len)`` drawn as ``lightpath_candidates`` draws them and
+    ``own_bound``; after the first, an option repeats an earlier route of the demand with another modulation format
+    and width with probability 0.3.  ``own_bound`` is per demand: -inf on every option (probability 0.2: every free
+    placement is feasible), +inf (0.2: none is) or, per option, uniform in ``bound_range`` (0.6: the spread of the
+    reference model's column-0 predictions, so that a few placements are feasible).  Returns
+    ``to_graph.LightpathDemands`` of CPU tensors (``.to(device)``)."""
+    import numpy as np
+    from .to_graph import LightpathDemands
+    rng = np.random.default_rng(seed)
+    S, _, L, _ = samples["data"].shape
+    lo, hi = int(options[0]), int(options[1])
+    if not 1 <= lo <= hi:
+        raise ValueError("options must be (lo, hi) with 1 <= lo <= hi")
+    smp, optr, lptr, links, widths, feats, bounds = [], [0], [0], [], [], [], []
+    for _ in range(S * per_sample):
+        smp.append(int(rng.integers(0, S)))
+        kind = rng.random()
+        routes = []
+        for k in range(int(rng.integers(lo, hi + 1))):
+            if routes and rng.random() < 0.3:
+                path = routes[int(rng.integers(0, len(routes)))]
+            else:
+                path = [int(l) for l in rng.choice(L, size=min(int(rng.integers(1, 7)), L), replace=False)]
+                routes.append(path)
+            links.extend(path)
+            lptr.append(len(links))
+            widths.append(int(rng.integers(1, 4)))
+            feats.append([rng.choice([4, 8, 16, 32, 64]), int(rng.integers(1, 107)), int(rng.integers(24214, 7834746))])
+            bounds.append(-np.inf if kind < 0.2 else np.inf if kind < 0.4 else rng.uniform(*bound_range))
+        optr.append(len(widths))
+    return LightpathDemands(torch.tensor(smp, dtype=torch.int64), torch.tensor(optr, dtype=torch.int64),
+                            torch.tensor(lptr, dtype=torch.int64), torch.tensor(links, dtype=torch.int32),
+                            torch.tensor(widths, dtype=torch.int32),
+                            torch.tensor(np.array(feats, dtype=np.float32).reshape(-1, 3)),
+                            torch.tensor(np.array(bounds, dtype=np.float32)))

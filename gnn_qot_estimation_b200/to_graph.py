@@ -181,6 +181,24 @@ class LightpathChanges(NamedTuple):
         return LightpathChanges(*(t.to(device) for t in self))
 
 
+class LightpathDemands(NamedTuple):
+    """Lightpath demands to place (device tensors; ``LightpathGNN.forward_placements``).  Demand d goes into sample
+    ``sample[d]`` of the state and offers options ``[opt_ptr[d], opt_ptr[d+1])`` (1..32).  Option p is the route
+    ``links[link_ptr[p]:link_ptr[p+1]]`` with slot width ``width[p]``, channel features ``feat[p] = (mod_order,
+    num_spans, path_len)`` and a bound ``own_bound[p]`` on its own predicted metric.  The same route with another
+    modulation format is another option."""
+    sample: torch.Tensor          # [D] int64
+    opt_ptr: torch.Tensor         # [D+1] int64
+    link_ptr: torch.Tensor        # [P+1] int64
+    links: torch.Tensor           # [sum of route lengths] int32
+    width: torch.Tensor           # [P] int32
+    feat: torch.Tensor            # [P, 3] float32
+    own_bound: torch.Tensor       # [P] float32
+
+    def to(self, device) -> "LightpathDemands":
+        return LightpathDemands(*(t.to(device) for t in self))
+
+
 def lightpath_nodes(state: LightpathNetworkState, sample: torch.Tensor, conn_id: torch.Tensor) -> torch.Tensor:
     """[K] int64: the node of ``state.batch`` that holds lightpath ``conn_id[k]`` in sample ``sample[k]``, -1 where the
     sample has no such lightpath (or ``sample[k]`` is outside the state).  Device tensor ops, no host synchronisation:

@@ -626,6 +626,47 @@ int qot_lightpath_change_sets(const qot_lp_graph_cfg_t* cfg, int64_t S, const do
                               float* out, int32_t* status, int32_t* set_status, int32_t* n_impact,
                               int64_t* impact_node, int8_t* impact_kind, float* impact_out, void* stream);
 
+/* qot_lightpath_placements (lp_placement_kernel, the same launch shape, one warp per demand): D demands, each a sample
+ * sample[d] and options [opt_ptr[d], opt_ptr[d+1]) (opt_ptr [D+1] int64, 1..QOT_PLACE_MAX_OPTIONS options).  Option p
+ * (P of them) is a route links[link_ptr[p] .. link_ptr[p+1]) (link_ptr [P+1] int64), a slot width width[p], channel
+ * features feat [P,3] = (mod_order, num_spans, path_len) and a bound own_bound [P] on its own metric.  A placement is
+ * an option with a start slot q0 in [0, Q - width] whose channels [q0, q0 + width) are free (chan_node -1) on every
+ * link of the route; its rows are, by definition, the qot_lightpath_candidates rows of the candidate (sample, route,
+ * q0, width, feat = (float32(freqs[q0]), mod_order, num_spans, path_len)).  A row's margin (fp32, round to nearest)
+ * is v - b if maximize, else b - v, with v its output column `metric` (0..2) and b own_bound[p] for the own row or
+ * bound[node] (bound [N] float32, may be NULL: impact rows unconstrained) for each impact row, every impact row
+ * counted whatever max_impact is.  A placement's margin is the minimum over its rows (NaN if one is NaN); it is
+ * feasible iff the margin is >= 0.  Among the feasible placements `policy` picks one, a tie going to the lower option
+ * and then the lower q0:
+ *   QOT_PLACE_FIRST_FIT    the first in (option, q0) order;
+ *   QOT_PLACE_BEST_QOT     the best own value (highest if maximize, lowest otherwise);
+ *   QOT_PLACE_MAX_MARGIN   the largest margin.
+ * Outputs per demand: option / q0 [D] int32 (option relative to opt_ptr[d]; -1 / -1 if none is feasible), out [D,3]
+ * the chosen own row (NaN if none), margin [D] (NaN if none), n_free / n_feasible [D] int32 over every placement of
+ * the demand, status [D] int32, and the chosen placement's n_impact / impact_node [D,max_impact] / impact_out
+ * [D,max_impact,3] exactly as qot_lightpath_candidates lays them out.  all_out [P,Q,3] / all_margin [P,Q] (both NULL,
+ * or both given): every free placement's own row and margin, NaN at every other (option, q0) of a demand's options.
+ * Status bits QOT_CAND_*: BAD_SAMPLE; BAD_PATH (an empty route, a link outside [0, L), a width outside [1, Q), zero
+ * or more than QOT_PLACE_MAX_OPTIONS options, a malformed opt_ptr or link_ptr range); BAD_STATE (a route's channel
+ * holds a node outside the sample, a bad in-row); IMPACT_OVERFLOW (the chosen placement has more than max_impact
+ * impact rows).  Any bit but IMPACT_OVERFLOW: option = q0 = -1, NaN rows, zero counts.  Q <= QOT_PLACE_MAX_SLOTS.
+ * No host synchronisation: capturable; a malformed demand never faults and never stops the launch. */
+#define QOT_PLACE_MAX_OPTIONS 32
+#define QOT_PLACE_MAX_SLOTS 1024
+#define QOT_PLACE_FIRST_FIT 0
+#define QOT_PLACE_BEST_QOT 1
+#define QOT_PLACE_MAX_MARGIN 2
+int qot_lightpath_placements(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
+                             const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N,
+                             int64_t E, const int32_t* chan_node, int64_t D, const int64_t* sample,
+                             const int64_t* opt_ptr, int64_t P, const int64_t* link_ptr, const int32_t* links,
+                             int64_t n_links, const int32_t* width, const float* feat, const float* own_bound,
+                             const float* bound, int32_t metric, int32_t maximize, int32_t policy,
+                             const float* prepared, int32_t is_lut_index, int32_t max_impact, int32_t* option,
+                             int32_t* q0, float* out, float* margin, int32_t* n_free, int32_t* n_feasible,
+                             int32_t* status, int32_t* n_impact, int64_t* impact_node, float* impact_out,
+                             float* all_out, float* all_margin, void* stream);
+
 /* The topological representation: to_graph.py::create_topological_graph (:62-184: one edge per
  * lightpath between its source and destination network node, lightpaths added in ascending conn_id,
  * nx.Graph keeps one edge per node pair -- position from the first, attributes from the last) fused
