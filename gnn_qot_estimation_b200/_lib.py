@@ -57,7 +57,7 @@ class QotParamSeg(C.Structure):
 
 class QotSgdHyper(C.Structure):
     _fields_ = [("lr", C.c_float), ("momentum", C.c_float), ("dampening", C.c_float), ("weight_decay", C.c_float),
-                ("nesterov", i32), ("maximize", i32), ("reserved", i32 * 2)]
+                ("nesterov", i32), ("maximize", i32), ("one_minus_dampening", C.c_float), ("reserved", i32)]
 
 
 class QotLpWireSlot(C.Structure):

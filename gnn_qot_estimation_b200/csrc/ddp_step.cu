@@ -78,7 +78,8 @@ ddp_sgd_step_kernel(float* __restrict__ grad, float* const* __restrict__ peers, 
       return;                                                     // no update: the replicas would diverge
     }
   }
-  const float lr = hyper->lr, mom = hyper->momentum, damp = hyper->dampening, wd = hyper->weight_decay;
+  // one_minus_dampening: rounded from double on the host, as torch's alpha = 1 - dampening (not 1.0f - float(dampening))
+  const float lr = hyper->lr, mom = hyper->momentum, omd = hyper->one_minus_dampening, wd = hyper->weight_decay;
   const bool nesterov = hyper->nesterov != 0, maximize = hyper->maximize != 0;
   const float inv_w = 1.0f / static_cast<float>(world);
   const bool first = mom != 0.f && state[1] == 0ull;             // torch: the first step clones the gradient into the buffer
@@ -119,7 +120,7 @@ ddp_sgd_step_kernel(float* __restrict__ grad, float* const* __restrict__ peers, 
       if (maximize) g = -g;
       if (wd != 0.f) g = fmaf(wd, p, g);
       if (mom != 0.f) {
-        float b = first ? g : fmaf(1.0f - damp, g, __fmul_rn(momentum_buf[i], mom));
+        float b = first ? g : fmaf(omd, g, __fmul_rn(momentum_buf[i], mom));
         momentum_buf[i] = b;
         g = nesterov ? fmaf(mom, b, g) : b;
       }

@@ -149,6 +149,15 @@ class PeerExchange:
         dist.barrier(group)                             # every rank's buffer is zeroed before anyone's first step
 
 
+def pack_sgd_hyper(lr: float, momentum: float, dampening: float, weight_decay: float, nesterov: bool,
+                   maximize: bool):
+    """``qot_sgd_hyper_t`` of one SGD parameter group.  ``one_minus_dampening`` is ``1 - dampening`` in double, rounded
+    to fp32 once: the ``alpha`` torch.optim.SGD hands its foreach kernels (``1.0f - float(dampening)`` is one ulp off
+    for dampening 0.6, 0.8, 0.9, 0.99 or 1/3)."""
+    from . import _lib
+    return _lib.QotSgdHyper(lr, momentum, dampening, weight_decay, int(nesterov), int(maximize), 1.0 - float(dampening))
+
+
 class FusedSGDStep:
     """``optimizer.step()`` of a plain ``torch.optim.SGD`` (one parameter group, fp32 CUDA parameters -- what
     topological_training/train.py:66 builds) fused with the data-parallel gradient exchange into ONE launch
@@ -210,14 +219,12 @@ class FusedSGDStep:
         self.state[1] = 0
 
     def sync_hyper(self) -> None:
-        import ctypes as C
-        from . import _lib
         g = self.opt.param_groups[0]
         key = (float(g["lr"]), float(g["momentum"]), float(g["dampening"]), float(g["weight_decay"]),
                bool(g["nesterov"]), bool(g.get("maximize", False)))
         if key == self._hyper_key:
             return
-        h = _lib.QotSgdHyper(key[0], key[1], key[2], key[3], int(key[4]), int(key[5]))
+        h = pack_sgd_hyper(*key)
         self._hyper_host.copy_(torch.frombuffer(bytearray(bytes(h)), dtype=torch.uint8))
         self.hyper.copy_(self._hyper_host, non_blocking=True)
         self._hyper_key = key

@@ -76,8 +76,13 @@ def check_status(clear: bool = True) -> None:
         by_dev.setdefault(t.device, []).append((what, t))
     bad = []
     for dev, items in by_dev.items():
-        vals = torch.cat([t.reshape(1) for _, t in items]).tolist()
-        bad += [f"{what} (status {v})" for (what, _), v in zip(items, vals) if v]
+        vals = iter(torch.cat([t.reshape(-1) for _, t in items]).tolist())
+        for what, t in items:                     # a tracked tensor may hold several words (one per batch): OR them
+            v = 0
+            for _ in range(t.numel()):
+                v |= next(vals)
+            if v:
+                bad.append(f"{what} (status {v})")
     if bad:
         raise RuntimeError("libqot_b200: input contract violated in: " + "; ".join(sorted(set(bad))[:8]) +
                            " -- out-of-range node ids / edge endpoints, edges not grouped by graph, or a graph "

@@ -742,7 +742,11 @@ int qot_topo_fused_bwd(const float* prepared, const float* emb, const int64_t* n
  *           reset it on one rank only), [1] != 0 once the momentum buffer holds a gradient (clear it to make the next
  *           step clone the gradient into the buffer, as torch does for a fresh optimizer).
  *   status  bit 0: a peer did not arrive within 4 s (no update was applied).
- * Sums in rank order on every rank: the replicas stay bit-identical. */
+ * Sums in rank order on every rank: the replicas stay bit-identical.
+ * `one_minus_dampening` is the momentum update's gradient factor, 1 - dampening computed in double and rounded to
+ * float once, as torch.optim.SGD passes it to its foreach kernels; float(1) - float(dampening) differs from it by one
+ * ulp for dampening 0.6, 0.8, 0.9, 0.99 or 1/3, and the trajectory would leave torch's in the low bits.  `dampening` itself is
+ * not read by the kernel. */
 typedef struct {
   float* param;          /* the parameter tensor (fp32, contiguous)           */
   int64_t offset;        /* its first element in the flat gradient            */
@@ -751,7 +755,8 @@ typedef struct {
 typedef struct {
   float lr, momentum, dampening, weight_decay;
   int32_t nesterov, maximize;
-  int32_t reserved[2];
+  float one_minus_dampening;
+  int32_t reserved;
 } qot_sgd_hyper_t;
 size_t qot_ddp_exchange_bytes(int64_t n);
 int qot_ddp_sgd_step(float* grad, float* const* peers, int32_t world, int32_t rank, int64_t n,

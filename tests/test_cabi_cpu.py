@@ -54,6 +54,25 @@ def test_ctypes_table_matches_header(lib_path):
     _lib.lib()                     # binds every symbol; raises AttributeError on a missing one
 
 
+@pytest.mark.parametrize("struct,ctype,size", [("qot_sgd_hyper_t", "QotSgdHyper", 32),
+                                               ("qot_param_seg_t", "QotParamSeg", 24)])
+def test_ctypes_structs_match_header(struct, ctype, size):
+    """Field names, order, offsets and size of the structs the kernels read from device memory."""
+    from gnn_qot_estimation_b200 import _lib
+    text = re.sub(r"/\*.*?\*/", "", HEADER.read_text(), flags=re.S)
+    body = re.search(r"typedef struct \{([^}]*)\}\s*" + struct + r"\s*;", text).group(1)
+    names = [re.sub(r"\[\d+\]$", "", n.strip().lstrip("*")) for decl in body.split(";") if decl.strip()
+             for n in decl.strip().split(None, 1)[1].split(",")]
+    cls = getattr(_lib, ctype)
+    assert [f[0] for f in cls._fields_] == names
+    assert ctypes.sizeof(cls) == size
+    if struct == "qot_sgd_hyper_t":
+        offs = {f[0]: getattr(cls, f[0]).offset for f in cls._fields_}
+        assert offs == {"lr": 0, "momentum": 4, "dampening": 8, "weight_decay": 12, "nesterov": 16, "maximize": 20,
+                        "one_minus_dampening": 24, "reserved": 28}
+        assert getattr(cls, "one_minus_dampening").size == 4 and cls._fields_[6][1] is ctypes.c_float
+
+
 def test_no_torch_types_in_the_abi():
     code = re.sub(r"/\*.*?\*/", "", HEADER.read_text(), flags=re.S)      # declarations only, no comments
     assert "torch" not in code.lower() and "at::" not in code and "Tensor" not in code

@@ -238,3 +238,24 @@ def test_derived_weight_cache_follows_parameter_updates():
     c5 = ops._derived("t", (a, b), make)                      # frozen weights: cached even with grad mode on
     c6 = ops._derived("t", (a, b), make)
     assert c5 is c6
+
+
+def test_check_status_reads_multi_word_status_tensors(monkeypatch):
+    """A tracked status tensor may hold one word per batch (the multi-batch lightpath stream): check_status() ORs its
+    words, raises only when one is set, and still reads single-word tensors tracked beside it."""
+    from gnn_qot_estimation_b200 import ops
+    monkeypatch.setattr(ops, "_status_words", {})
+    multi, single = torch.zeros(3, dtype=torch.int32), torch.zeros(1, dtype=torch.int32)
+    ops._track_status("multi", multi)
+    ops._track_status("single", single)
+    ops.check_status(clear=False)
+    multi[2] = 2
+    multi[0] = 1
+    with pytest.raises(RuntimeError, match=r"multi \(status 3\)") as e:
+        ops.check_status(clear=False)
+    assert "single" not in str(e.value)
+    multi.zero_()
+    single[0] = 4
+    with pytest.raises(RuntimeError, match=r"single \(status 4\)"):
+        ops.check_status()
+    ops.check_status()                               # cleared
