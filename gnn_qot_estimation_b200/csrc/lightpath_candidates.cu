@@ -1,38 +1,36 @@
-// LightpathGNN candidate QoT: a candidate lightpath evaluated against a resident network state without rebuilding
-// the state's graph.
+// LightpathGNN network-state queries: candidate lightpaths, reconfigurations, change sets and placements evaluated
+// against a resident network state without rebuilding the state's graph.
 //
-// Semantics: candidate k names a sample s_k of the state, a path (link indices), a contiguous slot range
-// [q0_k, q0_k + width_k) used on every link of the path and its raw feature vector (freq, mod_order, num_spans,
-// path_len).  sample' is sample s_k with the candidate written into every channel of its path and slot range (a new
-// conn_id, osnr = snr = ber = -1).  In sample''s lightpath graph (to_graph's construction):
-//   out[k]           = the eval-mode forward with the flag column one-hot at the candidate's node;
-//   impact row i     = the same with the flag at the candidate's i-th neighbour j, neighbours in ascending order of
-//                      their node index in the state batch.
 // Why no rebuild is needed: the model has one GAT layer and eval-mode BatchNorm is a per-node affine, so a row depends
-// only on its node and its in-neighbours.  Inserting the candidate adds exactly the edges candidate <-> j for the
-// lightpaths j that share a link with it at 0 < |df| < freq_threshold; every other row of the graph is unchanged.
+// only on its node and its in-neighbours.  Placing a lightpath adds exactly the edges new <-> j for the lightpaths j
+// that share a link with it at 0 < |df| < freq_threshold, and removing one drops its edges; every other row of the
+// graph is unchanged.
 //
 //   lp_channel_map_kernel (once per state): chan_node [S, L, Q] = state-batch node index of the lightpath on each
 //     channel, -1 on a free channel (occupancy and conn_id truncation as in to_graph.cu).
-//   lp_candidate_kernel: persistent, one warp per candidate.  Validate; scan the chan_node rows of the path's links
-//     with the fp64 df test of to_graph.cu, neighbours into a 256-bit per-warp mask (a state sample holds at most
-//     QOT_TG_MAX_NODES lightpaths), ranked ascending; then
-//       candidate row: query flag 1, the neighbours (flag 0), the appended self loop;
-//       impact row j:  query flag 1, j's in-row of the state graph = the destinations of j's out-run in the
-//                      source-sorted edge list (self loop dropped, flag 0), the candidate (flag 0), j's self loop.
-//     Every z row goes through the warp's 16-row buffer and head_rows16_tf32x3 (the mma.sync head of every-node mode).
 //
-// Reconfiguration (qot_lightpath_reconfigure, the kMove instantiation): a change is a candidate that also names the
-// lightpath j it moves (-1: a plain insertion, bit-identical to the candidate path).  j's old channels count as free,
-// its old neighbours (the destinations of its out-run, self loop dropped) go into a second 256-bit mask, and the impact
-// rows are the union of both masks, ranked ascending, with kind bits old | new << 1:
-//       j's row:         query flag 1, j's new neighbours (flag 0), the appended self loop (none for a teardown);
-//       impact row i:    query flag 1, i's state in-row without j (flag 0), j with its new x if i is a new
-//                        neighbour (flag 0), i's self loop.
-// Every other row of the sample is unchanged, for the same locality reason as a candidate's.
+// The query kernels are persistent, one warp per query, and built from the same pieces, each defined once below:
+//   cd_bad_route, cd_sample_nodes  a route (its link_ptr range, every link in [0, L)) and a sample's node range;
+//   cd_df_hit                      to_graph.cu's fp64 edge test: some slot of [c0, c0 + cw) at 0 < |df| < threshold;
+//   cd_scan                        the chan_node rows of a route, cd_df_hit against every channel of a known lightpath,
+//                                  neighbours into a 256-bit per-warp mask (a state sample holds at most
+//                                  QOT_TG_MAX_NODES lightpaths); the lightpaths a query removes count as free;
+//   cd_old_nbrs                    a removed lightpath's old neighbours: the destinations of its out-run;
+//   cd_rank                        a mask's bits in ascending order (the order of rows and messages);
+//   cd_xrow                        a new lightpath's scaled x row [freq, is_lut = 1, mod_order, num_spans, path_len];
+//   cd_in_row                      j's in-row of the state graph: the destinations of j's out-run in the source-sorted
+//                                  edge list, j's self loop and the removed lightpaths dropped;
+//   cd_head_prologue, cd_row       the head: every z row is staged in the warp's 16-row buffer and goes through
+//                                  head_rows16_tf32x3 (the mma.sync head of every-node mode) in cd_flush;
+//   cd_clear_impact                the empty result past the emitted impact rows: node -1, kind 0, NaN QoT.
+// A new lightpath's row is: query flag 1, its new neighbours ascending (flag 0), its appended self loop.  The impact
+// row of neighbour j is: query flag 1, j's in-row (flag 0), the new lightpath (flag 0) if j is a new neighbour, j's
+// self loop.  Because every kernel builds its rows from these pieces in this message order, an insertion through
+// qot_lightpath_reconfigure is bit-identical to a candidate, a set of one change to a reconfiguration, and a
+// placement's rows to the candidate on the same slots.
 //
-// Deterministic: integer mask bits only, fixed message order, no float atomics.  A malformed candidate gets status
-// bits and a NaN row; it never faults and never stops the launch.
+// Deterministic: integer mask bits only, fixed message order, no float atomics.  A malformed query gets status bits
+// and NaN rows; it never faults and never stops the launch.
 #include <algorithm>
 #include <climits>
 
@@ -115,55 +113,6 @@ struct CdX {
   }
 };
 
-__device__ __noinline__ void cd_flush(int w, int cnt, const float* __restrict__ prep, int lane) {
-  CdSmem& sm = cd_smem();
-  CdWarpSmem& ws = sm.w[w];
-  const int g8 = lane >> 2, t4 = lane & 3;
-  const bool va = g8 < cnt, vb = g8 + 8 < cnt;
-  float oa, ob;
-  head_rows16_tf32x3(sm.frag, sm.frag + 16 * 32, ws.z + g8 * kCdZPitch, ws.z + (g8 + 8) * kCdZPitch, va, vb, prep,
-                     lane, oa, ob);
-  if (t4 < QOT_OUT) {
-    if (va) reinterpret_cast<float*>(ws.orow[g8])[t4] = oa;
-    if (vb) reinterpret_cast<float*>(ws.orow[g8 + 8])[t4] = ob;
-  }
-  __syncwarp();
-}
-
-// attention of query node q over msg[0, M) into the next staged z row; the row's outputs go to `dst`
-template <typename XF>
-__device__ __forceinline__ int cd_row(CdWarpSmem& ws, int w, int zc, const int* msg, int M, int q, const XF& xf,
-                                      const float (&As)[kF], const float (&Ad)[kF], float* dst,
-                                      const float* __restrict__ prep, int lane) {
-  float d_q = 0.f;
-#pragma unroll
-  for (int k = 0; k < kF; ++k) d_q = fmaf(xf(q, k), Ad[k], d_q);
-  AttnState st;
-  attn_consume(st, msg, M, xf, As, d_q, lane);
-  attn_finish<kF>(st, ws.z + zc * kCdZPitch, lane);
-  if (lane == 0) ws.orow[zc] = reinterpret_cast<long long>(dst);
-  __syncwarp();
-  if (++zc == 16) {
-    cd_flush(w, 16, prep, lane);
-    zc = 0;
-  }
-  return zc;
-}
-
-// ranks the set bits of a 256-bit mask (lane t < 8 holds word t) ascending into dst[0, count); returns the count
-__device__ __forceinline__ int cd_rank(unsigned mw, int* dst, int lane) {
-  int pos = __popc(mw);
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const int up = __shfl_up_sync(kFull, pos, o);
-    if (lane >= o) pos += up;
-  }
-  const int cnt = __shfl_sync(kFull, pos, 31);
-  pos -= __popc(mw);
-  for (unsigned m = mw; m; m &= m - 1) dst[pos++] = 32 * lane + __ffs(m) - 1;
-  return cnt;
-}
-
 struct CdArgs {
   qot_lp_graph_cfg_t cfg;
   int64_t S, N, E, K, n_links;
@@ -190,26 +139,225 @@ struct CdArgs {
   float* impact_out;
 };
 
-// kMove = false: qot_lightpath_candidates; true: qot_lightpath_reconfigure (a.node, a.impact_kind)
-template <bool kMove>
-__global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __grid_constant__ CdArgs a) {
+// The helpers below read L, Q, the threshold and max_impact from the kernel parameters where they use them: hoisted
+// into registers, those values spill in the change-set kernel.
+
+// the head's fragment tables into shared memory (published by the caller's next block barrier) and this lane's head
+// column of the attention vectors into registers
+__device__ __forceinline__ void cd_head_prologue(const float* __restrict__ prep, float (&As)[kF], float (&Ad)[kF],
+                                                 int tid) {
   CdSmem& sm = cd_smem();
-  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
-  CdWarpSmem& ws = sm.w[w];
   for (int i = tid; i < kStHeadFrag4; i += kCdThreads)
-    sm.frag[i] = __ldg(reinterpret_cast<const float4*>(a.prep + kOffB1f) + i);
-  __syncthreads();
-  const float* __restrict__ prep = a.prep;
-  const int h = lane & 3;
-  float As[kF], Ad[kF];
+    sm.frag[i] = __ldg(reinterpret_cast<const float4*>(prep + kOffB1f) + i);
+  const int h = tid & 3;
 #pragma unroll
   for (int k = 0; k < kF; ++k) {
     As[k] = __ldg(prep + kOffAsrc + k * kHeads + h);
     Ad[k] = __ldg(prep + kOffAdst + k * kHeads + h);
   }
-  const int L = a.cfg.L, Q = a.cfg.Q, MI = a.max_impact;
-  const double thr = a.cfg.freq_threshold;
+}
+
+__device__ __noinline__ void cd_flush(int w, int cnt, const float* __restrict__ prep, int lane) {
+  CdSmem& sm = cd_smem();
+  CdWarpSmem& ws = sm.w[w];
+  const int g8 = lane >> 2, t4 = lane & 3;
+  const bool va = g8 < cnt, vb = g8 + 8 < cnt;
+  float oa, ob;
+  head_rows16_tf32x3(sm.frag, sm.frag + 16 * 32, ws.z + g8 * kCdZPitch, ws.z + (g8 + 8) * kCdZPitch, va, vb, prep,
+                     lane, oa, ob);
+  if (t4 < QOT_OUT) {
+    if (va) reinterpret_cast<float*>(ws.orow[g8])[t4] = oa;
+    if (vb) reinterpret_cast<float*>(ws.orow[g8 + 8])[t4] = ob;
+  }
+  __syncwarp();
+}
+
+// attention of query node q over msg[0, M) into staged z row zc, whose outputs go to `dst`; a full buffer of 16 rows
+// goes to `flush(16)`.  Returns the rows staged.
+template <typename XF, typename Flush>
+__device__ __forceinline__ int cd_row(CdWarpSmem& ws, int zc, const int* msg, int M, int q, const XF& xf,
+                                      const float (&As)[kF], const float (&Ad)[kF], float* dst, const Flush& flush,
+                                      int lane) {
+  float d_q = 0.f;
+#pragma unroll
+  for (int k = 0; k < kF; ++k) d_q = fmaf(xf(q, k), Ad[k], d_q);
+  AttnState st;
+  attn_consume(st, msg, M, xf, As, d_q, lane);
+  attn_finish<kF>(st, ws.z + zc * kCdZPitch, lane);
+  if (lane == 0) ws.orow[zc] = reinterpret_cast<long long>(dst);
+  __syncwarp();
+  if (++zc == 16) {
+    flush(16);
+    zc = 0;
+  }
+  return zc;
+}
+
+// ranks the set bits of a 256-bit mask (lane t < 8 holds word t) ascending into dst[0, count); returns the count
+__device__ __forceinline__ int cd_rank(unsigned mw, int* dst, int lane) {
+  int pos = __popc(mw);
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int up = __shfl_up_sync(kFull, pos, o);
+    if (lane >= o) pos += up;
+  }
+  const int cnt = __shfl_sync(kFull, pos, 31);
+  pos -= __popc(mw);
+  for (unsigned m = mw; m; m &= m - 1) dst[pos++] = 32 * lane + __ffs(m) - 1;
+  return cnt;
+}
+
+// to_graph.cu's edge test, in fp64: some slot c of [c0, c0 + cw) at 0 < |freqs[c] - fq| < thr
+__device__ __forceinline__ bool cd_df_hit(const double* freqs, double fq, int c0, int cw, double thr) {
+  bool hit = false;
+  for (int c = c0; c < c0 + cw && !hit; ++c) {
+    const double df = fabs(freqs[c] - fq);
+    hit = df < thr && df > 0.0;
+  }
+  return hit;
+}
+
+// removes no lightpath: the predicate of cd_scan and cd_in_row for candidates and placements
+struct CdNone {
+  __device__ __forceinline__ bool operator()(int) const { return false; }
+};
+
+// the new neighbours of placement [c0, c0 + cw) on route links[p0, p1) of sample s (nodes [n0, n0 + n)): the known
+// lightpath on every other channel of the route's chan_node rows that passes cd_df_hit sets its bit in `mask`.  A
+// channel of a lightpath `removed(j)` names (sample-local) counts as free.  Returns this lane's status bits:
+// QOT_CAND_OCCUPIED (a channel of the placement is taken), QOT_CAND_BAD_STATE (an owner outside the sample).
+template <typename Removed>
+__device__ __forceinline__ int cd_scan(const CdArgs& a, int64_t s, int64_t n0, int n, int64_t p0, int64_t p1, int c0,
+                                       int cw, unsigned* mask, const Removed& removed, int lane) {
+  bool occ = false, bad = false;
+  for (int64_t e = p0; e < p1; ++e) {
+    const int32_t* __restrict__ row = a.chan_node + (s * a.cfg.L + a.links[e]) * a.cfg.Q;
+    for (int q = lane; q < a.cfg.Q; q += 32) {
+      const int32_t v = row[q];
+      if (v == -1) continue;                                    // free
+      const int64_t j = v - n0;
+      const bool inside = v >= 0 && j >= 0 && j < n;
+      if (inside && removed(static_cast<int>(j))) continue;
+      if (q >= c0 && q < c0 + cw) { occ = true; continue; }
+      if (v < -1) continue;                                     // occupied by an unknown lightpath: no edge
+      if (!inside) { bad = true; continue; }
+      if (cd_df_hit(a.freqs, a.freqs[q], c0, cw, a.cfg.freq_threshold)) atomicOr(&mask[j >> 5], 1u << (j & 31));
+    }
+  }
+  return (occ ? QOT_CAND_OCCUPIED : 0) | (bad ? QOT_CAND_BAD_STATE : 0);
+}
+
+// the old neighbours of sample-local node jm: the destinations of its out-run, self loop dropped, into `mask`; false
+// (on this lane) when the run is malformed or leaves the sample
+__device__ __forceinline__ bool cd_old_nbrs(const CdArgs& a, int64_t n0, int n, int jm, unsigned* mask, int lane) {
+  const int64_t r0 = a.rowptr[n0 + jm], r1 = a.rowptr[n0 + jm + 1];
+  if (!(r0 >= 0 && r1 >= r0 && r1 <= a.E)) return false;
+  bool ok = true;
+  for (int64_t e = r0 + lane; e < r1; e += 32) {
+    const int64_t dg = a.edst[e] - n0;
+    if (dg < 0 || dg >= n) ok = false;
+    else if (dg != jm) atomicOr(&mask[dg >> 5], 1u << (dg & 31));
+  }
+  return ok;
+}
+
+// sample-local node j's in-row of the state graph: the destinations of j's out-run in the source-sorted edge list, in
+// edge order, without j's self loop and the nodes `drop` names, into msg.  Returns their count, or -1 (warp-uniform)
+// when the run is malformed, longer than a sample or leaves the sample.  kGather = false: the check alone.
+template <bool kGather = true, typename Drop = CdNone>
+__device__ __forceinline__ int cd_in_row(const CdArgs& a, int64_t n0, int n, int j, int* msg, int lane,
+                                         const Drop& drop = Drop()) {
+  const int64_t r0 = a.rowptr[n0 + j], r1 = a.rowptr[n0 + j + 1];
+  bool bad = !(r0 >= 0 && r1 >= r0 && r1 <= a.E && r1 - r0 <= kCdMaxN);
+  int m = 0;
+  if (!bad)
+    for (int64_t eb = r0; eb < r1; eb += 32) {
+      const int64_t e = eb + lane;
+      const int64_t dg = e < r1 ? a.edst[e] - n0 : -1;
+      const bool inside = dg >= 0 && dg < n;
+      bad |= e < r1 && !inside;
+      if (kGather) {
+        const bool keep = inside && dg != j && !drop(static_cast<int>(dg));
+        const unsigned ball = __ballot_sync(kFull, keep);
+        if (keep) msg[m + __popc(ball & ((1u << lane) - 1u))] = static_cast<int>(dg);
+        m += __popc(ball);
+      }
+    }
+  return __any_sync(kFull, bad) ? -1 : m;
+}
+
+// a new lightpath's x row [freq, is_lut, mod_order, num_spans, path_len] into cx: on lane t < 4, raw() gives raw
+// feature t (freq, mod_order, num_spans, path_len) as float32, scaled min-max in fp64 and rounded to fp32 (dataset.py's
+// scaling; feat_lo / feat_hi in that order); is_lut is 1, to_graph's value for a lightpath with unknown metrics
+template <typename Raw>
+__device__ __forceinline__ void cd_xrow(const CdArgs& a, float* cx, const Raw& raw, int lane) {
+  if (lane < 4) {
+    const double v = static_cast<double>(raw());
+    cx[lane == 0 ? 0 : lane + 1] =
+        static_cast<float>((v - a.cfg.feat_lo[lane]) / (a.cfg.feat_hi[lane] - a.cfg.feat_lo[lane]));
+  }
+  if (lane == 4) cx[1] = 1.0f;
+}
+
+// sample s's nodes [n0, n0 + n) of the state batch; false when node_ptr is malformed there or the sample holds more
+// than kCdMaxN lightpaths (n0 is read either way)
+__device__ __forceinline__ bool cd_sample_nodes(const CdArgs& a, int64_t s, int64_t& n0, int& n) {
+  n0 = a.node_ptr[s];
+  const int64_t n1 = a.node_ptr[s + 1];
+  if (!(n0 >= 0 && n1 >= n0 && n1 <= a.N && n1 - n0 <= kCdMaxN)) return false;
+  n = static_cast<int>(n1 - n0);
+  return true;
+}
+
+// the route check, warp-uniform: links[p0, p1) is a non-empty range of `links` (an empty one for a teardown) whose
+// links all lie in [0, L), and the caller's own checks `bad` (skipped for a teardown) pass; true when it fails.  L is
+// cfg.L, passed in: the placement kernel keeps it in a register, and reading it here again spills there.
+__device__ __forceinline__ bool cd_bad_route(const CdArgs& a, int L, int64_t p0, int64_t p1, bool tear, bool bad,
+                                             int lane) {
+  bad = tear ? !(p0 >= 0 && p0 <= a.n_links) : bad || !(p0 >= 0 && p1 > p0 && p1 <= a.n_links);
+  if (!bad)
+    for (int64_t e = p0 + lane; e < p1; e += 32) {
+      const int l = a.links[e];
+      bad |= l < 0 || l >= L;
+    }
+  return __any_sync(kFull, bad);
+}
+
+// the empty result in impact rows [from, MI) of output row k (MI = max_impact): node -1, kind 0 (when `kind`, the
+// kernel's optional impact_kind), NaN QoT; written by threads t, t + stride, ...
+__device__ __forceinline__ void cd_clear_impact(const CdArgs& a, int64_t k, int from, int MI, int8_t* kind, int t,
+                                                int stride) {
+  for (int i = from + t; i < MI; i += stride) {
+    a.impact_node[k * MI + i] = -1;
+    if (kind) kind[k * MI + i] = 0;
+  }
+  for (int i = from * QOT_OUT + t; i < MI * QOT_OUT; i += stride)
+    a.impact_out[k * MI * QOT_OUT + i] = __int_as_float(0x7fc00000);
+}
+
+// lp_candidate_kernel, one warp per candidate: candidate k names a sample s_k of the state, a path, a slot range
+// [q0_k, q0_k + width_k) used on every link of the path and its raw features (freq, mod_order, num_spans, path_len).
+// sample' is s_k with the candidate written into those channels (a new conn_id, osnr = snr = ber = -1); out[k] is the
+// candidate's row in sample''s lightpath graph with the flag column one-hot at the candidate, impact row i that of
+// its i-th neighbour, neighbours ascending by state-batch node index.
+//
+// kMove = true (qot_lightpath_reconfigure): a change is a candidate that also names the lightpath j it moves (-1: a
+// plain insertion, bit-identical to a candidate).  j's old channels count as free, its old neighbours go into a second
+// 256-bit mask, and the impact rows are the union of both masks, ranked ascending, with kind bits old | new << 1.  j's
+// row has its new neighbours (none for a teardown: NaN); impact row i drops j from i's in-row and takes j, with its
+// new x, only if i is a new neighbour.
+constexpr int kCdFatal =
+    QOT_CAND_BAD_SAMPLE | QOT_CAND_BAD_PATH | QOT_CAND_OCCUPIED | QOT_CAND_BAD_STATE | QOT_CAND_BAD_NODE;
+
+template <bool kMove>
+__global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __grid_constant__ CdArgs a) {
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  CdWarpSmem& ws = cd_smem().w[w];
+  float As[kF], Ad[kF];
+  cd_head_prologue(a.prep, As, Ad, tid);
+  __syncthreads();
   const float nan = __int_as_float(0x7fc00000);
+  const auto flush = [&](int cnt) { cd_flush(w, cnt, a.prep, lane); };
   int zc = 0;                                   // rows staged in this warp's head buffer
   for (int64_t k = static_cast<int64_t>(blockIdx.x) * kCdWarps + w; k < a.K;
        k += static_cast<int64_t>(gridDim.x) * kCdWarps) {
@@ -221,75 +369,33 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
     const int64_t p0 = a.link_ptr[k], p1 = a.link_ptr[k + 1];
     const bool tear = kMove && jg >= 0 && p1 == p0;       // a teardown: no new placement, q0 / width / feat unused
     const int c0 = a.q0[k], cw = a.width[k];
-    bool badp = !(p0 >= 0 && p1 > p0 && p1 <= a.n_links) || cw < 1 || c0 < 0 || static_cast<int64_t>(c0) + cw > Q;
-    if (kMove && tear) badp = !(p0 >= 0 && p0 <= a.n_links);
-    if (!badp)
-      for (int64_t e = p0 + lane; e < p1; e += 32) {
-        const int l = a.links[e];
-        badp |= l < 0 || l >= L;
-      }
-    if (__any_sync(kFull, badp)) st |= QOT_CAND_BAD_PATH;
+    if (cd_bad_route(a, a.cfg.L, p0, p1, tear, cw < 1 || c0 < 0 || static_cast<int64_t>(c0) + cw > a.cfg.Q, lane))
+      st |= QOT_CAND_BAD_PATH;
     if (kMove && jg != -1 && !(st & QOT_CAND_BAD_SAMPLE) && (jg < a.node_ptr[s] || jg >= a.node_ptr[s + 1]))
       st |= QOT_CAND_BAD_NODE;
     int64_t n0 = 0;
     int n = 0;
-    if (st == 0) {
-      n0 = a.node_ptr[s];
-      const int64_t n1 = a.node_ptr[s + 1];
-      if (n0 >= 0 && n1 >= n0 && n1 <= a.N && n1 - n0 <= kCdMaxN) n = static_cast<int>(n1 - n0);
-      else st |= QOT_CAND_BAD_STATE;
-    }
+    if (st == 0) st |= cd_sample_nodes(a, s, n0, n) ? 0 : QOT_CAND_BAD_STATE;
     const int jm = kMove && st == 0 && jg >= 0 ? static_cast<int>(jg - n0) : -1;   // sample-local; -1 matches no node
-    // ---- neighbours: chan_node rows of the path's links, the fp64 df test of to_graph.cu
+    // ---- new neighbours, with the moved lightpath's channels free; its old neighbours
     if (lane < kCdMaskWords) {
       ws.mask[lane] = 0u;
       if (kMove) ws.omask[lane] = 0u;
     }
     __syncwarp();
     if (st == 0) {
-      bool occ = false, bad = false;
-      for (int64_t e = p0; e < p1; ++e) {
-        const int32_t* __restrict__ row = a.chan_node + (s * L + a.links[e]) * Q;
-        for (int q = lane; q < Q; q += 32) {
-          const int32_t v = row[q];
-          if (v == -1 || (kMove && v == jg)) continue;            // free, or the moved lightpath's own channel
-          if (q >= c0 && q < c0 + cw) { occ = true; continue; }
-          if (v < -1) continue;                                   // occupied by an unknown lightpath: no edge
-          const int64_t j = v - n0;
-          if (j < 0 || j >= n) { bad = true; continue; }
-          const double fq = a.freqs[q];
-          bool hit = false;
-          for (int c = c0; c < c0 + cw && !hit; ++c) {
-            const double df = fabs(a.freqs[c] - fq);
-            hit = df < thr && df > 0.0;
-          }
-          if (hit) atomicOr(&ws.mask[j >> 5], 1u << (j & 31));
-        }
-      }
-      if (kMove && jm >= 0) {                 // old neighbours: destinations of j's out-run, self loop dropped
-        const int64_t r0 = a.rowptr[n0 + jm], r1 = a.rowptr[n0 + jm + 1];
-        if (!(r0 >= 0 && r1 >= r0 && r1 <= a.E)) bad = true;
-        else
-          for (int64_t e = r0 + lane; e < r1; e += 32) {
-            const int64_t dg = a.edst[e] - n0;
-            if (dg < 0 || dg >= n) bad = true;
-            else if (dg != jm) atomicOr(&ws.omask[dg >> 5], 1u << (dg & 31));
-          }
-      }
-      if (__any_sync(kFull, occ)) st |= QOT_CAND_OCCUPIED;
-      if (__any_sync(kFull, bad)) st |= QOT_CAND_BAD_STATE;
+      int sb = cd_scan(a, s, n0, n, p0, p1, c0, cw, ws.mask, [&](int j) { return kMove && j == jm; }, lane);
+      if (kMove && jm >= 0 && !cd_old_nbrs(a, n0, n, jm, ws.omask, lane)) sb |= QOT_CAND_BAD_STATE;
+      st |= __reduce_or_sync(kFull, sb);
     }
     __syncwarp();
-    if (st & (QOT_CAND_BAD_SAMPLE | QOT_CAND_BAD_PATH | QOT_CAND_OCCUPIED | QOT_CAND_BAD_STATE | QOT_CAND_BAD_NODE)) {
+    if (st & kCdFatal) {
       if (lane < QOT_OUT) a.out[k * QOT_OUT + lane] = nan;
       if (lane == 0) {
         a.status[k] = st;
         a.n_impact[k] = 0;
       }
-      for (int i = lane; i < MI; i += 32) a.impact_node[k * MI + i] = -1;
-      if (kMove && a.impact_kind)
-        for (int i = lane; i < MI; i += 32) a.impact_kind[k * MI + i] = 0;
-      for (int i = lane; i < MI * QOT_OUT; i += 32) a.impact_out[k * MI * QOT_OUT + i] = nan;
+      cd_clear_impact(a, k, 0, a.max_impact, kMove ? a.impact_kind : nullptr, lane, 32);
       continue;
     }
     // ---- neighbours of the new placement ranked ascending: lane t < 8 owns mask word t.  A candidate's impact rows
@@ -298,57 +404,35 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
     int* own = kMove ? ws.msg : ws.nbr;
     const int nn = cd_rank(mw, own, lane);
     if (lane == 0) own[nn] = kCand;                               // the candidate's appended self loop
-    // ---- the candidate's x row [freq, is_lut, mod_order, num_spans, path_len]: min-max in fp64 of the float32
-    // value, then fp32 (dataset.py's scaling; feat_lo / feat_hi in feat's order)
-    if (lane < 4) {
-      const double v = static_cast<double>(a.feat[k * 4 + lane]);
-      ws.cx[lane == 0 ? 0 : lane + 1] =
-          static_cast<float>((v - a.cfg.feat_lo[lane]) / (a.cfg.feat_hi[lane] - a.cfg.feat_lo[lane]));
-    }
-    if (lane == 4) ws.cx[1] = 1.0f;             // to_graph's is_lut of a lightpath with unknown metrics
+    cd_xrow(a, ws.cx, [&] { return a.feat[k * 4 + lane]; }, lane);
     __syncwarp();
     const float* xs = a.x + n0 * kF;
-    // ---- candidate row: neighbours (flag 0), then its self loop (flag 1)
     if (kMove && tear) {
       if (lane < QOT_OUT) a.out[k * QOT_OUT + lane] = nan;
     } else {
-      zc = cd_row(ws, w, zc, own, nn + 1, kCand, CdX{xs, ws.cx, kCand, a.lut_col}, As, Ad, a.out + k * QOT_OUT,
-                  prep, lane);
+      zc = cd_row(ws, zc, own, nn + 1, kCand, CdX{xs, ws.cx, kCand, a.lut_col}, As, Ad, a.out + k * QOT_OUT, flush,
+                  lane);
     }
     int cnt = nn;
     if (kMove) {                             // impact rows of a change: old and new neighbours
       cnt = cd_rank(mw | (lane < kCdMaskWords ? ws.omask[lane] : 0u), ws.nbr, lane);
       __syncwarp();
     }
+    const int MI = a.max_impact;
     if (cnt > MI) st |= QOT_CAND_IMPACT_OVERFLOW;
-    // ---- impact rows: neighbour j's in-row (flag 0), the candidate (flag 0), j's self loop (flag 1)
     const int rows = min(cnt, MI);
     for (int i = 0; i < rows; ++i) {
       const int j = ws.nbr[i];
       const int kind = kMove ? static_cast<int>((ws.omask[j >> 5] >> (j & 31) & 1u) |
                                                 (ws.mask[j >> 5] >> (j & 31) & 1u) << 1)
                              : 2;            // bit 0: was a neighbour of the moved lightpath, bit 1: is one now
-      const int64_t r0 = a.rowptr[n0 + j], r1 = a.rowptr[n0 + j + 1];
       float* dst = a.impact_out + (k * MI + i) * QOT_OUT;
       if (lane == 0) {
         a.impact_node[k * MI + i] = n0 + j;
         if (kMove && a.impact_kind) a.impact_kind[k * MI + i] = static_cast<int8_t>(kind);
       }
-      bool bad = !(r0 >= 0 && r1 >= r0 && r1 <= a.E && r1 - r0 <= kCdMaxN);
-      int m = 0;
-      if (!bad) {
-        for (int64_t eb = r0; eb < r1; eb += 32) {
-          const int64_t e = eb + lane;
-          const int64_t dg = e < r1 ? a.edst[e] - n0 : -1;
-          const bool inside = dg >= 0 && dg < n;
-          bad |= e < r1 && !inside;
-          const bool keep = inside && dg != j && (!kMove || dg != jm);
-          const unsigned ball = __ballot_sync(kFull, keep);
-          if (keep) ws.msg[m + __popc(ball & ((1u << lane) - 1u))] = static_cast<int>(dg);
-          m += __popc(ball);
-        }
-      }
-      if (__any_sync(kFull, bad)) {
+      const int m = cd_in_row(a, n0, n, j, ws.msg, lane, [&](int d) { return kMove && d == jm; });
+      if (m < 0) {
         st |= QOT_CAND_BAD_STATE;
         if (lane < QOT_OUT) dst[lane] = nan;
         __syncwarp();
@@ -360,19 +444,15 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
         ws.msg[m + mc] = j;
       }
       __syncwarp();
-      zc = cd_row(ws, w, zc, ws.msg, m + mc + 1, j, CdX{xs, ws.cx, j, a.lut_col}, As, Ad, dst, prep, lane);
+      zc = cd_row(ws, zc, ws.msg, m + mc + 1, j, CdX{xs, ws.cx, j, a.lut_col}, As, Ad, dst, flush, lane);
     }
-    for (int i = rows + lane; i < MI; i += 32) {
-      a.impact_node[k * MI + i] = -1;
-      if (kMove && a.impact_kind) a.impact_kind[k * MI + i] = 0;
-    }
-    for (int i = rows * QOT_OUT + lane; i < MI * QOT_OUT; i += 32) a.impact_out[k * MI * QOT_OUT + i] = nan;
+    cd_clear_impact(a, k, rows, MI, kMove ? a.impact_kind : nullptr, lane, 32);
     if (lane == 0) {
       a.status[k] = st;
       a.n_impact[k] = cnt;
     }
   }
-  if (zc) cd_flush(w, zc, prep, lane);
+  if (zc) flush(zc);
 }
 
 // ------------------------------------------------------------------------------------------------ change sets
@@ -385,8 +465,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_candidate_kernel(const __gri
 // with the same message order and values: bit-identical to lp_candidate_kernel<true>.
 constexpr int kCsMaxChanges = QOT_SET_MAX_CHANGES;
 constexpr int kCsMsgCap = kCdMaxN + kCsMaxChanges + 8;  // in-row (<= kCdMaxN) + changed lightpaths + self loop
-constexpr int kCsFatal = QOT_CAND_BAD_SAMPLE | QOT_CAND_BAD_PATH | QOT_CAND_OCCUPIED | QOT_CAND_BAD_STATE |
-                         QOT_CAND_BAD_NODE | QOT_SET_BAD_SET | QOT_SET_DUPLICATE | QOT_SET_CONFLICT;
+constexpr int kCsFatal = kCdFatal | QOT_SET_BAD_SET | QOT_SET_DUPLICATE | QOT_SET_CONFLICT;
 static_assert(kCsMaxChanges == 64, "the pairwise matrix and the per-set bit words hold 64 changes");
 
 struct CsWarpSmem {
@@ -399,7 +478,7 @@ struct CsWarpSmem {
   unsigned rmask[kCdMaskWords];                 // R: the lightpaths the set moves or tears down
   unsigned char tear[kCsMaxChanges];            // the change is a teardown
   long long k0, n0;                             // the set's first change and its sample's first node
-  int nc, cnt, any;                             // changes, impact rows, OR of the status words
+  int nc, n, cnt, any;                          // changes, the sample's nodes, impact rows, OR of the status words
 };
 struct CsSmem {
   CdSmem cd;                                    // head fragments and the candidate kernel's per-warp state
@@ -434,8 +513,8 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   CdWarpSmem& ws = sm.cd.w[w];
   CsWarpSmem& xw = sm.w[w];
-  for (int i = tid; i < kStHeadFrag4; i += kCdThreads)
-    sm.cd.frag[i] = __ldg(reinterpret_cast<const float4*>(a.prep + kOffB1f) + i);
+  float As[kF], Ad[kF];
+  cd_head_prologue(a.prep, As, Ad, tid);
   // set_ptr must partition [0, K): non-decreasing from 0 to K.  Otherwise sets could overlap, so none is evaluated:
   // every change and every set gets BAD_SET, each output written by exactly one thread of the grid.
   bool bad_ptr = false;
@@ -444,7 +523,6 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
     bad_ptr |= (g == 0 && v != 0) || (g == ca.G && v != a.K) || (g < ca.G && ca.set_ptr[g + 1] < v);
   }
   bad_ptr = __syncthreads_or(bad_ptr);
-  const float* __restrict__ prep = a.prep;
   const float nan = __int_as_float(0x7fc00000);
   if (bad_ptr) {
     const int64_t gt = static_cast<int64_t>(blockIdx.x) * kCdThreads + tid;
@@ -456,22 +534,11 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
     for (int64_t g = gt; g < ca.G; g += gs) {
       a.status[g] = QOT_SET_BAD_SET;
       a.n_impact[g] = 0;
-      for (int i = 0; i < a.max_impact; ++i) {
-        a.impact_node[g * a.max_impact + i] = -1;
-        if (a.impact_kind) a.impact_kind[g * a.max_impact + i] = 0;
-        for (int o = 0; o < QOT_OUT; ++o) a.impact_out[(g * a.max_impact + i) * QOT_OUT + o] = nan;
-      }
+      cd_clear_impact(a, g, 0, a.max_impact, a.impact_kind, 0, 1);
     }
     return;
   }
-  const int h = lane & 3;
-  float As[kF], Ad[kF];
-#pragma unroll
-  for (int k = 0; k < kF; ++k) {
-    As[k] = __ldg(prep + kOffAsrc + k * kHeads + h);
-    Ad[k] = __ldg(prep + kOffAdst + k * kHeads + h);
-  }
-  // L, Q, the threshold and max_impact are read from the kernel parameters where used: hoisted, they spill
+  const auto flush = [&](int cnt) { cd_flush(w, cnt, a.prep, lane); };
   int zc = 0;                                       // rows staged in this warp's head buffer
   for (int64_t g = static_cast<int64_t>(blockIdx.x) * kCdWarps + w; g < ca.G;
        g += static_cast<int64_t>(gridDim.x) * kCdWarps) {
@@ -480,13 +547,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
     const int64_t s = nc ? a.sample[k0] : -1;
     int64_t n0 = 0;
     int n = 0;
-    bool state_ok = s >= 0 && s < a.S;
-    if (state_ok) {
-      n0 = a.node_ptr[s];
-      const int64_t n1 = a.node_ptr[s + 1];
-      if (n0 >= 0 && n1 >= n0 && n1 <= a.N && n1 - n0 <= kCdMaxN) n = static_cast<int>(n1 - n0);
-      else state_ok = false;
-    }
+    const bool state_ok = s >= 0 && s < a.S && cd_sample_nodes(a, s, n0, n);
     if (lane < kCdMaskWords) {
       xw.rmask[lane] = 0u;
       ws.mask[lane] = 0u;
@@ -504,15 +565,8 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
       const int64_t p0 = a.link_ptr[k], p1 = a.link_ptr[k + 1];
       const bool tear = jg >= 0 && p1 == p0;        // a teardown: no new placement, q0 / width / feat unused
       const int c0 = a.q0[k], cw = a.width[k];
-      bool badp = tear ? !(p0 >= 0 && p0 <= a.n_links)
-                       : !(p0 >= 0 && p1 > p0 && p1 <= a.n_links) || cw < 1 || c0 < 0 ||
-                             static_cast<int64_t>(c0) + cw > a.cfg.Q;
-      if (!badp)
-        for (int64_t e = p0 + lane; e < p1; e += 32) {
-          const int l = a.links[e];
-          badp |= l < 0 || l >= a.cfg.L;
-        }
-      if (__any_sync(kFull, badp)) st |= QOT_CAND_BAD_PATH;
+      if (cd_bad_route(a, a.cfg.L, p0, p1, tear, cw < 1 || c0 < 0 || static_cast<int64_t>(c0) + cw > a.cfg.Q, lane))
+        st |= QOT_CAND_BAD_PATH;
       if (jg != -1 && !(st & QOT_CAND_BAD_SAMPLE) && (jg < a.node_ptr[sk] || jg >= a.node_ptr[sk + 1]))
         st |= QOT_CAND_BAD_NODE;
       if (st == 0 && !state_ok) st |= QOT_CAND_BAD_STATE;
@@ -527,13 +581,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
         xw.tear[c] = tear;
       }
       if (lane < kCdMaskWords) xw.nmask[c][lane] = 0u;
-      // x row [freq, is_lut, mod_order, num_spans, path_len]: dataset.py's scaling, as the candidate kernel
-      if (lane < 4) {
-        const double v = static_cast<double>(a.feat[k * 4 + lane]);
-        xw.cx[c][lane == 0 ? 0 : lane + 1] =
-            static_cast<float>((v - a.cfg.feat_lo[lane]) / (a.cfg.feat_hi[lane] - a.cfg.feat_lo[lane]));
-      }
-      if (lane == 4) xw.cx[c][1] = 1.0f;
+      cd_xrow(a, xw.cx[c], [&] { return a.feat[k * 4 + lane]; }, lane);
       __syncwarp();
     }
     if (lane == 0)                                  // every change removing a lightpath removed twice
@@ -549,48 +597,19 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
       for (int c = 0; c < nc; ++c) {
         if (xw.tear[c]) continue;
         const int64_t k = k0 + c;
-        const int64_t p0 = a.link_ptr[k], p1 = a.link_ptr[k + 1];
-        const int c0 = a.q0[k], cw = a.width[k];
-        bool occ = false, bad = false;
-        for (int64_t e = p0; e < p1; ++e) {
-          const int32_t* __restrict__ row = a.chan_node + (s * a.cfg.L + a.links[e]) * a.cfg.Q;
-          for (int q = lane; q < a.cfg.Q; q += 32) {
-            const int32_t v = row[q];
-            if (v == -1) continue;
-            const int64_t j = v - n0;
-            const bool inside = v >= 0 && j >= 0 && j < n;
-            if (inside && cs_bit(xw.rmask, static_cast<int>(j))) continue;
-            if (q >= c0 && q < c0 + cw) { occ = true; continue; }
-            if (v < -1) continue;                   // occupied by an unknown lightpath: no edge
-            if (!inside) { bad = true; continue; }
-            const double fq = a.freqs[q];
-            bool hit = false;
-            for (int cc = c0; cc < c0 + cw && !hit; ++cc) {
-              const double df = fabs(a.freqs[cc] - fq);
-              hit = df < a.cfg.freq_threshold && df > 0.0;
-            }
-            if (hit) atomicOr(&xw.nmask[c][j >> 5], 1u << (j & 31));
-          }
-        }
-        const bool o = __any_sync(kFull, occ), b = __any_sync(kFull, bad);
-        if (lane == 0) xw.st[c] |= (o ? QOT_CAND_OCCUPIED : 0) | (b ? QOT_CAND_BAD_STATE : 0);
+        const int sb = cd_scan(a, s, n0, n, a.link_ptr[k], a.link_ptr[k + 1], a.q0[k], a.width[k], xw.nmask[c],
+                               [&](int j) { return cs_bit(xw.rmask, j); }, lane);
+        const int sw = __reduce_or_sync(kFull, sb);
+        if (lane == 0) xw.st[c] |= sw;
       }
       // ---- old neighbours: the destinations of R's out-runs, self loops dropped
       for (int c = 0; c < nc; ++c) {
         const int jm = xw.jm[c];
         if (jm < 0) continue;
-        const int64_t r0 = a.rowptr[n0 + jm], r1 = a.rowptr[n0 + jm + 1];
-        bool bad = !(r0 >= 0 && r1 >= r0 && r1 <= a.E);
-        if (!bad)
-          for (int64_t e = r0 + lane; e < r1; e += 32) {
-            const int64_t dg = a.edst[e] - n0;
-            if (dg < 0 || dg >= n) bad = true;
-            else if (dg != jm) atomicOr(&ws.omask[dg >> 5], 1u << (dg & 31));
-          }
-        if (__any_sync(kFull, bad) && lane == 0) xw.st[c] |= QOT_CAND_BAD_STATE;
+        if (__any_sync(kFull, !cd_old_nbrs(a, n0, n, jm, ws.omask, lane)) && lane == 0) xw.st[c] |= QOT_CAND_BAD_STATE;
       }
       // ---- pairs of placed changes, one lane per pair: a shared link and a shared slot is a conflict, a shared link
-      // and 0 < |df| < threshold (to_graph's test on the grid) an edge
+      // and cd_df_hit between the two slot ranges an edge
       for (int c = lane; c < nc; c += 32) xw.adj[c] = 0ull;
       __syncwarp();
       for (int pr = lane; pr < nc * nc; pr += 32) {
@@ -608,11 +627,8 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
           continue;
         }
         bool hit = false;
-        for (int qc = c0; qc < c0 + cw && !hit; ++qc)
-          for (int qd = d0; qd < d0 + dw && !hit; ++qd) {
-            const double df = fabs(a.freqs[qc] - a.freqs[qd]);
-            hit = df < a.cfg.freq_threshold && df > 0.0;
-          }
+        for (int qd = d0; qd < d0 + dw && !hit; ++qd)
+          hit = cd_df_hit(a.freqs, a.freqs[qd], c0, cw, a.cfg.freq_threshold);
         if (hit) {
           atomicOr(&xw.adj[c], 1ull << d);
           atomicOr(&xw.adj[d], 1ull << c);
@@ -637,15 +653,9 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
       cnt = cd_rank(uw, ws.nbr, lane);
       __syncwarp();
       bool bad = false;
-      for (int i = 0; i < min(cnt, a.max_impact); ++i) {
-        const int64_t r0 = a.rowptr[n0 + ws.nbr[i]], r1 = a.rowptr[n0 + ws.nbr[i] + 1];
-        if (!(r0 >= 0 && r1 >= r0 && r1 <= a.E && r1 - r0 <= kCdMaxN)) { bad = true; break; }
-        for (int64_t e = r0 + lane; e < r1; e += 32) {
-          const int64_t dg = a.edst[e] - n0;
-          bad |= dg < 0 || dg >= n;
-        }
-      }
-      if (__any_sync(kFull, bad)) {
+      for (int i = 0; i < min(cnt, a.max_impact) && !bad; ++i)
+        bad = cd_in_row<false>(a, n0, n, ws.nbr[i], nullptr, lane) < 0;
+      if (bad) {
         if (lane == 0) xw.st[0] |= QOT_CAND_BAD_STATE;
         any |= QOT_CAND_BAD_STATE;
       }
@@ -663,11 +673,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
         a.status[g] = any;
         a.n_impact[g] = 0;
       }
-      for (int i = lane; i < a.max_impact; i += 32) {
-        a.impact_node[g * a.max_impact + i] = -1;
-        if (a.impact_kind) a.impact_kind[g * a.max_impact + i] = 0;
-      }
-      for (int i = lane; i < a.max_impact * QOT_OUT; i += 32) a.impact_out[g * a.max_impact * QOT_OUT + i] = nan;
+      cd_clear_impact(a, g, 0, a.max_impact, a.impact_kind, lane, 32);
       __syncwarp();
       continue;
     }
@@ -678,6 +684,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
       xw.k0 = k0;
       xw.n0 = n0;
       xw.nc = nc;
+      xw.n = n;
       xw.cnt = cnt;
       xw.any = any;
     }
@@ -700,22 +707,14 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
         }
         m = __shfl_sync(kFull, m, 0);
         q = -1 - r;
-      } else {                                      // impact row i = r - nc
+      } else {                                      // impact row i = r - nc (its in-row was checked above)
         const int i = r - ncr, j = ws.nbr[i];
         const int kind = static_cast<int>(cs_bit(ws.omask, j)) | static_cast<int>(cs_bit(ws.mask, j)) << 1;
-        const int64_t r0 = a.rowptr[n0r + j], r1 = a.rowptr[n0r + j + 1];
         if (lane == 0) {
           a.impact_node[g * a.max_impact + i] = n0r + j;
           if (a.impact_kind) a.impact_kind[g * a.max_impact + i] = static_cast<int8_t>(kind);
         }
-        for (int64_t eb = r0; eb < r1; eb += 32) {
-          const int64_t e = eb + lane;
-          const int dg = e < r1 ? static_cast<int>(a.edst[e] - n0r) : -1;
-          const bool keep = dg >= 0 && dg != j && !cs_bit(xw.rmask, dg);
-          const unsigned ball = __ballot_sync(kFull, keep);
-          if (keep) xw.msg[m + __popc(ball & ((1u << lane) - 1u))] = dg;
-          m += __popc(ball);
-        }
+        m = cd_in_row(a, n0r, xw.n, j, xw.msg, lane, [&](int d) { return cs_bit(xw.rmask, d); });
         if (kind >> 1)
           for (int cb = 0; cb < ncr; cb += 32) {
             const int c = cb + lane;
@@ -730,15 +729,9 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
         dst = a.impact_out + (g * a.max_impact + i) * QOT_OUT;
       }
       __syncwarp();
-      zc = cd_row(ws, w, zc, xw.msg, m, q, CsX{a.x + n0r * kF, xw.cx, q, a.lut_col}, As, Ad, dst, prep, lane);
+      zc = cd_row(ws, zc, xw.msg, m, q, CsX{a.x + n0r * kF, xw.cx, q, a.lut_col}, As, Ad, dst, flush, lane);
     }
-    const int rows = min(xw.cnt, a.max_impact);
-    for (int i = rows + lane; i < a.max_impact; i += 32) {
-      a.impact_node[g * a.max_impact + i] = -1;
-      if (a.impact_kind) a.impact_kind[g * a.max_impact + i] = 0;
-    }
-    for (int i = rows * QOT_OUT + lane; i < a.max_impact * QOT_OUT; i += 32)
-      a.impact_out[g * a.max_impact * QOT_OUT + i] = nan;
+    cd_clear_impact(a, g, min(xw.cnt, a.max_impact), a.max_impact, a.impact_kind, lane, 32);
     for (int c = lane; c < xw.nc; c += 32) ca.chg_status[xw.k0 + c] = xw.st[c];
     if (lane == 0) {
       a.status[g] = xw.any;
@@ -746,7 +739,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_change_set_kernel(const __gr
     }
     __syncwarp();
   }
-  if (zc) cd_flush(w, zc, prep, lane);
+  if (zc) flush(zc);
 }
 
 // ------------------------------------------------------------------------------------------------ placements
@@ -872,69 +865,15 @@ __device__ __noinline__ void pl_flush(const PlArgs& a, PlWarpSmem& pw, int w, in
   __syncwarp();
 }
 
-// cd_row with the row's destination, ring slot and bound index recorded for pl_fold
-template <typename XF>
-__device__ __forceinline__ int pl_row(const PlArgs& a, CdWarpSmem& ws, PlWarpSmem& pw, int w, int zc, const int* msg,
-                                      int M, int q, const XF& xf, const float (&As)[kF], const float (&Ad)[kF],
-                                      float* dst, int tag, long long node, int64_t o0, int lane) {
-  float d_q = 0.f;
-#pragma unroll
-  for (int k = 0; k < kF; ++k) d_q = fmaf(xf(q, k), Ad[k], d_q);
-  AttnState st;
-  attn_consume(st, msg, M, xf, As, d_q, lane);
-  attn_finish<kF>(st, ws.z + zc * kCdZPitch, lane);
-  if (lane == 0) {
-    ws.orow[zc] = reinterpret_cast<long long>(dst ? dst : pw.rout[zc]);
-    pw.rtag[zc] = tag;
-    pw.rnode[zc] = node;
-  }
-  __syncwarp();
-  if (++zc == 16) {
-    pl_flush(a, pw, w, 16, o0, lane);
-    zc = 0;
-  }
-  return zc;
-}
-
-// neighbours of placement [q0, q0 + cw) on a route, from the route's chan_node rows (the candidate kernel's scan; the
-// placement's own channels are free) into ws.mask
-__device__ __forceinline__ void pl_scan_mask(const CdArgs& a, CdWarpSmem& ws, int64_t s, int64_t n0, int64_t p0,
-                                             int64_t p1, int q0, int cw, int lane) {
-  const int Q = a.cfg.Q;
-  for (int64_t e = p0; e < p1; ++e) {
-    const int32_t* __restrict__ row = a.chan_node + (s * a.cfg.L + a.links[e]) * Q;
-    for (int q = lane; q < Q; q += 32) {
-      const int32_t v = row[q];
-      if (v < 0) continue;                                  // free, or occupied by an unknown lightpath
-      const int j = static_cast<int>(v - n0);               // inside the sample: checked when the route was read
-      const double fq = a.freqs[q];
-      bool hit = false;
-      for (int c = q0; c < q0 + cw && !hit; ++c) {
-        const double df = fabs(a.freqs[c] - fq);
-        hit = df < a.cfg.freq_threshold && df > 0.0;
-      }
-      if (hit) atomicOr(&ws.mask[j >> 5], 1u << (j & 31));
-    }
-  }
-}
-
 __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __grid_constant__ PlArgs pa) {
   const CdArgs& a = pa.c;
   PlSmem& sm = *reinterpret_cast<PlSmem*>(cd_smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   CdWarpSmem& ws = sm.cd.w[w];
   PlWarpSmem& pw = sm.w[w];
-  for (int i = tid; i < kStHeadFrag4; i += kCdThreads)
-    sm.cd.frag[i] = __ldg(reinterpret_cast<const float4*>(a.prep + kOffB1f) + i);
-  __syncthreads();
-  const float* __restrict__ prep = a.prep;
-  const int h = lane & 3;
   float As[kF], Ad[kF];
-#pragma unroll
-  for (int k = 0; k < kF; ++k) {
-    As[k] = __ldg(prep + kOffAsrc + k * kHeads + h);
-    Ad[k] = __ldg(prep + kOffAdst + k * kHeads + h);
-  }
+  cd_head_prologue(a.prep, As, Ad, tid);
+  __syncthreads();
   const float nan = __int_as_float(0x7fc00000);
   int zc = 0;                                             // rows staged in this warp's head buffer
   for (int64_t d = static_cast<int64_t>(blockIdx.x) * kCdWarps + w; d < a.K;
@@ -949,31 +888,29 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
     bool badp = !opts_ok;
     if (opts_ok)
       for (int64_t po = o0; po < o1 && !badp; ++po) {
-        const int64_t p0 = a.link_ptr[po], p1 = a.link_ptr[po + 1];
         const int cw = a.width[po];
-        bool b = !(p0 >= 0 && p1 > p0 && p1 <= a.n_links) || cw < 1 || cw > Q;
-        if (!b)
-          for (int64_t e = p0 + lane; e < p1; e += 32) {
-            const int l = a.links[e];
-            b |= l < 0 || l >= L;
-          }
-        badp = __any_sync(kFull, b);
+        badp = cd_bad_route(a, L, a.link_ptr[po], a.link_ptr[po + 1], false, cw < 1 || cw > Q, lane);
       }
     if (badp) st |= QOT_CAND_BAD_PATH;
     int64_t n0 = 0;
     int n = 0;
-    if (st == 0) {
-      n0 = a.node_ptr[s];
-      const int64_t n1 = a.node_ptr[s + 1];
-      if (n0 >= 0 && n1 >= n0 && n1 <= a.N && n1 - n0 <= kCdMaxN) n = static_cast<int>(n1 - n0);
-      else st |= QOT_CAND_BAD_STATE;
-    }
+    if (st == 0) st |= cd_sample_nodes(a, s, n0, n) ? 0 : QOT_CAND_BAD_STATE;
     if (lane == 0) {
       pw.key = 0ull;
       pw.n_free = pw.n_feas = 0;
     }
     __syncwarp();
     const float* xs = a.x + n0 * kF;
+    // a row of the search (ring slot `tag`, bound index `node`, -1 for an own row; its outputs staged for pl_fold) or
+    // of the winner (tag -1, its outputs to dst)
+    const auto row = [&](const int* msg, int M, int q, float* dst, int tag, long long node) {
+      if (lane == 0) {
+        pw.rtag[zc] = tag;
+        pw.rnode[zc] = node;
+      }
+      zc = cd_row(ws, zc, msg, M, q, CdX{xs, ws.cx, q, a.lut_col}, As, Ad, dst ? dst : pw.rout[zc],
+                  [&](int cnt) { pl_flush(pa, pw, w, cnt, o0, lane); }, lane);
+    };
     int seq = 0;                                          // placements of this demand, for the ring slots
     for (int64_t po = o0; st == 0 && po < o1; ++po) {
       const int64_t p0 = a.link_ptr[po], p1 = a.link_ptr[po + 1];
@@ -983,10 +920,10 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
       int ne = 0;
       bool bad = false;
       for (int64_t e = p0; e < p1; ++e) {
-        const int32_t* __restrict__ row = a.chan_node + (s * L + a.links[e]) * Q;
+        const int32_t* __restrict__ crow = a.chan_node + (s * L + a.links[e]) * Q;
         for (int qb = 0; qb < Q; qb += 32) {
           const int q = qb + lane;
-          const int32_t v = q < Q ? row[q] : -1;
+          const int32_t v = q < Q ? crow[q] : -1;
           const unsigned ob = __ballot_sync(kFull, v != -1);
           if (lane == qb >> 5) occ |= ob;
           const int64_t j = static_cast<int64_t>(v) - n0;
@@ -1022,7 +959,8 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
           pa.all_margin[at] = nan;
           for (int o = 0; o < QOT_OUT; ++o) pa.all_out[at * QOT_OUT + o] = nan;
         }
-      // ---- every free start in ascending order
+      // ---- every free start in ascending order; its neighbours from the collected entries (the placement's own
+      // channels are free), or from the chan_node rows again when the route held more than kPlEntCap of them
       for (int wd = 0; wd < 32 && 32 * wd < Q; ++wd) {
         for (unsigned bits = __shfl_sync(kFull, run, wd); bits; bits &= bits - 1u) {
           const int q0 = 32 * wd + __ffs(bits) - 1;
@@ -1031,27 +969,16 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
           if (ne <= kPlEntCap) {
             for (int i = lane; i < ne; i += 32) {
               const int en = pw.ent[i], q = en >> 8, j = en & 255;
-              const double fq = a.freqs[q];
-              bool hit = false;
-              for (int c = q0; c < q0 + cw && !hit; ++c) {
-                const double df = fabs(a.freqs[c] - fq);
-                hit = df < a.cfg.freq_threshold && df > 0.0;
-              }
-              if (hit) atomicOr(&ws.mask[j >> 5], 1u << (j & 31));
+              if (cd_df_hit(a.freqs, a.freqs[q], q0, cw, a.cfg.freq_threshold))
+                atomicOr(&ws.mask[j >> 5], 1u << (j & 31));
             }
           } else {
-            pl_scan_mask(a, ws, s, n0, p0, p1, q0, cw, lane);
+            cd_scan(a, s, n0, n, p0, p1, q0, cw, ws.mask, CdNone(), lane);
           }
           __syncwarp();
           const int nn = cd_rank(lane < kCdMaskWords ? ws.mask[lane] : 0u, ws.nbr, lane);
-          // x row of the placement: (float32(freqs[q0]), the option's features), scaled as the candidate kernel does
-          if (lane < 4) {
-            const double v = lane == 0 ? static_cast<double>(static_cast<float>(a.freqs[q0]))
-                                       : static_cast<double>(a.feat[po * 3 + lane - 1]);
-            ws.cx[lane == 0 ? 0 : lane + 1] =
-                static_cast<float>((v - a.cfg.feat_lo[lane]) / (a.cfg.feat_hi[lane] - a.cfg.feat_lo[lane]));
-          }
-          if (lane == 4) ws.cx[1] = 1.0f;
+          cd_xrow(a, ws.cx, [&] { return lane == 0 ? static_cast<float>(a.freqs[q0]) : a.feat[po * 3 + lane - 1]; },
+                  lane);
           const int slot = seq++ & (kPlRing - 1);
           const int nimp = pa.bound ? nn : 0;             // impact rows count against a bound, all of them
           if (lane == 0) {
@@ -1064,25 +991,11 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
             ++pw.n_free;
           }
           __syncwarp();
-          zc = pl_row(pa, ws, pw, w, zc, ws.nbr, nn + 1, kCand, CdX{xs, ws.cx, kCand, a.lut_col}, As, Ad, nullptr,
-                      slot, -1, o0, lane);
+          row(ws.nbr, nn + 1, kCand, nullptr, slot, -1);
           for (int i = 0; i < nimp; ++i) {                // whatever max_impact is
             const int j = ws.nbr[i];
-            const int64_t r0 = a.rowptr[n0 + j], r1 = a.rowptr[n0 + j + 1];
-            bool rb = !(r0 >= 0 && r1 >= r0 && r1 <= a.E && r1 - r0 <= kCdMaxN);
-            int m = 0;
-            if (!rb)
-              for (int64_t eb = r0; eb < r1; eb += 32) {
-                const int64_t e = eb + lane;
-                const int64_t dg = e < r1 ? a.edst[e] - n0 : -1;
-                const bool inside = dg >= 0 && dg < n;
-                rb |= e < r1 && !inside;
-                const bool keep = inside && dg != j;
-                const unsigned ball = __ballot_sync(kFull, keep);
-                if (keep) ws.msg[m + __popc(ball & ((1u << lane) - 1u))] = static_cast<int>(dg);
-                m += __popc(ball);
-              }
-            if (__any_sync(kFull, rb)) {
+            const int m = cd_in_row(a, n0, n, j, ws.msg, lane);
+            if (m < 0) {
               st |= QOT_CAND_BAD_STATE;
               break;
             }
@@ -1091,8 +1004,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
               ws.msg[m + 1] = j;
             }
             __syncwarp();
-            zc = pl_row(pa, ws, pw, w, zc, ws.msg, m + 2, j, CdX{xs, ws.cx, j, a.lut_col}, As, Ad, nullptr, slot,
-                        n0 + j, o0, lane);
+            row(ws.msg, m + 2, j, nullptr, slot, n0 + j);
           }
           if (st) break;
         }
@@ -1107,40 +1019,23 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
     const int MI = a.max_impact;
     const unsigned long long key = pw.key;
     int cnt = 0, rows = 0, bp = -1, bq = -1;
-    int64_t wp0 = 0, wp1 = 0;
     if (st == 0 && key) {
       const unsigned idx = 0xffffffffu - static_cast<unsigned>(key);
       bp = static_cast<int>(idx >> 10);
       bq = static_cast<int>(idx & 1023u);
       const int64_t po = o0 + bp;
-      wp0 = a.link_ptr[po];
-      wp1 = a.link_ptr[po + 1];
-      const int cw = a.width[po];
       if (lane < kCdMaskWords) ws.mask[lane] = 0u;
       __syncwarp();
-      pl_scan_mask(a, ws, s, n0, wp0, wp1, bq, cw, lane);
+      cd_scan(a, s, n0, n, a.link_ptr[po], a.link_ptr[po + 1], bq, a.width[po], ws.mask, CdNone(), lane);
       __syncwarp();
       cnt = cd_rank(lane < kCdMaskWords ? ws.mask[lane] : 0u, ws.nbr, lane);
       __syncwarp();
       rows = min(cnt, MI);
       bool bad = false;                                   // in-rows checked before any row is written
-      for (int i = 0; i < rows && !bad; ++i) {
-        const int64_t r0 = a.rowptr[n0 + ws.nbr[i]], r1 = a.rowptr[n0 + ws.nbr[i] + 1];
-        if (!(r0 >= 0 && r1 >= r0 && r1 <= a.E && r1 - r0 <= kCdMaxN)) { bad = true; break; }
-        for (int64_t e = r0 + lane; e < r1; e += 32) {
-          const int64_t dg = a.edst[e] - n0;
-          bad |= dg < 0 || dg >= n;
-        }
-        bad = __any_sync(kFull, bad);
-      }
-      if (__any_sync(kFull, bad)) st |= QOT_CAND_BAD_STATE;
-      if (lane < 4) {
-        const double v = lane == 0 ? static_cast<double>(static_cast<float>(a.freqs[bq]))
-                                   : static_cast<double>(a.feat[po * 3 + lane - 1]);
-        ws.cx[lane == 0 ? 0 : lane + 1] =
-            static_cast<float>((v - a.cfg.feat_lo[lane]) / (a.cfg.feat_hi[lane] - a.cfg.feat_lo[lane]));
-      }
-      if (lane == 4) ws.cx[1] = 1.0f;
+      for (int i = 0; i < rows && !bad; ++i) bad = cd_in_row<false>(a, n0, n, ws.nbr[i], nullptr, lane) < 0;
+      if (bad) st |= QOT_CAND_BAD_STATE;
+      cd_xrow(a, ws.cx, [&] { return lane == 0 ? static_cast<float>(a.freqs[bq]) : a.feat[po * 3 + lane - 1]; },
+              lane);
       __syncwarp();
     }
     if (st & kPlFatal) {
@@ -1152,8 +1047,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
         pa.margin[d] = nan;
         pa.n_free[d] = pa.n_feasible[d] = 0;
       }
-      for (int i = lane; i < MI; i += 32) a.impact_node[d * MI + i] = -1;
-      for (int i = lane; i < MI * QOT_OUT; i += 32) a.impact_out[d * MI * QOT_OUT + i] = nan;
+      cd_clear_impact(a, d, 0, MI, nullptr, lane, 32);
       if (pa.all_out && opts_ok)
         for (int64_t i = o0 * Q + lane; i < o1 * Q; i += 32) {
           pa.all_margin[i] = nan;
@@ -1162,30 +1056,19 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
       __syncwarp();
       continue;
     }
-    // ---- the winner's impact rows: its neighbour j's in-row (flag 0), the placement (flag 0), j's self loop (flag 1)
+    // ---- the winner's impact rows (their in-rows were checked above)
     for (int i = 0; i < rows; ++i) {
       const int j = ws.nbr[i];
-      const int64_t r0 = a.rowptr[n0 + j], r1 = a.rowptr[n0 + j + 1];
       if (lane == 0) a.impact_node[d * MI + i] = n0 + j;
-      int m = 0;
-      for (int64_t eb = r0; eb < r1; eb += 32) {
-        const int64_t e = eb + lane;
-        const int64_t dg = e < r1 ? a.edst[e] - n0 : -1;
-        const bool keep = dg >= 0 && dg != j;
-        const unsigned ball = __ballot_sync(kFull, keep);
-        if (keep) ws.msg[m + __popc(ball & ((1u << lane) - 1u))] = static_cast<int>(dg);
-        m += __popc(ball);
-      }
+      const int m = cd_in_row(a, n0, n, j, ws.msg, lane);
       if (lane == 0) {
         ws.msg[m] = kCand;
         ws.msg[m + 1] = j;
       }
       __syncwarp();
-      zc = pl_row(pa, ws, pw, w, zc, ws.msg, m + 2, j, CdX{xs, ws.cx, j, a.lut_col}, As, Ad,
-                  a.impact_out + (d * MI + i) * QOT_OUT, -1, -1, o0, lane);
+      row(ws.msg, m + 2, j, a.impact_out + (d * MI + i) * QOT_OUT, -1, -1);
     }
-    for (int i = rows + lane; i < MI; i += 32) a.impact_node[d * MI + i] = -1;
-    for (int i = rows * QOT_OUT + lane; i < MI * QOT_OUT; i += 32) a.impact_out[d * MI * QOT_OUT + i] = nan;
+    cd_clear_impact(a, d, rows, MI, nullptr, lane, 32);
     if (lane < QOT_OUT) a.out[d * QOT_OUT + lane] = key ? pw.best[lane] : nan;
     if (lane == 0) {
       a.status[d] = st | (cnt > MI ? QOT_CAND_IMPACT_OVERFLOW : 0);
@@ -1209,7 +1092,44 @@ static int cfg_check(const qot_lp_graph_cfg_t* cfg, const char* who) {
   return QOT_OK;
 }
 
-// shared by both entry points: argument checks, the once-per-device shared-memory opt-in, the launch
+// the checks every network-state entry point makes first: cfg, the sizes (sizes_ok), the head's table, the flag column
+static int cd_check_args(const char* who, const qot_lp_graph_cfg_t* cfg, bool sizes_ok, const float* prepared,
+                         int32_t is_lut_index) {
+  if (int rc = cfg_check(cfg, who)) return rc;
+  QOT_REQUIRE(sizes_ok, "%s: bad size", who);
+  QOT_REQUIRE(prepared && (reinterpret_cast<uintptr_t>(prepared) & 15) == 0, "%s: prepared must be 16-byte aligned",
+              who);
+  QOT_REQUIRE(is_lut_index >= 0 && is_lut_index < kF, "%s: is_lut_index out of range", who);
+  return QOT_OK;
+}
+
+// the opt-in to kSmem bytes of dynamic shared memory, once per device and kernel
+template <auto kKernel, int kSmem>
+static int cd_smem_opt_in() {
+  static std::atomic<unsigned long long> done{0};
+  return once_per_device(done, [] {
+    QOT_CUDA(cudaFuncSetAttribute(kKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem));
+    return static_cast<int>(QOT_OK);
+  });
+}
+
+// the state half of CdArgs (with the head's table and the output width), after the null-state check
+static int cd_state_args(const char* who, CdArgs& a, const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs,
+                         const float* x, const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index,
+                         int64_t N, int64_t E, const int32_t* chan_node, const float* prepared, int32_t is_lut_index,
+                         int32_t max_impact) {
+  QOT_REQUIRE(S == 0 || (freqs && x && node_ptr && rowptr && chan_node && (E == 0 || edge_index)),
+              "%s: null state array", who);
+  a.cfg = *cfg;
+  a.S = S; a.N = N; a.E = E;
+  a.freqs = freqs; a.x = x; a.node_ptr = node_ptr; a.rowptr = rowptr;
+  a.edst = edge_index ? edge_index + E : nullptr;
+  a.chan_node = chan_node;
+  a.prep = prepared; a.lut_col = is_lut_index; a.max_impact = max_impact;
+  return QOT_OK;
+}
+
+// qot_lightpath_candidates (kMove = false) and qot_lightpath_reconfigure (kMove = true)
 template <bool kMove>
 static int cd_launch(const char* who, const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
                      const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N, int64_t E,
@@ -1218,34 +1138,22 @@ static int cd_launch(const char* who, const qot_lp_graph_cfg_t* cfg, int64_t S, 
                      const int32_t* width, const float* feat, const float* prepared, int32_t is_lut_index,
                      int32_t max_impact, float* out, int32_t* status, int32_t* n_impact, int64_t* impact_node,
                      int8_t* impact_kind, float* impact_out, cudaStream_t stream) {
-  if (int rc = cfg_check(cfg, who)) return rc;
-  QOT_REQUIRE(S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && K >= 0 && n_links >= 0 && max_impact >= 0,
-              "%s: bad size", who);
-  QOT_REQUIRE(prepared && (reinterpret_cast<uintptr_t>(prepared) & 15) == 0, "%s: prepared must be 16-byte aligned",
-              who);
-  QOT_REQUIRE(is_lut_index >= 0 && is_lut_index < kF, "%s: is_lut_index out of range", who);
+  if (int rc = cd_check_args(who, cfg, S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && K >= 0 && n_links >= 0 &&
+                                           max_impact >= 0, prepared, is_lut_index))
+    return rc;
   if (K == 0) return QOT_OK;
   QOT_REQUIRE(sample && link_ptr && q0 && width && feat && out && status && n_impact && (n_links == 0 || links) &&
                   (max_impact == 0 || (impact_node && impact_out)) && (!kMove || node),
               "%s: null candidate or output array", who);
-  QOT_REQUIRE(S == 0 || (freqs && x && node_ptr && rowptr && chan_node && (E == 0 || edge_index)),
-              "%s: null state array", who);
-  static std::atomic<unsigned long long> done{0};
-  constexpr int smem = static_cast<int>(sizeof(CdSmem));
-  if (int rc = once_per_device(done, [] {
-        QOT_CUDA(cudaFuncSetAttribute(lp_candidate_kernel<kMove>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        return static_cast<int>(QOT_OK);
-      }))
-    return rc;
   CdArgs a;
-  a.cfg = *cfg;
-  a.S = S; a.N = N; a.E = E; a.K = K; a.n_links = n_links;
-  a.freqs = freqs; a.x = x; a.node_ptr = node_ptr; a.rowptr = rowptr;
-  a.edst = edge_index ? edge_index + E : nullptr;
-  a.chan_node = chan_node;
+  if (int rc = cd_state_args(who, a, cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, prepared,
+                             is_lut_index, max_impact))
+    return rc;
+  constexpr int smem = static_cast<int>(sizeof(CdSmem));
+  if (int rc = cd_smem_opt_in<lp_candidate_kernel<kMove>, smem>()) return rc;
+  a.K = K; a.n_links = n_links;
   a.node = node;
   a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = q0; a.width = width; a.feat = feat;
-  a.prep = prepared; a.lut_col = is_lut_index; a.max_impact = max_impact;
   a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_node;
   a.impact_kind = max_impact ? impact_kind : nullptr; a.impact_out = impact_out;
   const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, cdiv(K, kCdWarps)));
@@ -1263,36 +1171,24 @@ static int cs_launch(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* fre
                      int32_t* n_impact, int64_t* impact_node, int8_t* impact_kind, float* impact_out,
                      cudaStream_t stream) {
   const char* who = "qot_lightpath_change_sets";
-  if (int rc = cfg_check(cfg, who)) return rc;
-  QOT_REQUIRE(S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && K >= 0 && G >= 0 && n_links >= 0 && max_impact >= 0,
-              "%s: bad size", who);
-  QOT_REQUIRE(prepared && (reinterpret_cast<uintptr_t>(prepared) & 15) == 0, "%s: prepared must be 16-byte aligned",
-              who);
-  QOT_REQUIRE(is_lut_index >= 0 && is_lut_index < kF, "%s: is_lut_index out of range", who);
+  if (int rc = cd_check_args(who, cfg, S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && K >= 0 && G >= 0 &&
+                                           n_links >= 0 && max_impact >= 0, prepared, is_lut_index))
+    return rc;
   if (G == 0 && K == 0) return QOT_OK;
   QOT_REQUIRE(set_ptr && (G == 0 || (set_status && n_impact && (max_impact == 0 || (impact_node && impact_out)))),
               "%s: null set or set output array", who);
   QOT_REQUIRE(K == 0 || (node && sample && link_ptr && q0 && width && feat && out && status && (n_links == 0 || links)),
               "%s: null change or change output array", who);
-  QOT_REQUIRE(S == 0 || (freqs && x && node_ptr && rowptr && chan_node && (E == 0 || edge_index)),
-              "%s: null state array", who);
-  static std::atomic<unsigned long long> done{0};
-  constexpr int smem = static_cast<int>(sizeof(CsSmem));
-  if (int rc = once_per_device(done, [] {
-        QOT_CUDA(cudaFuncSetAttribute(lp_change_set_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        return static_cast<int>(QOT_OK);
-      }))
-    return rc;
   CsArgs ca;
   CdArgs& a = ca.c;
-  a.cfg = *cfg;
-  a.S = S; a.N = N; a.E = E; a.K = K; a.n_links = n_links;
-  a.freqs = freqs; a.x = x; a.node_ptr = node_ptr; a.rowptr = rowptr;
-  a.edst = edge_index ? edge_index + E : nullptr;
-  a.chan_node = chan_node;
+  if (int rc = cd_state_args(who, a, cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, prepared,
+                             is_lut_index, max_impact))
+    return rc;
+  constexpr int smem = static_cast<int>(sizeof(CsSmem));
+  if (int rc = cd_smem_opt_in<lp_change_set_kernel, smem>()) return rc;
+  a.K = K; a.n_links = n_links;
   a.node = node;
   a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = q0; a.width = width; a.feat = feat;
-  a.prep = prepared; a.lut_col = is_lut_index; a.max_impact = max_impact;
   a.out = nullptr; a.status = set_status; a.n_impact = n_impact; a.impact_node = impact_node;
   a.impact_kind = max_impact ? impact_kind : nullptr; a.impact_out = impact_out;
   ca.G = G; ca.set_ptr = set_ptr; ca.chg_out = out; ca.chg_status = status;
@@ -1312,41 +1208,29 @@ static int pl_launch(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* fre
                      int32_t* n_impact, int64_t* impact_node, float* impact_out, float* all_out, float* all_margin,
                      cudaStream_t stream) {
   const char* who = "qot_lightpath_placements";
-  if (int rc = cfg_check(cfg, who)) return rc;
+  if (int rc = cd_check_args(who, cfg, S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && D >= 0 && P >= 0 &&
+                                           n_links >= 0 && max_impact >= 0, prepared, is_lut_index))
+    return rc;
   QOT_REQUIRE(cfg->Q <= QOT_PLACE_MAX_SLOTS, "%s: Q = %d over QOT_PLACE_MAX_SLOTS", who, cfg->Q);
-  QOT_REQUIRE(S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && D >= 0 && P >= 0 && n_links >= 0 && max_impact >= 0,
-              "%s: bad size", who);
   QOT_REQUIRE(metric >= 0 && metric < QOT_OUT, "%s: metric must be an output column 0..2", who);
   QOT_REQUIRE(policy == QOT_PLACE_FIRST_FIT || policy == QOT_PLACE_BEST_QOT || policy == QOT_PLACE_MAX_MARGIN,
               "%s: unknown policy %d", who, policy);
-  QOT_REQUIRE(prepared && (reinterpret_cast<uintptr_t>(prepared) & 15) == 0, "%s: prepared must be 16-byte aligned",
-              who);
-  QOT_REQUIRE(is_lut_index >= 0 && is_lut_index < kF, "%s: is_lut_index out of range", who);
   if (D == 0) return QOT_OK;
   QOT_REQUIRE(sample && opt_ptr && link_ptr && (P == 0 || (width && feat && own_bound)) && (n_links == 0 || links),
               "%s: null demand array", who);
   QOT_REQUIRE(option && q0 && out && margin && n_free && n_feasible && status && n_impact &&
                   (max_impact == 0 || (impact_node && impact_out)) && (!all_out == !all_margin),
               "%s: null output array", who);
-  QOT_REQUIRE(S == 0 || (freqs && x && node_ptr && rowptr && chan_node && (E == 0 || edge_index)),
-              "%s: null state array", who);
-  static std::atomic<unsigned long long> done{0};
-  constexpr int smem = static_cast<int>(sizeof(PlSmem));
-  if (int rc = once_per_device(done, [] {
-        QOT_CUDA(cudaFuncSetAttribute(lp_placement_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        return static_cast<int>(QOT_OK);
-      }))
-    return rc;
   PlArgs pa;
   CdArgs& a = pa.c;
-  a.cfg = *cfg;
-  a.S = S; a.N = N; a.E = E; a.K = D; a.n_links = n_links;
-  a.freqs = freqs; a.x = x; a.node_ptr = node_ptr; a.rowptr = rowptr;
-  a.edst = edge_index ? edge_index + E : nullptr;
-  a.chan_node = chan_node;
+  if (int rc = cd_state_args(who, a, cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, prepared,
+                             is_lut_index, max_impact))
+    return rc;
+  constexpr int smem = static_cast<int>(sizeof(PlSmem));
+  if (int rc = cd_smem_opt_in<lp_placement_kernel, smem>()) return rc;
+  a.K = D; a.n_links = n_links;
   a.node = nullptr;
   a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = nullptr; a.width = width; a.feat = feat;
-  a.prep = prepared; a.lut_col = is_lut_index; a.max_impact = max_impact;
   a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_node;
   a.impact_kind = nullptr; a.impact_out = impact_out;
   pa.P = P; pa.opt_ptr = opt_ptr; pa.own_bound = own_bound; pa.bound = bound;

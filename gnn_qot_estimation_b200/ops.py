@@ -380,19 +380,28 @@ _CAND_DTYPES = {"sample": torch.int64, "link_ptr": torch.int64, "links": torch.i
                 "width": torch.int32, "feat": torch.float32}
 
 
+def _check_state_tensor(who: str, name: str, t, dev, dt) -> None:
+    """An input of a network-state query: a CUDA tensor on the state's device, of dtype dt."""
+    if not torch.is_tensor(t) or not t.is_cuda:
+        raise RuntimeError(f"{who}: {name} must be a CUDA tensor (no CPU path)")
+    if t.device != dev:
+        raise ValueError(f"{who}: {name} is on {t.device}, the state on {dev}")
+    if t.dtype != dt:
+        raise TypeError(f"{who}: {name} must be {dt}, got {t.dtype}")
+
+
+def _cptr(t):
+    """Pointer of a contiguous t, None for an absent or empty tensor."""
+    return ptr(t.contiguous()) if t is not None and t.numel() else None
+
+
 def _check_candidate_args(state, c, prepared, max_impact, who: str, arg: str, want: dict) -> int:
     """Host-side checks shared by forward_candidates and forward_reconfigurations; returns K."""
     if int(max_impact) != max_impact or max_impact < 0:
         raise ValueError(f"{who}: max_impact must be a non-negative integer")
     dev = state.batch.x.device
     for name, dt in want.items():
-        t = getattr(c, name)
-        if not torch.is_tensor(t) or not t.is_cuda:
-            raise RuntimeError(f"{who}: {arg}.{name} must be a CUDA tensor (no CPU path)")
-        if t.device != dev:
-            raise ValueError(f"{who}: {arg}.{name} is on {t.device}, the state on {dev}")
-        if t.dtype != dt:
-            raise TypeError(f"{who}: {arg}.{name} must be {dt}, got {t.dtype}")
+        _check_state_tensor(who, f"{arg}.{name}", getattr(c, name), dev, dt)
     if prepared.device != dev:
         raise ValueError(f"{who}: the model is on {prepared.device}, the state on {dev}")
     K = int(c.sample.shape[0]) if c.sample.dim() == 1 else -1
@@ -427,14 +436,13 @@ def lightpath_candidates(state, cands, prepared: torch.Tensor, is_lut_index: int
     impact_out = torch.empty(K, max_impact, 3, dtype=torch.float32, device=dev)
     if K == 0:
         return CandidateQoT(out, status, n_impact, impact_node, impact_out)
-    c = lambda t: ptr(t.contiguous()) if t.numel() else None
     keep = [t.contiguous() for t in cands]           # alive until the launch is enqueued
     with torch.cuda.device(dev):                     # stream() of the state's device
         check(_lib.lib().qot_lightpath_candidates(
             *_state_args(state, keep), K,
-            ptr(keep[0]), ptr(keep[1]), c(keep[2]), int(keep[2].numel()), ptr(keep[3]), ptr(keep[4]), ptr(keep[5]),
+            ptr(keep[0]), ptr(keep[1]), _cptr(keep[2]), int(keep[2].numel()), ptr(keep[3]), ptr(keep[4]), ptr(keep[5]),
             ptr(prepared), int(is_lut_index), max_impact, ptr(out), ptr(status), ptr(n_impact),
-            c(impact_node), c(impact_out), stream()), "qot_lightpath_candidates")
+            _cptr(impact_node), _cptr(impact_out), stream()), "qot_lightpath_candidates")
     return CandidateQoT(out, status, n_impact, impact_node, impact_out)
 
 
@@ -453,15 +461,14 @@ def lightpath_reconfigure(state, changes, prepared: torch.Tensor, is_lut_index: 
     impact_out = torch.empty(K, max_impact, 3, dtype=torch.float32, device=dev)
     if K == 0:
         return ReconfigQoT(out, status, n_impact, impact_node, impact_kind, impact_out)
-    c = lambda t: ptr(t.contiguous()) if t.numel() else None
     ch = changes
     keep = [t.contiguous() for t in (ch.node, ch.sample, ch.link_ptr, ch.links, ch.q0, ch.width, ch.feat)]
     with torch.cuda.device(dev):
         check(_lib.lib().qot_lightpath_reconfigure(
             *_state_args(state, keep), K, ptr(keep[0]),
-            ptr(keep[1]), ptr(keep[2]), c(keep[3]), int(keep[3].numel()), ptr(keep[4]), ptr(keep[5]), ptr(keep[6]),
+            ptr(keep[1]), ptr(keep[2]), _cptr(keep[3]), int(keep[3].numel()), ptr(keep[4]), ptr(keep[5]), ptr(keep[6]),
             ptr(prepared), int(is_lut_index), max_impact, ptr(out), ptr(status), ptr(n_impact),
-            c(impact_node), c(impact_kind), c(impact_out), stream()), "qot_lightpath_reconfigure")
+            _cptr(impact_node), _cptr(impact_kind), _cptr(impact_out), stream()), "qot_lightpath_reconfigure")
     return ReconfigQoT(out, status, n_impact, impact_node, impact_kind, impact_out)
 
 
@@ -475,12 +482,7 @@ def lightpath_change_sets(state, changes, set_ptr: torch.Tensor, prepared: torch
     K = _check_candidate_args(state, changes, prepared, max_impact, who, "changes", want)
     max_impact = int(max_impact)
     dev = state.batch.x.device
-    if not torch.is_tensor(set_ptr) or not set_ptr.is_cuda:
-        raise RuntimeError(f"{who}: set_ptr must be a CUDA tensor (no CPU path)")
-    if set_ptr.device != dev:
-        raise ValueError(f"{who}: set_ptr is on {set_ptr.device}, the state on {dev}")
-    if set_ptr.dtype != torch.int64:
-        raise TypeError(f"{who}: set_ptr must be torch.int64, got {set_ptr.dtype}")
+    _check_state_tensor(who, "set_ptr", set_ptr, dev, torch.int64)
     if set_ptr.dim() != 1 or set_ptr.shape[0] < 1:
         raise ValueError(f"{who}: need set_ptr [G+1] with G >= 0")
     G = int(set_ptr.shape[0]) - 1
@@ -494,15 +496,14 @@ def lightpath_change_sets(state, changes, set_ptr: torch.Tensor, prepared: torch
     res = ChangeSetQoT(out, status, set_status, n_impact, impact_node, impact_kind, impact_out)
     if K == 0 and G == 0:
         return res
-    c = lambda t: ptr(t.contiguous()) if t.numel() else None
     ch = changes
     keep = [t.contiguous() for t in (ch.node, ch.sample, ch.link_ptr, ch.links, ch.q0, ch.width, ch.feat, set_ptr)]
     with torch.cuda.device(dev):
         check(_lib.lib().qot_lightpath_change_sets(
-            *_state_args(state, keep), K, c(keep[0]),
-            c(keep[1]), ptr(keep[2]), c(keep[3]), int(keep[3].numel()), c(keep[4]), c(keep[5]), c(keep[6]), G,
-            ptr(keep[7]), ptr(prepared), int(is_lut_index), max_impact, c(out), c(status), c(set_status),
-            c(n_impact), c(impact_node), c(impact_kind), c(impact_out), stream()), "qot_lightpath_change_sets")
+            *_state_args(state, keep), K, _cptr(keep[0]), _cptr(keep[1]), ptr(keep[2]), _cptr(keep[3]),
+            int(keep[3].numel()), _cptr(keep[4]), _cptr(keep[5]), _cptr(keep[6]), G, ptr(keep[7]), ptr(prepared),
+            int(is_lut_index), max_impact, _cptr(out), _cptr(status), _cptr(set_status), _cptr(n_impact),
+            _cptr(impact_node), _cptr(impact_kind), _cptr(impact_out), stream()), "qot_lightpath_change_sets")
     return res
 
 
@@ -553,13 +554,7 @@ def lightpath_placements(state, demands, policy: int, metric: int, maximize: boo
     if bound is not None:
         named.append(("bound", bound, torch.float32))
     for name, t, dt in named:
-        arg = "" if name == "bound" else "demands."
-        if not torch.is_tensor(t) or not t.is_cuda:
-            raise RuntimeError(f"{who}: {arg}{name} must be a CUDA tensor (no CPU path)")
-        if t.device != dev:
-            raise ValueError(f"{who}: {arg}{name} is on {t.device}, the state on {dev}")
-        if t.dtype != dt:
-            raise TypeError(f"{who}: {arg}{name} must be {dt}, got {t.dtype}")
+        _check_state_tensor(who, name if name == "bound" else f"demands.{name}", t, dev, dt)
     if prepared.device != dev:
         raise ValueError(f"{who}: the model is on {prepared.device}, the state on {dev}")
     d = demands
@@ -581,17 +576,17 @@ def lightpath_placements(state, demands, policy: int, metric: int, maximize: boo
                        f32(P, Q, 3) if return_all else None, f32(P, Q) if return_all else None)
     if D == 0:
         return res
-    c = lambda t: ptr(t.contiguous()) if t is not None and t.numel() else None
     keep = [t.contiguous() for t in (d.sample, d.opt_ptr, d.link_ptr, d.links, d.width, d.feat, d.own_bound)]
     if bound is not None:
         keep.append(bound.contiguous())
     with torch.cuda.device(dev):
         check(_lib.lib().qot_lightpath_placements(
-            *_state_args(state, keep), D, ptr(keep[0]), ptr(keep[1]), P, ptr(keep[2]), c(keep[3]),
-            int(keep[3].numel()), c(keep[4]), c(keep[5]), c(keep[6]), c(bound), int(metric), int(bool(maximize)),
+            *_state_args(state, keep), D, ptr(keep[0]), ptr(keep[1]), P, ptr(keep[2]), _cptr(keep[3]),
+            int(keep[3].numel()), _cptr(keep[4]), _cptr(keep[5]), _cptr(keep[6]), _cptr(bound), int(metric),
+            int(bool(maximize)),
             int(policy), ptr(prepared), int(is_lut_index), max_impact, ptr(res.option), ptr(res.q0), ptr(res.out),
             ptr(res.margin), ptr(res.n_free), ptr(res.n_feasible), ptr(res.status), ptr(res.n_impact),
-            c(res.impact_node), c(res.impact_out), c(res.all_out), c(res.all_margin), stream()),
+            _cptr(res.impact_node), _cptr(res.impact_out), _cptr(res.all_out), _cptr(res.all_margin), stream()),
             "qot_lightpath_placements")
     return res
 
