@@ -117,6 +117,9 @@ SIGNATURES = {
     "qot_lightpath_placements": (C.c_int, [C.POINTER(QotLpGraphCfg), i64, P, P, P, P, P, i64, i64, P, i64, P, P, i64,
                                            P, P, i64, P, P, P, P, i32, i32, i32, P, i32, i32, P, P, P, P, P, P, P, P,
                                            P, P, P, P, vp]),
+    "qot_lightpath_provision": (C.c_int, [C.POINTER(QotLpGraphCfg), i64, P, P, P, P, P, i64, i64, P, P, i64, P, P, P,
+                                          P, i64, P, P, i64, P, P, P, P, i32, i32, i32, P, i32, i32, P, P, P, P, P, P,
+                                          P, P, P, P, P, P, P, vp]),
     "qot_topological_graph_scratch_bytes": (sz, [i64]),
     "qot_topological_graph_count": (C.c_int, [P, P, i64, C.POINTER(QotLpGraphCfg), i32, i32, i32, P, P, P, sz, P, vp]),
     "qot_topological_graph_fill": (C.c_int, [P, i64, P, P, P, P, P, vp]),

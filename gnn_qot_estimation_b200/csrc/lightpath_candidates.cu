@@ -1,5 +1,5 @@
-// LightpathGNN network-state queries: candidate lightpaths, reconfigurations, change sets and placements evaluated
-// against a resident network state without rebuilding the state's graph.
+// LightpathGNN network-state queries: candidate lightpaths, reconfigurations, change sets, placements and sequential
+// provisioning evaluated against a resident network state without rebuilding the state's graph.
 //
 // Why no rebuild is needed: the model has one GAT layer and eval-mode BatchNorm is a per-node affine, so a row depends
 // only on its node and its in-neighbours.  Placing a lightpath adds exactly the edges new <-> j for the lightpaths j
@@ -821,6 +821,28 @@ __device__ __forceinline__ unsigned pl_shr(unsigned x, int k, int lane) {
   return b ? (lo >> b) | (hi << (32 - b)) : lo;
 }
 
+// the free starts for width cw (lane t: word t): AND of the free bits over [q0, q0 + cw), in log2(cw) shift steps
+__device__ __forceinline__ unsigned pl_free_starts(unsigned occ, int Q, int cw, int lane) {
+  const int tail = Q - 32 * lane;
+  const unsigned valid = tail >= 32 ? 0xffffffffu : tail > 0 ? (1u << tail) - 1u : 0u;
+  unsigned run = ~occ & valid;
+  for (int have = 1; have < cw;) {
+    const int step = min(have, cw - have);
+    run &= pl_shr(run, step, lane);
+    have += step;
+  }
+  return run;
+}
+
+// the neighbour bits of placement [q0, q0 + cw) from a route's entries: cd_df_hit against each entry's slot
+__device__ __forceinline__ void pl_ent_mask(const CdArgs& a, const int* ent, int ne, int q0, int cw, unsigned* mask,
+                                            int lane) {
+  for (int i = lane; i < ne; i += 32) {
+    const int en = ent[i], q = en >> 8, j = en & 255;
+    if (cd_df_hit(a.freqs, a.freqs[q], q0, cw, a.cfg.freq_threshold)) atomicOr(&mask[j >> 5], 1u << (j & 31));
+  }
+}
+
 // the staged rows' outputs, in staging order, into their placements' margins; a placement whose last row is out goes
 // into the demand's count and running best, and into all_out / all_margin.  Lane 0.
 __device__ __noinline__ void pl_fold(const PlArgs& a, PlWarpSmem& pw, int cnt, int64_t o0) {
@@ -942,14 +964,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
       }
       __syncwarp();
       // ---- free starts for width cw: AND of the free bits over [q0, q0 + cw), in log2(cw) shift steps
-      const int tail = Q - 32 * lane;
-      const unsigned valid = tail >= 32 ? 0xffffffffu : tail > 0 ? (1u << tail) - 1u : 0u;
-      unsigned run = ~occ & valid;
-      for (int have = 1; have < cw;) {
-        const int step = min(have, cw - have);
-        run &= pl_shr(run, step, lane);
-        have += step;
-      }
+      const unsigned run = pl_free_starts(occ, Q, cw, lane);
       if (pa.all_out)                                     // NaN at every start that is not free
         for (int wd = 0; wd < 32 && 32 * wd < Q; ++wd) {
           const unsigned bits = __shfl_sync(kFull, run, wd);
@@ -967,11 +982,7 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
           if (lane < kCdMaskWords) ws.mask[lane] = 0u;
           __syncwarp();
           if (ne <= kPlEntCap) {
-            for (int i = lane; i < ne; i += 32) {
-              const int en = pw.ent[i], q = en >> 8, j = en & 255;
-              if (cd_df_hit(a.freqs, a.freqs[q], q0, cw, a.cfg.freq_threshold))
-                atomicOr(&ws.mask[j >> 5], 1u << (j & 31));
-            }
+            pl_ent_mask(a, pw.ent, ne, q0, cw, ws.mask, lane);
           } else {
             cd_scan(a, s, n0, n, p0, p1, q0, cw, ws.mask, CdNone(), lane);
           }
@@ -1080,6 +1091,462 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
       pa.n_feasible[d] = pw.n_feas;
     }
     __syncwarp();
+  }
+  if (zc) pl_flush(pa, pw, w, zc, 0, lane);
+}
+
+// ------------------------------------------------------------------------------------------------ provisioning
+// lp_provision_kernel: persistent, one block per sample (qot_lightpath_provision).  The sample's demands are taken in
+// order, each placed as lp_placement_kernel places it against the state with every earlier accepted demand of the
+// sample written in.  The block holds that state as a dense graph in node-rank order: a 256 x 256-bit adjacency from
+// the out-runs (self loops dropped), the x rows, the conn_ids and each node's first channel (link * Q + slot: the
+// graph builder orders nodes by it).  Accepted channels go into chan_work, the entry point's copy of chan_node, which
+// the block reads through L2 (__ldcg) because it writes it; a channel there holds n0 + the node's stable id (state
+// node j: j; the c-th accepted demand: n + c) and s2r maps a stable id to its rank.
+//   per demand and option: warp 0 scans the route into the free-start words (pl_free_starts) and (slot << 8 | rank)
+//     entries; the free placements are dealt round-robin to the warps, each evaluating its placements as the placement
+//     kernel does (own row: the neighbours by rank, then the self loop; impact row of rank r: r's adjacency row by
+//     rank, the placement, the self loop) and folding them with pl_fold into its own best key and counts;
+//   the block takes the largest key (unique: its low word is the placement's index) and the summed counts, so the
+//     choice does not depend on which warp evaluated what; warp 0 writes the winner's impact rows;
+//   an accepted demand is inserted at the rank its first channel (min route link, q0) gives it: every row's bits from
+//     that rank up move one place, its row and column go in, its channels into chan_work, its own_bound into
+//     bound_work (the bound of its impact rows from then on).
+// Message order and values are then those of lp_placement_kernel on the rebuilt state: bit-identical.
+struct PvSmem {
+  CdSmem cd;                                 // head fragments and the candidate kernel's per-warp state
+  PlWarpSmem w[kCdWarps];                    // the placement kernel's per-warp search state
+  unsigned adj[kCdMaxN][kCdMaskWords];       // the sample's graph by rank, self loops dropped
+  float x[kCdMaxN][kF];                      // x rows by rank
+  long long conn[kCdMaxN];                   // conn_id by rank
+  int key[kCdMaxN];                          // first channel (link * Q + slot) by rank
+  short r2s[kCdMaxN], s2r[kCdMaxN];          // rank <-> stable id
+  int ent[kPlEntCap];                        // the option's channels of known lightpaths: slot << 8 | rank
+  unsigned run[32];                          // the option's free-start words
+  unsigned wmask[kCdMaskWords];              // the winner's neighbours by rank
+  float best[4];                             // the winner's own row and margin
+  unsigned long long key_best, n_valid;
+  long long top;                             // the sample's largest conn_id (at least 0)
+  int n_tot, n_chan, ne, rbad, st, n_free, n_feas, acc, c_key;
+  long long c_po;
+  int c_q0;
+};
+static_assert(sizeof(PvSmem) + 16 <= 227 * 1024, "lp_provision_kernel: shared memory over the 227 KB block limit");
+static_assert(kCdThreads >= kCdMaxN + 1, "one thread per rank, and one more for the inserted row");
+
+struct PvArgs {
+  PlArgs p;                                // p.c.chan_node = chan_work, p.c.impact_node = impact_conn, p.bound =
+                                           // bound_work (or null)
+  const int64_t* order;                    // [D]: the demands grouped by sample, ascending within a sample
+  const int64_t* sample_ptr;               // [S+1]: sample s's demands are order[sample_ptr[s], sample_ptr[s+1])
+  const int64_t* conn_ids;                 // [N]
+  const float* bound;                      // [N] or null
+  int32_t* chan_work;                      // [S, L, Q]
+  float* bound_work;                       // [S, kCdMaxN] by stable id, or null
+  int64_t* conn_id;                        // [D]
+};
+
+// x of a message source: rank j of the block's graph or the placement (kCand)
+struct PvX {
+  const float (*x)[kF];
+  const float* cx;
+  int lut, col;
+  __device__ __forceinline__ float operator()(int j, int k) const {
+    if (k == col) return j == lut ? 1.0f : 0.0f;
+    return j == kCand ? cx[k] : x[j][k];
+  }
+};
+
+// the empty result of demand d with status st (option = q0 = -1, NaN rows, zero counts, conn_id -1), written by
+// threads t, t + stride, ...
+__device__ void pv_empty(const PvArgs& va, int64_t d, int st, int t, int stride) {
+  const PlArgs& pa = va.p;
+  const CdArgs& a = pa.c;
+  const float nan = __int_as_float(0x7fc00000);
+  if (t == 0) {
+    a.status[d] = st;
+    a.n_impact[d] = 0;
+    pa.option[d] = pa.q0[d] = -1;
+    pa.margin[d] = nan;
+    pa.n_free[d] = pa.n_feasible[d] = 0;
+    va.conn_id[d] = -1;
+  }
+  for (int o = t; o < QOT_OUT; o += stride) a.out[d * QOT_OUT + o] = nan;
+  cd_clear_impact(a, d, 0, a.max_impact, nullptr, t, stride);
+}
+
+// the neighbours by rank of placement [q0, q0 + cw) on route links[p0, p1), from chan_work (the route was scanned
+// before: every occupied channel is free, a known node's or unknown)
+__device__ __forceinline__ void pv_scan(const PvArgs& va, const PvSmem& sm, int64_t s, int64_t n0, int64_t p0,
+                                        int64_t p1, int q0, int cw, unsigned* mask, int lane) {
+  const CdArgs& a = va.p.c;
+  for (int64_t e = p0; e < p1; ++e) {
+    const int32_t* row = va.chan_work + (s * a.cfg.L + a.links[e]) * a.cfg.Q;
+    for (int q = lane; q < a.cfg.Q; q += 32) {
+      const int32_t v = __ldcg(row + q);
+      const int64_t j = static_cast<int64_t>(v) - n0;
+      if (v < 0 || j < 0 || j >= sm.n_tot || (q >= q0 && q < q0 + cw)) continue;
+      if (cd_df_hit(a.freqs, a.freqs[q], q0, cw, a.cfg.freq_threshold)) {
+        const int r = sm.s2r[j];
+        atomicOr(&mask[r >> 5], 1u << (r & 31));
+      }
+    }
+  }
+}
+
+// a 256-bit row with a bit inserted at position R (value v): the bits from R up move one place
+__device__ __forceinline__ void pv_insert_bit(unsigned (&r)[kCdMaskWords], int R, unsigned v) {
+  const int wr = R >> 5, b = R & 31;
+#pragma unroll
+  for (int k = kCdMaskWords - 1; k >= 0; --k) {
+    const unsigned prev = k ? r[k - 1] : 0u;
+    const unsigned keep = k < wr ? 0xffffffffu : k == wr ? (1u << b) - 1u : 0u;
+    r[k] = (r[k] & keep) | (r[k] & ~keep) << 1 | (k > wr ? prev >> 31 : 0u) | (k == wr ? v << b : 0u);
+  }
+}
+
+// the accepted demand into chan_work, bound_work and the block's graph: the new node inserted at rank R (the number of
+// nodes whose first channel comes before its own), every row's bits from R up moved one place.  All threads.
+__device__ __noinline__ void pv_commit(const PvArgs& va, PvSmem& sm, int64_t s, int64_t n0, int tid) {
+  const PlArgs& pa = va.p;
+  const CdArgs& a = pa.c;
+  const int L = a.cfg.L, Q = a.cfg.Q;
+  const int64_t po = sm.c_po, p0 = a.link_ptr[po], p1 = a.link_ptr[po + 1];
+  const int cw = a.width[po], q0 = sm.c_q0, ck = sm.c_key, nt = sm.n_tot;
+  const int64_t len = p1 - p0;
+  for (int64_t k = tid; k < len * cw; k += kCdThreads)
+    va.chan_work[(s * L + a.links[p0 + k / cw]) * Q + q0 + k % cw] = static_cast<int32_t>(n0 + nt);
+  if (va.bound_work && tid == 0) va.bound_work[s * kCdMaxN + nt] = pa.own_bound[po];
+  const int R = __syncthreads_count(tid < nt && sm.key[tid] < ck);
+  unsigned rw[kCdMaskWords];
+  float xr[kF];
+  long long cn = 0;
+  int ky = 0;
+  short sid = 0;
+  const bool old = tid < nt, ins = tid == kCdThreads - 1;
+  if (old || ins) {
+#pragma unroll
+    for (int k = 0; k < kCdMaskWords; ++k) rw[k] = ins ? sm.wmask[k] : sm.adj[tid][k];
+    pv_insert_bit(rw, R, ins ? 0u : sm.wmask[tid >> 5] >> (tid & 31) & 1u);
+#pragma unroll
+    for (int k = 0; k < kF; ++k) xr[k] = ins ? sm.cd.w[0].cx[k] : sm.x[tid][k];
+    cn = ins ? sm.top + 1 : sm.conn[tid];
+    ky = ins ? ck : sm.key[tid];
+    sid = ins ? static_cast<short>(nt) : sm.r2s[tid];
+  }
+  __syncthreads();
+  if (old || ins) {
+    const int to = ins ? R : tid < R ? tid : tid + 1;
+#pragma unroll
+    for (int k = 0; k < kCdMaskWords; ++k) sm.adj[to][k] = rw[k];
+#pragma unroll
+    for (int k = 0; k < kF; ++k) sm.x[to][k] = xr[k];
+    sm.conn[to] = cn;
+    sm.key[to] = ky;
+    sm.r2s[to] = sid;
+  }
+  __syncthreads();
+  for (int r = tid; r <= nt; r += kCdThreads) sm.s2r[sm.r2s[r]] = static_cast<short>(r);
+  if (tid == 0) {
+    sm.n_tot = nt + 1;
+    sm.n_chan += static_cast<int>(len * cw);
+    sm.top += 1;
+  }
+  __syncthreads();
+}
+
+__global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __grid_constant__ PvArgs va) {
+  const PlArgs& pa = va.p;
+  const CdArgs& a = pa.c;
+  PvSmem& sm = *reinterpret_cast<PvSmem*>(cd_smem_raw);
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  CdWarpSmem& ws = sm.cd.w[w];
+  PlWarpSmem& pw = sm.w[w];
+  float As[kF], Ad[kF];
+  cd_head_prologue(a.prep, As, Ad, tid);
+  if (tid == 0) sm.n_valid = 0ull;
+  // ---- the grouping, checked whole by every block: sample_ptr non-decreasing from 0; order[i] a demand of the sample
+  // whose range holds i, ascending within the range; the ranges hold every demand with a sample in [0, S).  Otherwise
+  // no demand is provisioned: every output says PROV_BAD_GROUPING, each written by exactly one thread of the grid.
+  const int64_t S = a.S, D = a.K;
+  bool bad = false;
+  for (int64_t g = tid; g <= S; g += kCdThreads) {
+    const int64_t v = va.sample_ptr[g];
+    bad |= (g == 0 && v != 0) || (g < S && va.sample_ptr[g + 1] < v) || (g == S && v > D);
+  }
+  bad = __syncthreads_or(bad);
+  if (!bad) {
+    const int64_t nv = va.sample_ptr[S];
+    unsigned long long cnt = 0;
+    for (int64_t i = tid; i < D; i += kCdThreads) {
+      const int64_t sd = a.sample[i];
+      cnt += sd >= 0 && sd < S;
+      if (i < nv) {
+        const int64_t d = va.order[i];
+        bool ok = d >= 0 && d < D;
+        const int64_t s = ok ? a.sample[d] : -1;
+        ok = ok && s >= 0 && s < S && va.sample_ptr[s] <= i && i < va.sample_ptr[s + 1];
+        if (ok && i + 1 < va.sample_ptr[s + 1]) ok = va.order[i + 1] > d;
+        bad |= !ok;
+      }
+    }
+    atomicAdd(&sm.n_valid, cnt);
+    bad = __syncthreads_or(bad) || sm.n_valid != static_cast<unsigned long long>(nv);
+  }
+  const int64_t gt = static_cast<int64_t>(blockIdx.x) * kCdThreads + tid;
+  const int64_t gs = static_cast<int64_t>(gridDim.x) * kCdThreads;
+  if (bad) {
+    for (int64_t d = gt; d < D; d += gs) pv_empty(va, d, QOT_PROV_BAD_GROUPING, 0, 1);
+    return;
+  }
+  for (int64_t d = gt; d < D; d += gs)
+    if (a.sample[d] < 0 || a.sample[d] >= S) pv_empty(va, d, QOT_CAND_BAD_SAMPLE, 0, 1);
+  const float nan = __int_as_float(0x7fc00000);
+  int zc = 0;                                             // rows staged in this warp's head buffer
+  for (int64_t s = blockIdx.x; s < S; s += gridDim.x) {
+    const int64_t i0 = va.sample_ptr[s], i1 = va.sample_ptr[s + 1];
+    if (i0 == i1) continue;
+    const int L = a.cfg.L, Q = a.cfg.Q;
+    int64_t n0 = 0;
+    int n = 0;
+    const bool state_ok = cd_sample_nodes(a, s, n0, n);
+    // ---- the sample's graph, in node order: adjacency from the out-runs, x, conn_ids, first channels, bounds
+    __syncthreads();                                      // the previous sample's graph is no longer read
+    for (int i = tid; i < kCdMaxN * kCdMaskWords; i += kCdThreads) (&sm.adj[0][0])[i] = 0u;
+    for (int r = tid; r < kCdMaxN; r += kCdThreads) {
+      sm.key[r] = INT_MAX;
+      sm.r2s[r] = sm.s2r[r] = static_cast<short>(r);
+    }
+    if (tid == 0) {
+      sm.n_tot = state_ok ? n : 0;
+      sm.n_chan = 0;
+      sm.top = 0;
+    }
+    __syncthreads();
+    bool sbad = !state_ok;
+    if (state_ok) {
+      for (int r = w; r < n; r += kCdWarps) sbad |= !cd_old_nbrs(a, n0, n, r, sm.adj[r], lane);
+      for (int i = tid; i < n * kF; i += kCdThreads) (&sm.x[0][0])[i] = a.x[n0 * kF + i];
+      long long top = 0;
+      for (int r = tid; r < n; r += kCdThreads) {
+        const long long c = va.conn_ids[n0 + r];
+        sm.conn[r] = c;
+        top = max(top, c);
+      }
+      atomicMax(&sm.top, top);
+      int nch = 0;
+      const int32_t* crow = va.chan_work + s * L * Q;
+      for (int ch = tid; ch < L * Q; ch += kCdThreads) {
+        const int32_t v = __ldcg(crow + ch);
+        if (v == -1) continue;
+        ++nch;
+        const int64_t j = static_cast<int64_t>(v) - n0;
+        if (v >= 0 && j >= 0 && j < n) atomicMin(&sm.key[j], ch);
+      }
+      atomicAdd(&sm.n_chan, nch);
+      if (va.bound_work)
+        for (int r = tid; r < n; r += kCdThreads) va.bound_work[s * kCdMaxN + r] = va.bound[n0 + r];
+    }
+    sbad = __syncthreads_or(sbad);
+    for (int64_t i = i0; i < i1; ++i) {
+      const int64_t d = va.order[i];
+      const int64_t o0 = pa.opt_ptr[d], o1 = pa.opt_ptr[d + 1];
+      // ---- validation (warp 0): the option range, every option's route and width; then the state
+      if (w == 0) {
+        const bool opts_ok = o0 >= 0 && o1 > o0 && o1 <= pa.P && o1 - o0 <= kPlMaxOptions;
+        bool badp = !opts_ok;
+        if (opts_ok)
+          for (int64_t po = o0; po < o1 && !badp; ++po) {
+            const int cw = a.width[po];
+            badp = cd_bad_route(a, L, a.link_ptr[po], a.link_ptr[po + 1], false, cw < 1 || cw > Q, lane);
+          }
+        if (lane == 0) sm.st = badp ? QOT_CAND_BAD_PATH : sbad ? QOT_CAND_BAD_STATE : 0;
+      }
+      if (lane == 0) {
+        pw.key = 0ull;
+        pw.n_free = pw.n_feas = 0;
+      }
+      __syncthreads();
+      const auto row = [&](const int* msg, int M, int q, float* dst, int tag, long long node) {
+        if (lane == 0) {
+          pw.rtag[zc] = tag;
+          pw.rnode[zc] = node;
+        }
+        zc = cd_row(ws, zc, msg, M, q, PvX{sm.x, ws.cx, q, a.lut_col}, As, Ad, dst ? dst : pw.rout[zc],
+                    [&](int cnt) { pl_flush(pa, pw, w, cnt, o0, lane); }, lane);
+      };
+      int st = sm.st;                                     // block-uniform
+      int seq = 0, wseq = 0;                              // placements of this demand: all, this warp's
+      for (int64_t po = o0; st == 0 && po < o1; ++po) {
+        const int64_t p0 = a.link_ptr[po], p1 = a.link_ptr[po + 1];
+        const int cw = a.width[po];
+        // ---- warp 0: the route's occupied bitmap and its channels of known lightpaths by rank, one read per row
+        if (w == 0) {
+          unsigned occ = 0u;
+          int ne = 0;
+          bool rbad = false;
+          const int nt = sm.n_tot;
+          for (int64_t e = p0; e < p1; ++e) {
+            const int32_t* crow = va.chan_work + (s * L + a.links[e]) * Q;
+            for (int qb = 0; qb < Q; qb += 32) {
+              const int q = qb + lane;
+              const int32_t v = q < Q ? __ldcg(crow + q) : -1;
+              const unsigned ob = __ballot_sync(kFull, v != -1);
+              if (lane == qb >> 5) occ |= ob;
+              const int64_t j = static_cast<int64_t>(v) - n0;
+              const bool known = v >= 0 && j >= 0 && j < nt;
+              rbad |= v >= 0 && !known;
+              const unsigned kb = __ballot_sync(kFull, known);
+              const int at = ne + __popc(kb & ((1u << lane) - 1u));
+              if (known && at < kPlEntCap) sm.ent[at] = q << 8 | sm.s2r[j];
+              ne += __popc(kb);
+            }
+          }
+          sm.run[lane] = pl_free_starts(occ, Q, cw, lane);
+          rbad = __any_sync(kFull, rbad);
+          if (lane == 0) {
+            sm.ne = ne;
+            sm.rbad = rbad;
+          }
+        }
+        __syncthreads();
+        if (sm.rbad) {
+          st |= QOT_CAND_BAD_STATE;
+          break;
+        }
+        // ---- the free starts in ascending order, dealt round-robin to the warps
+        const int ne = sm.ne;
+        for (int wd = 0; wd < 32 && 32 * wd < Q; ++wd) {
+          for (unsigned bits = sm.run[wd]; bits; bits &= bits - 1u) {
+            const int q0 = 32 * wd + __ffs(bits) - 1;
+            if (seq++ % kCdWarps != w) continue;
+            if (lane < kCdMaskWords) ws.mask[lane] = 0u;
+            __syncwarp();
+            if (ne <= kPlEntCap) pl_ent_mask(a, sm.ent, ne, q0, cw, ws.mask, lane);
+            else pv_scan(va, sm, s, n0, p0, p1, q0, cw, ws.mask, lane);
+            __syncwarp();
+            const int nn = cd_rank(lane < kCdMaskWords ? ws.mask[lane] : 0u, ws.nbr, lane);
+            cd_xrow(a, ws.cx, [&] { return lane == 0 ? static_cast<float>(a.freqs[q0]) : a.feat[po * 3 + lane - 1]; },
+                    lane);
+            const int slot = wseq++ & (kPlRing - 1);
+            const int nimp = pa.bound ? nn : 0;           // impact rows count against a bound, all of them
+            if (lane == 0) {
+              ws.nbr[nn] = kCand;
+              PlPending& pp = pw.ring[slot];
+              pp.mkey = 0xffffffffu;
+              pp.left = 1 + nimp;
+              pp.p = static_cast<int>(po);
+              pp.q0 = q0;
+              ++pw.n_free;
+            }
+            __syncwarp();
+            row(ws.nbr, nn + 1, kCand, nullptr, slot, -1);
+            for (int k = 0; k < nimp; ++k) {
+              const int r = ws.nbr[k];
+              const int m = cd_rank(lane < kCdMaskWords ? sm.adj[r][lane] : 0u, ws.msg, lane);
+              if (lane == 0) {
+                ws.msg[m] = kCand;
+                ws.msg[m + 1] = r;
+              }
+              __syncwarp();
+              row(ws.msg, m + 2, r, nullptr, slot, s * kCdMaxN + sm.r2s[r]);
+            }
+          }
+        }
+        __syncthreads();                                  // the entries and free words are read
+      }
+      // ---- every placement folded: the block's winner and counts
+      if (zc) {
+        pl_flush(pa, pw, w, zc, o0, lane);
+        zc = 0;
+      }
+      __syncthreads();
+      if (tid == 0) {
+        unsigned long long key = 0ull;
+        int nf = 0, nfe = 0, bw = -1;
+        for (int v = 0; v < kCdWarps; ++v) {
+          nf += sm.w[v].n_free;
+          nfe += sm.w[v].n_feas;
+          if (sm.w[v].key > key) {
+            key = sm.w[v].key;
+            bw = v;
+          }
+        }
+        sm.key_best = key;
+        sm.n_free = nf;
+        sm.n_feas = nfe;
+        if (bw >= 0)
+          for (int o = 0; o < 4; ++o) sm.best[o] = sm.w[bw].best[o];
+      }
+      __syncthreads();
+      // ---- warp 0: the winner's impact rows and the demand's outputs; acceptance
+      if (w == 0) {
+        const int MI = a.max_impact;
+        const unsigned long long key = sm.key_best;
+        int cnt = 0, rows = 0, bp = -1, bq = -1;
+        int64_t po = -1, p0 = 0, p1 = 0;
+        int cw = 0;
+        if (st == 0 && key) {
+          const unsigned idx = 0xffffffffu - static_cast<unsigned>(key);
+          bp = static_cast<int>(idx >> 10);
+          bq = static_cast<int>(idx & 1023u);
+          po = o0 + bp;
+          p0 = a.link_ptr[po];
+          p1 = a.link_ptr[po + 1];
+          cw = a.width[po];
+          if (lane < kCdMaskWords) sm.wmask[lane] = 0u;
+          __syncwarp();
+          pv_scan(va, sm, s, n0, p0, p1, bq, cw, sm.wmask, lane);
+          __syncwarp();
+          cnt = cd_rank(lane < kCdMaskWords ? sm.wmask[lane] : 0u, ws.nbr, lane);
+          rows = min(cnt, MI);
+          cd_xrow(a, ws.cx, [&] { return lane == 0 ? static_cast<float>(a.freqs[bq]) : a.feat[po * 3 + lane - 1]; },
+                  lane);
+          __syncwarp();
+          for (int k = 0; k < rows; ++k) {
+            const int r = ws.nbr[k];
+            if (lane == 0) a.impact_node[d * MI + k] = sm.conn[r];
+            const int m = cd_rank(lane < kCdMaskWords ? sm.adj[r][lane] : 0u, ws.msg, lane);
+            if (lane == 0) {
+              ws.msg[m] = kCand;
+              ws.msg[m + 1] = r;
+            }
+            __syncwarp();
+            row(ws.msg, m + 2, r, a.impact_out + (d * MI + k) * QOT_OUT, -1, -1);
+          }
+        }
+        if (st & kPlFatal) {
+          pv_empty(va, d, st, lane, 32);
+          if (lane == 0) sm.acc = 0;
+        } else {
+          cd_clear_impact(a, d, rows, MI, nullptr, lane, 32);
+          // the graph builder refuses a sample over QOT_TG_MAX_NODES lightpaths or QOT_TG_MAX_CHANNELS channels
+          const bool full = key && (sm.n_tot >= kCdMaxN || sm.n_chan + (p1 - p0) * cw > QOT_TG_MAX_CHANNELS);
+          const bool acc = key && !full;
+          int first = INT_MAX;                            // the accepted lightpath's first channel
+          for (int64_t e = p0 + lane; acc && e < p1; e += 32) first = min(first, a.links[e] * Q + bq);
+          first = __reduce_min_sync(kFull, first);
+          if (lane < QOT_OUT) a.out[d * QOT_OUT + lane] = key ? sm.best[lane] : nan;
+          if (lane == 0) {
+            a.status[d] = st | (cnt > MI ? QOT_CAND_IMPACT_OVERFLOW : 0) | (full ? QOT_PROV_FULL : 0);
+            a.n_impact[d] = cnt;
+            pa.option[d] = bp;
+            pa.q0[d] = bq;
+            pa.margin[d] = key ? sm.best[3] : nan;
+            pa.n_free[d] = sm.n_free;
+            pa.n_feasible[d] = sm.n_feas;
+            va.conn_id[d] = acc ? sm.top + 1 : -1;
+            sm.acc = acc;
+            sm.c_po = po;
+            sm.c_q0 = bq;
+            sm.c_key = first;
+          }
+        }
+      }
+      __syncthreads();
+      if (!sm.acc) continue;
+      pv_commit(va, sm, s, n0, tid);
+    }
   }
   if (zc) pl_flush(pa, pw, w, zc, 0, lane);
 }
@@ -1243,6 +1710,59 @@ static int pl_launch(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* fre
   return QOT_OK;
 }
 
+static int pv_launch(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
+                     const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N, int64_t E,
+                     const int32_t* chan_node, const int64_t* conn_ids, int64_t D, const int64_t* sample,
+                     const int64_t* order, const int64_t* sample_ptr, const int64_t* opt_ptr, int64_t P,
+                     const int64_t* link_ptr, const int32_t* links, int64_t n_links, const int32_t* width,
+                     const float* feat, const float* own_bound, const float* bound, int32_t metric, int32_t maximize,
+                     int32_t policy, const float* prepared, int32_t is_lut_index, int32_t max_impact,
+                     int32_t* chan_work, float* bound_work, int32_t* option, int32_t* q0, float* out, float* margin,
+                     int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact, int64_t* conn_id,
+                     int64_t* impact_conn, float* impact_out, cudaStream_t stream) {
+  const char* who = "qot_lightpath_provision";
+  if (int rc = cd_check_args(who, cfg, S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && D >= 0 && P >= 0 &&
+                                           n_links >= 0 && max_impact >= 0, prepared, is_lut_index))
+    return rc;
+  QOT_REQUIRE(cfg->Q <= QOT_PLACE_MAX_SLOTS, "%s: Q = %d over QOT_PLACE_MAX_SLOTS", who, cfg->Q);
+  QOT_REQUIRE(metric >= 0 && metric < QOT_OUT, "%s: metric must be an output column 0..2", who);
+  QOT_REQUIRE(policy == QOT_PLACE_FIRST_FIT || policy == QOT_PLACE_BEST_QOT || policy == QOT_PLACE_MAX_MARGIN,
+              "%s: unknown policy %d", who, policy);
+  if (D == 0) return QOT_OK;
+  QOT_REQUIRE(sample && order && sample_ptr && opt_ptr && link_ptr && (P == 0 || (width && feat && own_bound)) &&
+                  (n_links == 0 || links), "%s: null demand or grouping array", who);
+  QOT_REQUIRE(option && q0 && out && margin && n_free && n_feasible && status && n_impact && conn_id &&
+                  (max_impact == 0 || (impact_conn && impact_out)), "%s: null output array", who);
+  QOT_REQUIRE((S == 0 || chan_work) && (!bound || S == 0 || bound_work) && (N == 0 || conn_ids),
+              "%s: null work or conn_ids array", who);
+  PvArgs va;
+  PlArgs& pa = va.p;
+  CdArgs& a = pa.c;
+  if (int rc = cd_state_args(who, a, cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_work, prepared,
+                             is_lut_index, max_impact))
+    return rc;
+  constexpr int smem = static_cast<int>(sizeof(PvSmem));
+  if (int rc = cd_smem_opt_in<lp_provision_kernel, smem>()) return rc;
+  if (S > 0)
+    QOT_CUDA(cudaMemcpyAsync(chan_work, chan_node, static_cast<size_t>(S) * cfg->L * cfg->Q * sizeof(int32_t),
+                             cudaMemcpyDeviceToDevice, stream));
+  a.K = D; a.n_links = n_links;
+  a.node = nullptr;
+  a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = nullptr; a.width = width; a.feat = feat;
+  a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_conn;
+  a.impact_kind = nullptr; a.impact_out = impact_out;
+  pa.P = P; pa.opt_ptr = opt_ptr; pa.own_bound = own_bound; pa.bound = bound ? bound_work : nullptr;
+  pa.metric = metric; pa.maximize = maximize != 0; pa.policy = policy;
+  pa.option = option; pa.q0 = q0; pa.margin = margin; pa.n_free = n_free; pa.n_feasible = n_feasible;
+  pa.all_out = nullptr; pa.all_margin = nullptr;
+  va.order = order; va.sample_ptr = sample_ptr; va.conn_ids = conn_ids; va.bound = bound;
+  va.chan_work = chan_work; va.bound_work = bound ? bound_work : nullptr; va.conn_id = conn_id;
+  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, std::max<int64_t>(1, S)));
+  lp_provision_kernel<<<grid, kCdThreads, smem, stream>>>(va);
+  QOT_LAUNCH_CHECK();
+  return QOT_OK;
+}
+
 }  // namespace qot
 
 using namespace qot;
@@ -1323,4 +1843,24 @@ extern "C" int qot_lightpath_placements(const qot_lp_graph_cfg_t* cfg, int64_t S
                    links, n_links, width, feat, own_bound, bound, metric, maximize, policy, prepared, is_lut_index,
                    max_impact, option, q0, out, margin, n_free, n_feasible, status, n_impact, impact_node, impact_out,
                    all_out, all_margin, static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int qot_lightpath_provision(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
+                                       const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index,
+                                       int64_t N, int64_t E, const int32_t* chan_node, const int64_t* conn_ids,
+                                       int64_t D, const int64_t* sample, const int64_t* order,
+                                       const int64_t* sample_ptr, const int64_t* opt_ptr, int64_t P,
+                                       const int64_t* link_ptr, const int32_t* links, int64_t n_links,
+                                       const int32_t* width, const float* feat, const float* own_bound,
+                                       const float* bound, int32_t metric, int32_t maximize, int32_t policy,
+                                       const float* prepared, int32_t is_lut_index, int32_t max_impact,
+                                       int32_t* chan_work, float* bound_work, int32_t* option, int32_t* q0,
+                                       float* out, float* margin, int32_t* n_free, int32_t* n_feasible,
+                                       int32_t* status, int32_t* n_impact, int64_t* conn_id, int64_t* impact_conn,
+                                       float* impact_out, void* stream_) {
+  return pv_launch(cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, conn_ids, D, sample, order,
+                   sample_ptr, opt_ptr, P, link_ptr, links, n_links, width, feat, own_bound, bound, metric, maximize,
+                   policy, prepared, is_lut_index, max_impact, chan_work, bound_work, option, q0, out, margin, n_free,
+                   n_feasible, status, n_impact, conn_id, impact_conn, impact_out,
+                   static_cast<cudaStream_t>(stream_));
 }

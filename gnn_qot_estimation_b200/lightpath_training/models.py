@@ -251,6 +251,39 @@ class LightpathGNN(torch.nn.Module):
         return ops.lightpath_placements(state, demands, policy, metric, maximize, bound, self.prepared(),
                                         self.is_lut_index, max_impact, return_all)
 
+    def forward_provision(self, state, demands, policy: int, metric: int = 0, maximize: bool = True, bound=None,
+                          max_impact: int = 64) -> "ops.ProvisionQoT":
+        """Sequential provisioning of lightpath demands (eval mode only; csrc/lightpath_candidates.cu,
+        qot_lightpath_provision): the demands of each sample are placed in increasing index, each against the state
+        with the sample's earlier accepted demands set up.  Samples are independent; their demands may be interleaved.
+
+        Demand d is placed exactly as ``forward_placements`` places it against ``state_d`` =
+        ``lightpath_network_state(data_d, ...)``, where ``data_d`` is the raw samples with every earlier accepted demand
+        of d's sample written in as ``forward_candidates`` writes a candidate: the chosen route x ``[q0, q0 + width)``,
+        conn_id one above the sample's largest (top + 1, top + 2, ... for successive acceptances), ``freq =
+        float32(freqs[q0])``, the option's (mod_order, num_spans, path_len), osnr = snr = ber = -1, other rows 0.
+        With a ``bound`` ([N] float32 over ``state.batch``'s nodes), an accepted demand is bound from then on by its
+        option's ``own_bound``: a later placement that would take it below is infeasible; with ``bound=None`` impact
+        rows are unconstrained.  A demand is accepted when it has a feasible placement and no status bit but
+        ``CAND_IMPACT_OVERFLOW``; otherwise it commits nothing and the sample's later demands go on.
+
+        Returns ``ops.ProvisionQoT``: the fields of ``ops.PlacementQoT`` but ``all_out`` / ``all_margin``,
+        bit-identical to ``forward_placements(state_d, ...)`` for that demand, with the impact rows named by conn_id
+        (``impact_conn``, since node numbers change as lightpaths are added) and ``conn_id`` [D], the id the demand
+        was accepted under (-1 if not).  Status bits on top of ``ops.CAND_*``: ``ops.PROV_FULL`` (accepting would take
+        the sample past 256 lightpaths or 6144 occupied channels, which the graph builder refuses: not accepted, the
+        placement still reported).  ``state`` is not modified; ``to_graph.commit_provision`` writes the accepted
+        demands into the samples.  One copy and one launch, nothing read back: capturable in a CUDA graph.  Malformed
+        arguments raise on the host."""
+        if self.training:
+            raise RuntimeError("LightpathGNN.forward_provision is eval-only (in training mode BatchNorm couples the "
+                               "nodes): call model.eval()")
+        if not state.batch.x.is_cuda:
+            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
+        self._check_supported()
+        return ops.lightpath_provision(state, demands, policy, metric, maximize, bound, self.prepared(),
+                                       self.is_lut_index, max_impact)
+
     @_lib.on_tensor_device
     def forward_stream(self, plan, first: int = 0, count=None) -> None:
         """Enqueues batches [first, first+count) of ``plan`` (eval mode; no host synchronisation)."""

@@ -533,13 +533,8 @@ _DEMAND_DTYPES = {"sample": torch.int64, "opt_ptr": torch.int64, "link_ptr": tor
                   "width": torch.int32, "feat": torch.float32, "own_bound": torch.float32}
 
 
-def lightpath_placements(state, demands, policy: int, metric: int, maximize: bool, bound, prepared: torch.Tensor,
-                         is_lut_index: int, max_impact: int, return_all: bool = False) -> PlacementQoT:
-    """One launch of qot_lightpath_placements (the placement of each demand chosen over every free slot of its
-    options); nothing is read back (CUDA-graph capturable).  Refuses CPU tensors and mismatched devices, dtypes or
-    shapes, an unknown policy or metric and Q over PLACE_MAX_SLOTS; what can only be judged on the device comes back
-    as status bits."""
-    who = "forward_placements"
+def _check_demand_args(who: str, state, demands, policy: int, metric: int, bound, prepared, max_impact):
+    """Host-side checks shared by forward_placements and forward_provision; returns (D, P)."""
     if int(max_impact) != max_impact or max_impact < 0:
         raise ValueError(f"{who}: max_impact must be a non-negative integer")
     if policy not in (PLACE_FIRST_FIT, PLACE_BEST_QOT, PLACE_MAX_MARGIN):
@@ -567,6 +562,19 @@ def lightpath_placements(state, demands, policy: int, metric: int, maximize: boo
     N = int(state.batch.x.shape[0])
     if bound is not None and bound.shape != (N,):
         raise ValueError(f"{who}: need bound [N] with N = {N} nodes of the state batch")
+    return D, P
+
+
+def lightpath_placements(state, demands, policy: int, metric: int, maximize: bool, bound, prepared: torch.Tensor,
+                         is_lut_index: int, max_impact: int, return_all: bool = False) -> PlacementQoT:
+    """One launch of qot_lightpath_placements (the placement of each demand chosen over every free slot of its
+    options); nothing is read back (CUDA-graph capturable).  Refuses CPU tensors and mismatched devices, dtypes or
+    shapes, an unknown policy or metric and Q over PLACE_MAX_SLOTS; what can only be judged on the device comes back
+    as status bits."""
+    who = "forward_placements"
+    D, P = _check_demand_args(who, state, demands, policy, metric, bound, prepared, max_impact)
+    dev = state.batch.x.device
+    d = demands
     max_impact = int(max_impact)
     Q = state.Q
     i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=dev)
@@ -588,6 +596,69 @@ def lightpath_placements(state, demands, policy: int, metric: int, maximize: boo
             ptr(res.margin), ptr(res.n_free), ptr(res.n_feasible), ptr(res.status), ptr(res.n_impact),
             _cptr(res.impact_node), _cptr(res.impact_out), _cptr(res.all_out), _cptr(res.all_margin), stream()),
             "qot_lightpath_placements")
+    return res
+
+
+# status bits of qot_lightpath_provision, on top of the CAND_* bits
+PROV_FULL, PROV_BAD_GROUPING = 512, 1024
+TG_MAX_NODES, TG_MAX_CHANNELS = 256, 6144      # QOT_TG_MAX_NODES / QOT_TG_MAX_CHANNELS: a sample's graph capacity
+
+
+class ProvisionQoT(NamedTuple):
+    option: torch.Tensor         # [D] int32: the chosen option, relative to opt_ptr[d] (-1: no feasible placement)
+    q0: torch.Tensor             # [D] int32: its start slot (-1: none)
+    out: torch.Tensor            # [D,3]: the chosen placement's own QoT (NaN: none)
+    margin: torch.Tensor         # [D]: its margin (NaN: none)
+    n_free: torch.Tensor         # [D] int32: free placements over the demand's options
+    n_feasible: torch.Tensor     # [D] int32: feasible placements among them
+    status: torch.Tensor         # [D] int32, CAND_* | PROV_* bits
+    n_impact: torch.Tensor       # [D] int32: lightpaths the chosen placement interferes with (may exceed max_impact)
+    impact_conn: torch.Tensor    # [D, max_impact] int64: their conn_ids, ascending in node order; -1 past the rows
+    impact_out: torch.Tensor     # [D, max_impact, 3]: their QoT with the placement set up; NaN past the rows
+    conn_id: torch.Tensor        # [D] int64: the conn_id the demand was accepted under (-1: not accepted)
+
+
+def provision_grouping(sample: torch.Tensor, S: int):
+    """(order [D], sample_ptr [S+1]) int64: the demands grouped by sample, ascending within a sample (a stable sort),
+    samples outside [0, S) after the last range.  Device tensor ops, no host synchronisation."""
+    key = torch.where((sample >= 0) & (sample < S), sample, torch.full_like(sample, S))
+    skey, order = torch.sort(key, stable=True)
+    sample_ptr = torch.searchsorted(skey, torch.arange(S + 1, dtype=torch.int64, device=sample.device))
+    return order, sample_ptr
+
+
+def lightpath_provision(state, demands, policy: int, metric: int, maximize: bool, bound, prepared: torch.Tensor,
+                        is_lut_index: int, max_impact: int) -> ProvisionQoT:
+    """qot_lightpath_provision: each sample's demands placed in index order, each against the state with the earlier
+    accepted ones set up.  The grouping is computed on the device and the work arrays allocated here; one copy and one
+    launch, nothing read back (CUDA-graph capturable).  The host checks of ``lightpath_placements``."""
+    who = "forward_provision"
+    D, P = _check_demand_args(who, state, demands, policy, metric, bound, prepared, max_impact)
+    dev = state.batch.x.device
+    d = demands
+    max_impact = int(max_impact)
+    i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=dev)
+    f32 = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)
+    res = ProvisionQoT(i32(D), i32(D), f32(D, 3), f32(D), i32(D), i32(D), i32(D), i32(D),
+                       torch.empty(D, max_impact, dtype=torch.int64, device=dev), f32(D, max_impact, 3),
+                       torch.empty(D, dtype=torch.int64, device=dev))
+    if D == 0:
+        return res
+    order, sample_ptr = provision_grouping(d.sample, state.S)
+    keep = [t.contiguous() for t in (d.sample, d.opt_ptr, d.link_ptr, d.links, d.width, d.feat, d.own_bound)]
+    chan_work = torch.empty_like(state.chan_node)
+    bound_work = f32(state.S, TG_MAX_NODES) if bound is not None else None
+    if bound is not None:
+        keep.append(bound.contiguous())
+    with torch.cuda.device(dev):
+        check(_lib.lib().qot_lightpath_provision(
+            *_state_args(state, keep), ptr(state.conn_ids) if state.conn_ids.numel() else None, D, ptr(keep[0]),
+            ptr(order), ptr(sample_ptr), ptr(keep[1]), P, ptr(keep[2]), _cptr(keep[3]), int(keep[3].numel()),
+            _cptr(keep[4]), _cptr(keep[5]), _cptr(keep[6]), _cptr(bound), int(metric), int(bool(maximize)),
+            int(policy), ptr(prepared), int(is_lut_index), max_impact, _cptr(chan_work), _cptr(bound_work),
+            ptr(res.option), ptr(res.q0), ptr(res.out), ptr(res.margin), ptr(res.n_free), ptr(res.n_feasible),
+            ptr(res.status), ptr(res.n_impact), ptr(res.conn_id), _cptr(res.impact_conn), _cptr(res.impact_out),
+            stream()), "qot_lightpath_provision")
     return res
 
 

@@ -249,3 +249,48 @@ def lightpath_network_state(data: torch.Tensor, freqs: torch.Tensor, lp_feat: Se
     _track_status("qot_lightpath_channel_map (an occupied channel's conn_id is not among its sample's lightpaths)",
                   status)
     return LightpathNetworkState(batch, conn_ids, chan_node, rowptr, freqs, cfg, S, L, Q)
+
+
+def commit_provision(data: torch.Tensor, state: LightpathNetworkState, demands: LightpathDemands,
+                     res) -> LightpathNetworkState:
+    """Writes the demands ``LightpathGNN.forward_provision`` accepted (``res.conn_id >= 0``) into ``data`` [S, F, L, Q]
+    (float32, CUDA, the samples ``state`` was built from) in place, on the device, and returns
+    ``lightpath_network_state`` of the written samples: the state the next demand of each sample would be placed
+    against.  Each accepted demand goes onto its chosen route x ``[q0, q0 + width)`` with conn_id ``res.conn_id[d]``,
+    freq ``float32(state.freqs[q0])``, the option's (mod_order, num_spans, path_len), osnr = snr = ber = -1 and every
+    other row 0.  The new state is the builder's by construction (node order by first channel, so a new lightpath
+    lands among the existing nodes).  Not capturable: one host synchronisation gathers the written channels, and the
+    rebuild keeps the builder's own."""
+    if not (data.is_cuda and data.dtype == torch.float32 and data.is_contiguous()):
+        raise TypeError("commit_provision: data must be a contiguous float32 CUDA tensor (it is written in place)")
+    S, F, L, Q = (int(v) for v in data.shape)
+    if (S, L, Q) != (state.S, state.L, state.Q):
+        raise ValueError("commit_provision: data must be the [S, F, L, Q] samples the state was built from")
+    cfg, d, dev = state.cfg, demands, data.device
+    # chosen[p] = the accepted demand whose chosen option is p (an option belongs to one demand), else -1
+    P = int(d.width.shape[0])
+    acc = res.conn_id >= 0
+    po = d.opt_ptr[:-1] + res.option.to(torch.int64)
+    chosen = torch.full((P + 1,), -1, dtype=torch.int64, device=dev)
+    chosen.scatter_(0, torch.where(acc, po, torch.full_like(po, P)), torch.arange(po.shape[0], device=dev))
+    chosen[P] = -1
+    # every (route entry, slot) an accepted demand occupies; accepted placements of a sample are disjoint
+    opt = torch.searchsorted(d.link_ptr, torch.arange(d.links.shape[0], device=dev), right=True) - 1
+    dm = chosen[opt]
+    q0 = res.q0[dm.clamp(min=0)].to(torch.int64)
+    q = torch.arange(Q, device=dev)
+    on = (dm >= 0)[:, None] & (q[None, :] >= q0[:, None]) & (q[None, :] < (q0 + d.width[opt])[:, None])
+    e, c = on.nonzero(as_tuple=True)                            # the host synchronisation
+    dm, p = dm[e], opt[e]
+    vec = torch.zeros(int(e.shape[0]), F, dtype=torch.float32, device=dev)
+    vec[:, cfg.i_conn] = res.conn_id[dm].to(torch.float32)
+    vec[:, cfg.i_feat[0]] = state.freqs[q0[e]].to(torch.float32)
+    for k in range(3):
+        vec[:, cfg.i_feat[k + 1]] = d.feat[p, k]
+    vec[:, cfg.i_osnr] = vec[:, cfg.i_snr] = vec[:, cfg.i_ber] = -1.0
+    data[d.sample[dm], :, d.links[e].to(torch.int64), c] = vec
+    names = [f"row{f}" for f in range(F)]                       # the builder reads only the rows cfg names
+    names[cfg.i_conn], names[cfg.i_osnr], names[cfg.i_snr], names[cfg.i_ber] = "conn_id", "osnr", "snr", "ber"
+    for k, name in enumerate(("freq", "mod_order", "num_spans", "path_len")):
+        names[cfg.i_feat[k]] = name
+    return lightpath_network_state(data, state.freqs, names, float(cfg.freq_threshold))

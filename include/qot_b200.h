@@ -667,6 +667,43 @@ int qot_lightpath_placements(const qot_lp_graph_cfg_t* cfg, int64_t S, const dou
                              int32_t* status, int32_t* n_impact, int64_t* impact_node, float* impact_out,
                              float* all_out, float* all_margin, void* stream);
 
+/* qot_lightpath_provision (lp_provision_kernel, one block per sample, persistent over samples): sequential
+ * provisioning.  The demands and arguments of qot_lightpath_placements, plus order [D] / sample_ptr [S+1] int64, the
+ * demands grouped by sample: sample s's demands are order[sample_ptr[s] .. sample_ptr[s+1]), ascending, and the
+ * ranges hold every demand whose sample lies in [0, S).  Samples are independent; the demands of one sample are
+ * provisioned in that order, demand d placed exactly as qot_lightpath_placements places it against state_d, the state
+ * built from the samples with every earlier accepted demand of d's sample written in.  An accepted demand is written
+ * as qot_lightpath_candidates writes a candidate: its chosen option's route x [q0, q0 + width), conn_id one above the
+ * sample's largest (top + 1, top + 2, ... for successive acceptances; conn_ids [N] is the state's), freq =
+ * float32(freqs[q0]), the option's (mod_order, num_spans, path_len), osnr = snr = ber = -1.  With a bound, an accepted
+ * demand's impact rows are bound from then on by its option's own_bound.  A demand is accepted when it has a feasible
+ * placement and no status bit but IMPACT_OVERFLOW; otherwise it commits nothing and the sample's later demands go on.
+ * Outputs per demand as qot_lightpath_placements (no all_out / all_margin), bit-identical to its result against
+ * state_d, except: impact_conn [D, max_impact] int64 names the impact rows by conn_id (-1 past the rows), and conn_id
+ * [D] int64 is the id the demand was accepted under (-1: not accepted).  Status bits QOT_CAND_* as there, plus:
+ *   QOT_PROV_FULL           accepting would take the sample past QOT_TG_MAX_NODES lightpaths or QOT_TG_MAX_CHANNELS
+ *                           occupied channels (the graph builder refuses such a sample): not accepted, the placement
+ *                           is still reported;
+ *   QOT_PROV_BAD_GROUPING   order / sample_ptr are not such a grouping: no demand is provisioned, every demand gets
+ *                           this status alone, -1 / NaN rows and zero counts.
+ * A demand whose sample lies outside [0, S) gets BAD_SAMPLE.  Work arrays: chan_work [S, L, Q] int32 (the entry point
+ * copies chan_node into it, the kernel writes the accepted channels) and bound_work [S, QOT_TG_MAX_NODES] float32
+ * (required with a bound, else unused).  The state is not modified.  One copy and one launch, nothing read back:
+ * capturable; a malformed demand or grouping never faults and never stops the launch. */
+#define QOT_PROV_FULL 512
+#define QOT_PROV_BAD_GROUPING 1024
+int qot_lightpath_provision(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
+                            const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N,
+                            int64_t E, const int32_t* chan_node, const int64_t* conn_ids, int64_t D,
+                            const int64_t* sample, const int64_t* order, const int64_t* sample_ptr,
+                            const int64_t* opt_ptr, int64_t P, const int64_t* link_ptr, const int32_t* links,
+                            int64_t n_links, const int32_t* width, const float* feat, const float* own_bound,
+                            const float* bound, int32_t metric, int32_t maximize, int32_t policy,
+                            const float* prepared, int32_t is_lut_index, int32_t max_impact, int32_t* chan_work,
+                            float* bound_work, int32_t* option, int32_t* q0, float* out, float* margin,
+                            int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact,
+                            int64_t* conn_id, int64_t* impact_conn, float* impact_out, void* stream);
+
 /* The topological representation: to_graph.py::create_topological_graph (:62-184: one edge per
  * lightpath between its source and destination network node, lightpaths added in ascending conn_id,
  * nx.Graph keeps one edge per node pair -- position from the first, attributes from the last) fused
