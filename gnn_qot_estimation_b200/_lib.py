@@ -37,6 +37,23 @@ class QotLpGraphCfg(C.Structure):
                 ("freq_threshold", C.c_double)]
 
 
+class QotLpState(C.Structure):
+    _fields_ = [("cfg", QotLpGraphCfg), ("S", i64), ("N", i64), ("E", i64),
+                ("freqs", P), ("x", P), ("node_ptr", P), ("rowptr", P), ("edge_index", P), ("chan_node", P),
+                ("conn_ids", P)]
+
+
+class QotLpChanges(C.Structure):
+    _fields_ = [("K", i64), ("n_links", i64),
+                ("node", P), ("sample", P), ("link_ptr", P), ("links", P), ("q0", P), ("width", P), ("feat", P)]
+
+
+class QotLpDemands(C.Structure):
+    _fields_ = [("D", i64), ("P", i64), ("n_links", i64),
+                ("sample", P), ("opt_ptr", P), ("link_ptr", P), ("links", P), ("width", P), ("feat", P),
+                ("own_bound", P)]
+
+
 class QotLightpathParams(C.Structure):
     _fields_ = [("lin_w", P), ("att_src", P), ("att_dst", P), ("conv_bias", P),
                 ("bn_w", P), ("bn_b", P), ("bn_mean", P), ("bn_var", P),
@@ -108,18 +125,16 @@ SIGNATURES = {
     "qot_lightpath_graph_count": (C.c_int, [P, P, P, i64, C.POINTER(QotLpGraphCfg), P, P, P, sz, P, vp]),
     "qot_lightpath_graph_fill": (C.c_int, [P, i64, P, P, P, P, P, P, P, vp]),
     "qot_lightpath_channel_map": (C.c_int, [P, i64, C.POINTER(QotLpGraphCfg), P, P, i64, P, P, vp]),
-    "qot_lightpath_candidates": (C.c_int, [C.POINTER(QotLpGraphCfg), i64, P, P, P, P, P, i64, i64, P, i64, P, P, P,
-                                           i64, P, P, P, P, i32, i32, P, P, P, P, P, vp]),
-    "qot_lightpath_reconfigure": (C.c_int, [C.POINTER(QotLpGraphCfg), i64, P, P, P, P, P, i64, i64, P, i64, P, P, P,
-                                            P, i64, P, P, P, P, i32, i32, P, P, P, P, P, P, vp]),
-    "qot_lightpath_change_sets": (C.c_int, [C.POINTER(QotLpGraphCfg), i64, P, P, P, P, P, i64, i64, P, i64, P, P, P,
-                                            P, i64, P, P, P, i64, P, P, i32, i32, P, P, P, P, P, P, P, vp]),
-    "qot_lightpath_placements": (C.c_int, [C.POINTER(QotLpGraphCfg), i64, P, P, P, P, P, i64, i64, P, i64, P, P, i64,
-                                           P, P, i64, P, P, P, P, i32, i32, i32, P, i32, i32, P, P, P, P, P, P, P, P,
-                                           P, P, P, P, vp]),
-    "qot_lightpath_provision": (C.c_int, [C.POINTER(QotLpGraphCfg), i64, P, P, P, P, P, i64, i64, P, P, i64, P, P, P,
-                                          P, i64, P, P, i64, P, P, P, P, i32, i32, i32, P, i32, i32, P, P, P, P, P, P,
-                                          P, P, P, P, P, P, P, vp]),
+    "qot_lightpath_candidates": (C.c_int, [C.POINTER(QotLpState), C.POINTER(QotLpChanges), P, i32, i32, P, P, P, P, P,
+                                           vp]),
+    "qot_lightpath_reconfigure": (C.c_int, [C.POINTER(QotLpState), C.POINTER(QotLpChanges), P, i32, i32, P, P, P, P,
+                                            P, P, vp]),
+    "qot_lightpath_change_sets": (C.c_int, [C.POINTER(QotLpState), C.POINTER(QotLpChanges), i64, P, P, i32, i32, P, P,
+                                            P, P, P, P, P, vp]),
+    "qot_lightpath_placements": (C.c_int, [C.POINTER(QotLpState), C.POINTER(QotLpDemands), P, i32, i32, i32, P, i32,
+                                           i32, P, P, P, P, P, P, P, P, P, P, P, P, vp]),
+    "qot_lightpath_provision": (C.c_int, [C.POINTER(QotLpState), C.POINTER(QotLpDemands), P, P, P, i32, i32, i32, P,
+                                          i32, i32, P, P, P, P, P, P, P, P, P, P, P, P, P, vp]),
     "qot_topological_graph_scratch_bytes": (sz, [i64]),
     "qot_topological_graph_count": (C.c_int, [P, P, i64, C.POINTER(QotLpGraphCfg), i32, i32, i32, P, P, P, sz, P, vp]),
     "qot_topological_graph_fill": (C.c_int, [P, i64, P, P, P, P, P, vp]),

@@ -15,4 +15,4 @@ void set_error(const char* fmt, ...) {
 }  // namespace qot
 
 extern "C" const char* qot_last_error(void) { return qot::g_err; }
-extern "C" int qot_version(void) { return 100; }
+extern "C" int qot_version(void) { return 101; }

@@ -1559,11 +1559,13 @@ static int cfg_check(const qot_lp_graph_cfg_t* cfg, const char* who) {
   return QOT_OK;
 }
 
-// the checks every network-state entry point makes first: cfg, the sizes (sizes_ok), the head's table, the flag column
-static int cd_check_args(const char* who, const qot_lp_graph_cfg_t* cfg, bool sizes_ok, const float* prepared,
-                         int32_t is_lut_index) {
-  if (int rc = cfg_check(cfg, who)) return rc;
-  QOT_REQUIRE(sizes_ok, "%s: bad size", who);
+// the checks every network-state entry point makes first: cfg, the sizes (the state's, max_impact and the query's,
+// query_ok), the head's table, the flag column
+static int cd_check_args(const char* who, const qot_lp_state_t& st, bool query_ok, const float* prepared,
+                         int32_t is_lut_index, int32_t max_impact) {
+  if (int rc = cfg_check(&st.cfg, who)) return rc;
+  QOT_REQUIRE(st.S >= 0 && st.N >= 0 && st.N < INT_MAX && st.E >= 0 && max_impact >= 0 && query_ok, "%s: bad size",
+              who);
   QOT_REQUIRE(prepared && (reinterpret_cast<uintptr_t>(prepared) & 15) == 0, "%s: prepared must be 16-byte aligned",
               who);
   QOT_REQUIRE(is_lut_index >= 0 && is_lut_index < kF, "%s: is_lut_index out of range", who);
@@ -1581,184 +1583,75 @@ static int cd_smem_opt_in() {
 }
 
 // the state half of CdArgs (with the head's table and the output width), after the null-state check
-static int cd_state_args(const char* who, CdArgs& a, const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs,
-                         const float* x, const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index,
-                         int64_t N, int64_t E, const int32_t* chan_node, const float* prepared, int32_t is_lut_index,
-                         int32_t max_impact) {
-  QOT_REQUIRE(S == 0 || (freqs && x && node_ptr && rowptr && chan_node && (E == 0 || edge_index)),
+static int cd_state_args(const char* who, CdArgs& a, const qot_lp_state_t& st, const float* prepared,
+                         int32_t is_lut_index, int32_t max_impact) {
+  QOT_REQUIRE(st.S == 0 ||
+                  (st.freqs && st.x && st.node_ptr && st.rowptr && st.chan_node && (st.E == 0 || st.edge_index)),
               "%s: null state array", who);
-  a.cfg = *cfg;
-  a.S = S; a.N = N; a.E = E;
-  a.freqs = freqs; a.x = x; a.node_ptr = node_ptr; a.rowptr = rowptr;
-  a.edst = edge_index ? edge_index + E : nullptr;
-  a.chan_node = chan_node;
+  a.cfg = st.cfg;
+  a.S = st.S; a.N = st.N; a.E = st.E;
+  a.freqs = st.freqs; a.x = st.x; a.node_ptr = st.node_ptr; a.rowptr = st.rowptr;
+  a.edst = st.edge_index ? st.edge_index + st.E : nullptr;
+  a.chan_node = st.chan_node;
   a.prep = prepared; a.lut_col = is_lut_index; a.max_impact = max_impact;
+  return QOT_OK;
+}
+
+// the checks the three change entry points make before their empty-query return (sizes_ok: their own sizes), then the
+// change half of CdArgs
+static int cd_change_args(const char* who, CdArgs& a, const qot_lp_state_t* st, const qot_lp_changes_t* c,
+                          bool sizes_ok, const float* prepared, int32_t is_lut_index, int32_t max_impact) {
+  QOT_REQUIRE(st && c, "%s: null state or changes descriptor", who);
+  if (int rc = cd_check_args(who, *st, c->K >= 0 && c->n_links >= 0 && sizes_ok, prepared, is_lut_index, max_impact))
+    return rc;
+  a.K = c->K; a.n_links = c->n_links;
+  a.node = c->node;
+  a.sample = c->sample; a.link_ptr = c->link_ptr; a.links = c->links; a.q0 = c->q0; a.width = c->width;
+  a.feat = c->feat;
+  return QOT_OK;
+}
+
+// the checks the two demand entry points make before their empty-query return, then the demand half of PlArgs
+static int pl_demand_args(const char* who, PlArgs& pa, const qot_lp_state_t* st, const qot_lp_demands_t* d,
+                          int32_t metric, int32_t maximize, int32_t policy, const float* prepared, int32_t is_lut_index,
+                          int32_t max_impact) {
+  QOT_REQUIRE(st && d, "%s: null state or demands descriptor", who);
+  if (int rc = cd_check_args(who, *st, d->D >= 0 && d->P >= 0 && d->n_links >= 0, prepared, is_lut_index, max_impact))
+    return rc;
+  QOT_REQUIRE(st->cfg.Q <= QOT_PLACE_MAX_SLOTS, "%s: Q = %d over QOT_PLACE_MAX_SLOTS", who, st->cfg.Q);
+  QOT_REQUIRE(metric >= 0 && metric < QOT_OUT, "%s: metric must be an output column 0..2", who);
+  QOT_REQUIRE(policy == QOT_PLACE_FIRST_FIT || policy == QOT_PLACE_BEST_QOT || policy == QOT_PLACE_MAX_MARGIN,
+              "%s: unknown policy %d", who, policy);
+  CdArgs& a = pa.c;
+  a.K = d->D; a.n_links = d->n_links;
+  a.node = nullptr;
+  a.sample = d->sample; a.link_ptr = d->link_ptr; a.links = d->links; a.q0 = nullptr; a.width = d->width;
+  a.feat = d->feat;
+  a.impact_kind = nullptr;
+  pa.P = d->P; pa.opt_ptr = d->opt_ptr; pa.own_bound = d->own_bound;
+  pa.metric = metric; pa.maximize = maximize != 0; pa.policy = policy;
   return QOT_OK;
 }
 
 // qot_lightpath_candidates (kMove = false) and qot_lightpath_reconfigure (kMove = true)
 template <bool kMove>
-static int cd_launch(const char* who, const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
-                     const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N, int64_t E,
-                     const int32_t* chan_node, int64_t K, const int64_t* node, const int64_t* sample,
-                     const int64_t* link_ptr, const int32_t* links, int64_t n_links, const int32_t* q0,
-                     const int32_t* width, const float* feat, const float* prepared, int32_t is_lut_index,
-                     int32_t max_impact, float* out, int32_t* status, int32_t* n_impact, int64_t* impact_node,
-                     int8_t* impact_kind, float* impact_out, cudaStream_t stream) {
-  if (int rc = cd_check_args(who, cfg, S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && K >= 0 && n_links >= 0 &&
-                                           max_impact >= 0, prepared, is_lut_index))
-    return rc;
-  if (K == 0) return QOT_OK;
-  QOT_REQUIRE(sample && link_ptr && q0 && width && feat && out && status && n_impact && (n_links == 0 || links) &&
-                  (max_impact == 0 || (impact_node && impact_out)) && (!kMove || node),
-              "%s: null candidate or output array", who);
+static int cd_launch(const char* who, const qot_lp_state_t* state, const qot_lp_changes_t* changes,
+                     const float* prepared, int32_t is_lut_index, int32_t max_impact, float* out, int32_t* status,
+                     int32_t* n_impact, int64_t* impact_node, int8_t* impact_kind, float* impact_out, void* stream) {
   CdArgs a;
-  if (int rc = cd_state_args(who, a, cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, prepared,
-                             is_lut_index, max_impact))
-    return rc;
+  if (int rc = cd_change_args(who, a, state, changes, true, prepared, is_lut_index, max_impact)) return rc;
+  const qot_lp_changes_t& c = *changes;
+  if (c.K == 0) return QOT_OK;
+  QOT_REQUIRE(c.sample && c.link_ptr && c.q0 && c.width && c.feat && out && status && n_impact &&
+                  (c.n_links == 0 || c.links) && (max_impact == 0 || (impact_node && impact_out)) && (!kMove || c.node),
+              "%s: null candidate or output array", who);
+  if (int rc = cd_state_args(who, a, *state, prepared, is_lut_index, max_impact)) return rc;
   constexpr int smem = static_cast<int>(sizeof(CdSmem));
   if (int rc = cd_smem_opt_in<lp_candidate_kernel<kMove>, smem>()) return rc;
-  a.K = K; a.n_links = n_links;
-  a.node = node;
-  a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = q0; a.width = width; a.feat = feat;
   a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_node;
   a.impact_kind = max_impact ? impact_kind : nullptr; a.impact_out = impact_out;
-  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, cdiv(K, kCdWarps)));
-  lp_candidate_kernel<kMove><<<grid, kCdThreads, smem, stream>>>(a);
-  QOT_LAUNCH_CHECK();
-  return QOT_OK;
-}
-
-static int cs_launch(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
-                     const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N, int64_t E,
-                     const int32_t* chan_node, int64_t K, const int64_t* node, const int64_t* sample,
-                     const int64_t* link_ptr, const int32_t* links, int64_t n_links, const int32_t* q0,
-                     const int32_t* width, const float* feat, int64_t G, const int64_t* set_ptr, const float* prepared,
-                     int32_t is_lut_index, int32_t max_impact, float* out, int32_t* status, int32_t* set_status,
-                     int32_t* n_impact, int64_t* impact_node, int8_t* impact_kind, float* impact_out,
-                     cudaStream_t stream) {
-  const char* who = "qot_lightpath_change_sets";
-  if (int rc = cd_check_args(who, cfg, S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && K >= 0 && G >= 0 &&
-                                           n_links >= 0 && max_impact >= 0, prepared, is_lut_index))
-    return rc;
-  if (G == 0 && K == 0) return QOT_OK;
-  QOT_REQUIRE(set_ptr && (G == 0 || (set_status && n_impact && (max_impact == 0 || (impact_node && impact_out)))),
-              "%s: null set or set output array", who);
-  QOT_REQUIRE(K == 0 || (node && sample && link_ptr && q0 && width && feat && out && status && (n_links == 0 || links)),
-              "%s: null change or change output array", who);
-  CsArgs ca;
-  CdArgs& a = ca.c;
-  if (int rc = cd_state_args(who, a, cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, prepared,
-                             is_lut_index, max_impact))
-    return rc;
-  constexpr int smem = static_cast<int>(sizeof(CsSmem));
-  if (int rc = cd_smem_opt_in<lp_change_set_kernel, smem>()) return rc;
-  a.K = K; a.n_links = n_links;
-  a.node = node;
-  a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = q0; a.width = width; a.feat = feat;
-  a.out = nullptr; a.status = set_status; a.n_impact = n_impact; a.impact_node = impact_node;
-  a.impact_kind = max_impact ? impact_kind : nullptr; a.impact_out = impact_out;
-  ca.G = G; ca.set_ptr = set_ptr; ca.chg_out = out; ca.chg_status = status;
-  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, std::max<int64_t>(1, cdiv(G, kCdWarps))));
-  lp_change_set_kernel<<<grid, kCdThreads, smem, stream>>>(ca);
-  QOT_LAUNCH_CHECK();
-  return QOT_OK;
-}
-
-static int pl_launch(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
-                     const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N, int64_t E,
-                     const int32_t* chan_node, int64_t D, const int64_t* sample, const int64_t* opt_ptr, int64_t P,
-                     const int64_t* link_ptr, const int32_t* links, int64_t n_links, const int32_t* width,
-                     const float* feat, const float* own_bound, const float* bound, int32_t metric, int32_t maximize,
-                     int32_t policy, const float* prepared, int32_t is_lut_index, int32_t max_impact, int32_t* option,
-                     int32_t* q0, float* out, float* margin, int32_t* n_free, int32_t* n_feasible, int32_t* status,
-                     int32_t* n_impact, int64_t* impact_node, float* impact_out, float* all_out, float* all_margin,
-                     cudaStream_t stream) {
-  const char* who = "qot_lightpath_placements";
-  if (int rc = cd_check_args(who, cfg, S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && D >= 0 && P >= 0 &&
-                                           n_links >= 0 && max_impact >= 0, prepared, is_lut_index))
-    return rc;
-  QOT_REQUIRE(cfg->Q <= QOT_PLACE_MAX_SLOTS, "%s: Q = %d over QOT_PLACE_MAX_SLOTS", who, cfg->Q);
-  QOT_REQUIRE(metric >= 0 && metric < QOT_OUT, "%s: metric must be an output column 0..2", who);
-  QOT_REQUIRE(policy == QOT_PLACE_FIRST_FIT || policy == QOT_PLACE_BEST_QOT || policy == QOT_PLACE_MAX_MARGIN,
-              "%s: unknown policy %d", who, policy);
-  if (D == 0) return QOT_OK;
-  QOT_REQUIRE(sample && opt_ptr && link_ptr && (P == 0 || (width && feat && own_bound)) && (n_links == 0 || links),
-              "%s: null demand array", who);
-  QOT_REQUIRE(option && q0 && out && margin && n_free && n_feasible && status && n_impact &&
-                  (max_impact == 0 || (impact_node && impact_out)) && (!all_out == !all_margin),
-              "%s: null output array", who);
-  PlArgs pa;
-  CdArgs& a = pa.c;
-  if (int rc = cd_state_args(who, a, cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, prepared,
-                             is_lut_index, max_impact))
-    return rc;
-  constexpr int smem = static_cast<int>(sizeof(PlSmem));
-  if (int rc = cd_smem_opt_in<lp_placement_kernel, smem>()) return rc;
-  a.K = D; a.n_links = n_links;
-  a.node = nullptr;
-  a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = nullptr; a.width = width; a.feat = feat;
-  a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_node;
-  a.impact_kind = nullptr; a.impact_out = impact_out;
-  pa.P = P; pa.opt_ptr = opt_ptr; pa.own_bound = own_bound; pa.bound = bound;
-  pa.metric = metric; pa.maximize = maximize != 0; pa.policy = policy;
-  pa.option = option; pa.q0 = q0; pa.margin = margin; pa.n_free = n_free; pa.n_feasible = n_feasible;
-  pa.all_out = all_out; pa.all_margin = all_margin;
-  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, cdiv(D, kCdWarps)));
-  lp_placement_kernel<<<grid, kCdThreads, smem, stream>>>(pa);
-  QOT_LAUNCH_CHECK();
-  return QOT_OK;
-}
-
-static int pv_launch(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
-                     const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N, int64_t E,
-                     const int32_t* chan_node, const int64_t* conn_ids, int64_t D, const int64_t* sample,
-                     const int64_t* order, const int64_t* sample_ptr, const int64_t* opt_ptr, int64_t P,
-                     const int64_t* link_ptr, const int32_t* links, int64_t n_links, const int32_t* width,
-                     const float* feat, const float* own_bound, const float* bound, int32_t metric, int32_t maximize,
-                     int32_t policy, const float* prepared, int32_t is_lut_index, int32_t max_impact,
-                     int32_t* chan_work, float* bound_work, int32_t* option, int32_t* q0, float* out, float* margin,
-                     int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact, int64_t* conn_id,
-                     int64_t* impact_conn, float* impact_out, cudaStream_t stream) {
-  const char* who = "qot_lightpath_provision";
-  if (int rc = cd_check_args(who, cfg, S >= 0 && N >= 0 && N < INT_MAX && E >= 0 && D >= 0 && P >= 0 &&
-                                           n_links >= 0 && max_impact >= 0, prepared, is_lut_index))
-    return rc;
-  QOT_REQUIRE(cfg->Q <= QOT_PLACE_MAX_SLOTS, "%s: Q = %d over QOT_PLACE_MAX_SLOTS", who, cfg->Q);
-  QOT_REQUIRE(metric >= 0 && metric < QOT_OUT, "%s: metric must be an output column 0..2", who);
-  QOT_REQUIRE(policy == QOT_PLACE_FIRST_FIT || policy == QOT_PLACE_BEST_QOT || policy == QOT_PLACE_MAX_MARGIN,
-              "%s: unknown policy %d", who, policy);
-  if (D == 0) return QOT_OK;
-  QOT_REQUIRE(sample && order && sample_ptr && opt_ptr && link_ptr && (P == 0 || (width && feat && own_bound)) &&
-                  (n_links == 0 || links), "%s: null demand or grouping array", who);
-  QOT_REQUIRE(option && q0 && out && margin && n_free && n_feasible && status && n_impact && conn_id &&
-                  (max_impact == 0 || (impact_conn && impact_out)), "%s: null output array", who);
-  QOT_REQUIRE((S == 0 || chan_work) && (!bound || S == 0 || bound_work) && (N == 0 || conn_ids),
-              "%s: null work or conn_ids array", who);
-  PvArgs va;
-  PlArgs& pa = va.p;
-  CdArgs& a = pa.c;
-  if (int rc = cd_state_args(who, a, cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_work, prepared,
-                             is_lut_index, max_impact))
-    return rc;
-  constexpr int smem = static_cast<int>(sizeof(PvSmem));
-  if (int rc = cd_smem_opt_in<lp_provision_kernel, smem>()) return rc;
-  if (S > 0)
-    QOT_CUDA(cudaMemcpyAsync(chan_work, chan_node, static_cast<size_t>(S) * cfg->L * cfg->Q * sizeof(int32_t),
-                             cudaMemcpyDeviceToDevice, stream));
-  a.K = D; a.n_links = n_links;
-  a.node = nullptr;
-  a.sample = sample; a.link_ptr = link_ptr; a.links = links; a.q0 = nullptr; a.width = width; a.feat = feat;
-  a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_conn;
-  a.impact_kind = nullptr; a.impact_out = impact_out;
-  pa.P = P; pa.opt_ptr = opt_ptr; pa.own_bound = own_bound; pa.bound = bound ? bound_work : nullptr;
-  pa.metric = metric; pa.maximize = maximize != 0; pa.policy = policy;
-  pa.option = option; pa.q0 = q0; pa.margin = margin; pa.n_free = n_free; pa.n_feasible = n_feasible;
-  pa.all_out = nullptr; pa.all_margin = nullptr;
-  va.order = order; va.sample_ptr = sample_ptr; va.conn_ids = conn_ids; va.bound = bound;
-  va.chan_work = chan_work; va.bound_work = bound ? bound_work : nullptr; va.conn_id = conn_id;
-  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, std::max<int64_t>(1, S)));
-  lp_provision_kernel<<<grid, kCdThreads, smem, stream>>>(va);
+  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, cdiv(c.K, kCdWarps)));
+  lp_candidate_kernel<kMove><<<grid, kCdThreads, smem, static_cast<cudaStream_t>(stream)>>>(a);
   QOT_LAUNCH_CHECK();
   return QOT_OK;
 }
@@ -1782,85 +1675,122 @@ extern "C" int qot_lightpath_channel_map(const float* data, int64_t S, const qot
   return QOT_OK;
 }
 
-extern "C" int qot_lightpath_candidates(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs,
-                                        const float* x, const int64_t* node_ptr, const int64_t* rowptr,
-                                        const int64_t* edge_index, int64_t N, int64_t E, const int32_t* chan_node,
-                                        int64_t K, const int64_t* sample, const int64_t* link_ptr,
-                                        const int32_t* links, int64_t n_links, const int32_t* q0,
-                                        const int32_t* width, const float* feat, const float* prepared,
-                                        int32_t is_lut_index, int32_t max_impact, float* out, int32_t* status,
-                                        int32_t* n_impact, int64_t* impact_node, float* impact_out,
-                                        void* stream_) {
-  return cd_launch<false>("qot_lightpath_candidates", cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node,
-                          K, nullptr, sample, link_ptr, links, n_links, q0, width, feat, prepared, is_lut_index,
-                          max_impact, out, status, n_impact, impact_node, nullptr, impact_out,
-                          static_cast<cudaStream_t>(stream_));
+extern "C" int qot_lightpath_candidates(const qot_lp_state_t* state, const qot_lp_changes_t* cands,
+                                        const float* prepared, int32_t is_lut_index, int32_t max_impact, float* out,
+                                        int32_t* status, int32_t* n_impact, int64_t* impact_node, float* impact_out,
+                                        void* stream) {
+  return cd_launch<false>("qot_lightpath_candidates", state, cands, prepared, is_lut_index, max_impact, out, status,
+                          n_impact, impact_node, nullptr, impact_out, stream);
 }
 
-extern "C" int qot_lightpath_reconfigure(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs,
-                                         const float* x, const int64_t* node_ptr, const int64_t* rowptr,
-                                         const int64_t* edge_index, int64_t N, int64_t E, const int32_t* chan_node,
-                                         int64_t K, const int64_t* node, const int64_t* sample,
-                                         const int64_t* link_ptr, const int32_t* links, int64_t n_links,
-                                         const int32_t* q0, const int32_t* width, const float* feat,
+extern "C" int qot_lightpath_reconfigure(const qot_lp_state_t* state, const qot_lp_changes_t* changes,
                                          const float* prepared, int32_t is_lut_index, int32_t max_impact, float* out,
                                          int32_t* status, int32_t* n_impact, int64_t* impact_node,
-                                         int8_t* impact_kind, float* impact_out, void* stream_) {
-  return cd_launch<true>("qot_lightpath_reconfigure", cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E,
-                         chan_node, K, node, sample, link_ptr, links, n_links, q0, width, feat, prepared,
-                         is_lut_index, max_impact, out, status, n_impact, impact_node, impact_kind, impact_out,
-                         static_cast<cudaStream_t>(stream_));
+                                         int8_t* impact_kind, float* impact_out, void* stream) {
+  return cd_launch<true>("qot_lightpath_reconfigure", state, changes, prepared, is_lut_index, max_impact, out, status,
+                         n_impact, impact_node, impact_kind, impact_out, stream);
 }
 
-extern "C" int qot_lightpath_change_sets(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs,
-                                         const float* x, const int64_t* node_ptr, const int64_t* rowptr,
-                                         const int64_t* edge_index, int64_t N, int64_t E, const int32_t* chan_node,
-                                         int64_t K, const int64_t* node, const int64_t* sample,
-                                         const int64_t* link_ptr, const int32_t* links, int64_t n_links,
-                                         const int32_t* q0, const int32_t* width, const float* feat, int64_t G,
+extern "C" int qot_lightpath_change_sets(const qot_lp_state_t* state, const qot_lp_changes_t* changes, int64_t G,
                                          const int64_t* set_ptr, const float* prepared, int32_t is_lut_index,
                                          int32_t max_impact, float* out, int32_t* status, int32_t* set_status,
                                          int32_t* n_impact, int64_t* impact_node, int8_t* impact_kind,
-                                         float* impact_out, void* stream_) {
-  return cs_launch(cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, K, node, sample, link_ptr, links,
-                   n_links, q0, width, feat, G, set_ptr, prepared, is_lut_index, max_impact, out, status, set_status,
-                   n_impact, impact_node, impact_kind, impact_out, static_cast<cudaStream_t>(stream_));
+                                         float* impact_out, void* stream) {
+  const char* who = "qot_lightpath_change_sets";
+  CsArgs ca;
+  CdArgs& a = ca.c;
+  if (int rc = cd_change_args(who, a, state, changes, G >= 0, prepared, is_lut_index, max_impact)) return rc;
+  const qot_lp_changes_t& c = *changes;
+  if (G == 0 && c.K == 0) return QOT_OK;
+  QOT_REQUIRE(set_ptr && (G == 0 || (set_status && n_impact && (max_impact == 0 || (impact_node && impact_out)))),
+              "%s: null set or set output array", who);
+  QOT_REQUIRE(c.K == 0 || (c.node && c.sample && c.link_ptr && c.q0 && c.width && c.feat && out && status &&
+                           (c.n_links == 0 || c.links)),
+              "%s: null change or change output array", who);
+  if (int rc = cd_state_args(who, a, *state, prepared, is_lut_index, max_impact)) return rc;
+  constexpr int smem = static_cast<int>(sizeof(CsSmem));
+  if (int rc = cd_smem_opt_in<lp_change_set_kernel, smem>()) return rc;
+  a.out = nullptr; a.status = set_status; a.n_impact = n_impact; a.impact_node = impact_node;
+  a.impact_kind = max_impact ? impact_kind : nullptr; a.impact_out = impact_out;
+  ca.G = G; ca.set_ptr = set_ptr; ca.chg_out = out; ca.chg_status = status;
+  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, std::max<int64_t>(1, cdiv(G, kCdWarps))));
+  lp_change_set_kernel<<<grid, kCdThreads, smem, static_cast<cudaStream_t>(stream)>>>(ca);
+  QOT_LAUNCH_CHECK();
+  return QOT_OK;
 }
 
-extern "C" int qot_lightpath_placements(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs,
-                                        const float* x, const int64_t* node_ptr, const int64_t* rowptr,
-                                        const int64_t* edge_index, int64_t N, int64_t E, const int32_t* chan_node,
-                                        int64_t D, const int64_t* sample, const int64_t* opt_ptr, int64_t P,
-                                        const int64_t* link_ptr, const int32_t* links, int64_t n_links,
-                                        const int32_t* width, const float* feat, const float* own_bound,
+extern "C" int qot_lightpath_placements(const qot_lp_state_t* state, const qot_lp_demands_t* demands,
                                         const float* bound, int32_t metric, int32_t maximize, int32_t policy,
                                         const float* prepared, int32_t is_lut_index, int32_t max_impact,
                                         int32_t* option, int32_t* q0, float* out, float* margin, int32_t* n_free,
                                         int32_t* n_feasible, int32_t* status, int32_t* n_impact,
                                         int64_t* impact_node, float* impact_out, float* all_out, float* all_margin,
-                                        void* stream_) {
-  return pl_launch(cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, D, sample, opt_ptr, P, link_ptr,
-                   links, n_links, width, feat, own_bound, bound, metric, maximize, policy, prepared, is_lut_index,
-                   max_impact, option, q0, out, margin, n_free, n_feasible, status, n_impact, impact_node, impact_out,
-                   all_out, all_margin, static_cast<cudaStream_t>(stream_));
+                                        void* stream) {
+  const char* who = "qot_lightpath_placements";
+  PlArgs pa;
+  CdArgs& a = pa.c;
+  if (int rc = pl_demand_args(who, pa, state, demands, metric, maximize, policy, prepared, is_lut_index, max_impact))
+    return rc;
+  const qot_lp_demands_t& d = *demands;
+  if (d.D == 0) return QOT_OK;
+  QOT_REQUIRE(d.sample && d.opt_ptr && d.link_ptr && (d.P == 0 || (d.width && d.feat && d.own_bound)) &&
+                  (d.n_links == 0 || d.links),
+              "%s: null demand array", who);
+  QOT_REQUIRE(option && q0 && out && margin && n_free && n_feasible && status && n_impact &&
+                  (max_impact == 0 || (impact_node && impact_out)) && (!all_out == !all_margin),
+              "%s: null output array", who);
+  if (int rc = cd_state_args(who, a, *state, prepared, is_lut_index, max_impact)) return rc;
+  constexpr int smem = static_cast<int>(sizeof(PlSmem));
+  if (int rc = cd_smem_opt_in<lp_placement_kernel, smem>()) return rc;
+  a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_node; a.impact_out = impact_out;
+  pa.bound = bound;
+  pa.option = option; pa.q0 = q0; pa.margin = margin; pa.n_free = n_free; pa.n_feasible = n_feasible;
+  pa.all_out = all_out; pa.all_margin = all_margin;
+  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, cdiv(d.D, kCdWarps)));
+  lp_placement_kernel<<<grid, kCdThreads, smem, static_cast<cudaStream_t>(stream)>>>(pa);
+  QOT_LAUNCH_CHECK();
+  return QOT_OK;
 }
 
-extern "C" int qot_lightpath_provision(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
-                                       const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index,
-                                       int64_t N, int64_t E, const int32_t* chan_node, const int64_t* conn_ids,
-                                       int64_t D, const int64_t* sample, const int64_t* order,
-                                       const int64_t* sample_ptr, const int64_t* opt_ptr, int64_t P,
-                                       const int64_t* link_ptr, const int32_t* links, int64_t n_links,
-                                       const int32_t* width, const float* feat, const float* own_bound,
-                                       const float* bound, int32_t metric, int32_t maximize, int32_t policy,
-                                       const float* prepared, int32_t is_lut_index, int32_t max_impact,
-                                       int32_t* chan_work, float* bound_work, int32_t* option, int32_t* q0,
-                                       float* out, float* margin, int32_t* n_free, int32_t* n_feasible,
-                                       int32_t* status, int32_t* n_impact, int64_t* conn_id, int64_t* impact_conn,
-                                       float* impact_out, void* stream_) {
-  return pv_launch(cfg, S, freqs, x, node_ptr, rowptr, edge_index, N, E, chan_node, conn_ids, D, sample, order,
-                   sample_ptr, opt_ptr, P, link_ptr, links, n_links, width, feat, own_bound, bound, metric, maximize,
-                   policy, prepared, is_lut_index, max_impact, chan_work, bound_work, option, q0, out, margin, n_free,
-                   n_feasible, status, n_impact, conn_id, impact_conn, impact_out,
-                   static_cast<cudaStream_t>(stream_));
+extern "C" int qot_lightpath_provision(const qot_lp_state_t* state, const qot_lp_demands_t* demands,
+                                       const int64_t* order, const int64_t* sample_ptr, const float* bound,
+                                       int32_t metric, int32_t maximize, int32_t policy, const float* prepared,
+                                       int32_t is_lut_index, int32_t max_impact, int32_t* chan_work, float* bound_work,
+                                       int32_t* option, int32_t* q0, float* out, float* margin, int32_t* n_free,
+                                       int32_t* n_feasible, int32_t* status, int32_t* n_impact, int64_t* conn_id,
+                                       int64_t* impact_conn, float* impact_out, void* stream_) {
+  const char* who = "qot_lightpath_provision";
+  PvArgs va;
+  PlArgs& pa = va.p;
+  CdArgs& a = pa.c;
+  if (int rc = pl_demand_args(who, pa, state, demands, metric, maximize, policy, prepared, is_lut_index, max_impact))
+    return rc;
+  const qot_lp_state_t& st = *state;
+  const qot_lp_demands_t& d = *demands;
+  if (d.D == 0) return QOT_OK;
+  QOT_REQUIRE(d.sample && order && sample_ptr && d.opt_ptr && d.link_ptr &&
+                  (d.P == 0 || (d.width && d.feat && d.own_bound)) && (d.n_links == 0 || d.links),
+              "%s: null demand or grouping array", who);
+  QOT_REQUIRE(option && q0 && out && margin && n_free && n_feasible && status && n_impact && conn_id &&
+                  (max_impact == 0 || (impact_conn && impact_out)), "%s: null output array", who);
+  QOT_REQUIRE((st.S == 0 || chan_work) && (!bound || st.S == 0 || bound_work) && (st.N == 0 || st.conn_ids),
+              "%s: null work or conn_ids array", who);
+  if (int rc = cd_state_args(who, a, st, prepared, is_lut_index, max_impact)) return rc;
+  constexpr int smem = static_cast<int>(sizeof(PvSmem));
+  if (int rc = cd_smem_opt_in<lp_provision_kernel, smem>()) return rc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (st.S > 0)
+    QOT_CUDA(cudaMemcpyAsync(chan_work, st.chan_node, static_cast<size_t>(st.S) * st.cfg.L * st.cfg.Q * sizeof(int32_t),
+                             cudaMemcpyDeviceToDevice, stream));
+  a.chan_node = chan_work;
+  a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_conn; a.impact_out = impact_out;
+  pa.bound = bound ? bound_work : nullptr;
+  pa.option = option; pa.q0 = q0; pa.margin = margin; pa.n_free = n_free; pa.n_feasible = n_feasible;
+  pa.all_out = nullptr; pa.all_margin = nullptr;
+  va.order = order; va.sample_ptr = sample_ptr; va.conn_ids = st.conn_ids; va.bound = bound;
+  va.chan_work = chan_work; va.bound_work = bound ? bound_work : nullptr; va.conn_id = conn_id;
+  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, std::max<int64_t>(1, st.S)));
+  lp_provision_kernel<<<grid, kCdThreads, smem, stream>>>(va);
+  QOT_LAUNCH_CHECK();
+  return QOT_OK;
 }

@@ -156,12 +156,7 @@ class LightpathGNN(torch.nn.Module):
         a bad path or slot range, or an occupied channel gives a NaN row and no impact rows; more than ``max_impact``
         neighbours keeps the first ``max_impact`` rows and reports the true count in ``n_impact``.
         One launch, nothing read back: capturable in a CUDA graph.  Malformed arguments raise on the host."""
-        if self.training:
-            raise RuntimeError("LightpathGNN.forward_candidates is eval-only (in training mode BatchNorm couples the "
-                               "nodes): call model.eval()")
-        if not state.batch.x.is_cuda:
-            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
-        self._check_supported()
+        self._check_state_query("forward_candidates", state)
         return ops.lightpath_candidates(state, cands, self.prepared(), self.is_lut_index, max_impact)
 
     @_lib.on_tensor_device
@@ -181,12 +176,7 @@ class LightpathGNN(torch.nn.Module):
         ``forward_candidates``.  Changes are evaluated independently, each against the state alone.  ``status`` holds
         ``ops.CAND_*`` bits (``CAND_BAD_NODE``: the node is not in the sample; j's own channels are not OCCUPIED).
         One launch, nothing read back: capturable in a CUDA graph.  Malformed arguments raise on the host."""
-        if self.training:
-            raise RuntimeError("LightpathGNN.forward_reconfigurations is eval-only (in training mode BatchNorm couples "
-                               "the nodes): call model.eval()")
-        if not state.batch.x.is_cuda:
-            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
-        self._check_supported()
+        self._check_state_query("forward_reconfigurations", state)
         return ops.lightpath_reconfigure(state, changes, self.prepared(), self.is_lut_index, max_impact)
 
     @_lib.on_tensor_device
@@ -209,12 +199,7 @@ class LightpathGNN(torch.nn.Module):
         OR; any bit but ``CAND_IMPACT_OVERFLOW`` makes the whole set NaN with ``n_impact`` 0.  A set of one change is
         bit-identical to ``forward_reconfigurations``.  One launch, nothing read back: capturable in a CUDA graph.
         Malformed arguments raise on the host."""
-        if self.training:
-            raise RuntimeError("LightpathGNN.forward_change_sets is eval-only (in training mode BatchNorm couples the "
-                               "nodes): call model.eval()")
-        if not state.batch.x.is_cuda:
-            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
-        self._check_supported()
+        self._check_state_query("forward_change_sets", state)
         return ops.lightpath_change_sets(state, changes, set_ptr, self.prepared(), self.is_lut_index, max_impact)
 
     @_lib.on_tensor_device
@@ -242,15 +227,11 @@ class LightpathGNN(torch.nn.Module):
         3] and ``all_margin`` [P, Q], every free placement's own row and margin, NaN at the other slots of the demands'
         options.  Q is at most ``ops.PLACE_MAX_SLOTS``.  One launch, nothing read back: capturable in a CUDA graph.
         Malformed arguments raise on the host."""
-        if self.training:
-            raise RuntimeError("LightpathGNN.forward_placements is eval-only (in training mode BatchNorm couples the "
-                               "nodes): call model.eval()")
-        if not state.batch.x.is_cuda:
-            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
-        self._check_supported()
+        self._check_state_query("forward_placements", state)
         return ops.lightpath_placements(state, demands, policy, metric, maximize, bound, self.prepared(),
                                         self.is_lut_index, max_impact, return_all)
 
+    @_lib.on_tensor_device
     def forward_provision(self, state, demands, policy: int, metric: int = 0, maximize: bool = True, bound=None,
                           max_impact: int = 64) -> "ops.ProvisionQoT":
         """Sequential provisioning of lightpath demands (eval mode only; csrc/lightpath_candidates.cu,
@@ -275,12 +256,7 @@ class LightpathGNN(torch.nn.Module):
         placement still reported).  ``state`` is not modified; ``to_graph.commit_provision`` writes the accepted
         demands into the samples.  One copy and one launch, nothing read back: capturable in a CUDA graph.  Malformed
         arguments raise on the host."""
-        if self.training:
-            raise RuntimeError("LightpathGNN.forward_provision is eval-only (in training mode BatchNorm couples the "
-                               "nodes): call model.eval()")
-        if not state.batch.x.is_cuda:
-            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
-        self._check_supported()
+        self._check_state_query("forward_provision", state)
         return ops.lightpath_provision(state, demands, policy, metric, maximize, bound, self.prepared(),
                                        self.is_lut_index, max_impact)
 
@@ -307,6 +283,15 @@ class LightpathGNN(torch.nn.Module):
         if n_lut == 0:
             raise ValueError("No LUT node found in the batch.")
         return res.out[:n_lut].clone(), res.lut_batch[:n_lut].clone()   # the plan's buffers are reused by the next call
+
+    def _check_state_query(self, who: str, state):
+        """The checks every network-state query makes first: eval mode, the state on CUDA, the supported shape."""
+        if self.training:
+            raise RuntimeError(f"LightpathGNN.{who} is eval-only (in training mode BatchNorm couples the nodes): "
+                               "call model.eval()")
+        if not state.batch.x.is_cuda:
+            raise RuntimeError("LightpathGNN (B200) needs the network state on a CUDA device; there is no CPU path")
+        self._check_supported()
 
     def _check_supported(self):
         c = self.conv1

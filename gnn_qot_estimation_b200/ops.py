@@ -414,13 +414,24 @@ def _check_candidate_args(state, c, prepared, max_impact, who: str, arg: str, wa
     return K
 
 
-def _state_args(state, keep: list):
-    """The state's leading arguments of qot_lightpath_candidates / _reconfigure; converted tensors go into `keep`."""
+def _state_desc(state, keep: list) -> "_lib.QotLpState":
+    """The qot_lp_state_t of a ``LightpathNetworkState``; converted tensors go into `keep`.  Built on every call, never
+    cached on the state: a state made with ``_replace`` must not reuse another state's pointers."""
     b = state.batch
     x, ei = _f32(b.x), _i64(b.edge_index)
     keep += [x, ei]
-    return (C.byref(state.cfg), state.S, ptr(state.freqs), ptr(x), ptr(b.ptr), ptr(state.rowptr),
-            ptr(ei) if ei.numel() else None, int(x.shape[0]), int(ei.shape[1]), ptr(state.chan_node))
+    return _lib.QotLpState(state.cfg, state.S, int(x.shape[0]), int(ei.shape[1]), ptr(state.freqs), ptr(x), ptr(b.ptr),
+                           ptr(state.rowptr), ptr(ei) if ei.numel() else None, ptr(state.chan_node),
+                           ptr(state.conn_ids) if state.conn_ids.numel() else None)
+
+
+def _changes_desc(c, K: int, keep: list) -> "_lib.QotLpChanges":
+    """The qot_lp_changes_t of ``LightpathChanges`` or ``LightpathCandidates`` (node NULL); contiguous tensors go into
+    `keep`."""
+    node = getattr(c, "node", None)
+    ts = [None if t is None else t.contiguous() for t in (node, c.sample, c.link_ptr, c.links, c.q0, c.width, c.feat)]
+    keep += ts
+    return _lib.QotLpChanges(K, int(c.links.numel()), *(_cptr(t) for t in ts))
 
 
 def lightpath_candidates(state, cands, prepared: torch.Tensor, is_lut_index: int, max_impact: int) -> CandidateQoT:
@@ -436,13 +447,12 @@ def lightpath_candidates(state, cands, prepared: torch.Tensor, is_lut_index: int
     impact_out = torch.empty(K, max_impact, 3, dtype=torch.float32, device=dev)
     if K == 0:
         return CandidateQoT(out, status, n_impact, impact_node, impact_out)
-    keep = [t.contiguous() for t in cands]           # alive until the launch is enqueued
+    keep = []                                        # alive until the launch is enqueued
     with torch.cuda.device(dev):                     # stream() of the state's device
         check(_lib.lib().qot_lightpath_candidates(
-            *_state_args(state, keep), K,
-            ptr(keep[0]), ptr(keep[1]), _cptr(keep[2]), int(keep[2].numel()), ptr(keep[3]), ptr(keep[4]), ptr(keep[5]),
-            ptr(prepared), int(is_lut_index), max_impact, ptr(out), ptr(status), ptr(n_impact),
-            _cptr(impact_node), _cptr(impact_out), stream()), "qot_lightpath_candidates")
+            C.byref(_state_desc(state, keep)), C.byref(_changes_desc(cands, K, keep)), ptr(prepared),
+            int(is_lut_index), max_impact, ptr(out), ptr(status), ptr(n_impact), _cptr(impact_node),
+            _cptr(impact_out), stream()), "qot_lightpath_candidates")
     return CandidateQoT(out, status, n_impact, impact_node, impact_out)
 
 
@@ -461,14 +471,12 @@ def lightpath_reconfigure(state, changes, prepared: torch.Tensor, is_lut_index: 
     impact_out = torch.empty(K, max_impact, 3, dtype=torch.float32, device=dev)
     if K == 0:
         return ReconfigQoT(out, status, n_impact, impact_node, impact_kind, impact_out)
-    ch = changes
-    keep = [t.contiguous() for t in (ch.node, ch.sample, ch.link_ptr, ch.links, ch.q0, ch.width, ch.feat)]
+    keep = []
     with torch.cuda.device(dev):
         check(_lib.lib().qot_lightpath_reconfigure(
-            *_state_args(state, keep), K, ptr(keep[0]),
-            ptr(keep[1]), ptr(keep[2]), _cptr(keep[3]), int(keep[3].numel()), ptr(keep[4]), ptr(keep[5]), ptr(keep[6]),
-            ptr(prepared), int(is_lut_index), max_impact, ptr(out), ptr(status), ptr(n_impact),
-            _cptr(impact_node), _cptr(impact_kind), _cptr(impact_out), stream()), "qot_lightpath_reconfigure")
+            C.byref(_state_desc(state, keep)), C.byref(_changes_desc(changes, K, keep)), ptr(prepared),
+            int(is_lut_index), max_impact, ptr(out), ptr(status), ptr(n_impact), _cptr(impact_node),
+            _cptr(impact_kind), _cptr(impact_out), stream()), "qot_lightpath_reconfigure")
     return ReconfigQoT(out, status, n_impact, impact_node, impact_kind, impact_out)
 
 
@@ -496,14 +504,13 @@ def lightpath_change_sets(state, changes, set_ptr: torch.Tensor, prepared: torch
     res = ChangeSetQoT(out, status, set_status, n_impact, impact_node, impact_kind, impact_out)
     if K == 0 and G == 0:
         return res
-    ch = changes
-    keep = [t.contiguous() for t in (ch.node, ch.sample, ch.link_ptr, ch.links, ch.q0, ch.width, ch.feat, set_ptr)]
+    keep = [set_ptr.contiguous()]
     with torch.cuda.device(dev):
         check(_lib.lib().qot_lightpath_change_sets(
-            *_state_args(state, keep), K, _cptr(keep[0]), _cptr(keep[1]), ptr(keep[2]), _cptr(keep[3]),
-            int(keep[3].numel()), _cptr(keep[4]), _cptr(keep[5]), _cptr(keep[6]), G, ptr(keep[7]), ptr(prepared),
-            int(is_lut_index), max_impact, _cptr(out), _cptr(status), _cptr(set_status), _cptr(n_impact),
-            _cptr(impact_node), _cptr(impact_kind), _cptr(impact_out), stream()), "qot_lightpath_change_sets")
+            C.byref(_state_desc(state, keep)), C.byref(_changes_desc(changes, K, keep)), G, ptr(keep[0]),
+            ptr(prepared), int(is_lut_index), max_impact, _cptr(out), _cptr(status), _cptr(set_status),
+            _cptr(n_impact), _cptr(impact_node), _cptr(impact_kind), _cptr(impact_out), stream()),
+            "qot_lightpath_change_sets")
     return res
 
 
@@ -565,6 +572,22 @@ def _check_demand_args(who: str, state, demands, policy: int, metric: int, bound
     return D, P
 
 
+def _demands_desc(d, D: int, P: int, keep: list) -> "_lib.QotLpDemands":
+    """The qot_lp_demands_t of ``LightpathDemands``; contiguous tensors go into `keep`."""
+    ts = [t.contiguous() for t in (d.sample, d.opt_ptr, d.link_ptr, d.links, d.width, d.feat, d.own_bound)]
+    keep += ts
+    return _lib.QotLpDemands(D, P, int(d.links.numel()), *(_cptr(t) for t in ts))
+
+
+def _demand_outputs(D: int, max_impact: int, dev) -> list:
+    """Uninitialised outputs of a demand query, in PlacementQoT / ProvisionQoT field order: option, q0, out, margin,
+    n_free, n_feasible, status, n_impact, the impact rows' ids [D, max_impact] int64 and impact_out."""
+    i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=dev)
+    f32 = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)
+    return [i32(D), i32(D), f32(D, 3), f32(D), i32(D), i32(D), i32(D), i32(D),
+            torch.empty(D, max_impact, dtype=torch.int64, device=dev), f32(D, max_impact, 3)]
+
+
 def lightpath_placements(state, demands, policy: int, metric: int, maximize: bool, bound, prepared: torch.Tensor,
                          is_lut_index: int, max_impact: int, return_all: bool = False) -> PlacementQoT:
     """One launch of qot_lightpath_placements (the placement of each demand chosen over every free slot of its
@@ -574,28 +597,21 @@ def lightpath_placements(state, demands, policy: int, metric: int, maximize: boo
     who = "forward_placements"
     D, P = _check_demand_args(who, state, demands, policy, metric, bound, prepared, max_impact)
     dev = state.batch.x.device
-    d = demands
     max_impact = int(max_impact)
-    Q = state.Q
-    i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=dev)
     f32 = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)
-    res = PlacementQoT(i32(D), i32(D), f32(D, 3), f32(D), i32(D), i32(D), i32(D), i32(D),
-                       torch.empty(D, max_impact, dtype=torch.int64, device=dev), f32(D, max_impact, 3),
-                       f32(P, Q, 3) if return_all else None, f32(P, Q) if return_all else None)
+    res = PlacementQoT(*_demand_outputs(D, max_impact, dev), f32(P, state.Q, 3) if return_all else None,
+                       f32(P, state.Q) if return_all else None)
     if D == 0:
         return res
-    keep = [t.contiguous() for t in (d.sample, d.opt_ptr, d.link_ptr, d.links, d.width, d.feat, d.own_bound)]
-    if bound is not None:
-        keep.append(bound.contiguous())
+    bound = None if bound is None else bound.contiguous()
+    keep = []
     with torch.cuda.device(dev):
         check(_lib.lib().qot_lightpath_placements(
-            *_state_args(state, keep), D, ptr(keep[0]), ptr(keep[1]), P, ptr(keep[2]), _cptr(keep[3]),
-            int(keep[3].numel()), _cptr(keep[4]), _cptr(keep[5]), _cptr(keep[6]), _cptr(bound), int(metric),
-            int(bool(maximize)),
-            int(policy), ptr(prepared), int(is_lut_index), max_impact, ptr(res.option), ptr(res.q0), ptr(res.out),
-            ptr(res.margin), ptr(res.n_free), ptr(res.n_feasible), ptr(res.status), ptr(res.n_impact),
-            _cptr(res.impact_node), _cptr(res.impact_out), _cptr(res.all_out), _cptr(res.all_margin), stream()),
-            "qot_lightpath_placements")
+            C.byref(_state_desc(state, keep)), C.byref(_demands_desc(demands, D, P, keep)), _cptr(bound),
+            int(metric), int(bool(maximize)), int(policy), ptr(prepared), int(is_lut_index), max_impact,
+            ptr(res.option), ptr(res.q0), ptr(res.out), ptr(res.margin), ptr(res.n_free), ptr(res.n_feasible),
+            ptr(res.status), ptr(res.n_impact), _cptr(res.impact_node), _cptr(res.impact_out), _cptr(res.all_out),
+            _cptr(res.all_margin), stream()), "qot_lightpath_placements")
     return res
 
 
@@ -635,30 +651,22 @@ def lightpath_provision(state, demands, policy: int, metric: int, maximize: bool
     who = "forward_provision"
     D, P = _check_demand_args(who, state, demands, policy, metric, bound, prepared, max_impact)
     dev = state.batch.x.device
-    d = demands
     max_impact = int(max_impact)
-    i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=dev)
-    f32 = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)
-    res = ProvisionQoT(i32(D), i32(D), f32(D, 3), f32(D), i32(D), i32(D), i32(D), i32(D),
-                       torch.empty(D, max_impact, dtype=torch.int64, device=dev), f32(D, max_impact, 3),
-                       torch.empty(D, dtype=torch.int64, device=dev))
+    res = ProvisionQoT(*_demand_outputs(D, max_impact, dev), torch.empty(D, dtype=torch.int64, device=dev))
     if D == 0:
         return res
-    order, sample_ptr = provision_grouping(d.sample, state.S)
-    keep = [t.contiguous() for t in (d.sample, d.opt_ptr, d.link_ptr, d.links, d.width, d.feat, d.own_bound)]
+    order, sample_ptr = provision_grouping(demands.sample, state.S)
     chan_work = torch.empty_like(state.chan_node)
-    bound_work = f32(state.S, TG_MAX_NODES) if bound is not None else None
-    if bound is not None:
-        keep.append(bound.contiguous())
+    bound_work = torch.empty(state.S, TG_MAX_NODES, dtype=torch.float32, device=dev) if bound is not None else None
+    bound = None if bound is None else bound.contiguous()
+    keep = []
     with torch.cuda.device(dev):
         check(_lib.lib().qot_lightpath_provision(
-            *_state_args(state, keep), ptr(state.conn_ids) if state.conn_ids.numel() else None, D, ptr(keep[0]),
-            ptr(order), ptr(sample_ptr), ptr(keep[1]), P, ptr(keep[2]), _cptr(keep[3]), int(keep[3].numel()),
-            _cptr(keep[4]), _cptr(keep[5]), _cptr(keep[6]), _cptr(bound), int(metric), int(bool(maximize)),
-            int(policy), ptr(prepared), int(is_lut_index), max_impact, _cptr(chan_work), _cptr(bound_work),
-            ptr(res.option), ptr(res.q0), ptr(res.out), ptr(res.margin), ptr(res.n_free), ptr(res.n_feasible),
-            ptr(res.status), ptr(res.n_impact), ptr(res.conn_id), _cptr(res.impact_conn), _cptr(res.impact_out),
-            stream()), "qot_lightpath_provision")
+            C.byref(_state_desc(state, keep)), C.byref(_demands_desc(demands, D, P, keep)), ptr(order),
+            ptr(sample_ptr), _cptr(bound), int(metric), int(bool(maximize)), int(policy), ptr(prepared),
+            int(is_lut_index), max_impact, _cptr(chan_work), _cptr(bound_work), ptr(res.option), ptr(res.q0),
+            ptr(res.out), ptr(res.margin), ptr(res.n_free), ptr(res.n_feasible), ptr(res.status), ptr(res.n_impact),
+            ptr(res.conn_id), _cptr(res.impact_conn), _cptr(res.impact_out), stream()), "qot_lightpath_provision")
     return res
 
 

@@ -525,6 +525,54 @@ int qot_lightpath_graph_fill(const void* scratch, int64_t S, const int64_t* node
 int qot_lightpath_channel_map(const float* data, int64_t S, const qot_lp_graph_cfg_t* cfg, const int64_t* node_ptr,
                               const int64_t* conn_ids, int64_t N, int32_t* chan_node, int32_t* status, void* stream);
 
+/* The five network-state queries below take the state and their inputs as host structs (read during the call, not
+ * retained); the pointers in them are device pointers.
+ *
+ * A resident network state: the S samples' graphs collated in sample order (to_graph.lightpath_network_state).  x
+ * [N,5], node_ptr [S+1], rowptr [N+1] int64 (node v's out-edges are [rowptr[v], rowptr[v+1]) of edge_index [2,E]
+ * int64, which must be the layout qot_lightpath_graph_fill produces: sorted by source, every edge in both directions,
+ * so a node's in-neighbours are the destinations of its out-run), chan_node from qot_lightpath_channel_map.  With S ==
+ * 0 the arrays may be NULL; edge_index may be NULL when E == 0. */
+typedef struct {
+  qot_lp_graph_cfg_t cfg;      /* the configuration the graphs were built with, by value                    */
+  int64_t S, N, E;
+  const double* freqs;         /* [Q]                                                                       */
+  const float* x;              /* [N,5]                                                                     */
+  const int64_t* node_ptr;     /* [S+1]                                                                     */
+  const int64_t* rowptr;       /* [N+1]                                                                     */
+  const int64_t* edge_index;   /* [2,E]                                                                     */
+  const int32_t* chan_node;    /* [S,L,Q]                                                                   */
+  const int64_t* conn_ids;     /* [N]; read by qot_lightpath_provision only, may be NULL elsewhere          */
+} qot_lp_state_t;              /* 264 bytes */
+
+/* Candidates, reconfigurations and change-set changes: K of them, change k naming sample[k], the path
+ * links[link_ptr[k] .. link_ptr[k+1]) (n_links entries of links in all), the slots [q0[k], q0[k] + width[k]) and the
+ * raw channel vector feat[k]; node[k] is the lightpath a change moves. */
+typedef struct {
+  int64_t K, n_links;
+  const int64_t* node;         /* [K]; ignored by qot_lightpath_candidates                                  */
+  const int64_t* sample;       /* [K]                                                                       */
+  const int64_t* link_ptr;     /* [K+1]                                                                     */
+  const int32_t* links;        /* [n_links]                                                                 */
+  const int32_t* q0;           /* [K]                                                                       */
+  const int32_t* width;        /* [K]                                                                       */
+  const float* feat;           /* [K,4]                                                                     */
+} qot_lp_changes_t;            /* 72 bytes */
+
+/* Placement and provisioning demands: D of them, demand d naming sample[d] and the options [opt_ptr[d],
+ * opt_ptr[d+1]); option p (P of them) is the route links[link_ptr[p] .. link_ptr[p+1]) (n_links entries in all), a
+ * slot width, channel features and a bound on its own metric. */
+typedef struct {
+  int64_t D, P, n_links;
+  const int64_t* sample;       /* [D]                                                                       */
+  const int64_t* opt_ptr;      /* [D+1]                                                                     */
+  const int64_t* link_ptr;     /* [P+1]                                                                     */
+  const int32_t* links;        /* [n_links]                                                                 */
+  const int32_t* width;        /* [P]                                                                       */
+  const float* feat;           /* [P,3]                                                                     */
+  const float* own_bound;      /* [P]                                                                       */
+} qot_lp_demands_t;            /* 80 bytes */
+
 /* qot_lightpath_candidates (lp_candidate_kernel): K candidates, one warp each, one launch.  Candidate k names sample
  * sample[k], a path links[link_ptr[k] .. link_ptr[k+1]) (int32 link indices; duplicates change nothing), the slot
  * range [q0[k], q0[k] + width[k]) used on every link of the path and its raw channel vector feat [K,4] = (freq,
@@ -533,16 +581,12 @@ int qot_lightpath_channel_map(const float* data, int64_t S, const qot_lp_graph_c
  * ber = -1).  In sample''s lightpath graph, with the flag column x[:, is_lut_index] one-hot:
  *   out [K,3]          row k: the reference LightpathGNN.forward under eval() with the flag at the candidate's node;
  *   impact rows        one per existing lightpath j adjacent to the candidate (sharing a link at 0 < |freqs[qc] -
- *                      freqs[qj]| < cfg->freq_threshold in fp64): the same forward with the flag at j, in ascending
+ *                      freqs[qj]| < cfg.freq_threshold in fp64): the same forward with the flag at j, in ascending
  *                      order of j's state-batch node index.  impact_node [K,max_impact] int64 = j, impact_out
  *                      [K,max_impact,3]; slots past the rows written hold -1 / NaN.  n_impact [K] int32 = the number
  *                      of neighbours (may exceed max_impact).
  * Candidates are independent of each other.  The candidate's x row is feat scaled as qot_lightpath_graph_count scales
- * node features (min-max in fp64 of the float32 value with cfg->feat_lo / feat_hi, then fp32).
- * State: freqs [Q] float64, x [N,5], node_ptr [S+1], rowptr [N+1] int64 (node v's out-edges are
- * [rowptr[v], rowptr[v+1]) of edge_index [2,E] int64, which must be the layout qot_lightpath_graph_fill produces:
- * sorted by source, every edge in both directions, so a node's in-neighbours are the destinations of its out-run),
- * chan_node from qot_lightpath_channel_map.  n_links: entries of `links`.  `prepared` as for
+ * node features (min-max in fp64 of the float32 value with cfg.feat_lo / feat_hi, then fp32).  `prepared` as for
  * qot_lightpath_infer_stream.  status [K] int32 (written for every candidate), bits QOT_CAND_*: with BAD_SAMPLE,
  * BAD_PATH, OCCUPIED or BAD_STATE before the scan ends the out row is NaN and n_impact is 0; with IMPACT_OVERFLOW the
  * out row and the first max_impact impact rows are written.  No host synchronisation: capturable; a malformed
@@ -553,12 +597,8 @@ int qot_lightpath_channel_map(const float* data, int64_t S, const qot_lp_graph_c
 #define QOT_CAND_IMPACT_OVERFLOW 8   /* more neighbours than max_impact                                           */
 #define QOT_CAND_BAD_STATE 16        /* the state arrays are inconsistent (offsets, chan_node, rowptr); the
                                         affected rows are NaN                                                     */
-int qot_lightpath_candidates(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
-                             const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N,
-                             int64_t E, const int32_t* chan_node, int64_t K, const int64_t* sample,
-                             const int64_t* link_ptr, const int32_t* links, int64_t n_links, const int32_t* q0,
-                             const int32_t* width, const float* feat, const float* prepared, int32_t is_lut_index,
-                             int32_t max_impact, float* out, int32_t* status, int32_t* n_impact,
+int qot_lightpath_candidates(const qot_lp_state_t* state, const qot_lp_changes_t* cands, const float* prepared,
+                             int32_t is_lut_index, int32_t max_impact, float* out, int32_t* status, int32_t* n_impact,
                              int64_t* impact_node, float* impact_out, void* stream);
 
 /* qot_lightpath_reconfigure (lp_candidate_kernel, the same launch shape): K changes to the state, evaluated
@@ -581,11 +621,7 @@ int qot_lightpath_candidates(const qot_lp_graph_cfg_t* cfg, int64_t S, const dou
  * its self loop; row i = i's state in-row ascending without j and without i's self loop, then j if bit 1 is set, then
  * i's self loop.  Status bits QOT_CAND_*, plus BAD_NODE; with BAD_NODE the out row is NaN and n_impact is 0. */
 #define QOT_CAND_BAD_NODE 32         /* node[k] is neither -1 nor a node of sample[k]                             */
-int qot_lightpath_reconfigure(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
-                              const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N,
-                              int64_t E, const int32_t* chan_node, int64_t K, const int64_t* node,
-                              const int64_t* sample, const int64_t* link_ptr, const int32_t* links, int64_t n_links,
-                              const int32_t* q0, const int32_t* width, const float* feat, const float* prepared,
+int qot_lightpath_reconfigure(const qot_lp_state_t* state, const qot_lp_changes_t* changes, const float* prepared,
                               int32_t is_lut_index, int32_t max_impact, float* out, int32_t* status, int32_t* n_impact,
                               int64_t* impact_node, int8_t* impact_kind, float* impact_out, void* stream);
 
@@ -617,11 +653,7 @@ int qot_lightpath_reconfigure(const qot_lp_graph_cfg_t* cfg, int64_t S, const do
                                         first), the set has more than 64 changes, or set_ptr is malformed            */
 #define QOT_SET_DUPLICATE 128        /* a lightpath is moved or torn down by two changes of the set (on both)       */
 #define QOT_SET_CONFLICT 256         /* this change's placement shares a channel with another change's placement    */
-int qot_lightpath_change_sets(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
-                              const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N,
-                              int64_t E, const int32_t* chan_node, int64_t K, const int64_t* node,
-                              const int64_t* sample, const int64_t* link_ptr, const int32_t* links, int64_t n_links,
-                              const int32_t* q0, const int32_t* width, const float* feat, int64_t G,
+int qot_lightpath_change_sets(const qot_lp_state_t* state, const qot_lp_changes_t* changes, int64_t G,
                               const int64_t* set_ptr, const float* prepared, int32_t is_lut_index, int32_t max_impact,
                               float* out, int32_t* status, int32_t* set_status, int32_t* n_impact,
                               int64_t* impact_node, int8_t* impact_kind, float* impact_out, void* stream);
@@ -656,16 +688,11 @@ int qot_lightpath_change_sets(const qot_lp_graph_cfg_t* cfg, int64_t S, const do
 #define QOT_PLACE_FIRST_FIT 0
 #define QOT_PLACE_BEST_QOT 1
 #define QOT_PLACE_MAX_MARGIN 2
-int qot_lightpath_placements(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
-                             const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N,
-                             int64_t E, const int32_t* chan_node, int64_t D, const int64_t* sample,
-                             const int64_t* opt_ptr, int64_t P, const int64_t* link_ptr, const int32_t* links,
-                             int64_t n_links, const int32_t* width, const float* feat, const float* own_bound,
-                             const float* bound, int32_t metric, int32_t maximize, int32_t policy,
-                             const float* prepared, int32_t is_lut_index, int32_t max_impact, int32_t* option,
-                             int32_t* q0, float* out, float* margin, int32_t* n_free, int32_t* n_feasible,
-                             int32_t* status, int32_t* n_impact, int64_t* impact_node, float* impact_out,
-                             float* all_out, float* all_margin, void* stream);
+int qot_lightpath_placements(const qot_lp_state_t* state, const qot_lp_demands_t* demands, const float* bound,
+                             int32_t metric, int32_t maximize, int32_t policy, const float* prepared,
+                             int32_t is_lut_index, int32_t max_impact, int32_t* option, int32_t* q0, float* out,
+                             float* margin, int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact,
+                             int64_t* impact_node, float* impact_out, float* all_out, float* all_margin, void* stream);
 
 /* qot_lightpath_provision (lp_provision_kernel, one block per sample, persistent over samples): sequential
  * provisioning.  The demands and arguments of qot_lightpath_placements, plus order [D] / sample_ptr [S+1] int64, the
@@ -692,16 +719,11 @@ int qot_lightpath_placements(const qot_lp_graph_cfg_t* cfg, int64_t S, const dou
  * capturable; a malformed demand or grouping never faults and never stops the launch. */
 #define QOT_PROV_FULL 512
 #define QOT_PROV_BAD_GROUPING 1024
-int qot_lightpath_provision(const qot_lp_graph_cfg_t* cfg, int64_t S, const double* freqs, const float* x,
-                            const int64_t* node_ptr, const int64_t* rowptr, const int64_t* edge_index, int64_t N,
-                            int64_t E, const int32_t* chan_node, const int64_t* conn_ids, int64_t D,
-                            const int64_t* sample, const int64_t* order, const int64_t* sample_ptr,
-                            const int64_t* opt_ptr, int64_t P, const int64_t* link_ptr, const int32_t* links,
-                            int64_t n_links, const int32_t* width, const float* feat, const float* own_bound,
-                            const float* bound, int32_t metric, int32_t maximize, int32_t policy,
-                            const float* prepared, int32_t is_lut_index, int32_t max_impact, int32_t* chan_work,
-                            float* bound_work, int32_t* option, int32_t* q0, float* out, float* margin,
-                            int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact,
+int qot_lightpath_provision(const qot_lp_state_t* state, const qot_lp_demands_t* demands, const int64_t* order,
+                            const int64_t* sample_ptr, const float* bound, int32_t metric, int32_t maximize,
+                            int32_t policy, const float* prepared, int32_t is_lut_index, int32_t max_impact,
+                            int32_t* chan_work, float* bound_work, int32_t* option, int32_t* q0, float* out,
+                            float* margin, int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact,
                             int64_t* conn_id, int64_t* impact_conn, float* impact_out, void* stream);
 
 /* The topological representation: to_graph.py::create_topological_graph (:62-184: one edge per

@@ -55,17 +55,23 @@ def test_ctypes_table_matches_header(lib_path):
 
 
 @pytest.mark.parametrize("struct,ctype,size", [("qot_sgd_hyper_t", "QotSgdHyper", 32),
-                                               ("qot_param_seg_t", "QotParamSeg", 24)])
+                                               ("qot_param_seg_t", "QotParamSeg", 24),
+                                               ("qot_lp_state_t", "QotLpState", 264),
+                                               ("qot_lp_changes_t", "QotLpChanges", 72),
+                                               ("qot_lp_demands_t", "QotLpDemands", 80)])
 def test_ctypes_structs_match_header(struct, ctype, size):
-    """Field names, order, offsets and size of the structs the kernels read from device memory."""
+    """Field names, order, offsets and size of the structs the kernels read from device memory, and of the network-state
+    queries' argument structs."""
     from gnn_qot_estimation_b200 import _lib
     text = re.sub(r"/\*.*?\*/", "", HEADER.read_text(), flags=re.S)
     body = re.search(r"typedef struct \{([^}]*)\}\s*" + struct + r"\s*;", text).group(1)
     names = [re.sub(r"\[\d+\]$", "", n.strip().lstrip("*")) for decl in body.split(";") if decl.strip()
-             for n in decl.strip().split(None, 1)[1].split(",")]
+             for n in decl.strip().removeprefix("const ").split(None, 1)[1].split(",")]
     cls = getattr(_lib, ctype)
     assert [f[0] for f in cls._fields_] == names
     assert ctypes.sizeof(cls) == size
+    if struct == "qot_lp_state_t":
+        assert cls._fields_[0][1] is _lib.QotLpGraphCfg and ctypes.sizeof(_lib.QotLpGraphCfg) == cls.S.offset == 184
     if struct == "qot_sgd_hyper_t":
         offs = {f[0]: getattr(cls, f[0]).offset for f in cls._fields_}
         assert offs == {"lr": 0, "momentum": 4, "dampening": 8, "weight_decay": 12, "nesterov": 16, "maximize": 20,
@@ -91,13 +97,48 @@ def test_cpu_arguments_fail_through_the_abi(lib_path):
     """Argument validation works without a GPU: bad sizes return QOT_E_BADARG + a message."""
     from gnn_qot_estimation_b200 import _lib
     L = _lib.lib()
-    assert L.qot_version() >= 100
+    assert L.qot_version() >= 101
     rc = L.qot_build_csr(None, -1, 4, 1, 0, None, None, None, None, None, 0, None)
     assert rc == -1 and b"negative" in L.qot_last_error()
     rc = L.qot_tconv_fwd(None, None, None, None, None, None, 10, 17, 1.0, None, None, None, None, None)
     assert rc == -1 and b"H must be" in L.qot_last_error()
     assert L.qot_csr_workspace_bytes(1000, 5000) > 0
     assert L.qot_lightpath_prepared_floats() >= 5 * 4 * 2 + 128 * 5 + 128 + 128 * 32 + 32 + 96 + 3
+
+
+STATE_QUERIES = {"qot_lightpath_candidates": 2, "qot_lightpath_reconfigure": 2, "qot_lightpath_change_sets": 4,
+                 "qot_lightpath_placements": 6, "qot_lightpath_provision": 8}      # name -> position of `prepared`
+
+
+@pytest.mark.parametrize("name", sorted(STATE_QUERIES))
+def test_state_query_arguments_fail_through_the_abi(lib_path, name):
+    """The network-state queries validate their arguments before any CUDA call: with an empty query the call returns 0
+    without a GPU, and a NULL descriptor, a negative count, a misaligned `prepared` or an `is_lut_index` out of range
+    each returns QOT_E_BADARG with a message naming the entry point."""
+    from gnn_qot_estimation_b200 import _lib
+    L = _lib.lib()
+    argtypes = _lib.SIGNATURES[name][1]
+    query_cls, at = argtypes[1]._type_, STATE_QUERIES[name]
+    assert argtypes[0] is ctypes.POINTER(_lib.QotLpState)
+    assert query_cls in (_lib.QotLpChanges, _lib.QotLpDemands)
+    assert argtypes[at:at + 3] == [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32]   # prepared, lut index, max_impact
+
+    def call(state=True, query=True, S=0, count=0, prepared=1 << 20, lut=1):
+        st = _lib.QotLpState(cfg=_lib.QotLpGraphCfg(F=8, L=4, Q=16), S=S)
+        q = query_cls(**{query_cls._fields_[0][0]: count})                      # K or D
+        args = [ctypes.byref(st) if state else None, ctypes.byref(q) if query else None]
+        args += [0 if t in (ctypes.c_int32, ctypes.c_int64) else None for t in argtypes[2:]]
+        args[at], args[at + 1] = prepared, lut
+        return getattr(L, name)(*args)
+
+    assert call() == 0
+    for bad, why in ((dict(state=False), b"descriptor"), (dict(query=False), b"descriptor"), (dict(S=-1), b"bad size"),
+                     (dict(count=-1), b"bad size"), (dict(prepared=(1 << 20) + 4), b"16-byte aligned"),
+                     (dict(prepared=None), b"16-byte aligned"), (dict(lut=5), b"is_lut_index"),
+                     (dict(lut=-1), b"is_lut_index")):
+        assert call(**bad) == -1, bad
+        msg = L.qot_last_error()
+        assert msg.startswith(name.encode() + b":") and why in msg, (bad, msg)
 
 
 def test_product_refuses_cpu_tensors():

@@ -1,6 +1,7 @@
 """CPU checks of LightpathGNN's candidate QoT: the C ABI declares and binds it, the literal reference definition
 (tests/candidates_ref.py) agrees with every-node mode by leave-one-out on the oracle, the seeded candidate generator
 uses free channels only, and the timing script's argument parsing and byte arithmetic."""
+import ctypes as C
 import importlib.util
 import re
 from pathlib import Path
@@ -24,12 +25,15 @@ def _header_arity(name):
     return m.group(1).count(",") + 1
 
 
-def test_header_declares_and_ctypes_binds_candidate_family():
+def test_candidate_family_takes_state_and_changes_structs():
     from gnn_qot_estimation_b200 import _lib, ops
     for name in CANDIDATES:
         assert name in _lib.SIGNATURES, name
         assert len(_lib.SIGNATURES[name][1]) == _header_arity(name), name
-    assert _header_arity("qot_lightpath_candidates") == 27
+    assert _header_arity("qot_lightpath_candidates") == 11
+    # the state, then the candidates
+    assert _lib.SIGNATURES["qot_lightpath_candidates"][1][:2] == [C.POINTER(_lib.QotLpState),
+                                                                  C.POINTER(_lib.QotLpChanges)]
     text = HEADER.read_text()
     bits = {name: int(re.search(r"#define " + name + r"\s+(\d+)", text).group(1))
             for name in ("QOT_CAND_BAD_SAMPLE", "QOT_CAND_BAD_PATH", "QOT_CAND_OCCUPIED", "QOT_CAND_IMPACT_OVERFLOW",

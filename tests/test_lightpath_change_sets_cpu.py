@@ -1,6 +1,7 @@
 """CPU checks of LightpathGNN's change-set QoT: the C ABI declares and binds it, the literal reference definition
 (tests/change_set_ref.py) agrees with the reconfiguration reference and with every-node mode on the oracle, the seeded
 set generator, and the timing script's arguments and byte arithmetic."""
+import ctypes as C
 import importlib.util
 import re
 from pathlib import Path
@@ -14,13 +15,14 @@ from test_lightpath_reconfig_cpu import HEADER, TOL, _every, _header_arity, _ora
 ROOT = Path(__file__).resolve().parents[1]
 
 
-def test_header_declares_and_ctypes_binds_change_sets():
+def test_change_sets_take_state_and_changes_structs():
     from gnn_qot_estimation_b200 import _lib, ops
     name = "qot_lightpath_change_sets"
     assert name in _lib.SIGNATURES
-    assert len(_lib.SIGNATURES[name][1]) == _header_arity(name) == 32
-    # the reconfiguration arguments up to feat, then G and set_ptr
-    assert _lib.SIGNATURES[name][1][:19] == _lib.SIGNATURES["qot_lightpath_reconfigure"][1][:19]
+    assert len(_lib.SIGNATURES[name][1]) == _header_arity(name) == 15
+    # the state, the changes, then G and set_ptr
+    assert _lib.SIGNATURES[name][1][:4] == [C.POINTER(_lib.QotLpState), C.POINTER(_lib.QotLpChanges), C.c_int64,
+                                            C.c_void_p]
     text = HEADER.read_text()
     bits = {n: int(re.search(r"#define QOT_SET_" + n + r"\s+(\d+)", text).group(1))
             for n in ("MAX_CHANGES", "BAD_SET", "DUPLICATE", "CONFLICT")}

@@ -1,6 +1,7 @@
 """CPU checks of LightpathGNN's placement search: the C ABI declares and binds it, the literal reference definition
 (tests/placement_ref.py) agrees with candidates_ref, with its own per-placement table and with every-node mode on the
 oracle, the seeded demand generator, and the timing script's arguments and arithmetic."""
+import ctypes as C
 import importlib.util
 import re
 from pathlib import Path
@@ -14,13 +15,13 @@ from test_lightpath_reconfig_cpu import HEADER, TOL, _every, _header_arity, _ora
 ROOT = Path(__file__).resolve().parents[1]
 
 
-def test_header_declares_and_ctypes_binds_placements():
+def test_placements_take_state_and_demands_structs():
     from gnn_qot_estimation_b200 import _lib, ops
     name = "qot_lightpath_placements"
     assert name in _lib.SIGNATURES
-    assert len(_lib.SIGNATURES[name][1]) == _header_arity(name) == 40
-    # the state arguments of the candidate entry point, in its order
-    assert _lib.SIGNATURES[name][1][:10] == _lib.SIGNATURES["qot_lightpath_candidates"][1][:10]
+    assert len(_lib.SIGNATURES[name][1]) == _header_arity(name) == 22
+    # the state, then the demands
+    assert _lib.SIGNATURES[name][1][:2] == [C.POINTER(_lib.QotLpState), C.POINTER(_lib.QotLpDemands)]
     text = HEADER.read_text()
     vals = {n: int(re.search(r"#define QOT_PLACE_" + n + r"\s+(\d+)", text).group(1))
             for n in ("MAX_OPTIONS", "MAX_SLOTS", "FIRST_FIT", "BEST_QOT", "MAX_MARGIN")}

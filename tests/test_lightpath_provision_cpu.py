@@ -1,9 +1,22 @@
-"""CPU checks of sequential provisioning's host side: the literal reference (tests/provision_ref.py) is consistent with
-placement_ref and insert_candidate, and the device grouping of demands by sample is a stable sort."""
+"""CPU checks of sequential provisioning's host side: the C ABI declares and binds it, the literal reference
+(tests/provision_ref.py) is consistent with placement_ref and insert_candidate, and the device grouping of demands by
+sample is a stable sort."""
+import ctypes as C
+
 import numpy as np
 import torch
 
 from conftest import load_golden
+from test_lightpath_reconfig_cpu import _header_arity
+
+
+def test_header_declares_and_ctypes_binds_provision():
+    from gnn_qot_estimation_b200 import _lib
+    name = "qot_lightpath_provision"
+    assert len(_lib.SIGNATURES[name][1]) == _header_arity(name) == 25
+    # the state, the demands, then the grouping
+    assert _lib.SIGNATURES[name][1][:4] == [C.POINTER(_lib.QotLpState), C.POINTER(_lib.QotLpDemands), C.c_void_p,
+                                            C.c_void_p]
 
 
 def _oracle():

@@ -342,7 +342,7 @@ def test_capacity(cuda):
 def _c_call(m, state, d, order, sample_ptr, bound=None, max_impact=4):
     """qot_lightpath_provision through the C entry point with a caller-made grouping."""
     from gnn_qot_estimation_b200 import _lib, ops
-    from gnn_qot_estimation_b200.ops import _state_args, ptr, stream
+    from gnn_qot_estimation_b200.ops import _demands_desc, _state_desc, ptr, stream
     D, P, dev = int(d.sample.shape[0]), int(d.width.shape[0]), state.batch.x.device
     res = ops.ProvisionQoT(*(torch.full((D,), 99, dtype=torch.int32, device=dev) for _ in range(2)),
                            torch.zeros(D, 3, device=dev), torch.zeros(D, device=dev),
@@ -353,16 +353,15 @@ def _c_call(m, state, d, order, sample_ptr, bound=None, max_impact=4):
     keep = []
     cw = torch.empty_like(state.chan_node)
     rc = _lib.lib().qot_lightpath_provision(
-        *_state_args(state, keep), ptr(state.conn_ids), D, ptr(d.sample), ptr(order), ptr(sample_ptr),
-        ptr(d.opt_ptr), P, ptr(d.link_ptr), ptr(d.links), int(d.links.numel()), ptr(d.width), ptr(d.feat),
-        ptr(d.own_bound), None, 0, 1, 0, ptr(m.prepared()), 1, max_impact, ptr(cw), None, ptr(res.option),
+        C.byref(_state_desc(state, keep)), C.byref(_demands_desc(d, D, P, keep)), ptr(order),
+        ptr(sample_ptr), None, 0, 1, 0, ptr(m.prepared()), 1, max_impact, ptr(cw), None, ptr(res.option),
         ptr(res.q0), ptr(res.out), ptr(res.margin), ptr(res.n_free), ptr(res.n_feasible), ptr(res.status),
         ptr(res.n_impact), ptr(res.conn_id), ptr(res.impact_conn), ptr(res.impact_out), stream())
     torch.cuda.synchronize()
     return rc, res
 
 
-def test_status_bits(cuda):
+def test_status_bits_and_c_groupings_through_structs(cuda):
     """BAD_SAMPLE, BAD_PATH (each kind), BAD_STATE, IMPACT_OVERFLOW (accepted), PROV_FULL (above), BAD_GROUPING through
     the C entry point (each malformation), an empty sample and D = 0."""
     from gnn_qot_estimation_b200 import ops, synthetic

@@ -1,6 +1,7 @@
 """CPU checks of LightpathGNN's reconfiguration QoT: the C ABI declares and binds it, the literal reference definition
 (tests/reconfig_ref.py) agrees with every-node mode and with the candidate reference on the oracle, the seeded change
 generator, and the timing script's argument parsing, byte arithmetic and expansion inputs."""
+import ctypes as C
 import importlib.util
 import re
 from pathlib import Path
@@ -24,13 +25,13 @@ def _header_arity(name):
     return m.group(1).count(",") + 1
 
 
-def test_header_declares_and_ctypes_binds_reconfigure():
+def test_reconfigure_takes_state_and_changes_structs():
     from gnn_qot_estimation_b200 import _lib, ops
     name = "qot_lightpath_reconfigure"
     assert name in _lib.SIGNATURES
-    assert len(_lib.SIGNATURES[name][1]) == _header_arity(name) == 29
-    # the candidate arguments plus node and impact_kind, in the candidate order
-    assert _lib.SIGNATURES[name][1][:11] == _lib.SIGNATURES["qot_lightpath_candidates"][1][:11]
+    assert len(_lib.SIGNATURES[name][1]) == _header_arity(name) == 12
+    # the state, then the changes
+    assert _lib.SIGNATURES[name][1][:2] == [C.POINTER(_lib.QotLpState), C.POINTER(_lib.QotLpChanges)]
     bit = int(re.search(r"#define QOT_CAND_BAD_NODE\s+(\d+)", HEADER.read_text()).group(1))
     assert bit == ops.CAND_BAD_NODE == 32
     assert (ops.KIND_LOST, ops.KIND_GAINED, ops.KIND_KEPT) == (1, 2, 3)
