@@ -389,6 +389,17 @@ __device__ __noinline__ void st_generic(int cw, unsigned todo, const float* __re
       }
     }
     if (lane == 0 && found != gl1 - gl0) atomicOr(ga.status, 1);
+    // rows lut_ptr gives the graph beyond its LUT nodes: out NaN and lut_node -1, never what the buffers held (split
+    // head: lp_stream_head_kernel writes the NaN for lut_node -1)
+    for (int64_t r = orow; r < gl1; ++r) {
+      if constexpr (kHead) {
+        if (lane < QOT_OUT) ga.out[r * QOT_OUT + lane] = __int_as_float(0x7fffffff);
+      }
+      if (lane == 0) {
+        ga.lut_batch[r] = ga.g0 + s;
+        ga.lut_node[r] = -1;
+      }
+    }
   }
   __syncwarp();
   if (lane == 0) {
@@ -729,7 +740,8 @@ __device__ __forceinline__ void st_consume_tile(int k, int cw, const float* __re
       }
     }
   }
-  const bool generic = !ok && active && (!fits || (cnt == lrows && cnt > 0));
+  // also a staged graph whose lut_ptr disagrees with x: the generic path fills every row lut_ptr gives it
+  const bool generic = !ok && active && (!fits || cnt > 0 || lrows > 0);
   const unsigned todo = __ballot_sync(kFull, generic && sl == 0);      // bit 8*s: graph s of this warp
   if (todo) {
     StGenericArgs& ga = gs.gargs;
@@ -1072,9 +1084,9 @@ lp_stream_head_kernel(const qot_lp_batch_t* __restrict__ batches, const float* _
     const bool va = ra < L, vb = rb < L;
     float oa, ob;
     head_rows16_tf32x3(f1, f2, zbuf + ra * (kHeads * kF), zbuf + rb * (kHeads * kF), va, vb, prep, lane, oa, ob);
-    if (t4 < QOT_OUT) {
-      if (va) out[ra * QOT_OUT + t4] = oa;
-      if (vb) out[rb * QOT_OUT + t4] = ob;
+    if (t4 < QOT_OUT) {                    // lut_node -1: lut_ptr gave the graph a row its x has no LUT node for: NaN
+      if (va) out[ra * QOT_OUT + t4] = d.lut_node[ra] < 0 ? __int_as_float(0x7fffffff) : oa;
+      if (vb) out[rb * QOT_OUT + t4] = d.lut_node[rb] < 0 ? __int_as_float(0x7fffffff) : ob;
     }
   }
 }

@@ -290,7 +290,8 @@ typedef struct {
  * ascending node order:
  *   out [L,3], lut_batch [L] int64 (graph id), lut_node [L] int32, n_lut[0] = L = lut_ptr[B].
  * status (int32[1], zeroed by the caller): bit 0 is set when lut_ptr does not describe x (a
- * graph holds a different number of LUT nodes); rows of such a graph are not written. */
+ * graph holds a different number of LUT nodes); the rows lut_ptr gives such a graph hold its LUT
+ * nodes in order as far as they go, every other row out = NaN, lut_node = -1. */
 size_t qot_lightpath_lut_ptr_workspace_bytes(int64_t B);
 int qot_lightpath_lut_ptr(const float* x, const int64_t* gptr, int64_t N, int64_t B,
                           int32_t is_lut_index, int64_t* lut_ptr, void* ws, size_t ws_bytes,
