@@ -1113,6 +1113,19 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_placement_kernel(const __gri
 //     that rank up move one place, its row and column go in, its channels into chan_work, its own_bound into
 //     bound_work (the bound of its impact rows from then on).
 // Message order and values are then those of lp_placement_kernel on the rebuilt state: bit-identical.
+//
+// Releases (qot_lightpath_traffic; none for qot_lightpath_provision): before demand d the block applies the sample's
+// releases with before <= d, after its last demand the rest.  A release finds its lightpath's rank by conn_id
+// (conn_id[demand] for a release by demand, written earlier by this block), evaluates the rows of its neighbours
+// (adj[R]'s bits by rank, each its adjacency row by rank with bit R cleared, then its self loop: the KIND_LOST rows of
+// lp_candidate_kernel<true> for the teardown) and folds their margins against bound_work, then pv_release takes the
+// lightpath out: its channels in chan_work become -1, the highest stable id takes over its freed id (stable ids stay
+// dense in [0, n_tot), which the j < n_tot checks of the route scans rely on), and rank R leaves the graph, every row's
+// bits above R moving down one place.  top is not lowered, so conn_ids are never reused within a call.
+//
+// The kernel is templated on kReleases: the release path takes the kernel from 28 to 148 bytes of spill loads, and a
+// launch without releases (qot_lightpath_provision, and qot_lightpath_traffic with R = 0) runs the code it ran before
+// releases existed.
 struct PvSmem {
   CdSmem cd;                                 // head fragments and the candidate kernel's per-warp state
   PlWarpSmem w[kCdWarps];                    // the placement kernel's per-warp search state
@@ -1130,6 +1143,10 @@ struct PvSmem {
   int n_tot, n_chan, ne, rbad, st, n_free, n_feas, acc, c_key;
   long long c_po;
   int c_q0;
+  unsigned long long n_rvalid;               // releases with a sample in [0, S), counted by the grouping check
+  long long r_conn;                          // the release's conn_id
+  int r_st, r_rank;                          // its status so far and its rank (-1: not in the sample)
+  unsigned r_mkey;                           // min of its neighbour rows' margin keys
 };
 static_assert(sizeof(PvSmem) + 16 <= 227 * 1024, "lp_provision_kernel: shared memory over the 227 KB block limit");
 static_assert(kCdThreads >= kCdMaxN + 1, "one thread per rank, and one more for the inserted row");
@@ -1144,6 +1161,15 @@ struct PvArgs {
   int32_t* chan_work;                      // [S, L, Q]
   float* bound_work;                       // [S, kCdMaxN] by stable id, or null
   int64_t* conn_id;                        // [D]
+  qot_lp_releases_t rel;                   // R = 0: none (qot_lightpath_provision)
+  const int64_t* rel_order;                // [R]: the releases grouped by sample, by (before, k) within a sample
+  const int64_t* rel_ptr;                  // [S+1], or null with R = 0
+  int32_t* rel_status;                     // [R]
+  int64_t* rel_conn_id;                    // [R]
+  int32_t* rel_n_impact;                   // [R]
+  int64_t* rel_impact_conn;                // [R, max_impact]
+  float* rel_impact_out;                   // [R, max_impact, 3]
+  float* rel_margin;                       // [R]
 };
 
 // x of a message source: rank j of the block's graph or the placement (kCand)
@@ -1173,6 +1199,104 @@ __device__ void pv_empty(const PvArgs& va, int64_t d, int st, int t, int stride)
   }
   for (int o = t; o < QOT_OUT; o += stride) a.out[d * QOT_OUT + o] = nan;
   cd_clear_impact(a, d, 0, a.max_impact, nullptr, t, stride);
+}
+
+// the empty result of release k with status st (conn_id -1, n_impact 0, margin NaN) and its impact rows from `from`
+// on (-1 / NaN), written by threads t, t + stride, ...
+__device__ void pv_rel_empty(const PvArgs& va, int64_t k, int st, int from, int t, int stride) {
+  const int MI = va.p.c.max_impact;
+  if (t == 0 && from == 0) {
+    va.rel_status[k] = st;
+    va.rel_conn_id[k] = -1;
+    va.rel_n_impact[k] = 0;
+    va.rel_margin[k] = __int_as_float(0x7fc00000);
+  }
+  for (int i = from + t; i < MI; i += stride) va.rel_impact_conn[k * MI + i] = -1;
+  for (int i = from * QOT_OUT + t; i < MI * QOT_OUT; i += stride)
+    va.rel_impact_out[k * MI * QOT_OUT + i] = __int_as_float(0x7fc00000);
+}
+
+// the staged neighbour rows of release k, in staging order: rows with a tag (their index, < max_impact) into
+// rel_impact_out, and with a bound every row's margin into r_mkey.  Lane 0.
+__device__ __noinline__ void pv_rel_fold(const PvArgs& va, PvSmem& sm, const PlWarpSmem& pw, int cnt, int64_t k) {
+  const PlArgs& pa = va.p;
+  const int MI = pa.c.max_impact;
+  for (int r = 0; r < cnt; ++r) {
+    const int t = pw.rtag[r];
+    if (t >= 0)
+      for (int o = 0; o < QOT_OUT; ++o) va.rel_impact_out[(k * MI + t) * QOT_OUT + o] = pw.rout[r][o];
+    if (pa.bound) {
+      const float v = pw.rout[r][pa.metric], b = pa.bound[pw.rnode[r]];
+      sm.r_mkey = min(sm.r_mkey, pl_okey(pa.maximize ? __fsub_rn(v, b) : __fsub_rn(b, v)));
+    }
+  }
+}
+
+// a 256-bit row with the bit at position R taken out: the bits above R move down one place
+__device__ __forceinline__ void pv_remove_bit(unsigned (&r)[kCdMaskWords], int R) {
+  const int wr = R >> 5, b = R & 31;
+#pragma unroll
+  for (int k = 0; k < kCdMaskWords; ++k) {
+    const unsigned next = k + 1 < kCdMaskWords ? r[k + 1] : 0u;
+    const unsigned keep = k < wr ? 0xffffffffu : k == wr ? (1u << b) - 1u : 0u;
+    r[k] = (r[k] & keep) | (r[k] >> 1 & ~keep) | (k >= wr ? next << 31 : 0u);
+  }
+}
+
+// the lightpath at rank sm.r_rank out of chan_work, bound_work and the block's graph: its channels -1, the highest
+// stable id relabelled to its freed one, rank R removed and every row's bits above R moved down one place.  All
+// threads; the caller's neighbour rows are staged before.
+__device__ __noinline__ void pv_release(const PvArgs& va, PvSmem& sm, int64_t s, int64_t n0, int tid) {
+  const CdArgs& a = va.p.c;
+  __syncthreads();                                        // the neighbour rows are staged
+  const int R = sm.r_rank, nt = sm.n_tot, last = nt - 1;
+  const short sid = sm.r2s[R];
+  const int LQ = a.cfg.L * a.cfg.Q;
+  int32_t* row = va.chan_work + s * LQ;
+  const int32_t vs = static_cast<int32_t>(n0 + sid), vl = static_cast<int32_t>(n0 + last);
+  int freed = 0;
+  for (int ch = tid; ch < LQ; ch += kCdThreads) {
+    const int32_t v = __ldcg(row + ch);
+    if (v == vs) {
+      row[ch] = -1;
+      ++freed;
+    } else if (v == vl) {
+      row[ch] = vs;
+    }
+  }
+  if (freed) atomicSub(&sm.n_chan, freed);
+  if (va.bound_work && tid == 0) va.bound_work[s * kCdMaxN + sid] = va.bound_work[s * kCdMaxN + last];
+  unsigned rw[kCdMaskWords];
+  float xr[kF];
+  long long cn = 0;
+  int ky = 0;
+  short st = 0;
+  const bool keep = tid < nt && tid != R;
+  if (keep) {
+#pragma unroll
+    for (int k = 0; k < kCdMaskWords; ++k) rw[k] = sm.adj[tid][k];
+    pv_remove_bit(rw, R);
+#pragma unroll
+    for (int k = 0; k < kF; ++k) xr[k] = sm.x[tid][k];
+    cn = sm.conn[tid];
+    ky = sm.key[tid];
+    st = sm.r2s[tid] == last ? sid : sm.r2s[tid];
+  }
+  __syncthreads();
+  if (keep) {
+    const int to = tid < R ? tid : tid - 1;
+#pragma unroll
+    for (int k = 0; k < kCdMaskWords; ++k) sm.adj[to][k] = rw[k];
+#pragma unroll
+    for (int k = 0; k < kF; ++k) sm.x[to][k] = xr[k];
+    sm.conn[to] = cn;
+    sm.key[to] = ky;
+    sm.r2s[to] = st;
+  }
+  __syncthreads();
+  for (int r = tid; r < last; r += kCdThreads) sm.s2r[sm.r2s[r]] = static_cast<short>(r);
+  if (tid == 0) sm.n_tot = last;
+  __syncthreads();
 }
 
 // the neighbours by rank of placement [q0, q0 + cw) on route links[p0, p1), from chan_work (the route was scanned
@@ -1255,6 +1379,7 @@ __device__ __noinline__ void pv_commit(const PvArgs& va, PvSmem& sm, int64_t s, 
   __syncthreads();
 }
 
+template <bool kReleases>
 __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __grid_constant__ PvArgs va) {
   const PlArgs& pa = va.p;
   const CdArgs& a = pa.c;
@@ -1264,11 +1389,12 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __gri
   PlWarpSmem& pw = sm.w[w];
   float As[kF], Ad[kF];
   cd_head_prologue(a.prep, As, Ad, tid);
-  if (tid == 0) sm.n_valid = 0ull;
+  if (tid == 0) sm.n_valid = sm.n_rvalid = 0ull;
   // ---- the grouping, checked whole by every block: sample_ptr non-decreasing from 0; order[i] a demand of the sample
-  // whose range holds i, ascending within the range; the ranges hold every demand with a sample in [0, S).  Otherwise
-  // no demand is provisioned: every output says PROV_BAD_GROUPING, each written by exactly one thread of the grid.
-  const int64_t S = a.S, D = a.K;
+  // whose range holds i, ascending within the range; the ranges hold every demand with a sample in [0, S).  The same
+  // for the releases, ordered by (before, k) within a range.  Otherwise no demand is provisioned and no release
+  // applied: every output says PROV_BAD_GROUPING, each written by exactly one thread of the grid.
+  const int64_t S = a.S, D = a.K, NR = kReleases ? va.rel.R : 0;
   bool bad = false;
   for (int64_t g = tid; g <= S; g += kCdThreads) {
     const int64_t v = va.sample_ptr[g];
@@ -1293,19 +1419,53 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __gri
     atomicAdd(&sm.n_valid, cnt);
     bad = __syncthreads_or(bad) || sm.n_valid != static_cast<unsigned long long>(nv);
   }
+  if (!bad && NR > 0) {
+    const int64_t* rp = va.rel_ptr;
+    const int64_t* bf = va.rel.before;
+    for (int64_t g = tid; g <= S; g += kCdThreads) {
+      const int64_t v = rp[g];
+      bad |= (g == 0 && v != 0) || (g < S && rp[g + 1] < v) || (g == S && v > NR);
+    }
+    bad = __syncthreads_or(bad);
+    if (!bad) {
+      const int64_t nv = rp[S];
+      unsigned long long cnt = 0;
+      for (int64_t i = tid; i < NR; i += kCdThreads) {
+        const int64_t sk = va.rel.sample[i];
+        cnt += sk >= 0 && sk < S;
+        if (i < nv) {
+          const int64_t k = va.rel_order[i];
+          bool ok = k >= 0 && k < NR;
+          const int64_t s = ok ? va.rel.sample[k] : -1;
+          ok = ok && s >= 0 && s < S && rp[s] <= i && i < rp[s + 1];
+          if (ok && i + 1 < rp[s + 1]) {
+            const int64_t k2 = va.rel_order[i + 1];
+            ok = k2 >= 0 && k2 < NR && (bf[k2] > bf[k] || (bf[k2] == bf[k] && k2 > k));
+          }
+          bad |= !ok;
+        }
+      }
+      atomicAdd(&sm.n_rvalid, cnt);
+      bad = __syncthreads_or(bad) || sm.n_rvalid != static_cast<unsigned long long>(nv);
+    }
+  }
   const int64_t gt = static_cast<int64_t>(blockIdx.x) * kCdThreads + tid;
   const int64_t gs = static_cast<int64_t>(gridDim.x) * kCdThreads;
   if (bad) {
     for (int64_t d = gt; d < D; d += gs) pv_empty(va, d, QOT_PROV_BAD_GROUPING, 0, 1);
+    for (int64_t k = gt; k < NR; k += gs) pv_rel_empty(va, k, QOT_PROV_BAD_GROUPING, 0, 0, 1);
     return;
   }
   for (int64_t d = gt; d < D; d += gs)
     if (a.sample[d] < 0 || a.sample[d] >= S) pv_empty(va, d, QOT_CAND_BAD_SAMPLE, 0, 1);
+  for (int64_t k = gt; k < NR; k += gs)
+    if (va.rel.sample[k] < 0 || va.rel.sample[k] >= S) pv_rel_empty(va, k, QOT_CAND_BAD_SAMPLE, 0, 0, 1);
   const float nan = __int_as_float(0x7fc00000);
   int zc = 0;                                             // rows staged in this warp's head buffer
   for (int64_t s = blockIdx.x; s < S; s += gridDim.x) {
     const int64_t i0 = va.sample_ptr[s], i1 = va.sample_ptr[s + 1];
-    if (i0 == i1) continue;
+    const int64_t j0 = NR > 0 ? va.rel_ptr[s] : 0, j1 = NR > 0 ? va.rel_ptr[s + 1] : 0;
+    if (i0 == i1 && j0 == j1) continue;
     const int L = a.cfg.L, Q = a.cfg.Q;
     int64_t n0 = 0;
     int n = 0;
@@ -1348,8 +1508,79 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __gri
         for (int r = tid; r < n; r += kCdThreads) va.bound_work[s * kCdMaxN + r] = va.bound[n0 + r];
     }
     sbad = __syncthreads_or(sbad);
-    for (int64_t i = i0; i < i1; ++i) {
-      const int64_t d = va.order[i];
+    int64_t j = j0;                                       // the sample's next release
+    for (int64_t i = i0; i <= i1; ++i) {
+      const int64_t d = i < i1 ? va.order[i] : -1;
+      // ---- the releases due before demand d (after the last demand: the rest)
+      for (; j < j1 && (i == i1 || va.rel.before[va.rel_order[j]] <= d); ++j) {
+        const int64_t k = va.rel_order[j];
+        if (tid == 0) {                                   // what it names: status and conn_id
+          const int64_t b = va.rel.before[k], dm = va.rel.demand[k];
+          int rs = 0;
+          long long c = -1;
+          if (sbad) rs = QOT_CAND_BAD_STATE;
+          else if (b < 0 || b > D || dm < -1 || (dm >= 0 && (dm >= D || dm >= b || a.sample[dm] != s)))
+            rs = QOT_TRAF_BAD_REF;
+          else if (dm >= 0 && (c = __ldcg(va.conn_id + dm)) < 0) rs = QOT_TRAF_NOT_ACCEPTED;
+          else if (dm == -1) c = va.rel.conn_id[k];
+          sm.r_st = rs;
+          sm.r_conn = c;
+          sm.r_rank = -1;
+          sm.r_mkey = 0xffffffffu;
+        }
+        __syncthreads();
+        if (sm.r_st == 0 && tid < sm.n_tot && sm.conn[tid] == sm.r_conn) sm.r_rank = tid;
+        __syncthreads();
+        const int R = sm.r_rank;
+        // ---- warp 0: the former neighbours' rows (all of them against a bound) and the release's outputs
+        if (w == 0) {
+          if (zc) {                                       // the previous demand's winner rows
+            pl_flush(pa, pw, w, zc, 0, lane);
+            zc = 0;
+          }
+          const int rs = sm.r_st ? sm.r_st : R < 0 ? QOT_TRAF_BAD_REF : 0;
+          if (rs) {
+            pv_rel_empty(va, k, rs, 0, lane, 32);
+          } else {
+            const int MI = a.max_impact;
+            const int cnt = cd_rank(lane < kCdMaskWords ? sm.adj[R][lane] : 0u, ws.nbr, lane);
+            __syncwarp();
+            const int rows = min(cnt, MI), nev = pa.bound ? cnt : rows;
+            const auto flush = [&](int c) {
+              cd_flush(w, c, a.prep, lane);
+              if (lane == 0) pv_rel_fold(va, sm, pw, c, k);
+              __syncwarp();
+            };
+            for (int e = 0; e < nev; ++e) {
+              const int r = ws.nbr[e];
+              if (lane == 0 && e < rows) va.rel_impact_conn[k * MI + e] = sm.conn[r];
+              const unsigned rb = lane == R >> 5 ? 1u << (R & 31) : 0u;
+              const int m = cd_rank(lane < kCdMaskWords ? sm.adj[r][lane] & ~rb : 0u, ws.msg, lane);
+              if (lane == 0) {
+                ws.msg[m] = r;
+                pw.rtag[zc] = e < rows ? e : -1;
+                pw.rnode[zc] = s * kCdMaxN + sm.r2s[r];
+              }
+              __syncwarp();
+              zc = cd_row(ws, zc, ws.msg, m + 1, r, PvX{sm.x, ws.cx, r, a.lut_col}, As, Ad, pw.rout[zc], flush, lane);
+            }
+            if (zc) {
+              flush(zc);
+              zc = 0;
+            }
+            pv_rel_empty(va, k, 0, rows, lane, 32);
+            if (lane == 0) {
+              va.rel_status[k] = cnt > MI ? QOT_CAND_IMPACT_OVERFLOW : 0;
+              va.rel_conn_id[k] = sm.r_conn;
+              va.rel_n_impact[k] = cnt;
+              va.rel_margin[k] = pa.bound && cnt ? pl_unkey(sm.r_mkey) : nan;
+            }
+          }
+        }
+        if (R >= 0) pv_release(va, sm, s, n0, tid);
+        __syncthreads();                                  // the release's shared state is read
+      }
+      if (i == i1) break;
       const int64_t o0 = pa.opt_ptr[d], o1 = pa.opt_ptr[d + 1];
       // ---- validation (warp 0): the option range, every option's route and width; then the state
       if (w == 0) {
@@ -1656,6 +1887,66 @@ static int cd_launch(const char* who, const qot_lp_state_t* state, const qot_lp_
   return QOT_OK;
 }
 
+// qot_lightpath_provision (rel = null: no releases) and qot_lightpath_traffic: the checks, the copy of chan_node and
+// the launch
+static int pv_launch(const char* who, const qot_lp_state_t* state, const qot_lp_demands_t* demands,
+                     const int64_t* order, const int64_t* sample_ptr, const float* bound, int32_t metric,
+                     int32_t maximize, int32_t policy, const float* prepared, int32_t is_lut_index, int32_t max_impact,
+                     int32_t* chan_work, float* bound_work, int32_t* option, int32_t* q0, float* out, float* margin,
+                     int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact, int64_t* conn_id,
+                     int64_t* impact_conn, float* impact_out, const qot_lp_releases_t* rel, const int64_t* rel_order,
+                     const int64_t* rel_ptr, int32_t* rel_status, int64_t* rel_conn_id, int32_t* rel_n_impact,
+                     int64_t* rel_impact_conn, float* rel_impact_out, float* rel_margin, cudaStream_t stream) {
+  PvArgs va;
+  PlArgs& pa = va.p;
+  CdArgs& a = pa.c;
+  if (int rc = pl_demand_args(who, pa, state, demands, metric, maximize, policy, prepared, is_lut_index, max_impact))
+    return rc;
+  const qot_lp_state_t& st = *state;
+  const qot_lp_demands_t& d = *demands;
+  const int64_t NR = rel ? rel->R : 0;
+  QOT_REQUIRE(NR >= 0, "%s: bad release count", who);
+  if (d.D == 0 && NR == 0) return QOT_OK;
+  QOT_REQUIRE(d.D == 0 || (d.sample && order && d.opt_ptr && d.link_ptr &&
+                           (d.P == 0 || (d.width && d.feat && d.own_bound)) && (d.n_links == 0 || d.links)),
+              "%s: null demand or grouping array", who);
+  QOT_REQUIRE(sample_ptr, "%s: null demand or grouping array", who);
+  QOT_REQUIRE(d.D == 0 || (option && q0 && out && margin && n_free && n_feasible && status && n_impact && conn_id &&
+                           (max_impact == 0 || (impact_conn && impact_out))), "%s: null output array", who);
+  QOT_REQUIRE((st.S == 0 || chan_work) && (!bound || st.S == 0 || bound_work) && (st.N == 0 || st.conn_ids),
+              "%s: null work or conn_ids array", who);
+  if (NR > 0) {
+    QOT_REQUIRE(rel->sample && rel->before && rel->demand && rel->conn_id && rel_order && rel_ptr,
+                "%s: null release or release grouping array", who);
+    QOT_REQUIRE(rel_status && rel_conn_id && rel_n_impact && rel_margin &&
+                    (max_impact == 0 || (rel_impact_conn && rel_impact_out)), "%s: null release output array", who);
+  }
+  if (int rc = cd_state_args(who, a, st, prepared, is_lut_index, max_impact)) return rc;
+  constexpr int smem = static_cast<int>(sizeof(PvSmem));
+  if (int rc = NR > 0 ? cd_smem_opt_in<lp_provision_kernel<true>, smem>()
+                      : cd_smem_opt_in<lp_provision_kernel<false>, smem>())
+    return rc;
+  if (st.S > 0)
+    QOT_CUDA(cudaMemcpyAsync(chan_work, st.chan_node, static_cast<size_t>(st.S) * st.cfg.L * st.cfg.Q * sizeof(int32_t),
+                             cudaMemcpyDeviceToDevice, stream));
+  a.chan_node = chan_work;
+  a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_conn; a.impact_out = impact_out;
+  pa.bound = bound ? bound_work : nullptr;
+  pa.option = option; pa.q0 = q0; pa.margin = margin; pa.n_free = n_free; pa.n_feasible = n_feasible;
+  pa.all_out = nullptr; pa.all_margin = nullptr;
+  va.order = order; va.sample_ptr = sample_ptr; va.conn_ids = st.conn_ids; va.bound = bound;
+  va.chan_work = chan_work; va.bound_work = bound ? bound_work : nullptr; va.conn_id = conn_id;
+  va.rel = NR > 0 ? *rel : qot_lp_releases_t{0, nullptr, nullptr, nullptr, nullptr};
+  va.rel_order = rel_order; va.rel_ptr = NR > 0 ? rel_ptr : nullptr;
+  va.rel_status = rel_status; va.rel_conn_id = rel_conn_id; va.rel_n_impact = rel_n_impact;
+  va.rel_impact_conn = rel_impact_conn; va.rel_impact_out = rel_impact_out; va.rel_margin = rel_margin;
+  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, std::max<int64_t>(1, st.S)));
+  if (NR > 0) lp_provision_kernel<true><<<grid, kCdThreads, smem, stream>>>(va);
+  else lp_provision_kernel<false><<<grid, kCdThreads, smem, stream>>>(va);
+  QOT_LAUNCH_CHECK();
+  return QOT_OK;
+}
+
 }  // namespace qot
 
 using namespace qot;
@@ -1758,39 +2049,27 @@ extern "C" int qot_lightpath_provision(const qot_lp_state_t* state, const qot_lp
                                        int32_t is_lut_index, int32_t max_impact, int32_t* chan_work, float* bound_work,
                                        int32_t* option, int32_t* q0, float* out, float* margin, int32_t* n_free,
                                        int32_t* n_feasible, int32_t* status, int32_t* n_impact, int64_t* conn_id,
-                                       int64_t* impact_conn, float* impact_out, void* stream_) {
-  const char* who = "qot_lightpath_provision";
-  PvArgs va;
-  PlArgs& pa = va.p;
-  CdArgs& a = pa.c;
-  if (int rc = pl_demand_args(who, pa, state, demands, metric, maximize, policy, prepared, is_lut_index, max_impact))
-    return rc;
-  const qot_lp_state_t& st = *state;
-  const qot_lp_demands_t& d = *demands;
-  if (d.D == 0) return QOT_OK;
-  QOT_REQUIRE(d.sample && order && sample_ptr && d.opt_ptr && d.link_ptr &&
-                  (d.P == 0 || (d.width && d.feat && d.own_bound)) && (d.n_links == 0 || d.links),
-              "%s: null demand or grouping array", who);
-  QOT_REQUIRE(option && q0 && out && margin && n_free && n_feasible && status && n_impact && conn_id &&
-                  (max_impact == 0 || (impact_conn && impact_out)), "%s: null output array", who);
-  QOT_REQUIRE((st.S == 0 || chan_work) && (!bound || st.S == 0 || bound_work) && (st.N == 0 || st.conn_ids),
-              "%s: null work or conn_ids array", who);
-  if (int rc = cd_state_args(who, a, st, prepared, is_lut_index, max_impact)) return rc;
-  constexpr int smem = static_cast<int>(sizeof(PvSmem));
-  if (int rc = cd_smem_opt_in<lp_provision_kernel, smem>()) return rc;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (st.S > 0)
-    QOT_CUDA(cudaMemcpyAsync(chan_work, st.chan_node, static_cast<size_t>(st.S) * st.cfg.L * st.cfg.Q * sizeof(int32_t),
-                             cudaMemcpyDeviceToDevice, stream));
-  a.chan_node = chan_work;
-  a.out = out; a.status = status; a.n_impact = n_impact; a.impact_node = impact_conn; a.impact_out = impact_out;
-  pa.bound = bound ? bound_work : nullptr;
-  pa.option = option; pa.q0 = q0; pa.margin = margin; pa.n_free = n_free; pa.n_feasible = n_feasible;
-  pa.all_out = nullptr; pa.all_margin = nullptr;
-  va.order = order; va.sample_ptr = sample_ptr; va.conn_ids = st.conn_ids; va.bound = bound;
-  va.chan_work = chan_work; va.bound_work = bound ? bound_work : nullptr; va.conn_id = conn_id;
-  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, std::max<int64_t>(1, st.S)));
-  lp_provision_kernel<<<grid, kCdThreads, smem, stream>>>(va);
-  QOT_LAUNCH_CHECK();
-  return QOT_OK;
+                                       int64_t* impact_conn, float* impact_out, void* stream) {
+  return pv_launch("qot_lightpath_provision", state, demands, order, sample_ptr, bound, metric, maximize, policy,
+                   prepared, is_lut_index, max_impact, chan_work, bound_work, option, q0, out, margin, n_free,
+                   n_feasible, status, n_impact, conn_id, impact_conn, impact_out, nullptr, nullptr, nullptr, nullptr,
+                   nullptr, nullptr, nullptr, nullptr, nullptr, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int qot_lightpath_traffic(const qot_lp_state_t* state, const qot_lp_demands_t* demands,
+                                     const int64_t* order, const int64_t* sample_ptr, const float* bound,
+                                     int32_t metric, int32_t maximize, int32_t policy, const float* prepared,
+                                     int32_t is_lut_index, int32_t max_impact, int32_t* chan_work, float* bound_work,
+                                     int32_t* option, int32_t* q0, float* out, float* margin, int32_t* n_free,
+                                     int32_t* n_feasible, int32_t* status, int32_t* n_impact, int64_t* conn_id,
+                                     int64_t* impact_conn, float* impact_out, const qot_lp_releases_t* releases,
+                                     const int64_t* rel_order, const int64_t* rel_ptr, int32_t* rel_status,
+                                     int64_t* rel_conn_id, int32_t* rel_n_impact, int64_t* rel_impact_conn,
+                                     float* rel_impact_out, float* rel_margin, void* stream) {
+  const char* who = "qot_lightpath_traffic";
+  QOT_REQUIRE(releases, "%s: null releases descriptor", who);
+  return pv_launch(who, state, demands, order, sample_ptr, bound, metric, maximize, policy, prepared, is_lut_index,
+                   max_impact, chan_work, bound_work, option, q0, out, margin, n_free, n_feasible, status, n_impact,
+                   conn_id, impact_conn, impact_out, releases, rel_order, rel_ptr, rel_status, rel_conn_id,
+                   rel_n_impact, rel_impact_conn, rel_impact_out, rel_margin, static_cast<cudaStream_t>(stream));
 }

@@ -261,6 +261,39 @@ class LightpathGNN(torch.nn.Module):
                                        self.is_lut_index, max_impact)
 
     @_lib.on_tensor_device
+    def forward_traffic(self, state, demands, releases, policy: int, metric: int = 0, maximize: bool = True,
+                        bound=None, max_impact: int = 64) -> "ops.TrafficQoT":
+        """Dynamic traffic: lightpath arrivals and departures in one pass (eval mode only;
+        csrc/lightpath_candidates.cu, qot_lightpath_traffic).  Each sample's demands and releases form one sequence of
+        events: release k (``to_graph.LightpathReleases``) happens after the sample's demands with index ``<
+        releases.before[k]`` and before the others.  Each event is evaluated against the state with every earlier
+        event of its sample applied; samples are independent.
+
+        A demand is handled exactly as ``forward_provision`` handles it against that state.  A demand accepted here
+        gets one above the largest conn_id its sample has held in the call, released lightpaths included, so conn_ids
+        are never reused within a call; with no releases that is ``forward_provision``'s rule, and every demand output
+        equals ``forward_provision``'s bit for bit.  A release removes the lightpath from the sample (every channel of
+        it zeroed, as a teardown in ``forward_reconfigurations``) and, with a ``bound``, its bound stops applying;
+        ``PROV_FULL`` is judged on the occupancy at the time of the demand, so a release can make room.
+
+        Returns ``ops.TrafficQoT``: the fields of ``ops.ProvisionQoT`` over the demands, then per release
+        ``release_status``, ``release_conn_id`` (the conn_id released, -1 if nothing was), ``release_n_impact``,
+        ``release_impact_conn`` / ``release_impact_out`` (the rows of the released lightpath's former neighbours after
+        the release, ascending in node order: bit-identical to the ``KIND_LOST`` rows ``forward_reconfigurations``
+        gives for that teardown against the state just before it) and ``release_margin`` (with a ``bound``, the
+        minimum margin over every neighbour row whatever ``max_impact`` is; NaN without a bound or without
+        neighbours).  A departure can take a neighbour below its bound -- GAT attention is not monotone -- and is
+        reported there, never refused.  Release status bits: ``ops.TRAF_BAD_REF`` (the release names nothing in the
+        sample at that point: an unknown or released conn_id, a demand of another sample or not ``< before``, a
+        ``before`` outside [0, D]), ``ops.TRAF_NOT_ACCEPTED`` (the named demand was not accepted), ``CAND_BAD_SAMPLE``,
+        ``CAND_BAD_STATE`` and ``CAND_IMPACT_OVERFLOW``; nothing is removed with the first four.  ``state`` is not
+        modified; ``to_graph.commit_traffic`` writes the end state into the samples.  One copy and one launch,
+        nothing read back: capturable in a CUDA graph.  Malformed arguments raise on the host."""
+        self._check_state_query("forward_traffic", state)
+        return ops.lightpath_traffic(state, demands, releases, policy, metric, maximize, bound, self.prepared(),
+                                     self.is_lut_index, max_impact)
+
+    @_lib.on_tensor_device
     def forward_stream(self, plan, first: int = 0, count=None) -> None:
         """Enqueues batches [first, first+count) of ``plan`` (eval mode; no host synchronisation)."""
         if self.training:

@@ -670,6 +670,92 @@ def lightpath_provision(state, demands, policy: int, metric: int, maximize: bool
     return res
 
 
+
+# status bits of qot_lightpath_traffic's releases, on top of the CAND_* and PROV_* bits
+TRAF_BAD_REF, TRAF_NOT_ACCEPTED = 2048, 4096
+
+
+class TrafficQoT(NamedTuple):
+    option: torch.Tensor         # [D] int32: the chosen option, relative to opt_ptr[d] (-1: no feasible placement)
+    q0: torch.Tensor             # [D] int32: its start slot (-1: none)
+    out: torch.Tensor            # [D,3]: the chosen placement's own QoT (NaN: none)
+    margin: torch.Tensor         # [D]: its margin (NaN: none)
+    n_free: torch.Tensor         # [D] int32: free placements over the demand's options
+    n_feasible: torch.Tensor     # [D] int32: feasible placements among them
+    status: torch.Tensor         # [D] int32, CAND_* | PROV_* bits
+    n_impact: torch.Tensor       # [D] int32: lightpaths the chosen placement interferes with (may exceed max_impact)
+    impact_conn: torch.Tensor    # [D, max_impact] int64: their conn_ids, ascending in node order; -1 past the rows
+    impact_out: torch.Tensor     # [D, max_impact, 3]: their QoT with the placement set up; NaN past the rows
+    conn_id: torch.Tensor        # [D] int64: the conn_id the demand was accepted under (-1: not accepted)
+    release_status: torch.Tensor       # [R] int32, CAND_* | PROV_BAD_GROUPING | TRAF_* bits
+    release_conn_id: torch.Tensor      # [R] int64: the conn_id released (-1: nothing released)
+    release_n_impact: torch.Tensor     # [R] int32: the released lightpath's former neighbours (may exceed max_impact)
+    release_impact_conn: torch.Tensor  # [R, max_impact] int64: their conn_ids, in node order; -1 past the rows
+    release_impact_out: torch.Tensor   # [R, max_impact, 3]: their QoT after the release; NaN past the rows
+    release_margin: torch.Tensor       # [R]: with a bound, the minimum margin over every neighbour row (else NaN)
+
+
+_RELEASE_FIELDS = ("sample", "before", "demand", "conn_id")
+
+
+def traffic_grouping(sample: torch.Tensor, before: torch.Tensor, S: int, D: int):
+    """(rel_order [R], rel_ptr [S+1]) int64: the releases grouped by sample, by (before, k) within a sample (a stable
+    sort on (sample, before)), samples outside [0, S) after the last range.  ``before`` outside [0, D] stays in its
+    sample's range (the kernel reports it).  Device tensor ops, no host synchronisation."""
+    R = sample.shape[0]
+    dev = sample.device
+    if R == 0:
+        return torch.zeros(0, dtype=torch.int64, device=dev), torch.zeros(S + 1, dtype=torch.int64, device=dev)
+    skey = torch.where((sample >= 0) & (sample < S), sample, torch.full_like(sample, S))
+    o1 = torch.sort(before, stable=True)[1]
+    o2 = torch.sort(skey[o1], stable=True)[1]
+    order = o1[o2]
+    sample_ptr = torch.searchsorted(skey[order], torch.arange(S + 1, dtype=torch.int64, device=dev))
+    return order, sample_ptr
+
+
+def lightpath_traffic(state, demands, releases, policy: int, metric: int, maximize: bool, bound,
+                      prepared: torch.Tensor, is_lut_index: int, max_impact: int) -> TrafficQoT:
+    """qot_lightpath_traffic: each sample's demands and releases as one sequence of events, each against the state
+    with every earlier event of its sample applied.  Both groupings are computed on the device and the work arrays
+    allocated here; one copy and one launch, nothing read back (CUDA-graph capturable).  The host checks of
+    ``lightpath_provision`` plus the dtypes, shapes and device of the four release tensors."""
+    who = "forward_traffic"
+    D, P = _check_demand_args(who, state, demands, policy, metric, bound, prepared, max_impact)
+    dev = state.batch.x.device
+    for name in _RELEASE_FIELDS:
+        _check_state_tensor(who, f"releases.{name}", getattr(releases, name), dev, torch.int64)
+    R = int(releases.sample.shape[0]) if releases.sample.dim() == 1 else -1
+    if R < 0 or any(getattr(releases, n).shape != (R,) for n in _RELEASE_FIELDS):
+        raise ValueError(f"{who}: need releases.sample, before, demand, conn_id, each [R]")
+    max_impact = int(max_impact)
+    i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=dev)
+    i64 = lambda *s: torch.empty(*s, dtype=torch.int64, device=dev)
+    f32 = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)
+    res = TrafficQoT(*_demand_outputs(D, max_impact, dev), i64(D), i32(R), i64(R), i32(R), i64(R, max_impact),
+                     f32(R, max_impact, 3), f32(R))
+    if D == 0 and R == 0:
+        return res
+    order, sample_ptr = provision_grouping(demands.sample, state.S)
+    rel = [getattr(releases, n).contiguous() for n in _RELEASE_FIELDS]
+    rel_order, rel_ptr = traffic_grouping(rel[0], rel[1], state.S, D)
+    chan_work = torch.empty_like(state.chan_node)
+    bound_work = torch.empty(state.S, TG_MAX_NODES, dtype=torch.float32, device=dev) if bound is not None else None
+    bound = None if bound is None else bound.contiguous()
+    keep = list(rel)
+    with torch.cuda.device(dev):
+        check(_lib.lib().qot_lightpath_traffic(
+            C.byref(_state_desc(state, keep)), C.byref(_demands_desc(demands, D, P, keep)), _cptr(order),
+            ptr(sample_ptr), _cptr(bound), int(metric), int(bool(maximize)), int(policy), ptr(prepared),
+            int(is_lut_index), max_impact, _cptr(chan_work), _cptr(bound_work), _cptr(res.option), _cptr(res.q0),
+            _cptr(res.out), _cptr(res.margin), _cptr(res.n_free), _cptr(res.n_feasible), _cptr(res.status),
+            _cptr(res.n_impact), _cptr(res.conn_id), _cptr(res.impact_conn), _cptr(res.impact_out),
+            C.byref(_lib.QotLpReleases(R, *(_cptr(t) for t in rel))), _cptr(rel_order), ptr(rel_ptr),
+            _cptr(res.release_status), _cptr(res.release_conn_id), _cptr(res.release_n_impact),
+            _cptr(res.release_impact_conn), _cptr(res.release_impact_out), _cptr(res.release_margin), stream()),
+            "qot_lightpath_traffic")
+    return res
+
 class GraphIndex:
     """Lazily built, cached index structures of one batch: the destination-sorted CSR
     (forward), its GAT variant (self loops replaced) and the source-sorted transposed

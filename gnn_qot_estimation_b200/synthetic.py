@@ -537,3 +537,69 @@ def lightpath_demands(samples, per_sample: int, options=(1, 4), seed: int = 0, b
                             torch.tensor(widths, dtype=torch.int32),
                             torch.tensor(np.array(feats, dtype=np.float32).reshape(-1, 3)),
                             torch.tensor(np.array(bounds, dtype=np.float32)))
+
+
+def lightpath_traffic(samples, per_sample: int, load: float, options=(1, 4), seed: int = 0, bound_range=(0.1, 0.6),
+                      release_existing: float = 0.0):
+    """Seeded dynamic traffic for the network-status ``samples``, for ``LightpathGNN.forward_traffic``: returns
+    ``(demands, releases)``, ``to_graph.LightpathDemands`` and ``to_graph.LightpathReleases`` of CPU tensors.
+
+    Per sample, ``per_sample`` demands arrive as a Poisson process of rate ``load`` (in Erlang, with unit-mean
+    exponential holding times) and each holds its lightpath for its holding time.  Options are drawn as
+    ``lightpath_demands`` draws them.  The demands of all samples are ordered by arrival time, so samples interleave.
+    Each demand's departure is a release by demand whose ``before`` is the number of demands that arrived before the
+    departure (one ``searchsorted`` over all arrivals); departures after the last arrival get ``before = D``.
+    ``release_existing``: the fraction of each sample's lightpaths (the conn_ids on its channels) released by conn_id
+    at uniform random times over the sample's arrival window."""
+    import numpy as np
+    from .to_graph import LightpathReleases
+    if load <= 0:
+        raise ValueError("load must be positive (Erlang)")
+    rng = np.random.default_rng(seed)
+    S = samples["data"].shape[0]
+    base = lightpath_demands(samples, per_sample, options, seed=int(rng.integers(1 << 31)), bound_range=bound_range)
+    optr = base.opt_ptr.numpy()
+    # arrival times per sample, then one global order by time
+    smp, t_arr, t_dep, opts = [], [], [], []
+    for s in range(S):
+        t = np.cumsum(rng.exponential(1.0 / load, per_sample))
+        smp += [s] * per_sample
+        t_arr.append(t)
+        t_dep.append(t + rng.exponential(1.0, per_sample))
+    t_arr, t_dep = np.concatenate(t_arr), np.concatenate(t_dep)
+    order = np.argsort(t_arr, kind="stable")
+    smp = np.asarray(smp, dtype=np.int64)[order]
+    t_arr, t_dep = t_arr[order], t_dep[order]
+    D = smp.shape[0]
+    # demand k takes the options of base demand k (whose sample is redrawn here)
+    sub = [list(range(int(optr[k]), int(optr[k + 1]))) for k in range(D)]
+    lptr = base.link_ptr.numpy()
+    o_idx = [p for k in range(D) for p in sub[k]]
+    l_idx = [e for p in o_idx for e in range(int(lptr[p]), int(lptr[p + 1]))]
+    from .to_graph import LightpathDemands
+    t = lambda v: torch.tensor(np.asarray(v, dtype=np.int64))
+    demands = LightpathDemands(t(smp), t(np.cumsum([0] + [len(x) for x in sub])),
+                               t(np.cumsum([0] + [int(lptr[p + 1] - lptr[p]) for p in o_idx])),
+                               base.links[t(l_idx)], base.width[t(o_idx)], base.feat[t(o_idx)],
+                               base.own_bound[t(o_idx)])
+    # departures of the demands: before = arrivals strictly earlier than the departure
+    r_s, r_b, r_d, r_c, r_t = [], [], [], [], []
+    before = np.searchsorted(t_arr, t_dep, side="left")
+    for k in range(D):
+        r_s.append(int(smp[k])); r_b.append(int(before[k])); r_d.append(k); r_c.append(-1); r_t.append(t_dep[k])
+    # a share of the initial lightpaths released by conn_id at uniform times over the sample's arrivals
+    if release_existing > 0:
+        fi = {n: i for i, n in enumerate(samples["lp_feat"])}
+        for s in range(S):
+            d = samples["data"][s]
+            conns = np.unique(np.trunc(d[fi["conn_id"]][np.any(d != 0, axis=0)]).astype(np.int64))
+            pick = conns[rng.random(conns.shape[0]) < release_existing]
+            mine = t_arr[smp == s]
+            end = float(mine[-1]) if mine.size else 1.0
+            for c in pick:
+                tr = rng.uniform(0.0, end)
+                r_s.append(s); r_b.append(int(np.searchsorted(t_arr, tr, side="left"))); r_d.append(-1)
+                r_c.append(int(c)); r_t.append(tr)
+    ro = np.argsort(np.asarray(r_t), kind="stable")            # releases in time order (the index is cosmetic)
+    pick = lambda v: torch.tensor(np.asarray(v, dtype=np.int64)[ro] if len(v) else np.zeros(0, dtype=np.int64))
+    return demands, LightpathReleases(pick(r_s), pick(r_b), pick(r_d), pick(r_c))

@@ -14,6 +14,7 @@ against golden vectors made by the reference's own code); edges are emitted sort
 from __future__ import annotations
 
 import ctypes as C
+from types import SimpleNamespace
 from typing import NamedTuple, Optional, Sequence
 
 import torch
@@ -199,6 +200,21 @@ class LightpathDemands(NamedTuple):
         return LightpathDemands(*(t.to(device) for t in self))
 
 
+class LightpathReleases(NamedTuple):
+    """Lightpath releases for ``LightpathGNN.forward_traffic`` (device tensors).  Release k happens in sample
+    ``sample[k]`` after every demand of that sample with index ``< before[k]`` and before every demand with index
+    ``>= before[k]`` (``before = D``: after the sample's last demand; equal ``before`` in increasing k).  It removes the
+    lightpath demand ``demand[k]`` was accepted under (``demand[k] >= 0``: a demand of the same sample, ``<
+    before[k]``), or the lightpath with conn_id ``conn_id[k]`` present at that point (``demand[k] == -1``)."""
+    sample: torch.Tensor          # [R] int64
+    before: torch.Tensor          # [R] int64
+    demand: torch.Tensor          # [R] int64
+    conn_id: torch.Tensor         # [R] int64
+
+    def to(self, device) -> "LightpathReleases":
+        return LightpathReleases(*(t.to(device) for t in self))
+
+
 def lightpath_nodes(state: LightpathNetworkState, sample: torch.Tensor, conn_id: torch.Tensor) -> torch.Tensor:
     """[K] int64: the node of ``state.batch`` that holds lightpath ``conn_id[k]`` in sample ``sample[k]``, -1 where the
     sample has no such lightpath (or ``sample[k]`` is outside the state).  Device tensor ops, no host synchronisation:
@@ -294,3 +310,32 @@ def commit_provision(data: torch.Tensor, state: LightpathNetworkState, demands: 
     for k, name in enumerate(("freq", "mod_order", "num_spans", "path_len")):
         names[cfg.i_feat[k]] = name
     return lightpath_network_state(data, state.freqs, names, float(cfg.freq_threshold))
+
+
+def commit_traffic(data: torch.Tensor, state: LightpathNetworkState, demands: LightpathDemands,
+                   releases: LightpathReleases, r) -> LightpathNetworkState:
+    """Writes the end state of ``LightpathGNN.forward_traffic`` (result ``r``) into ``data`` [S, F, L, Q] (float32,
+    CUDA, the samples ``state`` was built from) in place and returns ``lightpath_network_state`` of it: every lightpath
+    of the initial state that a release removed is zeroed, then every accepted demand still present at the end is
+    written as ``commit_provision`` writes it (``commit_provision`` with conn_id -1 for the demands released later).
+    The conn_ids are the call's: unique within the call.  A later call numbers its new lightpaths from the new state's
+    largest conn_id, so an id released in one call can come back in the next.  Not capturable, like
+    ``commit_provision``."""
+    if not (data.is_cuda and data.dtype == torch.float32 and data.is_contiguous()):
+        raise TypeError("commit_traffic: data must be a contiguous float32 CUDA tensor (it is written in place)")
+    S, F, L, Q = (int(v) for v in data.shape)
+    if (S, L, Q) != (state.S, state.L, state.Q):
+        raise ValueError("commit_traffic: data must be the [S, F, L, Q] samples the state was built from")
+    lo, span = -(1 << 31), 1 << 32                           # conn_ids are int32 values (a float32 row truncated)
+    done = r.release_conn_id >= 0
+    gone = releases.sample[done] * span + (r.release_conn_id[done] - lo)
+    # the released lightpaths of the initial state: every channel with a released (sample, conn_id) zeroed
+    conn = data[:, state.cfg.i_conn].to(torch.int64)                       # truncated toward zero, as the builder
+    key = torch.arange(S, device=data.device)[:, None, None] * span + (conn - lo)
+    hit = torch.isin(key, gone) & (data != 0).any(1)
+    data.masked_fill_(hit[:, None], 0.0)
+    # the accepted demands still present at the end
+    acc = r.conn_id >= 0
+    kept = acc & ~torch.isin(demands.sample * span + (r.conn_id - lo), gone)
+    present = torch.where(kept, r.conn_id, torch.full_like(r.conn_id, -1))
+    return commit_provision(data, state, demands, SimpleNamespace(conn_id=present, option=r.option, q0=r.q0))

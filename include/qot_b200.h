@@ -574,6 +574,18 @@ typedef struct {
   const float* own_bound;      /* [P]                                                                       */
 } qot_lp_demands_t;            /* 80 bytes */
 
+/* Lightpath releases for qot_lightpath_traffic: R of them.  Release k happens in sample sample[k] after every demand of
+ * that sample with index < before[k] and before every demand with index >= before[k] (before = D: after the last);
+ * releases with equal before happen in increasing k.  It removes the lightpath demand demand[k] was accepted under
+ * (demand[k] >= 0), or the lightpath with conn_id conn_id[k] that is in the sample at that point (demand[k] == -1). */
+typedef struct {
+  int64_t R;
+  const int64_t* sample;       /* [R]                                                                       */
+  const int64_t* before;       /* [R]                                                                       */
+  const int64_t* demand;       /* [R]                                                                       */
+  const int64_t* conn_id;      /* [R]; read where demand[k] == -1                                           */
+} qot_lp_releases_t;           /* 40 bytes */
+
 /* qot_lightpath_candidates (lp_candidate_kernel): K candidates, one warp each, one launch.  Candidate k names sample
  * sample[k], a path links[link_ptr[k] .. link_ptr[k+1]) (int32 link indices; duplicates change nothing), the slot
  * range [q0[k], q0[k] + width[k]) used on every link of the path and its raw channel vector feat [K,4] = (freq,
@@ -726,6 +738,45 @@ int qot_lightpath_provision(const qot_lp_state_t* state, const qot_lp_demands_t*
                             int32_t* chan_work, float* bound_work, int32_t* option, int32_t* q0, float* out,
                             float* margin, int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact,
                             int64_t* conn_id, int64_t* impact_conn, float* impact_out, void* stream);
+
+/* qot_lightpath_traffic (lp_provision_kernel, the launch of qot_lightpath_provision): dynamic traffic, arrivals and
+ * departures.  The arguments and outputs of qot_lightpath_provision, then the releases and their grouping:
+ * rel_order [R] / rel_ptr [S+1] int64, sample s's releases are rel_order[rel_ptr[s] .. rel_ptr[s+1]), sorted by
+ * (before, k), and the ranges hold every release whose sample lies in [0, S).  Per sample the demands and releases are
+ * events in one sequence: before demand d every release of the sample with before <= d is applied, after the last
+ * demand the rest.
+ * Each demand and each release is evaluated against the state with every earlier event of its sample applied; a
+ * demand exactly as qot_lightpath_provision evaluates it (with R = 0 every demand output is bit-identical to it).  A
+ * release removes the lightpath from the sample: every channel of it is zeroed.  A demand accepted here gets one above
+ * the largest conn_id its sample has held, released lightpaths included, so conn_ids are never reused within a call.
+ * With a bound, a released lightpath's bound stops applying.  Outputs per release:
+ *   rel_status [R] int32     QOT_CAND_BAD_SAMPLE (sample outside [0, S)), QOT_CAND_BAD_STATE (the sample's state is
+ *                            inconsistent), QOT_TRAF_BAD_REF, QOT_TRAF_NOT_ACCEPTED (nothing removed with these),
+ *                            QOT_CAND_IMPACT_OVERFLOW (more neighbour rows than max_impact), QOT_PROV_BAD_GROUPING;
+ *   rel_conn_id [R] int64    the conn_id released (-1: none);
+ *   rel_n_impact [R] int32, rel_impact_conn [R, max_impact] int64, rel_impact_out [R, max_impact, 3]: the rows of the
+ *                            released lightpath's former neighbours after the release, ascending in node order, each
+ *                            bit-identical to the KIND_LOST row qot_lightpath_reconfigure gives for that teardown
+ *                            against the state just before it (message order: the neighbour's in-row ascending
+ *                            without the released lightpath, then its self loop); -1 / NaN past the rows;
+ *   rel_margin [R] float     with a bound, the minimum margin (placement rule, fp32) over every neighbour row,
+ *                            whatever max_impact is; NaN without a bound or without neighbours.  A release below a
+ *                            bound is reported, never refused.
+ * If rel_order / rel_ptr (or order / sample_ptr) are not such a grouping, nothing is provisioned or released: every
+ * demand and every release gets QOT_PROV_BAD_GROUPING alone, -1 / NaN rows and zero counts.  One copy and one launch,
+ * nothing read back: capturable; a malformed demand, release or grouping never faults and never stops the launch. */
+#define QOT_TRAF_BAD_REF 2048        /* the release names nothing in the sample at that point: an unknown or released
+                                        conn_id, a demand of another sample or not < before, before outside [0, D] */
+#define QOT_TRAF_NOT_ACCEPTED 4096   /* the named demand was not accepted: nothing to release                     */
+int qot_lightpath_traffic(const qot_lp_state_t* state, const qot_lp_demands_t* demands, const int64_t* order,
+                          const int64_t* sample_ptr, const float* bound, int32_t metric, int32_t maximize,
+                          int32_t policy, const float* prepared, int32_t is_lut_index, int32_t max_impact,
+                          int32_t* chan_work, float* bound_work, int32_t* option, int32_t* q0, float* out,
+                          float* margin, int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact,
+                          int64_t* conn_id, int64_t* impact_conn, float* impact_out,
+                          const qot_lp_releases_t* releases, const int64_t* rel_order, const int64_t* rel_ptr,
+                          int32_t* rel_status, int64_t* rel_conn_id, int32_t* rel_n_impact,
+                          int64_t* rel_impact_conn, float* rel_impact_out, float* rel_margin, void* stream);
 
 /* The topological representation: to_graph.py::create_topological_graph (:62-184: one edge per
  * lightpath between its source and destination network node, lightpaths added in ascending conn_id,
