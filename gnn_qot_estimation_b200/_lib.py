@@ -58,6 +58,10 @@ class QotLpReleases(C.Structure):
     _fields_ = [("R", i64), ("sample", P), ("before", P), ("demand", P), ("conn_id", P)]
 
 
+class QotLpFailures(C.Structure):
+    _fields_ = [("F", i64), ("n_links", i64), ("sample", P), ("link_ptr", P), ("links", P)]
+
+
 class QotLightpathParams(C.Structure):
     _fields_ = [("lin_w", P), ("att_src", P), ("att_dst", P), ("conv_bias", P),
                 ("bn_w", P), ("bn_b", P), ("bn_mean", P), ("bn_var", P),
@@ -142,6 +146,9 @@ SIGNATURES = {
     "qot_lightpath_traffic": (C.c_int, [C.POINTER(QotLpState), C.POINTER(QotLpDemands), P, P, P, i32, i32, i32, P,
                                         i32, i32, P, P, P, P, P, P, P, P, P, P, P, P, P,
                                         C.POINTER(QotLpReleases), P, P, P, P, P, P, P, P, vp]),
+    "qot_lightpath_restore": (C.c_int, [C.POINTER(QotLpState), C.POINTER(QotLpDemands), C.POINTER(QotLpFailures),
+                                        i32, i32, i32, P, P, i32, i32, P, P, i32, P, P, P, P, P, P, P, P, P, P, P, P, P,
+                                        P, P, vp]),
     "qot_topological_graph_scratch_bytes": (sz, [i64]),
     "qot_topological_graph_count": (C.c_int, [P, P, i64, C.POINTER(QotLpGraphCfg), i32, i32, i32, P, P, P, sz, P, vp]),
     "qot_topological_graph_fill": (C.c_int, [P, i64, P, P, P, P, P, vp]),

@@ -1782,6 +1782,405 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __gri
   if (zc) pl_flush(pa, pw, w, zc, 0, lane);
 }
 
+// ------------------------------------------------------------------------------------------------ restoration
+// lp_restore_kernel: persistent, one block per failure scenario (qot_lightpath_restore).  Scenario f names a sample s
+// and a set of failed links; any number of scenarios may name one sample, so the block works on its own slabs,
+// chan_work[b] and bound_work[b] (b = blockIdx.x), never on a slab of the sample's.  Per scenario:
+//   s's chan_node row is copied into chan_work[b], bound into bound_work[b] and the dense graph loaded as
+//     lp_provision_kernel loads it (rank = node order);
+//   the failed links' chan_node rows give the cut set C, a 256-bit mask by sample-local node; pv_release takes each
+//     cut lightpath out, highest node first (a release relabels only the highest stable id, so a lower node's stable
+//     id is still its node index when its turn comes), without its neighbours' rows;
+//   each c in C, ascending, is a demand with c's options (options.opt_ptr[n0 + c]), placed as lp_provision_kernel
+//     places a demand; an option whose route touches a failed link is skipped (bit po - o0 of `skip`): never scanned,
+//     never counted.  Option indices stay those of c's full list, so the tie rule (the lower index wins) is that of
+//     the filtered list.  An accepted demand goes in with pv_commit, then takes c's conn_id back;
+//   every remaining rank's row (its adjacency row by rank, then its self loop: the every-node row of the end state)
+//     goes through the same head, 12 warps round-robin, folded into end_margin / n_below and written to end_out.
+// The demand body is lp_provision_kernel's without the impact rows, so a restoration's outputs are bit-identical to
+// qot_lightpath_traffic's for the same releases and filtered demands.
+struct RsSmem {
+  PvSmem v;                                  // lp_provision_kernel's block state (head, warps, dense graph)
+  unsigned cut[kCdMaskWords];                // the cut set by sample-local node
+  unsigned skip;                             // the current demand's options that touch a failed link
+  unsigned e_mkey;                           // min of the end rows' margin keys
+  int e_below, f_st, n_rest;
+  long long c_conn;                          // the current demand's conn_id
+};
+static_assert(sizeof(RsSmem) + 16 <= 227 * 1024, "lp_restore_kernel: shared memory over the 227 KB block limit");
+
+struct RsArgs {
+  PvArgs v;                                // v.p.c.chan_node = v.chan_work = the [blocks, L, Q] slabs, v.p.bound =
+                                           // v.bound_work (or null); demand outputs at f * max_cut + i
+  const int32_t* chan_node;                // the state's [S, L, Q]
+  qot_lp_failures_t fail;
+  int max_cut;
+  int64_t* cut_node;                       // [F, max_cut]
+  int32_t* status;                         // [F]
+  int32_t* n_cut;
+  int32_t* n_restored;
+  float* end_margin;
+  int32_t* n_below;
+  int64_t* end_conn;                       // [F, kCdMaxN] or null
+  float* end_out;                          // [F, kCdMaxN, 3] or null
+};
+
+// the staged end rows, in staging order: their outputs into end_out (rtag: the rank) and, with a bound, their margins
+// into e_mkey / e_below.  Lane 0.
+__device__ __noinline__ void rs_end_fold(const RsArgs& ra, RsSmem& rs, const PlWarpSmem& pw, int cnt, int64_t f) {
+  const PlArgs& pa = ra.v.p;
+  for (int r = 0; r < cnt; ++r) {
+    if (ra.end_out)
+      for (int o = 0; o < QOT_OUT; ++o) ra.end_out[(f * kCdMaxN + pw.rtag[r]) * QOT_OUT + o] = pw.rout[r][o];
+    if (pa.bound) {
+      const float v = pw.rout[r][pa.metric], b = pa.bound[pw.rnode[r]];
+      const unsigned k = pl_okey(pa.maximize ? __fsub_rn(v, b) : __fsub_rn(b, v));
+      atomicMin(&rs.e_mkey, k);
+      if (k < 0x80000000u) atomicAdd(&rs.e_below, 1);    // margin < 0 or NaN
+    }
+  }
+}
+
+__global__ void __launch_bounds__(kCdThreads, 1) lp_restore_kernel(const __grid_constant__ RsArgs ra) {
+  const PvArgs& va = ra.v;
+  const PlArgs& pa = va.p;
+  const CdArgs& a = pa.c;
+  RsSmem& rs = *reinterpret_cast<RsSmem*>(cd_smem_raw);
+  PvSmem& sm = rs.v;
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  CdWarpSmem& ws = sm.cd.w[w];
+  PlWarpSmem& pw = sm.w[w];
+  float As[kF], Ad[kF];
+  cd_head_prologue(a.prep, As, Ad, tid);
+  const float nan = __int_as_float(0x7fc00000);
+  const int64_t b = blockIdx.x;                           // the block's slabs
+  const int MC = ra.max_cut;
+  int zc = 0;                                             // rows staged in this warp's head buffer
+  for (int64_t f = blockIdx.x; f < ra.fail.F; f += gridDim.x) {
+    const int L = a.cfg.L, Q = a.cfg.Q;
+    // ---- the scenario: its sample, its failed links, the sample's offsets
+    const int64_t s = ra.fail.sample[f];
+    const int64_t l0 = ra.fail.link_ptr[f], l1 = ra.fail.link_ptr[f + 1];
+    int fst = s < 0 || s >= a.S ? QOT_CAND_BAD_SAMPLE
+              : !(l0 >= 0 && l1 > l0 && l1 <= ra.fail.n_links) ? QOT_REST_BAD_FAILURE : 0;
+    bool lbad = false;
+    for (int64_t e = l0 + tid; fst == 0 && e < l1; e += kCdThreads) lbad |= ra.fail.links[e] < 0 || ra.fail.links[e] >= L;
+    int64_t n0 = 0;
+    int n = 0;
+    if (__syncthreads_or(lbad)) fst = QOT_REST_BAD_FAILURE;   // also: the previous scenario's state is no longer read
+    if (fst == 0 && !cd_sample_nodes(a, s, n0, n)) fst = QOT_CAND_BAD_STATE;
+    // ---- the sample's graph, in node order, and the block's slabs
+    for (int i = tid; i < kCdMaxN * kCdMaskWords; i += kCdThreads) (&sm.adj[0][0])[i] = 0u;
+    for (int r = tid; r < kCdMaxN; r += kCdThreads) {
+      sm.key[r] = INT_MAX;
+      sm.r2s[r] = sm.s2r[r] = static_cast<short>(r);
+    }
+    if (tid < kCdMaskWords) rs.cut[tid] = 0u;
+    if (tid == 0) {
+      sm.n_tot = fst == 0 ? n : 0;
+      sm.n_chan = 0;
+      sm.top = 0;
+      rs.e_mkey = 0xffffffffu;
+      rs.e_below = rs.n_rest = 0;
+    }
+    __syncthreads();
+    bool sbad = false;
+    if (fst == 0) {
+      for (int r = w; r < n; r += kCdWarps) sbad |= !cd_old_nbrs(a, n0, n, r, sm.adj[r], lane);
+      for (int i = tid; i < n * kF; i += kCdThreads) (&sm.x[0][0])[i] = a.x[n0 * kF + i];
+      for (int r = tid; r < n; r += kCdThreads) sm.conn[r] = va.conn_ids[n0 + r];
+      int nch = 0;
+      const int32_t* crow = ra.chan_node + s * L * Q;
+      int32_t* wrow = va.chan_work + b * L * Q;
+      for (int ch = tid; ch < L * Q; ch += kCdThreads) {
+        const int32_t v = crow[ch];
+        wrow[ch] = v;
+        if (v == -1) continue;
+        ++nch;
+        const int64_t j = static_cast<int64_t>(v) - n0;
+        if (v >= 0 && j >= 0 && j < n) atomicMin(&sm.key[j], ch);
+      }
+      atomicAdd(&sm.n_chan, nch);
+      if (va.bound_work)
+        for (int r = tid; r < n; r += kCdThreads) va.bound_work[b * kCdMaxN + r] = va.bound[n0 + r];
+      // the cut set: every known lightpath with a channel on a failed link
+      for (int64_t e = l0; e < l1; ++e) {
+        const int32_t* frow = crow + static_cast<int64_t>(ra.fail.links[e]) * Q;
+        for (int q = tid; q < Q; q += kCdThreads) {
+          const int64_t j = static_cast<int64_t>(frow[q]) - n0;
+          if (frow[q] >= 0 && j >= 0 && j < n) atomicOr(&rs.cut[j >> 5], 1u << (j & 31));
+        }
+      }
+    }
+    if (__syncthreads_or(sbad)) fst = QOT_CAND_BAD_STATE;
+    if (fst) {
+      if (tid < kCdMaskWords) rs.cut[tid] = 0u;
+      if (tid == 0) sm.n_tot = 0;
+      __syncthreads();
+    }
+    // ---- the cut lightpaths out, highest node first
+    int ncut = 0;
+#pragma unroll 1
+    for (int wd = kCdMaskWords - 1; wd >= 0; --wd)
+      for (unsigned bits = rs.cut[wd]; bits; ++ncut) {
+        const int hb = 31 - __clz(bits);
+        bits &= ~(1u << hb);
+        if (tid == 0) sm.r_rank = sm.s2r[32 * wd + hb];
+        pv_release(va, sm, b, n0, tid);
+      }
+    // ---- each cut lightpath, ascending, placed on its options that avoid the failed links
+    int i = 0;                                            // the cut lightpath's ordinal
+#pragma unroll 1
+    for (int wd = 0; wd < kCdMaskWords; ++wd)
+      for (unsigned bits = rs.cut[wd]; bits; bits &= bits - 1u, ++i) {
+        const int c = 32 * wd + __ffs(bits) - 1;
+        const int64_t v = n0 + c, k = f * MC + i;         // k: the output row (i < max_cut)
+        const int64_t o0 = pa.opt_ptr[v], o1 = pa.opt_ptr[v + 1];
+        // ---- validation (warp 0): the sample, the option range, every option's route and width; the skip mask
+        if (w == 0) {
+          const bool opts_ok = o0 >= 0 && o1 >= o0 && o1 <= pa.P && o1 - o0 <= kPlMaxOptions;
+          bool badp = !opts_ok;
+          unsigned skip = 0u;
+          for (int64_t po = o0; opts_ok && po < o1 && !badp; ++po) {
+            const int cw = a.width[po];
+            const int64_t p0 = a.link_ptr[po], p1 = a.link_ptr[po + 1];
+            badp = cd_bad_route(a, L, p0, p1, false, cw < 1 || cw > Q, lane);
+            bool hit = false;
+            for (int64_t e = p0 + lane; !badp && e < p1; e += 32)
+              for (int64_t g = l0; g < l1 && !hit; ++g) hit = a.links[e] == ra.fail.links[g];
+            if (__any_sync(kFull, hit)) skip |= 1u << (po - o0);
+          }
+          if (lane == 0) {
+            const unsigned all = o1 - o0 >= 32 ? 0xffffffffu : (1u << (o1 - o0)) - 1u;
+            sm.st = a.sample[v] != s ? QOT_CAND_BAD_SAMPLE : badp ? QOT_CAND_BAD_PATH
+                    : skip == all ? QOT_REST_NO_OPTION : 0;
+            rs.skip = skip;
+            rs.c_conn = va.conn_ids[v];
+          }
+        }
+        if (lane == 0) {
+          pw.key = 0ull;
+          pw.n_free = pw.n_feas = 0;
+        }
+        __syncthreads();
+        const auto row = [&](const int* msg, int M, int q, float* dst, int tag, long long node) {
+          if (lane == 0) {
+            pw.rtag[zc] = tag;
+            pw.rnode[zc] = node;
+          }
+          zc = cd_row(ws, zc, msg, M, q, PvX{sm.x, ws.cx, q, a.lut_col}, As, Ad, dst ? dst : pw.rout[zc],
+                      [&](int cnt) { pl_flush(pa, pw, w, cnt, o0, lane); }, lane);
+        };
+        int st = sm.st;                                   // block-uniform
+        const unsigned skip = rs.skip;
+        int seq = 0, wseq = 0;                            // placements of this demand: all, this warp's
+        for (int64_t po = o0; st == 0 && po < o1; ++po) {
+          if (skip >> (po - o0) & 1u) continue;
+          const int64_t p0 = a.link_ptr[po], p1 = a.link_ptr[po + 1];
+          const int cw = a.width[po];
+          // ---- warp 0: the route's occupied bitmap and its channels of known lightpaths by rank, one read per row
+          if (w == 0) {
+            unsigned occ = 0u;
+            int ne = 0;
+            bool rbad = false;
+            const int nt = sm.n_tot;
+            for (int64_t e = p0; e < p1; ++e) {
+              const int32_t* crow = va.chan_work + (b * L + a.links[e]) * Q;
+              for (int qb = 0; qb < Q; qb += 32) {
+                const int q = qb + lane;
+                const int32_t cv = q < Q ? __ldcg(crow + q) : -1;
+                const unsigned ob = __ballot_sync(kFull, cv != -1);
+                if (lane == qb >> 5) occ |= ob;
+                const int64_t j = static_cast<int64_t>(cv) - n0;
+                const bool known = cv >= 0 && j >= 0 && j < nt;
+                rbad |= cv >= 0 && !known;
+                const unsigned kb = __ballot_sync(kFull, known);
+                const int at = ne + __popc(kb & ((1u << lane) - 1u));
+                if (known && at < kPlEntCap) sm.ent[at] = q << 8 | sm.s2r[j];
+                ne += __popc(kb);
+              }
+            }
+            sm.run[lane] = pl_free_starts(occ, Q, cw, lane);
+            rbad = __any_sync(kFull, rbad);
+            if (lane == 0) {
+              sm.ne = ne;
+              sm.rbad = rbad;
+            }
+          }
+          __syncthreads();
+          if (sm.rbad) {
+            st |= QOT_CAND_BAD_STATE;
+            break;
+          }
+          // ---- the free starts in ascending order, dealt round-robin to the warps
+          const int ne = sm.ne;
+          for (int wd2 = 0; wd2 < 32 && 32 * wd2 < Q; ++wd2) {
+            for (unsigned fb = sm.run[wd2]; fb; fb &= fb - 1u) {
+              const int q0 = 32 * wd2 + __ffs(fb) - 1;
+              if (seq++ % kCdWarps != w) continue;
+              if (lane < kCdMaskWords) ws.mask[lane] = 0u;
+              __syncwarp();
+              if (ne <= kPlEntCap) pl_ent_mask(a, sm.ent, ne, q0, cw, ws.mask, lane);
+              else pv_scan(va, sm, b, n0, p0, p1, q0, cw, ws.mask, lane);
+              __syncwarp();
+              const int nn = cd_rank(lane < kCdMaskWords ? ws.mask[lane] : 0u, ws.nbr, lane);
+              cd_xrow(a, ws.cx, [&] { return lane == 0 ? static_cast<float>(a.freqs[q0]) : a.feat[po * 3 + lane - 1]; },
+                      lane);
+              const int slot = wseq++ & (kPlRing - 1);
+              const int nimp = pa.bound ? nn : 0;         // impact rows count against a bound, all of them
+              if (lane == 0) {
+                ws.nbr[nn] = kCand;
+                PlPending& pp = pw.ring[slot];
+                pp.mkey = 0xffffffffu;
+                pp.left = 1 + nimp;
+                pp.p = static_cast<int>(po);
+                pp.q0 = q0;
+                ++pw.n_free;
+              }
+              __syncwarp();
+              row(ws.nbr, nn + 1, kCand, nullptr, slot, -1);
+              for (int e = 0; e < nimp; ++e) {
+                const int r = ws.nbr[e];
+                const int m = cd_rank(lane < kCdMaskWords ? sm.adj[r][lane] : 0u, ws.msg, lane);
+                if (lane == 0) {
+                  ws.msg[m] = kCand;
+                  ws.msg[m + 1] = r;
+                }
+                __syncwarp();
+                row(ws.msg, m + 2, r, nullptr, slot, b * kCdMaxN + sm.r2s[r]);
+              }
+            }
+          }
+          __syncthreads();                                // the entries and free words are read
+        }
+        // ---- every placement folded: the block's winner and counts
+        if (zc) {
+          pl_flush(pa, pw, w, zc, o0, lane);
+          zc = 0;
+        }
+        __syncthreads();
+        if (tid == 0) {
+          unsigned long long key = 0ull;
+          int nf = 0, nfe = 0, bw = -1;
+          for (int u = 0; u < kCdWarps; ++u) {
+            nf += sm.w[u].n_free;
+            nfe += sm.w[u].n_feas;
+            if (sm.w[u].key > key) {
+              key = sm.w[u].key;
+              bw = u;
+            }
+          }
+          sm.key_best = key;
+          sm.n_free = nf;
+          sm.n_feas = nfe;
+          if (bw >= 0)
+            for (int o = 0; o < 4; ++o) sm.best[o] = sm.w[bw].best[o];
+        }
+        __syncthreads();
+        // ---- warp 0: the winner's neighbours (for pv_commit) and the demand's outputs; acceptance
+        if (w == 0) {
+          const unsigned long long key = st ? 0ull : sm.key_best;
+          int bp = -1, bq = -1;
+          int64_t po = -1, p0 = 0, p1 = 0;
+          int cw = 0;
+          if (key) {
+            const unsigned idx = 0xffffffffu - static_cast<unsigned>(key);
+            bp = static_cast<int>(idx >> 10);
+            bq = static_cast<int>(idx & 1023u);
+            po = o0 + bp;
+            p0 = a.link_ptr[po];
+            p1 = a.link_ptr[po + 1];
+            cw = a.width[po];
+            if (lane < kCdMaskWords) sm.wmask[lane] = 0u;
+            __syncwarp();
+            pv_scan(va, sm, b, n0, p0, p1, bq, cw, sm.wmask, lane);
+            cd_xrow(a, ws.cx, [&] { return lane == 0 ? static_cast<float>(a.freqs[bq]) : a.feat[po * 3 + lane - 1]; },
+                    lane);
+            __syncwarp();
+          }
+          const bool fatal = st & (kPlFatal | QOT_REST_NO_OPTION);
+          // the graph builder refuses a sample over QOT_TG_MAX_NODES lightpaths or QOT_TG_MAX_CHANNELS channels
+          const bool full = key && (sm.n_tot >= kCdMaxN || sm.n_chan + (p1 - p0) * cw > QOT_TG_MAX_CHANNELS);
+          const bool acc = key && !full;
+          int first = INT_MAX;                            // the accepted lightpath's first channel
+          for (int64_t e = p0 + lane; acc && e < p1; e += 32) first = min(first, a.links[e] * Q + bq);
+          first = __reduce_min_sync(kFull, first);
+          if (i < MC) {
+            if (lane < QOT_OUT) a.out[k * QOT_OUT + lane] = key ? sm.best[lane] : nan;
+            if (lane == 0) {
+              ra.cut_node[k] = v;
+              a.status[k] = st | (full ? QOT_PROV_FULL : 0);
+              pa.option[k] = bp;
+              pa.q0[k] = bq;
+              pa.margin[k] = key ? sm.best[3] : nan;
+              pa.n_free[k] = fatal ? 0 : sm.n_free;
+              pa.n_feasible[k] = fatal ? 0 : sm.n_feas;
+            }
+          }
+          if (lane == 0) {
+            sm.acc = acc;
+            sm.c_po = po;
+            sm.c_q0 = bq;
+            sm.c_key = first;
+          }
+        }
+        __syncthreads();
+        if (!sm.acc) continue;
+        pv_commit(va, sm, b, n0, tid);
+        if (tid == 0) {                                   // the restored lightpath keeps its conn_id
+          sm.conn[sm.s2r[sm.n_tot - 1]] = rs.c_conn;
+          ++rs.n_rest;
+        }
+      }
+    // ---- the end state: every rank's row through the head, its margin against its bound
+    __syncthreads();
+    const int nt = sm.n_tot;
+    if (pa.bound || ra.end_out) {
+      const auto flush = [&](int cnt) {
+        cd_flush(w, cnt, a.prep, lane);
+        if (lane == 0) rs_end_fold(ra, rs, pw, cnt, f);
+        __syncwarp();
+      };
+      for (int r = w; r < nt; r += kCdWarps) {
+        const int m = cd_rank(lane < kCdMaskWords ? sm.adj[r][lane] : 0u, ws.msg, lane);
+        if (lane == 0) {
+          ws.msg[m] = r;
+          pw.rtag[zc] = r;
+          pw.rnode[zc] = b * kCdMaxN + sm.r2s[r];
+        }
+        __syncwarp();
+        zc = cd_row(ws, zc, ws.msg, m + 1, r, PvX{sm.x, ws.cx, r, a.lut_col}, As, Ad, pw.rout[zc], flush, lane);
+      }
+      if (zc) {
+        flush(zc);
+        zc = 0;
+      }
+    }
+    __syncthreads();
+    // ---- the scenario's outputs, the unused cut rows and end rows
+    if (tid == 0) {
+      ra.status[f] = fst | (ncut > MC ? QOT_REST_CUT_OVERFLOW : 0);
+      ra.n_cut[f] = ncut;
+      ra.n_restored[f] = rs.n_rest;
+      ra.end_margin[f] = pa.bound && nt ? pl_unkey(rs.e_mkey) : nan;
+      ra.n_below[f] = pa.bound ? rs.e_below : 0;
+    }
+    for (int64_t u = f * MC + min(ncut, MC) + tid; u < (f + 1) * MC; u += kCdThreads) {
+      ra.cut_node[u] = -1;
+      a.status[u] = 0;
+      pa.option[u] = pa.q0[u] = -1;
+      pa.margin[u] = nan;
+      pa.n_free[u] = pa.n_feasible[u] = 0;
+      for (int o = 0; o < QOT_OUT; ++o) a.out[u * QOT_OUT + o] = nan;
+    }
+    if (ra.end_conn) {
+      for (int r = tid; r < kCdMaxN; r += kCdThreads) ra.end_conn[f * kCdMaxN + r] = r < nt ? sm.conn[r] : -1;
+      for (int u = nt * QOT_OUT + tid; u < kCdMaxN * QOT_OUT; u += kCdThreads)
+        ra.end_out[f * kCdMaxN * QOT_OUT + u] = nan;
+    }
+  }
+}
+
 static int cfg_check(const qot_lp_graph_cfg_t* cfg, const char* who) {
   QOT_REQUIRE(cfg, "%s: null cfg", who);
   QOT_REQUIRE(cfg->F > 0 && cfg->L > 0 && cfg->Q > 0 && cfg->L <= 65535 && cfg->Q <= 65535 &&
@@ -1947,6 +2346,58 @@ static int pv_launch(const char* who, const qot_lp_state_t* state, const qot_lp_
   return QOT_OK;
 }
 
+// qot_lightpath_restore: the checks and the launch (the kernel copies each scenario's chan_node row itself)
+static int rs_launch(const qot_lp_state_t* state, const qot_lp_demands_t* options, const qot_lp_failures_t* failures,
+                     int32_t policy, int32_t metric, int32_t maximize, const float* bound, const float* prepared,
+                     int32_t is_lut_index, int32_t max_cut, int32_t* chan_work, float* bound_work, int32_t n_blocks,
+                     int64_t* cut_node, int32_t* option, int32_t* q0, float* out, float* margin, int32_t* n_free,
+                     int32_t* n_feasible, int32_t* cut_status, int32_t* status, int32_t* n_cut, int32_t* n_restored,
+                     float* end_margin, int32_t* n_below, int64_t* end_conn, float* end_out, cudaStream_t stream) {
+  const char* who = "qot_lightpath_restore";
+  RsArgs ra;
+  PvArgs& va = ra.v;
+  PlArgs& pa = va.p;
+  CdArgs& a = pa.c;
+  QOT_REQUIRE(failures, "%s: null failures descriptor", who);
+  if (int rc = pl_demand_args(who, pa, state, options, metric, maximize, policy, prepared, is_lut_index, 0)) return rc;
+  const qot_lp_state_t& st = *state;
+  const qot_lp_demands_t& d = *options;
+  const qot_lp_failures_t& fl = *failures;
+  QOT_REQUIRE(fl.F >= 0 && fl.n_links >= 0 && max_cut >= 0 && n_blocks >= 1, "%s: bad size", who);
+  QOT_REQUIRE(d.D == st.N, "%s: the options hold %lld demands, the state %lld nodes (one demand per node)", who,
+              static_cast<long long>(d.D), static_cast<long long>(st.N));
+  if (fl.F == 0) return QOT_OK;
+  QOT_REQUIRE(fl.sample && fl.link_ptr && (fl.n_links == 0 || fl.links), "%s: null failure array", who);
+  QOT_REQUIRE(d.D == 0 || (d.sample && d.opt_ptr && d.link_ptr && (d.P == 0 || (d.width && d.feat && d.own_bound)) &&
+                           (d.n_links == 0 || d.links)),
+              "%s: null option array", who);
+  QOT_REQUIRE(status && n_cut && n_restored && end_margin && n_below && !end_conn == !end_out &&
+                  (max_cut == 0 || (cut_node && option && q0 && out && margin && n_free && n_feasible && cut_status)),
+              "%s: null output array", who);
+  QOT_REQUIRE(chan_work && (!bound || bound_work) && (st.N == 0 || st.conn_ids), "%s: null work or conn_ids array",
+              who);
+  if (int rc = cd_state_args(who, a, st, prepared, is_lut_index, 0)) return rc;
+  constexpr int smem = static_cast<int>(sizeof(RsSmem));
+  if (int rc = cd_smem_opt_in<lp_restore_kernel, smem>()) return rc;
+  a.chan_node = chan_work;
+  a.out = out; a.status = cut_status; a.n_impact = nullptr; a.impact_node = nullptr; a.impact_out = nullptr;
+  pa.bound = bound ? bound_work : nullptr;
+  pa.option = option; pa.q0 = q0; pa.margin = margin; pa.n_free = n_free; pa.n_feasible = n_feasible;
+  pa.all_out = nullptr; pa.all_margin = nullptr;
+  va = PvArgs{pa, nullptr, nullptr, st.conn_ids, bound, chan_work, bound ? bound_work : nullptr, nullptr,
+              qot_lp_releases_t{0, nullptr, nullptr, nullptr, nullptr}, nullptr, nullptr, nullptr, nullptr, nullptr,
+              nullptr, nullptr, nullptr};
+  ra.chan_node = st.chan_node;
+  ra.fail = fl;
+  ra.max_cut = max_cut;
+  ra.cut_node = cut_node; ra.status = status; ra.n_cut = n_cut; ra.n_restored = n_restored;
+  ra.end_margin = end_margin; ra.n_below = n_below; ra.end_conn = end_conn; ra.end_out = end_out;
+  const unsigned grid = static_cast<unsigned>(std::min<int64_t>(n_blocks, fl.F));
+  lp_restore_kernel<<<grid, kCdThreads, smem, stream>>>(ra);
+  QOT_LAUNCH_CHECK();
+  return QOT_OK;
+}
+
 }  // namespace qot
 
 using namespace qot;
@@ -2072,4 +2523,18 @@ extern "C" int qot_lightpath_traffic(const qot_lp_state_t* state, const qot_lp_d
                    max_impact, chan_work, bound_work, option, q0, out, margin, n_free, n_feasible, status, n_impact,
                    conn_id, impact_conn, impact_out, releases, rel_order, rel_ptr, rel_status, rel_conn_id,
                    rel_n_impact, rel_impact_conn, rel_impact_out, rel_margin, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int qot_lightpath_restore(const qot_lp_state_t* state, const qot_lp_demands_t* options,
+                                     const qot_lp_failures_t* failures, int32_t policy, int32_t metric,
+                                     int32_t maximize, const float* bound, const float* prepared, int32_t is_lut_index,
+                                     int32_t max_cut, int32_t* chan_work, float* bound_work, int32_t n_blocks,
+                                     int64_t* cut_node, int32_t* option, int32_t* q0, float* out, float* margin,
+                                     int32_t* n_free, int32_t* n_feasible, int32_t* cut_status, int32_t* status,
+                                     int32_t* n_cut, int32_t* n_restored, float* end_margin, int32_t* n_below,
+                                     int64_t* end_conn, float* end_out, void* stream) {
+  return rs_launch(state, options, failures, policy, metric, maximize, bound, prepared, is_lut_index, max_cut,
+                   chan_work, bound_work, n_blocks, cut_node, option, q0, out, margin, n_free, n_feasible, cut_status,
+                   status, n_cut, n_restored, end_margin, n_below, end_conn, end_out,
+                   static_cast<cudaStream_t>(stream));
 }

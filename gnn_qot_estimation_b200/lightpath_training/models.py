@@ -294,6 +294,45 @@ class LightpathGNN(torch.nn.Module):
                                      self.is_lut_index, max_impact)
 
     @_lib.on_tensor_device
+    def forward_restoration(self, state, options, failures, policy: int, metric: int = 0, maximize: bool = True,
+                            bound=None, max_cut: int = 64, return_end: bool = False) -> "ops.RestorationQoT":
+        """Failure restoration: for every link failure scenario, the lightpaths it cuts released and restored on routes
+        that avoid it, and the end state's QoT, in one pass (eval mode only; csrc/lightpath_candidates.cu,
+        qot_lightpath_restore).
+
+        ``failures``: ``to_graph.LightpathFailures`` (``to_graph.single_link_failures`` gives every single-link one);
+        ``options``: ``to_graph.LightpathDemands`` with one demand per node of ``state.batch`` (``sample[v] ==
+        state.batch.batch[v]``), demand v holding lightpath v's restoration options (0..32;
+        ``synthetic.lightpath_restoration_options`` draws such options).  Scenario f is defined by ``forward_traffic``
+        on a copy of its sample s alone: the cut set C is every lightpath of s with an occupied channel on a failed
+        link, in ascending node order; every lightpath of C is released by conn_id at ``before = 0`` (no release rows);
+        then each c in C, in order, is one demand whose options are c's options whose route uses no failed link, in
+        their order (none left: status ``ops.REST_NO_OPTION``, no demand), placed exactly as ``forward_traffic`` places
+        it (policy, metric, maximize, ``bound`` by node, ``PROV_FULL``, the tie rule).  A restored lightpath keeps its
+        conn_id, and from then on its bound is its chosen option's ``own_bound``.
+
+        Returns ``ops.RestorationQoT``.  Per cut lightpath (the first ``max_cut`` of C, ``[f, i]``): ``cut_node``,
+        then ``option`` (the index in c's full option list), ``q0``, ``out``, ``margin``, ``n_free``, ``n_feasible``
+        and ``cut_status``, bit-identical to that ``forward_traffic`` call's demand outputs (options crossing the
+        failure are neither scanned nor counted); ``CAND_BAD_PATH`` covers a bad option route, width or option count,
+        ``CAND_BAD_SAMPLE`` an ``options.sample[v]`` that is not v's sample.  Per scenario: ``status``
+        (``CAND_BAD_SAMPLE``, ``CAND_BAD_STATE``, ``ops.REST_BAD_FAILURE`` -- an empty link set, a link outside [0, L)
+        or a malformed ``link_ptr`` -- with which nothing is done; ``ops.REST_CUT_OVERFLOW`` when more than ``max_cut``
+        lightpaths are cut: all are restored and counted, the first ``max_cut`` reported), ``n_cut``, ``n_restored``,
+        and on the end state (the sample after the cuts and every restoration), with a ``bound``, ``end_margin`` (the
+        minimum margin over every lightpath present, by the fp32 rule of placements, against ``bound[node]`` for a
+        survivor and the chosen option's ``own_bound`` for a restored one; NaN without a bound or lightpaths) and
+        ``n_below`` (lightpaths whose margin is not >= 0).  GAT attention is not monotone: a survivor can end below its
+        bound.  ``return_end=True`` adds ``end_conn`` [F, 256] / ``end_out`` [F, 256, 3], every end-state lightpath in
+        the builder's node order (first channel) with the row ``forward_every_node`` gives on the committed end state,
+        -1 / NaN past them.  ``state`` is never modified; scenarios are independent, any number naming one sample.
+        Work memory is per resident block (one per SM), not per scenario.  One launch, nothing read back: capturable
+        in a CUDA graph.  Malformed arguments raise on the host."""
+        self._check_state_query("forward_restoration", state)
+        return ops.lightpath_restoration(state, options, failures, policy, metric, maximize, bound, self.prepared(),
+                                         self.is_lut_index, max_cut, return_end)
+
+    @_lib.on_tensor_device
     def forward_stream(self, plan, first: int = 0, count=None) -> None:
         """Enqueues batches [first, first+count) of ``plan`` (eval mode; no host synchronisation)."""
         if self.training:

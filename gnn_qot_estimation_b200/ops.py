@@ -756,6 +756,77 @@ def lightpath_traffic(state, demands, releases, policy: int, metric: int, maximi
             "qot_lightpath_traffic")
     return res
 
+
+# status bits of qot_lightpath_restore, on top of the CAND_* and PROV_* bits: per cut lightpath REST_NO_OPTION, per
+# scenario REST_BAD_FAILURE and REST_CUT_OVERFLOW
+REST_NO_OPTION, REST_BAD_FAILURE, REST_CUT_OVERFLOW = 8192, 16384, 32768
+
+
+class RestorationQoT(NamedTuple):
+    cut_node: torch.Tensor       # [F, max_cut] int64: the cut lightpaths, ascending state-batch nodes; -1 past them
+    option: torch.Tensor         # [F, max_cut] int32: the chosen option, in the lightpath's full list (-1: none)
+    q0: torch.Tensor             # [F, max_cut] int32: its start slot (-1: none)
+    out: torch.Tensor            # [F, max_cut, 3]: the restored lightpath's own QoT (NaN: none)
+    margin: torch.Tensor         # [F, max_cut]: its margin (NaN: none)
+    n_free: torch.Tensor         # [F, max_cut] int32: free placements over the options that avoid the failure
+    n_feasible: torch.Tensor     # [F, max_cut] int32: feasible placements among them
+    cut_status: torch.Tensor     # [F, max_cut] int32, CAND_* | PROV_FULL | REST_NO_OPTION bits
+    status: torch.Tensor         # [F] int32: CAND_BAD_SAMPLE | CAND_BAD_STATE | REST_BAD_FAILURE | REST_CUT_OVERFLOW
+    n_cut: torch.Tensor          # [F] int32: lightpaths the failure cuts (may exceed max_cut)
+    n_restored: torch.Tensor     # [F] int32: those restored
+    end_margin: torch.Tensor     # [F]: with a bound, the minimum margin over the end state's lightpaths (else NaN)
+    n_below: torch.Tensor        # [F] int32: with a bound, the end state's lightpaths whose margin is not >= 0
+    end_conn: Optional[torch.Tensor] = None    # [F, 256] int64 (return_end): the end state's conn_ids in node order
+    end_out: Optional[torch.Tensor] = None     # [F, 256, 3] (return_end): their every-node rows; NaN past them
+
+
+_FAILURE_DTYPES = {"sample": torch.int64, "link_ptr": torch.int64, "links": torch.int32}
+
+
+def lightpath_restoration(state, options, failures, policy: int, metric: int, maximize: bool, bound,
+                          prepared: torch.Tensor, is_lut_index: int, max_cut: int,
+                          return_end: bool = False) -> RestorationQoT:
+    """qot_lightpath_restore: every failure scenario's cut lightpaths released and restored on routes that avoid the
+    failure, one block per scenario.  The work slabs are allocated here at one block per SM; one launch, nothing read
+    back (CUDA-graph capturable).  The host checks of ``lightpath_provision`` (``options`` as the demands) plus one
+    demand per state node and the dtypes, shapes and device of the three failure tensors."""
+    who = "forward_restoration"
+    if int(max_cut) != max_cut or max_cut < 0:
+        raise ValueError(f"{who}: max_cut must be a non-negative integer")
+    D, P = _check_demand_args(who, state, options, policy, metric, bound, prepared, 0)
+    N = int(state.batch.x.shape[0])
+    if D != N:
+        raise ValueError(f"{who}: options must hold one demand per state node ({N}), got {D}")
+    dev = state.batch.x.device
+    for name, dt in _FAILURE_DTYPES.items():
+        _check_state_tensor(who, f"failures.{name}", getattr(failures, name), dev, dt)
+    F = int(failures.sample.shape[0]) if failures.sample.dim() == 1 else -1
+    if F < 0 or failures.link_ptr.shape != (F + 1,) or failures.links.dim() != 1:
+        raise ValueError(f"{who}: need failures.sample [F], link_ptr [F+1], links [n]")
+    max_cut = int(max_cut)
+    i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=dev)
+    f32 = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)
+    res = RestorationQoT(torch.empty(F, max_cut, dtype=torch.int64, device=dev), i32(F, max_cut), i32(F, max_cut),
+                         f32(F, max_cut, 3), f32(F, max_cut), i32(F, max_cut), i32(F, max_cut), i32(F, max_cut),
+                         i32(F), i32(F), i32(F), f32(F), i32(F),
+                         torch.empty(F, TG_MAX_NODES, dtype=torch.int64, device=dev) if return_end else None,
+                         f32(F, TG_MAX_NODES, 3) if return_end else None)
+    if F == 0:
+        return res
+    blocks = torch.cuda.get_device_properties(dev).multi_processor_count
+    chan_work = torch.empty(blocks, state.L, state.Q, dtype=torch.int32, device=dev)
+    bound_work = torch.empty(blocks, TG_MAX_NODES, dtype=torch.float32, device=dev) if bound is not None else None
+    bound = None if bound is None else bound.contiguous()
+    fl = [getattr(failures, n).contiguous() for n in _FAILURE_DTYPES]
+    keep = list(fl)
+    with torch.cuda.device(dev):
+        check(_lib.lib().qot_lightpath_restore(
+            C.byref(_state_desc(state, keep)), C.byref(_demands_desc(options, D, P, keep)),
+            C.byref(_lib.QotLpFailures(F, int(fl[2].numel()), *(_cptr(t) for t in fl))), int(policy), int(metric),
+            int(bool(maximize)), _cptr(bound), ptr(prepared), int(is_lut_index), max_cut, ptr(chan_work),
+            _cptr(bound_work), blocks, *(_cptr(t) for t in res), stream()), "qot_lightpath_restore")
+    return res
+
 class GraphIndex:
     """Lazily built, cached index structures of one batch: the destination-sorted CSR
     (forward), its GAT variant (self loops replaced) and the source-sorted transposed

@@ -603,3 +603,59 @@ def lightpath_traffic(samples, per_sample: int, load: float, options=(1, 4), see
     ro = np.argsort(np.asarray(r_t), kind="stable")            # releases in time order (the index is cosmetic)
     pick = lambda v: torch.tensor(np.asarray(v, dtype=np.int64)[ro] if len(v) else np.zeros(0, dtype=np.int64))
     return demands, LightpathReleases(pick(r_s), pick(r_b), pick(r_d), pick(r_c))
+
+
+def lightpath_restoration_options(samples, state, options=(1, 4), seed: int = 0, bound_range=(0.1, 0.6)):
+    """Seeded restoration options for every lightpath of ``state`` (built from the network-status ``samples``), for
+    ``LightpathGNN.forward_restoration``: ``to_graph.LightpathDemands`` of CPU tensors with one demand per node of
+    ``state.batch`` (``sample[v]`` = v's sample) and ``options[0]..options[1]`` options each.  Option 0 is the
+    lightpath's current route (the links it occupies, ascending) and width (its slots on its first link) with its own
+    (mod_order, num_spans, path_len), so a failure of one of its links always filters it out; the others are drawn as
+    ``lightpath_demands`` draws them, as is ``own_bound`` (one kind per lightpath: -inf, +inf or uniform in
+    ``bound_range`` per option).  One host copy of the state's channel map."""
+    import numpy as np
+    from .to_graph import LightpathDemands
+    rng = np.random.default_rng(seed)
+    lo, hi = int(options[0]), int(options[1])
+    if not 1 <= lo <= hi:
+        raise ValueError("options must be (lo, hi) with 1 <= lo <= hi")
+    data = samples["data"]
+    L = data.shape[2]
+    fi = {k: i for i, k in enumerate(samples["lp_feat"])}
+    chan = state.chan_node.cpu().numpy()
+    node_ptr = state.batch.ptr.cpu().numpy()
+    smp, optr, lptr, links, widths, feats, bounds = [], [0], [0], [], [], [], []
+    for s in range(state.S):
+        n0, n1 = int(node_ptr[s]), int(node_ptr[s + 1])
+        c = chan[s]
+        for v in range(n0, n1):
+            ll, qq = np.nonzero(c == v)
+            route = sorted(set(ll.tolist()))
+            width = int((ll == route[0]).sum()) if route else 1
+            l0, q0 = (int(ll[0]), int(qq[0])) if route else (0, 0)
+            smp.append(s)
+            kind = rng.random()
+            routes = [route] if route else []
+            for k in range(int(rng.integers(lo, hi + 1))):
+                if k == 0 and route:
+                    path, w = route, width
+                    f = [float(data[s, fi[n], l0, q0]) for n in ("mod_order", "num_spans", "path_len")]
+                else:
+                    if routes and rng.random() < 0.3:
+                        path = routes[int(rng.integers(0, len(routes)))]
+                    else:
+                        path = [int(l) for l in rng.choice(L, size=min(int(rng.integers(1, 7)), L), replace=False)]
+                        routes.append(path)
+                    w = int(rng.integers(1, 4))
+                    f = [rng.choice([4, 8, 16, 32, 64]), int(rng.integers(1, 107)), int(rng.integers(24214, 7834746))]
+                links.extend(path)
+                lptr.append(len(links))
+                widths.append(w)
+                feats.append(f)
+                bounds.append(-np.inf if kind < 0.2 else np.inf if kind < 0.4 else rng.uniform(*bound_range))
+            optr.append(len(widths))
+    return LightpathDemands(torch.tensor(smp, dtype=torch.int64), torch.tensor(optr, dtype=torch.int64),
+                            torch.tensor(lptr, dtype=torch.int64), torch.tensor(links, dtype=torch.int32),
+                            torch.tensor(widths, dtype=torch.int32),
+                            torch.tensor(np.array(feats, dtype=np.float32).reshape(-1, 3)),
+                            torch.tensor(np.array(bounds, dtype=np.float32)))

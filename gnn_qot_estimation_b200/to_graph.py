@@ -215,6 +215,29 @@ class LightpathReleases(NamedTuple):
         return LightpathReleases(*(t.to(device) for t in self))
 
 
+class LightpathFailures(NamedTuple):
+    """Link failure scenarios for ``LightpathGNN.forward_restoration`` (device tensors).  Scenario f fails the links
+    ``links[link_ptr[f]:link_ptr[f+1]]`` (non-empty; several links: a shared-risk group) of sample ``sample[f]``."""
+    sample: torch.Tensor          # [F] int64
+    link_ptr: torch.Tensor        # [F+1] int64
+    links: torch.Tensor           # [sum of set sizes] int32
+
+    def to(self, device) -> "LightpathFailures":
+        return LightpathFailures(*(t.to(device) for t in self))
+
+
+def single_link_failures(state: LightpathNetworkState) -> LightpathFailures:
+    """Every single-link failure that cuts something: one scenario per (sample, link) with an occupied channel of a
+    lightpath the state knows, in (sample, link) order, on the state's device.  One host synchronisation (the number
+    of scenarios), so not capturable; build the failures once and reuse them."""
+    used = (state.chan_node >= 0).any(2)                        # [S, L]
+    sl = used.nonzero()                                         # the host synchronisation; row-major: (sample, link)
+    F = int(sl.shape[0])
+    dev = state.chan_node.device
+    return LightpathFailures(sl[:, 0].contiguous(), torch.arange(F + 1, dtype=torch.int64, device=dev),
+                             sl[:, 1].to(torch.int32).contiguous())
+
+
 def lightpath_nodes(state: LightpathNetworkState, sample: torch.Tensor, conn_id: torch.Tensor) -> torch.Tensor:
     """[K] int64: the node of ``state.batch`` that holds lightpath ``conn_id[k]`` in sample ``sample[k]``, -1 where the
     sample has no such lightpath (or ``sample[k]`` is outside the state).  Device tensor ops, no host synchronisation:

@@ -586,6 +586,16 @@ typedef struct {
   const int64_t* conn_id;      /* [R]; read where demand[k] == -1                                           */
 } qot_lp_releases_t;           /* 40 bytes */
 
+/* Link failure scenarios for qot_lightpath_restore: F of them.  Scenario f names sample sample[f] of the state and the
+ * non-empty set of failed links links[link_ptr[f] .. link_ptr[f+1]) (int32; several links: a shared-risk group). */
+typedef struct {
+  int64_t F;
+  int64_t n_links;
+  const int64_t* sample;       /* [F]                                                                       */
+  const int64_t* link_ptr;     /* [F+1]                                                                     */
+  const int32_t* links;        /* [n_links]                                                                 */
+} qot_lp_failures_t;           /* 40 bytes */
+
 /* qot_lightpath_candidates (lp_candidate_kernel): K candidates, one warp each, one launch.  Candidate k names sample
  * sample[k], a path links[link_ptr[k] .. link_ptr[k+1]) (int32 link indices; duplicates change nothing), the slot
  * range [q0[k], q0[k] + width[k]) used on every link of the path and its raw channel vector feat [K,4] = (freq,
@@ -777,6 +787,49 @@ int qot_lightpath_traffic(const qot_lp_state_t* state, const qot_lp_demands_t* d
                           const qot_lp_releases_t* releases, const int64_t* rel_order, const int64_t* rel_ptr,
                           int32_t* rel_status, int64_t* rel_conn_id, int32_t* rel_n_impact,
                           int64_t* rel_impact_conn, float* rel_impact_out, float* rel_margin, void* stream);
+
+/* qot_lightpath_restore (lp_restore_kernel, one block of 12 warps per scenario, one launch): failure restoration.
+ * options: one demand per node of the state batch (D = N), demand v holding lightpath v's restoration options (0..32;
+ * options->sample[v] must be v's sample).  Scenario f (qot_lp_failures_t) is defined by qot_lightpath_traffic on a
+ * copy of sample s = sample[f] alone:
+ *   the cut set C: every lightpath of s with an occupied channel on a failed link, in ascending node order;
+ *   every lightpath of C released by conn_id before the first demand (no release rows);
+ *   for each c in C, in order, one demand: c's options whose route uses no failed link, in their order; a cut
+ *   lightpath with none is no demand (QOT_REST_NO_OPTION);
+ *   each demand placed exactly as qot_lightpath_traffic places it (policy, metric, maximize, bound by node, PROV_FULL,
+ *   the tie rule); a restored lightpath keeps its conn_id, and from then on its bound is its option's own_bound.
+ * Outputs per cut lightpath, the first max_cut of C at [f, i] (-1 / NaN / 0 past them), bit-identical to that call's
+ * demand outputs: cut_node [F, max_cut] int64 (the state-batch node), option (the index in c's full option list, -1:
+ * none), q0, out [.., 3], margin, n_free, n_feasible (options crossing a failed link neither scanned nor counted) and
+ * cut_status (QOT_CAND_BAD_SAMPLE: options->sample[v] is not v's sample; QOT_CAND_BAD_PATH: a bad option route, width
+ * or option count; QOT_CAND_BAD_STATE, QOT_PROV_FULL, QOT_REST_NO_OPTION; never QOT_CAND_IMPACT_OVERFLOW).
+ * Outputs per scenario, on the end state (the sample after the cuts and every restoration):
+ *   status [F] int32          QOT_CAND_BAD_SAMPLE (sample outside [0, S)), QOT_CAND_BAD_STATE (the sample's state is
+ *                             inconsistent), QOT_REST_BAD_FAILURE (nothing is done with these three: zero counts,
+ *                             -1 / NaN rows), QOT_REST_CUT_OVERFLOW (every cut lightpath is restored and counted, the
+ *                             first max_cut reported);
+ *   n_cut, n_restored [F] int32;
+ *   end_margin [F] float      with a bound, the minimum margin (placement rule, fp32) over every lightpath present at
+ *                             the end: bound[node] for a survivor, its option's own_bound for a restored one (NaN
+ *                             without a bound or without lightpaths);
+ *   n_below [F] int32         with a bound, the lightpaths whose margin is not >= 0 (0 without a bound);
+ *   end_conn [F, 256] int64, end_out [F, 256, 3] (both or neither): every end-state lightpath in the graph builder's
+ *                             node order (first channel), its conn_id and its every-node row (the row
+ *                             LightpathGNN.forward_every_node gives on the committed end state); -1 / NaN past them.
+ * Work arrays, per resident block b < n_blocks (>= 1; the grid is min(n_blocks, F)), never per scenario: chan_work
+ * [n_blocks, L, Q] int32 and bound_work [n_blocks, QOT_TG_MAX_NODES] float32 (required with a bound, else unused).
+ * Requires Q <= QOT_PLACE_MAX_SLOTS.  The state is not modified and scenarios are independent, any number of them
+ * naming one sample.  One launch, nothing read back: capturable; malformed input never faults and never stops it. */
+#define QOT_REST_NO_OPTION 8192      /* every option of the cut lightpath crosses a failed link, or it has none     */
+#define QOT_REST_BAD_FAILURE 16384   /* an empty link set, a link outside [0, L) or a malformed link_ptr          */
+#define QOT_REST_CUT_OVERFLOW 32768  /* more cut lightpaths than max_cut: all restored, the first max_cut reported */
+int qot_lightpath_restore(const qot_lp_state_t* state, const qot_lp_demands_t* options,
+                          const qot_lp_failures_t* failures, int32_t policy, int32_t metric, int32_t maximize,
+                          const float* bound, const float* prepared, int32_t is_lut_index, int32_t max_cut,
+                          int32_t* chan_work, float* bound_work, int32_t n_blocks, int64_t* cut_node, int32_t* option,
+                          int32_t* q0, float* out, float* margin, int32_t* n_free, int32_t* n_feasible,
+                          int32_t* cut_status, int32_t* status, int32_t* n_cut, int32_t* n_restored,
+                          float* end_margin, int32_t* n_below, int64_t* end_conn, float* end_out, void* stream);
 
 /* The topological representation: to_graph.py::create_topological_graph (:62-184: one edge per
  * lightpath between its source and destination network node, lightpaths added in ascending conn_id,
