@@ -146,6 +146,9 @@ SIGNATURES = {
     "qot_lightpath_traffic": (C.c_int, [C.POINTER(QotLpState), C.POINTER(QotLpDemands), P, P, P, i32, i32, i32, P,
                                         i32, i32, P, P, P, P, P, P, P, P, P, P, P, P, P,
                                         C.POINTER(QotLpReleases), P, P, P, P, P, P, P, P, vp]),
+    "qot_lightpath_protect": (C.c_int, [C.POINTER(QotLpState), C.POINTER(QotLpDemands), P, P, P, i32, i32, i32, P,
+                                        i32, i32, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P,
+                                        P, P, vp]),
     "qot_lightpath_restore": (C.c_int, [C.POINTER(QotLpState), C.POINTER(QotLpDemands), C.POINTER(QotLpFailures),
                                         i32, i32, i32, P, P, i32, i32, P, P, i32, P, P, P, P, P, P, P, P, P, P, P, P, P,
                                         P, P, vp]),

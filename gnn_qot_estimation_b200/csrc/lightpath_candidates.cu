@@ -33,6 +33,7 @@
 // and NaN rows; it never faults and never stops the launch.
 #include <algorithm>
 #include <climits>
+#include <type_traits>
 
 #include "lightpath_common.cuh"
 
@@ -1379,11 +1380,59 @@ __device__ __noinline__ void pv_commit(const PvArgs& va, PvSmem& sm, int64_t s, 
   __syncthreads();
 }
 
-template <bool kReleases>
-__global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __grid_constant__ PvArgs va) {
+// Protection (qot_lightpath_protect; kProtect): a protected demand (protect[d] != 0) is placed twice against the
+// block's state.  First the working path, over the options that have a link-disjoint partner among the demand's
+// options (the others are skipped as restoration skips options crossing a failed link: never scanned, never counted;
+// none left: QOT_PROT_NO_PARTNER).  An acceptable working path goes in with pv_commit (conn_id top + 1, its own_bound),
+// then the backup path is placed the same way over the options whose route shares no link with the working route,
+// its outputs written through bk (PtArgs: the backup output arrays).  An acceptable backup goes in as top + 2; else
+// pv_release takes the working path out again (stable id n_tot - 1, the highest: nothing is relabelled) and top goes
+// back, so the state is what it was before the demand.  The link sets are 1024-bit bitmaps (QOT_TG_MAX_LINKS), word
+// t held in bm[t].  An unprotected demand is handled exactly as without kProtect, its backup outputs empty.
+struct PtSmem {
+  PvSmem v;                                  // lp_provision_kernel's block state
+  unsigned bm[QOT_TG_MAX_LINKS / 32];        // a route's links
+  unsigned skip;                             // the current search's options skipped (bit po - o0)
+};
+static_assert(sizeof(PtSmem) + 16 <= 227 * 1024, "lp_provision_kernel<.., true>: shared memory over the 227 KB limit");
+static_assert(QOT_TG_MAX_LINKS == 32 * 32 && kPlMaxOptions <= 32, "one bitmap word per lane, one skip bit per option");
+
+struct PtArgs : PvArgs {
+  PvArgs bk;                               // the same arguments with the backup output arrays
+  const uint8_t* protect;                  // [D] or null (none protected)
+};
+template <bool kProtect>
+using PvKernelArgs = std::conditional_t<kProtect, PtArgs, PvArgs>;
+
+// route links[p0, p1) into the bitmap bm (all lanes of one warp; links checked to lie in [0, QOT_TG_MAX_LINKS))
+__device__ __forceinline__ void pt_route_bits(const CdArgs& a, int64_t p0, int64_t p1, unsigned* bm, int lane) {
+  bm[lane] = 0u;
+  __syncwarp();
+  for (int64_t e = p0 + lane; e < p1; e += 32) atomicOr(&bm[a.links[e] >> 5], 1u << (a.links[e] & 31));
+  __syncwarp();
+}
+
+// true on every lane when route links[p0, p1) shares a link with bm
+__device__ __forceinline__ bool pt_touches(const CdArgs& a, int64_t p0, int64_t p1, const unsigned* bm, int lane) {
+  bool hit = false;
+  for (int64_t e = p0 + lane; e < p1 && !hit; e += 32) hit = bm[a.links[e] >> 5] >> (a.links[e] & 31) & 1u;
+  return __any_sync(kFull, hit);
+}
+
+// the arguments a search writes its outputs through: the backup's in the backup search (ph = 1), else the demand's
+template <bool kProtect>
+__device__ __forceinline__ const PvArgs& pv_out_args(const PvKernelArgs<kProtect>& args, int ph) {
+  if constexpr (kProtect) return ph ? static_cast<const PvArgs&>(args.bk) : static_cast<const PvArgs&>(args);
+  else return args;
+}
+
+template <bool kReleases, bool kProtect = false>
+__global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __grid_constant__ PvKernelArgs<kProtect> args) {
+  const PvArgs& va = args;
   const PlArgs& pa = va.p;
   const CdArgs& a = pa.c;
   PvSmem& sm = *reinterpret_cast<PvSmem*>(cd_smem_raw);
+  PtSmem& pt = *reinterpret_cast<PtSmem*>(cd_smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   CdWarpSmem& ws = sm.cd.w[w];
   PlWarpSmem& pw = sm.w[w];
@@ -1454,10 +1503,15 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __gri
   if (bad) {
     for (int64_t d = gt; d < D; d += gs) pv_empty(va, d, QOT_PROV_BAD_GROUPING, 0, 1);
     for (int64_t k = gt; k < NR; k += gs) pv_rel_empty(va, k, QOT_PROV_BAD_GROUPING, 0, 0, 1);
+    if constexpr (kProtect)
+      for (int64_t d = gt; d < D; d += gs) pv_empty(args.bk, d, 0, 0, 1);
     return;
   }
   for (int64_t d = gt; d < D; d += gs)
     if (a.sample[d] < 0 || a.sample[d] >= S) pv_empty(va, d, QOT_CAND_BAD_SAMPLE, 0, 1);
+  if constexpr (kProtect)
+    for (int64_t d = gt; d < D; d += gs)
+      if (a.sample[d] < 0 || a.sample[d] >= S) pv_empty(args.bk, d, 0, 0, 1);
   for (int64_t k = gt; k < NR; k += gs)
     if (va.rel.sample[k] < 0 || va.rel.sample[k] >= S) pv_rel_empty(va, k, QOT_CAND_BAD_SAMPLE, 0, 0, 1);
   const float nan = __int_as_float(0x7fc00000);
@@ -1582,6 +1636,10 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __gri
       }
       if (i == i1) break;
       const int64_t o0 = pa.opt_ptr[d], o1 = pa.opt_ptr[d + 1];
+      [[maybe_unused]] bool prot = false;                 // kProtect: d is protected
+      [[maybe_unused]] int ph = 0;                        // kProtect: 0 the working path, 1 the backup
+      if constexpr (kProtect) prot = args.protect && args.protect[d];
+    search:                                               // kProtect: the backup search starts here again
       // ---- validation (warp 0): the option range, every option's route and width; then the state
       if (w == 0) {
         const bool opts_ok = o0 >= 0 && o1 > o0 && o1 <= pa.P && o1 - o0 <= kPlMaxOptions;
@@ -1592,6 +1650,30 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __gri
             badp = cd_bad_route(a, L, a.link_ptr[po], a.link_ptr[po + 1], false, cw < 1 || cw > Q, lane);
           }
         if (lane == 0) sm.st = badp ? QOT_CAND_BAD_PATH : sbad ? QOT_CAND_BAD_STATE : 0;
+        if constexpr (kProtect) {
+          // working: the options without a link-disjoint partner; backup: those sharing a link with the working route
+          unsigned skip = 0u;
+          if (prot && !badp) {
+            if (ph == 0) {
+              for (int64_t po = o0; po < o1; ++po) {
+                pt_route_bits(a, a.link_ptr[po], a.link_ptr[po + 1], pt.bm, lane);
+                bool partner = false;
+                for (int64_t p2 = o0; p2 < o1 && !partner; ++p2)
+                  partner = !pt_touches(a, a.link_ptr[p2], a.link_ptr[p2 + 1], pt.bm, lane);
+                if (!partner) skip |= 1u << (po - o0);
+              }
+            } else {                                      // sm.c_po: the working option, committed
+              pt_route_bits(a, a.link_ptr[sm.c_po], a.link_ptr[sm.c_po + 1], pt.bm, lane);
+              for (int64_t po = o0; po < o1; ++po)
+                if (pt_touches(a, a.link_ptr[po], a.link_ptr[po + 1], pt.bm, lane)) skip |= 1u << (po - o0);
+            }
+          }
+          if (lane == 0) {
+            pt.skip = skip;
+            if (prot && !badp && !sbad && skip == (o1 - o0 >= 32 ? 0xffffffffu : (1u << (o1 - o0)) - 1u))
+              sm.st = QOT_PROT_NO_PARTNER;
+          }
+        }
       }
       if (lane == 0) {
         pw.key = 0ull;
@@ -1608,7 +1690,11 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __gri
       };
       int st = sm.st;                                     // block-uniform
       int seq = 0, wseq = 0;                              // placements of this demand: all, this warp's
+      [[maybe_unused]] unsigned skip = 0u;
+      if constexpr (kProtect) skip = pt.skip;
       for (int64_t po = o0; st == 0 && po < o1; ++po) {
+        if constexpr (kProtect)
+          if (skip >> (po - o0) & 1u) continue;
         const int64_t p0 = a.link_ptr[po], p1 = a.link_ptr[po + 1];
         const int cw = a.width[po];
         // ---- warp 0: the route's occupied bitmap and its channels of known lightpaths by rank, one read per row
@@ -1712,6 +1798,10 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __gri
       __syncthreads();
       // ---- warp 0: the winner's impact rows and the demand's outputs; acceptance
       if (w == 0) {
+        // the outputs written: the demand's, or with kProtect in the backup search the backup's
+        const PvArgs& vo = pv_out_args<kProtect>(args, ph);
+        const PlArgs& po_ = vo.p;
+        const CdArgs& ao = po_.c;
         const int MI = a.max_impact;
         const unsigned long long key = sm.key_best;
         int cnt = 0, rows = 0, bp = -1, bq = -1;
@@ -1736,47 +1826,70 @@ __global__ void __launch_bounds__(kCdThreads, 1) lp_provision_kernel(const __gri
           __syncwarp();
           for (int k = 0; k < rows; ++k) {
             const int r = ws.nbr[k];
-            if (lane == 0) a.impact_node[d * MI + k] = sm.conn[r];
+            if (lane == 0) ao.impact_node[d * MI + k] = sm.conn[r];
             const int m = cd_rank(lane < kCdMaskWords ? sm.adj[r][lane] : 0u, ws.msg, lane);
             if (lane == 0) {
               ws.msg[m] = kCand;
               ws.msg[m + 1] = r;
             }
             __syncwarp();
-            row(ws.msg, m + 2, r, a.impact_out + (d * MI + k) * QOT_OUT, -1, -1);
+            row(ws.msg, m + 2, r, ao.impact_out + (d * MI + k) * QOT_OUT, -1, -1);
           }
         }
-        if (st & kPlFatal) {
-          pv_empty(va, d, st, lane, 32);
+        if (st & (kProtect ? kPlFatal | QOT_PROT_NO_PARTNER : kPlFatal)) {
+          pv_empty(vo, d, st, lane, 32);
           if (lane == 0) sm.acc = 0;
         } else {
-          cd_clear_impact(a, d, rows, MI, nullptr, lane, 32);
+          cd_clear_impact(ao, d, rows, MI, nullptr, lane, 32);
           // the graph builder refuses a sample over QOT_TG_MAX_NODES lightpaths or QOT_TG_MAX_CHANNELS channels
           const bool full = key && (sm.n_tot >= kCdMaxN || sm.n_chan + (p1 - p0) * cw > QOT_TG_MAX_CHANNELS);
           const bool acc = key && !full;
           int first = INT_MAX;                            // the accepted lightpath's first channel
           for (int64_t e = p0 + lane; acc && e < p1; e += 32) first = min(first, a.links[e] * Q + bq);
           first = __reduce_min_sync(kFull, first);
-          if (lane < QOT_OUT) a.out[d * QOT_OUT + lane] = key ? sm.best[lane] : nan;
+          if (lane < QOT_OUT) ao.out[d * QOT_OUT + lane] = key ? sm.best[lane] : nan;
           if (lane == 0) {
-            a.status[d] = st | (cnt > MI ? QOT_CAND_IMPACT_OVERFLOW : 0) | (full ? QOT_PROV_FULL : 0);
-            a.n_impact[d] = cnt;
-            pa.option[d] = bp;
-            pa.q0[d] = bq;
-            pa.margin[d] = key ? sm.best[3] : nan;
-            pa.n_free[d] = sm.n_free;
-            pa.n_feasible[d] = sm.n_feas;
-            va.conn_id[d] = acc ? sm.top + 1 : -1;
+            ao.status[d] = st | (cnt > MI ? QOT_CAND_IMPACT_OVERFLOW : 0) | (full ? QOT_PROV_FULL : 0);
+            ao.n_impact[d] = cnt;
+            po_.option[d] = bp;
+            po_.q0[d] = bq;
+            po_.margin[d] = key ? sm.best[3] : nan;
+            po_.n_free[d] = sm.n_free;
+            po_.n_feasible[d] = sm.n_feas;
+            vo.conn_id[d] = acc ? sm.top + 1 : -1;
             sm.acc = acc;
             sm.c_po = po;
             sm.c_q0 = bq;
             sm.c_key = first;
           }
         }
+        if constexpr (kProtect) {
+          __syncwarp();
+          const bool acc = sm.acc;
+          if (ph == 0 && !(prot && acc)) pv_empty(args.bk, d, 0, lane, 32);   // no backup search: empty
+          if (ph == 1 && !acc && lane == 0) {             // no backup: the demand is not accepted
+            a.status[d] |= QOT_PROT_NO_BACKUP;
+            va.conn_id[d] = -1;
+          }
+        }
       }
       __syncthreads();
+      if constexpr (kProtect) {
+        if (ph == 1 && !sm.acc) {                         // the working path out again, top back
+          if (tid == 0) {
+            sm.r_rank = sm.s2r[sm.n_tot - 1];
+            sm.top -= 1;
+          }
+          pv_release(va, sm, s, n0, tid);
+          continue;
+        }
+      }
       if (!sm.acc) continue;
       pv_commit(va, sm, s, n0, tid);
+      if (kProtect && prot && ph == 0) {                  // the working path is in: its backup
+        ph = 1;
+        goto search;
+      }
     }
   }
   if (zc) pl_flush(pa, pw, w, zc, 0, lane);
@@ -2286,8 +2399,18 @@ static int cd_launch(const char* who, const qot_lp_state_t* state, const qot_lp_
   return QOT_OK;
 }
 
-// qot_lightpath_provision (rel = null: no releases) and qot_lightpath_traffic: the checks, the copy of chan_node and
-// the launch
+// qot_lightpath_protect's additions: the protect flags and the backup outputs
+struct PtOut {
+  const uint8_t* protect;
+  int32_t *option, *q0;
+  float *out, *margin;
+  int32_t *n_free, *n_feasible, *status, *n_impact;
+  int64_t *conn_id, *impact_conn;
+  float* impact_out;
+};
+
+// qot_lightpath_provision (rel = pt = null), qot_lightpath_traffic (pt = null) and qot_lightpath_protect (rel = null):
+// the checks, the copy of chan_node and the launch
 static int pv_launch(const char* who, const qot_lp_state_t* state, const qot_lp_demands_t* demands,
                      const int64_t* order, const int64_t* sample_ptr, const float* bound, int32_t metric,
                      int32_t maximize, int32_t policy, const float* prepared, int32_t is_lut_index, int32_t max_impact,
@@ -2295,7 +2418,8 @@ static int pv_launch(const char* who, const qot_lp_state_t* state, const qot_lp_
                      int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact, int64_t* conn_id,
                      int64_t* impact_conn, float* impact_out, const qot_lp_releases_t* rel, const int64_t* rel_order,
                      const int64_t* rel_ptr, int32_t* rel_status, int64_t* rel_conn_id, int32_t* rel_n_impact,
-                     int64_t* rel_impact_conn, float* rel_impact_out, float* rel_margin, cudaStream_t stream) {
+                     int64_t* rel_impact_conn, float* rel_impact_out, float* rel_margin, cudaStream_t stream,
+                     const PtOut* pt = nullptr) {
   PvArgs va;
   PlArgs& pa = va.p;
   CdArgs& a = pa.c;
@@ -2305,7 +2429,12 @@ static int pv_launch(const char* who, const qot_lp_state_t* state, const qot_lp_
   const qot_lp_demands_t& d = *demands;
   const int64_t NR = rel ? rel->R : 0;
   QOT_REQUIRE(NR >= 0, "%s: bad release count", who);
+  QOT_REQUIRE(!pt || st.cfg.L <= QOT_TG_MAX_LINKS, "%s: L = %d over QOT_TG_MAX_LINKS (the link bitmaps)", who,
+              st.cfg.L);
   if (d.D == 0 && NR == 0) return QOT_OK;
+  QOT_REQUIRE(!pt || (pt->option && pt->q0 && pt->out && pt->margin && pt->n_free && pt->n_feasible && pt->status &&
+                      pt->n_impact && pt->conn_id && (max_impact == 0 || (pt->impact_conn && pt->impact_out))),
+              "%s: null backup output array", who);
   QOT_REQUIRE(d.D == 0 || (d.sample && order && d.opt_ptr && d.link_ptr &&
                            (d.P == 0 || (d.width && d.feat && d.own_bound)) && (d.n_links == 0 || d.links)),
               "%s: null demand or grouping array", who);
@@ -2321,9 +2450,10 @@ static int pv_launch(const char* who, const qot_lp_state_t* state, const qot_lp_
                     (max_impact == 0 || (rel_impact_conn && rel_impact_out)), "%s: null release output array", who);
   }
   if (int rc = cd_state_args(who, a, st, prepared, is_lut_index, max_impact)) return rc;
-  constexpr int smem = static_cast<int>(sizeof(PvSmem));
-  if (int rc = NR > 0 ? cd_smem_opt_in<lp_provision_kernel<true>, smem>()
-                      : cd_smem_opt_in<lp_provision_kernel<false>, smem>())
+  constexpr int smem = static_cast<int>(sizeof(PvSmem)), pt_smem = static_cast<int>(sizeof(PtSmem));
+  if (int rc = pt        ? cd_smem_opt_in<lp_provision_kernel<false, true>, pt_smem>()
+               : NR > 0  ? cd_smem_opt_in<lp_provision_kernel<true>, smem>()
+                         : cd_smem_opt_in<lp_provision_kernel<false>, smem>())
     return rc;
   if (st.S > 0)
     QOT_CUDA(cudaMemcpyAsync(chan_work, st.chan_node, static_cast<size_t>(st.S) * st.cfg.L * st.cfg.Q * sizeof(int32_t),
@@ -2340,8 +2470,22 @@ static int pv_launch(const char* who, const qot_lp_state_t* state, const qot_lp_
   va.rel_status = rel_status; va.rel_conn_id = rel_conn_id; va.rel_n_impact = rel_n_impact;
   va.rel_impact_conn = rel_impact_conn; va.rel_impact_out = rel_impact_out; va.rel_margin = rel_margin;
   const unsigned grid = static_cast<unsigned>(std::min<int64_t>(kNumSMs, std::max<int64_t>(1, st.S)));
-  if (NR > 0) lp_provision_kernel<true><<<grid, kCdThreads, smem, stream>>>(va);
-  else lp_provision_kernel<false><<<grid, kCdThreads, smem, stream>>>(va);
+  if (pt) {
+    PtArgs ta;
+    static_cast<PvArgs&>(ta) = va;
+    ta.bk = va;
+    ta.bk.p.c.out = pt->out; ta.bk.p.c.status = pt->status; ta.bk.p.c.n_impact = pt->n_impact;
+    ta.bk.p.c.impact_node = pt->impact_conn; ta.bk.p.c.impact_out = pt->impact_out;
+    ta.bk.p.option = pt->option; ta.bk.p.q0 = pt->q0; ta.bk.p.margin = pt->margin;
+    ta.bk.p.n_free = pt->n_free; ta.bk.p.n_feasible = pt->n_feasible;
+    ta.bk.conn_id = pt->conn_id;
+    ta.protect = pt->protect;
+    lp_provision_kernel<false, true><<<grid, kCdThreads, pt_smem, stream>>>(ta);
+  } else if (NR > 0) {
+    lp_provision_kernel<true><<<grid, kCdThreads, smem, stream>>>(va);
+  } else {
+    lp_provision_kernel<false><<<grid, kCdThreads, smem, stream>>>(va);
+  }
   QOT_LAUNCH_CHECK();
   return QOT_OK;
 }
@@ -2523,6 +2667,25 @@ extern "C" int qot_lightpath_traffic(const qot_lp_state_t* state, const qot_lp_d
                    max_impact, chan_work, bound_work, option, q0, out, margin, n_free, n_feasible, status, n_impact,
                    conn_id, impact_conn, impact_out, releases, rel_order, rel_ptr, rel_status, rel_conn_id,
                    rel_n_impact, rel_impact_conn, rel_impact_out, rel_margin, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int qot_lightpath_protect(const qot_lp_state_t* state, const qot_lp_demands_t* demands,
+                                     const int64_t* order, const int64_t* sample_ptr, const float* bound,
+                                     int32_t metric, int32_t maximize, int32_t policy, const float* prepared,
+                                     int32_t is_lut_index, int32_t max_impact, int32_t* chan_work, float* bound_work,
+                                     int32_t* option, int32_t* q0, float* out, float* margin, int32_t* n_free,
+                                     int32_t* n_feasible, int32_t* status, int32_t* n_impact, int64_t* conn_id,
+                                     int64_t* impact_conn, float* impact_out, const uint8_t* protect,
+                                     int32_t* backup_option, int32_t* backup_q0, float* backup_out,
+                                     float* backup_margin, int32_t* backup_n_free, int32_t* backup_n_feasible,
+                                     int32_t* backup_status, int32_t* backup_n_impact, int64_t* backup_conn_id,
+                                     int64_t* backup_impact_conn, float* backup_impact_out, void* stream) {
+  const PtOut pt{protect, backup_option, backup_q0, backup_out, backup_margin, backup_n_free, backup_n_feasible,
+                 backup_status, backup_n_impact, backup_conn_id, backup_impact_conn, backup_impact_out};
+  return pv_launch("qot_lightpath_protect", state, demands, order, sample_ptr, bound, metric, maximize, policy,
+                   prepared, is_lut_index, max_impact, chan_work, bound_work, option, q0, out, margin, n_free,
+                   n_feasible, status, n_impact, conn_id, impact_conn, impact_out, nullptr, nullptr, nullptr, nullptr,
+                   nullptr, nullptr, nullptr, nullptr, nullptr, static_cast<cudaStream_t>(stream), &pt);
 }
 
 extern "C" int qot_lightpath_restore(const qot_lp_state_t* state, const qot_lp_demands_t* options,

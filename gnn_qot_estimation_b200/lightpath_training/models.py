@@ -261,6 +261,35 @@ class LightpathGNN(torch.nn.Module):
                                        self.is_lut_index, max_impact)
 
     @_lib.on_tensor_device
+    def forward_protection(self, state, demands, protect, policy: int, metric: int = 0, maximize: bool = True,
+                           bound=None, max_impact: int = 64) -> "ops.ProtectionQoT":
+        """Provisioning with dedicated 1+1 protection (eval mode only; csrc/lightpath_candidates.cu,
+        qot_lightpath_protect): a demand with ``protect[d]`` ([D] bool) is admitted only with a working path and a
+        link-disjoint backup path, both set up and both meeting their bounds.  Demands are grouped and taken in order
+        as in ``forward_provision``; an unprotected demand is handled exactly as there (every output bit-identical, the
+        backup outputs -1 / NaN / 0), so with ``protect`` all False the call is ``forward_provision``.
+
+        A protected demand d, against ``state_d`` (the samples with every earlier committed lightpath of d's sample
+        written in): an option is eligible as the working path iff some option of d has a route sharing no link with
+        its route (none: ``ops.PROT_NO_PARTNER``, nothing placed).  The working path is placed exactly as
+        ``forward_placements`` places d with the eligible options (option indices stay those of the full list); if it
+        is not acceptable the demand is blocked.  Otherwise it is set up as ``forward_provision`` sets up an accepted
+        demand (conn_id top + 1, its option's ``own_bound``) and the backup is placed the same way over d's options
+        whose route shares no link with the working route, against that state (``PROV_FULL`` counts the working path).
+        An acceptable backup is set up as top + 2 and the demand is accepted; otherwise the working path is removed,
+        the state is exactly what it was before d (no conn_id consumed), ``status`` gets ``ops.PROT_NO_BACKUP`` and
+        both conn_ids are -1, the working placement still reported.  Working first, then backup: greedy, not a joint
+        search over pairs.
+
+        Returns ``ops.ProtectionQoT``: ``forward_provision``'s fields for the working path, then the same fields for
+        the backup (``backup_*``).  ``state`` is not modified; ``to_graph.commit_protection`` writes both paths into
+        the samples.  One copy and one launch, nothing read back: capturable in a CUDA graph.  Malformed arguments
+        raise on the host."""
+        self._check_state_query("forward_protection", state)
+        return ops.lightpath_protection(state, demands, protect, policy, metric, maximize, bound, self.prepared(),
+                                        self.is_lut_index, max_impact)
+
+    @_lib.on_tensor_device
     def forward_traffic(self, state, demands, releases, policy: int, metric: int = 0, maximize: bool = True,
                         bound=None, max_impact: int = 64) -> "ops.TrafficQoT":
         """Dynamic traffic: lightpath arrivals and departures in one pass (eval mode only;

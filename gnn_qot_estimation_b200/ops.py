@@ -670,6 +670,69 @@ def lightpath_provision(state, demands, policy: int, metric: int, maximize: bool
     return res
 
 
+# status bits of qot_lightpath_protect, on top of the CAND_* and PROV_* bits
+PROT_NO_PARTNER, PROT_NO_BACKUP = 65536, 131072
+TG_MAX_LINKS = 1024                            # QOT_TG_MAX_LINKS: the route bitmaps of the partner and backup filters
+_C_ORDER = (0, 1, 2, 3, 4, 5, 6, 7, 10, 8, 9)  # ProvisionQoT's fields in the C argument order (conn_id before impact_*)
+
+
+class ProtectionQoT(NamedTuple):
+    option: torch.Tensor         # [D] int32: the working path's option, in the demand's full list (-1: none)
+    q0: torch.Tensor             # [D] int32: its start slot (-1: none)
+    out: torch.Tensor            # [D,3]: the working placement's own QoT (NaN: none)
+    margin: torch.Tensor         # [D]: its margin (NaN: none)
+    n_free: torch.Tensor         # [D] int32: free placements over the eligible options
+    n_feasible: torch.Tensor     # [D] int32: feasible placements among them
+    status: torch.Tensor         # [D] int32, CAND_* | PROV_* | PROT_* bits
+    n_impact: torch.Tensor       # [D] int32: lightpaths the working placement interferes with
+    impact_conn: torch.Tensor    # [D, max_impact] int64: their conn_ids, ascending in node order; -1 past the rows
+    impact_out: torch.Tensor     # [D, max_impact, 3]: their QoT with the working placement set up; NaN past the rows
+    conn_id: torch.Tensor        # [D] int64: the working path's conn_id (-1: not accepted)
+    backup_option: torch.Tensor      # [D] int32: the backup's option, in the full list (-1: none or no search)
+    backup_q0: torch.Tensor          # [D] int32
+    backup_out: torch.Tensor         # [D,3]
+    backup_margin: torch.Tensor      # [D]
+    backup_n_free: torch.Tensor      # [D] int32: free placements over the options link-disjoint from the working one
+    backup_n_feasible: torch.Tensor  # [D] int32
+    backup_status: torch.Tensor      # [D] int32, CAND_* | PROV_FULL bits
+    backup_n_impact: torch.Tensor    # [D] int32
+    backup_impact_conn: torch.Tensor  # [D, max_impact] int64
+    backup_impact_out: torch.Tensor  # [D, max_impact, 3]
+    backup_conn_id: torch.Tensor     # [D] int64: the backup path's conn_id (-1: not accepted)
+
+
+def lightpath_protection(state, demands, protect: torch.Tensor, policy: int, metric: int, maximize: bool, bound,
+                         prepared: torch.Tensor, is_lut_index: int, max_impact: int) -> ProtectionQoT:
+    """qot_lightpath_protect: ``lightpath_provision`` where a demand with ``protect[d]`` gets a working path and a
+    link-disjoint backup path or nothing.  The grouping is computed on the device and the work arrays allocated here;
+    one copy and one launch, nothing read back (CUDA-graph capturable).  The host checks of ``lightpath_provision``
+    plus ``protect``'s dtype (bool), shape [D] and device."""
+    who = "forward_protection"
+    D, P = _check_demand_args(who, state, demands, policy, metric, bound, prepared, max_impact)
+    dev = state.batch.x.device
+    _check_state_tensor(who, "protect", protect, dev, torch.bool)
+    if protect.shape != (D,):
+        raise ValueError(f"{who}: need protect [D] with D = {D} demands")
+    if state.L > TG_MAX_LINKS:
+        raise ValueError(f"{who}: L = {state.L} links, at most {TG_MAX_LINKS} (the route bitmaps)")
+    max_impact = int(max_impact)
+    i64 = lambda *s: torch.empty(*s, dtype=torch.int64, device=dev)
+    res = ProtectionQoT(*_demand_outputs(D, max_impact, dev), i64(D), *_demand_outputs(D, max_impact, dev), i64(D))
+    if D == 0:
+        return res
+    order, sample_ptr = provision_grouping(demands.sample, state.S)
+    chan_work = torch.empty_like(state.chan_node)
+    bound_work = torch.empty(state.S, TG_MAX_NODES, dtype=torch.float32, device=dev) if bound is not None else None
+    bound = None if bound is None else bound.contiguous()
+    keep = [protect.contiguous()]
+    with torch.cuda.device(dev):
+        check(_lib.lib().qot_lightpath_protect(
+            C.byref(_state_desc(state, keep)), C.byref(_demands_desc(demands, D, P, keep)), ptr(order),
+            ptr(sample_ptr), _cptr(bound), int(metric), int(bool(maximize)), int(policy), ptr(prepared),
+            int(is_lut_index), max_impact, _cptr(chan_work), _cptr(bound_work), *(_cptr(res[k]) for k in _C_ORDER),
+            ptr(keep[0]), *(_cptr(res[11 + k]) for k in _C_ORDER), stream()), "qot_lightpath_protect")
+    return res
+
 
 # status bits of qot_lightpath_traffic's releases, on top of the CAND_* and PROV_* bits
 TRAF_BAD_REF, TRAF_NOT_ACCEPTED = 2048, 4096

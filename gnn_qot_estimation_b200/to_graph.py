@@ -290,6 +290,56 @@ def lightpath_network_state(data: torch.Tensor, freqs: torch.Tensor, lp_feat: Se
     return LightpathNetworkState(batch, conn_ids, chan_node, rowptr, freqs, cfg, S, L, Q)
 
 
+def _write_lightpaths(data: torch.Tensor, state: LightpathNetworkState, demands: LightpathDemands, dm: torch.Tensor,
+                      option: torch.Tensor, q0: torch.Tensor, conn_id: torch.Tensor) -> None:
+    """Writes lightpath k (``conn_id[k] >= 0``; the others are skipped) of demand ``dm[k]`` onto its option
+    ``option[k]`` (relative to the demand's first) x ``[q0[k], q0[k] + width)`` into ``data`` in place, as
+    ``commit_provision`` documents.  An option is written at most once, and the written placements of a sample are
+    disjoint.  One host synchronisation gathers the written channels."""
+    S, F, L, Q = (int(v) for v in data.shape)
+    cfg, d, dev = state.cfg, demands, data.device
+    # chosen[p] = the written row whose option is p, else -1
+    P = int(d.width.shape[0])
+    acc = conn_id >= 0
+    po = d.opt_ptr[dm] + option.to(torch.int64)
+    chosen = torch.full((P + 1,), -1, dtype=torch.int64, device=dev)
+    chosen.scatter_(0, torch.where(acc, po, torch.full_like(po, P)), torch.arange(po.shape[0], device=dev))
+    chosen[P] = -1
+    # every (route entry, slot) a written row occupies
+    opt = torch.searchsorted(d.link_ptr, torch.arange(d.links.shape[0], device=dev), right=True) - 1
+    k = chosen[opt]
+    q0 = q0[k.clamp(min=0)].to(torch.int64)
+    q = torch.arange(Q, device=dev)
+    on = (k >= 0)[:, None] & (q[None, :] >= q0[:, None]) & (q[None, :] < (q0 + d.width[opt])[:, None])
+    e, c = on.nonzero(as_tuple=True)                            # the host synchronisation
+    k, p = k[e], opt[e]
+    vec = torch.zeros(int(e.shape[0]), F, dtype=torch.float32, device=dev)
+    vec[:, cfg.i_conn] = conn_id[k].to(torch.float32)
+    vec[:, cfg.i_feat[0]] = state.freqs[q0[e]].to(torch.float32)
+    for j in range(3):
+        vec[:, cfg.i_feat[j + 1]] = d.feat[p, j]
+    vec[:, cfg.i_osnr] = vec[:, cfg.i_snr] = vec[:, cfg.i_ber] = -1.0
+    data[d.sample[dm[k]], :, d.links[e].to(torch.int64), c] = vec
+
+
+def _rebuild(data: torch.Tensor, state: LightpathNetworkState) -> LightpathNetworkState:
+    """``lightpath_network_state`` of the written samples, with the state's frequencies and threshold."""
+    cfg, F = state.cfg, int(data.shape[1])
+    names = [f"row{f}" for f in range(F)]                       # the builder reads only the rows cfg names
+    names[cfg.i_conn], names[cfg.i_osnr], names[cfg.i_snr], names[cfg.i_ber] = "conn_id", "osnr", "snr", "ber"
+    for k, name in enumerate(("freq", "mod_order", "num_spans", "path_len")):
+        names[cfg.i_feat[k]] = name
+    return lightpath_network_state(data, state.freqs, names, float(cfg.freq_threshold))
+
+
+def _check_commit_data(who: str, data: torch.Tensor, state: LightpathNetworkState) -> None:
+    if not (data.is_cuda and data.dtype == torch.float32 and data.is_contiguous()):
+        raise TypeError(f"{who}: data must be a contiguous float32 CUDA tensor (it is written in place)")
+    S, F, L, Q = (int(v) for v in data.shape)
+    if (S, L, Q) != (state.S, state.L, state.Q):
+        raise ValueError(f"{who}: data must be the [S, F, L, Q] samples the state was built from")
+
+
 def commit_provision(data: torch.Tensor, state: LightpathNetworkState, demands: LightpathDemands,
                      res) -> LightpathNetworkState:
     """Writes the demands ``LightpathGNN.forward_provision`` accepted (``res.conn_id >= 0``) into ``data`` [S, F, L, Q]
@@ -300,39 +350,25 @@ def commit_provision(data: torch.Tensor, state: LightpathNetworkState, demands: 
     other row 0.  The new state is the builder's by construction (node order by first channel, so a new lightpath
     lands among the existing nodes).  Not capturable: one host synchronisation gathers the written channels, and the
     rebuild keeps the builder's own."""
-    if not (data.is_cuda and data.dtype == torch.float32 and data.is_contiguous()):
-        raise TypeError("commit_provision: data must be a contiguous float32 CUDA tensor (it is written in place)")
-    S, F, L, Q = (int(v) for v in data.shape)
-    if (S, L, Q) != (state.S, state.L, state.Q):
-        raise ValueError("commit_provision: data must be the [S, F, L, Q] samples the state was built from")
-    cfg, d, dev = state.cfg, demands, data.device
-    # chosen[p] = the accepted demand whose chosen option is p (an option belongs to one demand), else -1
-    P = int(d.width.shape[0])
-    acc = res.conn_id >= 0
-    po = d.opt_ptr[:-1] + res.option.to(torch.int64)
-    chosen = torch.full((P + 1,), -1, dtype=torch.int64, device=dev)
-    chosen.scatter_(0, torch.where(acc, po, torch.full_like(po, P)), torch.arange(po.shape[0], device=dev))
-    chosen[P] = -1
-    # every (route entry, slot) an accepted demand occupies; accepted placements of a sample are disjoint
-    opt = torch.searchsorted(d.link_ptr, torch.arange(d.links.shape[0], device=dev), right=True) - 1
-    dm = chosen[opt]
-    q0 = res.q0[dm.clamp(min=0)].to(torch.int64)
-    q = torch.arange(Q, device=dev)
-    on = (dm >= 0)[:, None] & (q[None, :] >= q0[:, None]) & (q[None, :] < (q0 + d.width[opt])[:, None])
-    e, c = on.nonzero(as_tuple=True)                            # the host synchronisation
-    dm, p = dm[e], opt[e]
-    vec = torch.zeros(int(e.shape[0]), F, dtype=torch.float32, device=dev)
-    vec[:, cfg.i_conn] = res.conn_id[dm].to(torch.float32)
-    vec[:, cfg.i_feat[0]] = state.freqs[q0[e]].to(torch.float32)
-    for k in range(3):
-        vec[:, cfg.i_feat[k + 1]] = d.feat[p, k]
-    vec[:, cfg.i_osnr] = vec[:, cfg.i_snr] = vec[:, cfg.i_ber] = -1.0
-    data[d.sample[dm], :, d.links[e].to(torch.int64), c] = vec
-    names = [f"row{f}" for f in range(F)]                       # the builder reads only the rows cfg names
-    names[cfg.i_conn], names[cfg.i_osnr], names[cfg.i_snr], names[cfg.i_ber] = "conn_id", "osnr", "snr", "ber"
-    for k, name in enumerate(("freq", "mod_order", "num_spans", "path_len")):
-        names[cfg.i_feat[k]] = name
-    return lightpath_network_state(data, state.freqs, names, float(cfg.freq_threshold))
+    _check_commit_data("commit_provision", data, state)
+    D = int(res.conn_id.shape[0])
+    _write_lightpaths(data, state, demands, torch.arange(D, device=data.device), res.option, res.q0, res.conn_id)
+    return _rebuild(data, state)
+
+
+def commit_protection(data: torch.Tensor, state: LightpathNetworkState, demands: LightpathDemands,
+                      res) -> LightpathNetworkState:
+    """Writes what ``LightpathGNN.forward_protection`` accepted (result ``res``) into ``data`` [S, F, L, Q] in place
+    and returns ``lightpath_network_state`` of it: each accepted demand's working path (``res.conn_id``, ``option``,
+    ``q0``) and backup path (``res.backup_conn_id``, ``backup_option``, ``backup_q0``), each written as
+    ``commit_provision`` writes a demand; rolled-back demands write nothing.  One rebuild.  Not capturable, like
+    ``commit_provision``."""
+    _check_commit_data("commit_protection", data, state)
+    D = int(res.conn_id.shape[0])
+    dm = torch.arange(D, device=data.device)
+    _write_lightpaths(data, state, demands, torch.cat([dm, dm]), torch.cat([res.option, res.backup_option]),
+                      torch.cat([res.q0, res.backup_q0]), torch.cat([res.conn_id, res.backup_conn_id]))
+    return _rebuild(data, state)
 
 
 def commit_traffic(data: torch.Tensor, state: LightpathNetworkState, demands: LightpathDemands,

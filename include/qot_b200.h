@@ -831,6 +831,42 @@ int qot_lightpath_restore(const qot_lp_state_t* state, const qot_lp_demands_t* o
                           int32_t* cut_status, int32_t* status, int32_t* n_cut, int32_t* n_restored,
                           float* end_margin, int32_t* n_below, int64_t* end_conn, float* end_out, void* stream);
 
+/* qot_lightpath_protect (lp_provision_kernel<.., kProtect>, the launch of qot_lightpath_provision): provisioning with
+ * dedicated 1+1 protection.  The arguments and outputs of qot_lightpath_provision, then protect [D] (nonzero: the
+ * demand is protected; NULL: none is, which gives qot_lightpath_provision's outputs bit for bit) and the backup
+ * outputs.  Demands are grouped and taken in order as there; an unprotected demand is handled exactly as there, its
+ * backup outputs -1 / NaN / 0.  A protected demand d, against state_d (every earlier committed lightpath of d's sample
+ * written in):
+ *   partner filter: option p may be the working path iff some option of d has a route sharing no link with p's (link
+ *     sets compared as sets); the others are neither scanned nor counted, option indices stay those of d's full list
+ *     (the tie rule is the filtered list's); none left: QOT_PROT_NO_PARTNER, nothing placed (-1 / NaN / 0);
+ *   working path: placed exactly as qot_lightpath_placements places d with the eligible options against state_d; its
+ *     outputs are option .. impact_out.  Not acceptable (nothing feasible, or a status bit but IMPACT_OVERFLOW): the
+ *     demand is blocked, no backup search;
+ *   backup path: the working path set up (conn_id top + 1, its option's own_bound), the backup is placed the same way
+ *     over d's options whose route shares no link with the working route, against state_d + working (PROV_FULL counts
+ *     the working path); its outputs are backup_option .. backup_impact_out (impact rows: shared third-party
+ *     neighbours; the working path is never one);
+ *   accept: an acceptable backup is set up as top + 2: conn_id[d] = top + 1, backup_conn_id[d] = top + 2;
+ *   roll back: otherwise the working path is removed and the state is exactly what it was before d, top included (a
+ *     rolled-back demand consumes no conn_id); status[d] gets QOT_PROT_NO_BACKUP, conn_id[d] = backup_conn_id[d] = -1,
+ *     the working placement is still reported.
+ * The choice is greedy: the working path first, then its backup.  Requires L <= QOT_TG_MAX_LINKS.  Malformed demands
+ * and groupings never fault: as in qot_lightpath_provision (QOT_PROV_BAD_GROUPING, QOT_CAND_BAD_SAMPLE), with empty
+ * backup outputs.  One copy and one launch, nothing read back: capturable. */
+#define QOT_PROT_NO_PARTNER 65536    /* no option of the demand has a link-disjoint partner: nothing placed          */
+#define QOT_PROT_NO_BACKUP 131072    /* the working path had no acceptable backup: rolled back, not accepted        */
+int qot_lightpath_protect(const qot_lp_state_t* state, const qot_lp_demands_t* demands, const int64_t* order,
+                          const int64_t* sample_ptr, const float* bound, int32_t metric, int32_t maximize,
+                          int32_t policy, const float* prepared, int32_t is_lut_index, int32_t max_impact,
+                          int32_t* chan_work, float* bound_work, int32_t* option, int32_t* q0, float* out,
+                          float* margin, int32_t* n_free, int32_t* n_feasible, int32_t* status, int32_t* n_impact,
+                          int64_t* conn_id, int64_t* impact_conn, float* impact_out, const uint8_t* protect,
+                          int32_t* backup_option, int32_t* backup_q0, float* backup_out, float* backup_margin,
+                          int32_t* backup_n_free, int32_t* backup_n_feasible, int32_t* backup_status,
+                          int32_t* backup_n_impact, int64_t* backup_conn_id, int64_t* backup_impact_conn,
+                          float* backup_impact_out, void* stream);
+
 /* The topological representation: to_graph.py::create_topological_graph (:62-184: one edge per
  * lightpath between its source and destination network node, lightpaths added in ascending conn_id,
  * nx.Graph keeps one edge per node pair -- position from the first, attributes from the last) fused
